@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the prior-fit hot path (BASELINE.json metric: prior-fit pixel-samples/sec, fwd+bwd+step).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|f16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|f16] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE configs[1] -- the convexity prior ``ConvexNextNet(h=130, L=2, C=2)``
 fitted per frame on a synthetic FBMS-shaped 640x480 frame (unaries = soft UNet-like blob), loss
@@ -16,10 +16,15 @@ events), e2e (same metric through the public fit API with the step's unaries com
 memory and the step's loss read back, copies inside the timed region), roofline (dominant kernel,
 timed live with CUDA events on the launch stream), cpu_baseline (the oracle port on the host cores,
 rank 0, bounded sample), clocks, gpu_launches.
+
+``--dump-outputs DIR`` writes what the K timed steps computed (rank 0): ``params.npy`` = the fitted parameters of the
+G priors after the last timed step [G,P] (float32, each row in ``parameters()`` order), ``loss.npy`` = the loss of that
+step per frame [G] (float64).  The inputs depend on the arguments only, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import ctypes as C
 import json
 import os
@@ -31,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark may run from a read-only tree: it writes nothing into it
 
 H, W = 480, 640
 N_PIX = H * W
@@ -94,8 +100,14 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.index), f"--query-gpu={self.QUERY}",
                                           "--format=csv,noheader,nounits", "-lms", "20"],
                                          stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(self._kill)          # no sampler outlives the benchmark, also when it fails before stop()
         except Exception:
             self.proc = None
+
+    def _kill(self):
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.kill()
+            self.proc.wait()
 
     @staticmethod
     def _epoch(ts: str) -> float:
@@ -550,6 +562,17 @@ def eager_gpu_throughput(dev, steps: int = 10):
             "sample": f"{steps} fit steps on the full 640x480 frame, eager PyTorch fp32 ops of the reference's loop on cuda"}
 
 
+def dump_outputs(out_dir: str, fitter, G: int) -> None:
+    """What a caller of the timed path receives after its last step: the G fitted priors and that step's loss per frame
+    (kept by the optimizer state on the device).  Called right after the timed region, before any other leg fits."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    params = fitter.params.detach().reshape(G, -1).cpu().numpy().astype(np.float32)
+    loss = np.array([fitter.scalars(o).last_loss for o in range(G)], dtype=np.float64)
+    np.save(os.path.join(out_dir, "params.npy"), params)
+    np.save(os.path.join(out_dir, "loss.npy"), loss)
+
+
 def run_reference(args, rank: int, world: int):
     if rank != 0:
         return
@@ -583,7 +606,11 @@ def main():
     ap.add_argument("--no-joint", action="store_true", help="skip the joint UNet + prior step leg (BASELINE configs[4])")
     ap.add_argument("--no-frames", action="store_true", help="skip the measured frames/s leg (60-frame sharded sequence fit)")
     ap.add_argument("--sustained-seconds", type=float, default=10.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the fitted parameters and the per-frame loss of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE line, the JSON: everything any library prints to file descriptor 1 (NCCL's version
     # banner, warnings of child processes) is sent to stderr, and the JSON line is written to the saved descriptor.
     global _JSON_OUT
@@ -659,6 +686,8 @@ def main():
     barrier()
     launches = lib.awb_launch_count() - launches0
     ms_total = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fitter, G)
 
     # ---- end to end through the public API: the step's unaries arrive from pinned host memory, loss read back
     fitter.set_target_pool(None)

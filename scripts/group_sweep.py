@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import awesome_b200 as A
 import bench as B
 dev = torch.device("cuda", 0)

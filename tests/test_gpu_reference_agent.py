@@ -1,32 +1,6 @@
-"""The drop-in under the REAL reference agent: the reference's ``TorchAgent`` / ``WrapperModule`` / ``PriorDataset`` /
-``PriorCache`` (installed in ``baseline/_ref`` by ``baseline/install_reference.py``; non-numeric packages missing offline
-are stubbed by ``oracle/ref_shim.py``) drive ``awesome_b200.real_nvp_path_connected_net`` through ``TorchAgent._pretrain``
-(``awesome/agent/torch_agent.py:553-627``) on three synthetic frames; the saved ``pretrain_state_path`` is reloaded with
-the reference's own ``PriorCache``; and a ``PriorCache`` file written by the reference loads into ``DevicePriorCache``."""
-import os
-
-import pytest
+"""A ``PriorCache`` file written by the reference's ``PriorCache.save`` (stored fixture ``prior_cache_ref.pth``) loads
+into ``DevicePriorCache`` and is written back in the same format."""
 import torch
-
-import __graft_entry__ as entry
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
-DEV = "cuda:0"
-
-
-def _reference():
-    if not os.path.isdir(os.path.join(REF, "awesome")):
-        pytest.skip("reference package not installed (python baseline/install_reference.py)")
-    from oracle import ref_shim
-    if not ref_shim._installed:
-        ref_shim.REFERENCE_ROOT = REF
-    ref_shim.install()
-
-
-def blob(H, W, cx=0.5, cy=0.5, rx=0.22, ry=0.27, tau=0.08):
-    yy, xx = torch.meshgrid(torch.linspace(0, 1, H), torch.linspace(0, 1, W), indexing="ij")
-    return torch.sigmoid((torch.sqrt(((xx - cx) / rx) ** 2 + ((yy - cy) / ry) ** 2) - 1) / tau)
 
 
 def test_reference_prior_cache_file_loads_into_device_cache(golden):
@@ -50,256 +24,3 @@ def test_reference_prior_cache_file_loads_into_device_cache(golden):
     assert set(back) == set(state) and saved_type.endswith("ConvexNextNet")
     for k, v in state["cache"]["5"].items():
         assert torch.equal(back["cache"]["5"][k].cpu(), v)
-
-
-@pytest.mark.gpu
-def test_pretrain_under_the_reference_torch_agent(tmp_path):
-    entry.build()
-    _reference()
-    import awesome_b200 as A
-    from awesome.agent.torch_agent import TorchAgent
-    from awesome.dataset.prior_dataset import PriorDataset, prior
-    from awesome.dataset.torch_datasource import TorchDataSource
-    from awesome.model.pretrainable_module import PretrainableModule
-    from awesome.model.wrapper_module import WrapperModule
-    from awesome.util.prior_cache import PriorCache
-
-    assert A.integrate_with_reference(force=True)
-    H, W, T = 40, 56, 3
-    prior_args = dict(channels=2, hidden_units=32, flow_n_flows=6, flow_output_fn="tanh", norm="minmax",
-                      convex_net_hidden_units=130, convex_net_hidden_layers=2, precision="f16")
-
-    class SynthFrames(PriorDataset, TorchDataSource):
-        """Three synthetic frames in the item format of ``AwesomeDataset`` (image mode, ``param_clean_grid``): inputs =
-        (image [4,H,W], feature grid, clean coordinate grid [2,H,W]), label map."""
-
-        def __init__(self, **kw):
-            super().__init__(returns_index=False, **kw)
-            self.frames = [blob(H, W, cx=0.42 + 0.05 * i) for i in range(T)]
-            self.grid = A.GridSpecHost("linspace", 1, H, W).materialize(2, "cpu")[0]
-
-        def __len__(self):
-            return T
-
-        @prior()
-        def __getitem__(self, i):
-            u = self.frames[i]
-            image = torch.stack([u, u * 0.5, 1 - u, torch.zeros_like(u)])
-            return (image, self.grid.clone(), self.grid.clone()), (u > 0.5).float()[None]
-
-    class TinySeg(torch.nn.Module):
-        """Frozen "UNet": its logit is a fixed function of the image's first channel (so that sigmoid gives back the blob)."""
-
-        def __init__(self):
-            super().__init__()
-            self.conv = torch.nn.Conv2d(4, 1, 1)
-            with torch.no_grad():
-                self.conv.weight.zero_()
-                self.conv.weight[0, 0] = 8.0
-                self.conv.bias.fill_(-4.0)
-
-        def forward(self, image, *args, **kwargs):
-            return self.conv(image)
-
-    ds = SynthFrames(prior_model_type=A.real_nvp_path_connected_net, prior_model_args=prior_args)
-    assert ds.has_prior and isinstance(ds.__prior_cache__, PriorCache)
-    prior_module = A.real_nvp_path_connected_net(**prior_args)
-    assert isinstance(prior_module, PretrainableModule)              # the reference's gate (wrapper_module.py:325-340)
-    state_path = str(tmp_path / "pretrain_state.pth")
-    agent = TorchAgent(
-        name="awb_integration", model_type=WrapperModule,
-        model_args=dict(segmentation_module=TinySeg(), prior_module=prior_module, mode="multi", input_mode="image",
-                        prior_arg_mode="param_clean_grid", use_segmentation_sigmoid=True),
-        optimizer_type=A.FusedAdam, optimizer_args=dict(lr=1e-3), loss=torch.nn.MSELoss(), training_dataset=ds,
-        agent_directory=str(tmp_path / "agent"), runs_directory=str(tmp_path / "runs"), do_pretraining=True,
-        pretrain_args=dict(num_epochs=250, reuse_state_epochs=60, lr=3e-3, prefit_flow_net_identity=True,
-                           prefit_flow_net_identity_num_epochs=15, prefit_convex_net=True, prefit_convex_net_num_epochs=25,
-                           do_pretrain_checkpoints=True, pretrain_checkpoint_dir=str(tmp_path / "ck")),
-        pretrain_state_path=state_path, force_pretrain=True, pretrain_only=True, device=DEV)
-    model = agent._get_prepared_model()
-    assert isinstance(model, WrapperModule) and next(model.parameters()).is_cuda
-    saved = {}
-    agent.save = lambda *a, **k: saved.setdefault("called", True)      # checkpoint serialisation of the agent needs jsonpickle
-    agent._pretrain(model, ds, ds, use_progress_bar=False)
-    assert os.path.exists(state_path) and saved.get("called")
-    assert sorted(os.listdir(tmp_path / "ck")) == [f"pretrain_checkpoint_{i}.pth" for i in range(T)]
-    # the saved state is the reference's PriorCache format; the reference's own class reloads it
-    state = torch.load(state_path, map_location="cpu", weights_only=False)
-    assert set(state) == {"model_type", "model_args", "store_device", "cache"} and set(state["cache"]) == {"0", "1", "2"}
-    assert state["model_type"].endswith("real_nvp_path_connected_net")
-    pc = PriorCache(None, None)
-    pc.set_state(state)
-    assert pc.model_type is A.real_nvp_path_connected_net
-    # each frame's cached prior, applied by the reference's PriorManager path, reproduces that frame's mask
-    from awesome.dataset.prior_dataset import PriorManager
-    grid = ds.grid[None].to(DEV)
-    for i in range(T):
-        with PriorManager(model, prior_state=(i, pc[i]), prior_cache=pc, model_device=torch.device(DEV)):
-            with torch.no_grad():
-                prob = torch.sigmoid(model.prior_module(grid))
-        assert A.mask_iou(prob.reshape(1, -1), ds.frames[i].to(DEV).reshape(1, -1)) > 0.85, i
-    # and pretrain_load_state through the agent: a second agent finds the state file and does not fit again
-    ds2 = SynthFrames(prior_model_type=A.real_nvp_path_connected_net, prior_model_args=prior_args)
-    agent2 = TorchAgent(
-        name="awb_integration2", model_type=WrapperModule,
-        model_args=dict(segmentation_module=TinySeg(), prior_module=A.real_nvp_path_connected_net(**prior_args), mode="multi",
-                        input_mode="image", prior_arg_mode="param_clean_grid"),
-        optimizer_type=A.FusedAdam, optimizer_args=dict(lr=1e-3), loss=torch.nn.MSELoss(), training_dataset=ds2,
-        agent_directory=str(tmp_path / "agent2"), runs_directory=str(tmp_path / "runs"), do_pretraining=True,
-        pretrain_args=dict(num_epochs=250), pretrain_state_path=state_path, force_pretrain=False, device=DEV)
-    agent2.save = lambda *a, **k: None
-    m2 = agent2._get_prepared_model()
-    fits = []
-    orig = m2.prior_module.pretrain
-    m2.prior_module.pretrain = lambda *a, **k: fits.append(1) or orig(*a, **k)
-    agent2._pretrain(m2, ds2, ds2, use_progress_bar=False)
-    assert not fits and 1 in ds2.__prior_cache__
-    for k, v in state["cache"]["1"].items():
-        assert torch.equal(ds2.__prior_cache__[1][k].cpu(), v.cpu()), k
-
-
-@pytest.mark.gpu
-def test_awesome_runner_builds_and_pretrains_the_drop_in_from_dotted_names(tmp_path):
-    """``AwesomeRunner(config).build()`` (``awesome/run/awesome_runner.py:107-123, 222-297, 492-494``) with
-    ``prior_model_type: awesome_b200.real_nvp_path_connected_net`` and ``optimizer_type: awesome_b200.FusedAdam``: the runner
-    resolves the dotted names, mints the per-frame ``PriorCache`` from ``prior_model_type(**args).state_dict()``, builds the
-    ``WrapperModule`` and the ``TorchAgent`` and attaches its ``_enforce_convexity`` batch hook; the agent then pretrains."""
-    import sys
-    entry.build()
-    _reference()
-    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-    import awesome_b200 as A
-    import ref_support
-    from awesome.agent.util.learning_mode import LearningMode
-    from awesome.event.torch_model_step_event_args import TorchModelStepEventArgs
-    from awesome.model.wrapper_module import WrapperModule
-    from awesome.run.awesome_config import AwesomeConfig
-    from awesome.run.awesome_runner import AwesomeRunner
-    from awesome.util.prior_cache import PriorCache
-
-    prior_args = dict(channels=2, hidden_units=32, flow_n_flows=6, flow_output_fn="tanh", norm="minmax",
-                      convex_net_hidden_units=130, convex_net_hidden_layers=2, precision="f16")
-    cfg = AwesomeConfig(
-        name_experiment="awb_runner", runs_path=str(tmp_path / "runs"), output_folder=str(tmp_path / "out"),
-        dataset_type="ref_support.SynthFrames", dataset_args=dict(),
-        segmentation_model_type="ref_support.TinySeg", segmentation_model_args=dict(), segmentation_training_mode="multi",
-        combined_segmentation_module_args=dict(input_mode="image", prior_arg_mode="param_clean_grid"),
-        prior_model_type="awesome_b200.real_nvp_path_connected_net", prior_model_args=prior_args, use_prior_model=True,
-        loss_type="torch.nn.MSELoss", loss_args=dict(), optimizer_type="awesome_b200.FusedAdam", optimizer_args=dict(lr=1e-3),
-        device=DEV, num_epochs=0, use_progress_bar=False, save_images_after_pretraining=False,
-        use_lr_stop_training_watchdog=False,
-        agent_args=dict(do_pretraining=True, force_pretrain=True, pretrain_only=True,
-                        pretrain_state_path=str(tmp_path / "state.pth"),
-                        pretrain_args=dict(num_epochs=200, reuse_state_epochs=50, lr=3e-3, prefit_flow_net_identity=True,
-                                           prefit_flow_net_identity_num_epochs=15, prefit_convex_net=True,
-                                           prefit_convex_net_num_epochs=25)))
-    runner = AwesomeRunner(cfg)
-    runner.build()
-    agent, ds = runner.agent, runner.dataloader
-    assert runner.prior_model_type is A.real_nvp_path_connected_net and runner.optim_type is A.FusedAdam
-    assert isinstance(ds, ref_support.SynthFrames) and isinstance(ds.__prior_cache__, PriorCache)
-    # the cache mints fresh per-frame states from the drop-in's factory (prior_cache.py:29-32)
-    fresh = ds.__prior_cache__[2]
-    assert list(fresh.keys()) == list(A.real_nvp_path_connected_net(**prior_args).state_dict().keys())
-    model = agent._get_prepared_model()
-    assert isinstance(model, WrapperModule) and isinstance(model.prior_module, A.PathConnectedNet)
-    # the runner's batch hook (awesome_runner.py:294-297) reaches the fused clamp
-    with torch.no_grad():
-        model.prior_module.convex_net.skip[0].ln.weight[0, :4] = -1.0
-    hooks = [f for f in agent.batch_processed.observers if getattr(f, "__name__", "") == "_enforce_convexity"]
-    assert len(hooks) == 1          # attached by AwesomeRunner.build_agent; the other observers are tensorboard loggers
-    hooks[0](dict(source=agent), TorchModelStepEventArgs(model=model, model_args=agent.model_args, mode=LearningMode.TRAINING))
-    assert float(model.prior_module.convex_net.skip[0].ln.weight.min()) >= 0.0
-    # pretraining through the agent; the runner's plotting / metric handles need the FBMS dataset API and jsonpickle
-    for handle in list(agent.after_pretrain.observers):
-        agent.after_pretrain.remove(handle)
-    agent.save = lambda *a, **k: None
-    agent._pretrain(model, ds, ds, use_progress_bar=False)
-    state = torch.load(str(tmp_path / "state.pth"), map_location="cpu", weights_only=False)
-    assert set(state["cache"]) == {"0", "1", "2"} and state["model_type"].endswith("real_nvp_path_connected_net")
-    grid = ds.grid[None].to(DEV)
-    for i in range(3):
-        model.prior_module.load_state_dict(state["cache"][str(i)])
-        with torch.no_grad():
-            prob = torch.sigmoid(model.prior_module(grid))
-        assert A.mask_iou(prob.reshape(1, -1), ds.frames[i].to(DEV).reshape(1, -1)) > 0.85, i
-
-
-@pytest.mark.gpu
-def test_joint_step_equals_the_reference_wrapper_loss_and_optimizer(tmp_path):
-    """The joint UNet + prior step (``TorchAgent._perform_step``, ``torch_agent.py:428-492``) written with the REFERENCE's
-    ``WrapperModule`` forward, the REFERENCE's ``FBMSJointLoss(WeightedLoss(BCELoss, "sssdms", noneclass=2), SE)`` and
-    ``torch.optim.Adam`` + ``enforce_convexity`` -- against ``awesome_b200.JointTrainer`` (own loss objects, ``FusedAdam``, flat
-    gradient bucket) on the same weights and data: losses and parameters after three steps."""
-    entry.build()
-    _reference()
-    import awesome_b200 as A
-    from awesome.measures.fbms_joint_loss import FBMSJointLoss
-    from awesome.measures.se import SE
-    from awesome.measures.weighted_loss import WeightedLoss
-    from awesome.model.wrapper_module import WrapperModule
-
-    B, H, W = 1, 32, 40            # the reference wrapper evaluates the prior per batch item: one frame per step
-    prior_args = dict(channels=3, hidden_units=32, flow_n_flows=6, flow_output_fn="tanh", convex_net_hidden_layers=2)
-
-    class Seg(torch.nn.Module):
-        """Like the reference UNet: forward(image, feature_encoding, ...) (awesome/model/unet.py:33-35); the features are unused."""
-
-        def __init__(self):
-            super().__init__()
-            self.net = torch.nn.Sequential(torch.nn.Conv2d(4, 8, 3, padding=1), torch.nn.ReLU(), torch.nn.Conv2d(8, 1, 3, padding=1))
-
-        def forward(self, image, *args, **kwargs):
-            return self.net(image)
-
-    def nets():
-        torch.manual_seed(6)
-        return Seg().to(DEV), A.real_nvp_path_connected_net(**prior_args).to(DEV)
-
-    g = torch.Generator().manual_seed(0)
-    img = torch.randn(B, 4, H, W, generator=g).to(DEV)
-    grid = A.GridSpecHost("linspace", B, H, W, t0=0.2, t_step=0.1).materialize(3, DEV)
-    lab = torch.full((B, 1, H, W), 2.0)
-    lab[torch.rand(B, 1, H, W, generator=g) < 0.15] = 0.0
-    lab[torch.rand(B, 1, H, W, generator=g) < 0.3] = 1.0
-    lab = lab.to(DEV)
-
-    seg, pri = nets()
-    with torch.no_grad():
-        pri(grid)                                                   # ActNorm data-dependent init
-    init = ({k: v.clone() for k, v in seg.state_dict().items()}, {k: v.clone() for k, v in pri.state_dict().items()})
-    tr = A.JointTrainer(seg, pri, A.measures.FBMSJointLoss(), optimizer_args=dict(lr=1e-3))
-    l_ours = [float(tr.step(img, grid, lab)) for _ in range(3)]
-
-    seg2, pri2 = nets()
-    seg2.load_state_dict(init[0]); pri2.load_state_dict(init[1])
-    model = WrapperModule(segmentation_module=seg2, prior_module=pri2, mode="multi", input_mode="image",
-                          prior_arg_mode="param_clean_grid").to(DEV)
-    model.train()
-    crit = FBMSJointLoss(criterion=WeightedLoss(torch.nn.BCELoss(), mode="sssdms", noneclass=2.),
-                         penalty_criterion=SE(reduction="mean"), alpha=1.0, beta=1.0)
-    crit.log = lambda *a, **k: None                                  # tensorboard side channel of the loss
-    opt = torch.optim.Adam(model.parameters(), lr=1e-3)
-    l_ref = []
-    for _ in range(3):
-        opt.zero_grad()
-        out = model(img, grid, grid)                                 # (image, feature grid, clean grid) as AwesomeDataset yields them
-        loss = crit(out, lab)
-        loss.backward()
-        opt.step()
-        model.enforce_convexity()                                    # the runner's batch hook (awesome_runner.py:294-297)
-        l_ref.append(float(loss.detach()))
-    torch.testing.assert_close(torch.tensor(l_ours), torch.tensor(l_ref), rtol=2e-5, atol=1e-7)
-    # Adam normalises every entry by its own gradient history: an entry whose gradient is at the fp32 noise floor (hidden units
-    # of the zero-initialised coupling layers that are active on a handful of pixels) moves by up to lr per step in a direction
-    # the last bits of the two loss implementations decide.  Everything above the noise floor must agree; nothing may differ
-    # by more than the 3 x lr Adam can move an entry in three steps.
-    close, total = 0, 0
-    for (k, a), b in zip(pri.state_dict().items(), pri2.state_dict().values()):
-        if a.dtype.is_floating_point:
-            ok = (a - b).abs() <= 2e-6 + 1e-4 * b.abs()
-            close += int(ok.sum()); total += ok.numel()
-            assert float((a - b).abs().max()) <= 3.05e-3, k
-    assert close >= 0.995 * total, (close, total)
-    for a, b in zip(seg.parameters(), seg2.parameters()):
-        torch.testing.assert_close(a, b, rtol=1e-5, atol=1e-7)
