@@ -6,7 +6,8 @@ Drop-in names for the reference's YAML configs (``prior_model_type`` / ``optimiz
 All arithmetic runs in ``csrc/libawb.so`` (hand-written sm_100a CUDA); there is no CPU fallback.
 """
 from .core import GridSpecHost, Prior, iou_counts, target_counts  # noqa: F401
-from .fit import FlowIdentityFitter, LossConfig, OptimConfig, PriorFitter  # noqa: F401
+from .fit import (FlowIdentityFitter, LossConfig, OptimConfig, PriorFitter, SlicedFitter, rank_slices,  # noqa: F401
+                  slice_plan)
 from .optim import FusedAdam, FusedAdamax  # noqa: F401
 from .pretrain import (FitSchedule, FrameResult, collect_unaries, evaluate_frames, fit_frames, fit_frames_grouped,  # noqa: F401
                        fit_sequence, load_pretrain_checkpoint, mask_iou, noisy_unaries, save_pretrain_checkpoint)

@@ -85,6 +85,10 @@ SYMBOLS = [
     ("awb_prior_fit_host_frames", C.c_int, [_P, _P, _P, C.POINTER(GridSpec), C.POINTER(_P), C.c_int32, C.c_int32,
                                             C.POINTER(LossSpec), C.POINTER(OptHyper), _P, _P, _P, C.c_size_t,
                                             C.c_int32, _P]),
+    ("awb_prior_grad_row_floats", C.c_int64, [_P]),
+    ("awb_prior_slice_grads", C.c_int, [_P, _P, C.POINTER(GridSpec), C.c_int64, C.c_int64, _P, C.POINTER(LossSpec), _P,
+                                        _P, C.c_size_t, C.c_int32, _P]),
+    ("awb_prior_rows_opt_step", C.c_int, [_P, _P, _P, _P, C.c_int32, C.POINTER(OptHyper), _P, _P, C.c_size_t, _P]),
     ("awb_flow_identity_step", C.c_int, [_P, _P, _P, C.POINTER(GridSpec), C.POINTER(OptHyper), _P, _P,
                                          C.c_size_t, _P]),
     ("awb_optim_step", C.c_int, [_P, _P, _P, _P, C.POINTER(OptHyper), _P]),

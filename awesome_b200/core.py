@@ -161,6 +161,35 @@ class Prior:
     def enforce_convexity(self, params: torch.Tensor) -> None:
         L.check(self.lib.awb_prior_enforce_convexity(self._h, params.data_ptr(), L.stream_ptr()))
 
+    # ---- pixel-sliced fit step (awb_prior_slice_grads / awb_prior_rows_opt_step)
+    @property
+    def grad_row_floats(self) -> int:
+        """``P + 1``: a slice's gradient in state_dict order, then its loss sum."""
+        return int(self.lib.awb_prior_grad_row_floats(self._h))
+
+    def slice_grads(self, params: torch.Tensor, grid: GridSpecHost, row_begin: int, row_end: int, target: torch.Tensor,
+                    loss, grad_row: torch.Tensor, ws: torch.Tensor, reuse_packed: bool = False) -> None:
+        """Gradient row of pixel rows ``[row_begin, row_end)`` of the batch into ``grad_row`` (``[P + 1]`` fp32, device).
+        ``target`` is the FULL batch ``[N]``; ``loss`` the ``LossSpec`` of the full batch.  ``ws``:
+        ``workspace_bytes(row_end - row_begin, 2)``.  ``reuse_packed``: the previous call on ``ws`` was a slice of the
+        same parameters."""
+        gs = grid.to_c()
+        L.check(self.lib.awb_prior_slice_grads(self._h, params.data_ptr(), C.byref(gs), int(row_begin), int(row_end),
+                                               target.data_ptr(), C.byref(loss), grad_row.data_ptr(), ws.data_ptr(),
+                                               ws.numel(), L.AWB_FIT_REUSE_PACKED if reuse_packed else 0,
+                                               L.stream_ptr()))
+
+    def rows_opt_step(self, params: torch.Tensor, opt_state: torch.Tensor, rows: torch.Tensor, hyper,
+                      loss_out: Optional[torch.Tensor] = None) -> None:
+        """Sum of the gradient rows ``rows`` (``[S, P + 1]`` fp32, device) in a fixed order, then the optimizer step of
+        the fused fit step.  ``loss_out`` (optional, one device float) receives the summed loss."""
+        if rows.dim() != 2 or rows.shape[1] != self.grad_row_floats or not rows.is_contiguous():
+            raise ValueError(f"rows must be a contiguous [S, {self.grad_row_floats}] tensor, got {tuple(rows.shape)}")
+        L.check(self.lib.awb_prior_rows_opt_step(self._h, params.data_ptr(), opt_state.data_ptr(), rows.data_ptr(),
+                                                 rows.shape[0], C.byref(hyper),
+                                                 loss_out.data_ptr() if loss_out is not None else None, None, 0,
+                                                 L.stream_ptr()))
+
 
 def iou_counts(pred: torch.Tensor, target: torch.Tensor, pred_is_logit: bool, n_objects: int = 1) -> torch.Tensor:
     """``[O,4]`` int64 counts {intersection, pred_fg, target_fg, n}; fg = value <= 0.5.

@@ -92,6 +92,7 @@ Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool f
   w.flowseg = (training && rnvp && flow_seg_scratch_floats(h, S) > 0) ? (float*)take(4 * flow_seg_scratch_floats(h, S)) : nullptr;
   w.tc = (h->desc.precision == AWB_PREC_F16 && tc_supported(h)) ? (void*)take(O * (int64_t)tc_image_bytes(L.L)) : nullptr;
   w.bytes = off;
+  w.row0 = 0; w.N = N;
   return w;
 }
 
@@ -269,15 +270,22 @@ int awb_prior_set_flow_eval(awb_handle h, int32_t mode) {
   return AWB_OK;
 }
 
+// window (optional, {row_begin, row_end}): the call works on the pixel rows [row_begin, row_end) of the batch, which must
+// be a non-empty range inside [0, N), and the workspace is sized for them
 static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, bool training, int64_t* N,
-                        bool fit_only = false) {
+                        bool fit_only = false, const int64_t* window = nullptr) {
   if (!h || !g || !ws) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (g->B < 1 || g->H < 1 || g->W < 1) { set_error("empty grid %dx%dx%d", g->B, g->H, g->W); return AWB_ERR_INVALID; }
   if (g->mode == AWB_GRID_EXPLICIT && !g->grid) { set_error("explicit grid needs a pointer"); return AWB_ERR_INVALID; }
   if (g->mode < 0 || g->mode > 2) { set_error("unknown grid mode %d", g->mode); return AWB_ERR_INVALID; }
   *N = (int64_t)g->B * g->H * g->W;
   if (*N > (int64_t)1 << 30) { set_error("too many pixel rows"); return AWB_ERR_UNSUPPORTED; }
-  int64_t need = carve(h, *N, training, nullptr, fit_only).bytes;
+  if (window && (window[0] < 0 || window[0] >= window[1] || window[1] > *N)) {
+    set_error("pixel-row window [%lld, %lld) is empty or outside [0, %lld)", (long long)window[0], (long long)window[1],
+              (long long)*N);
+    return AWB_ERR_INVALID;
+  }
+  int64_t need = carve(h, window ? window[1] - window[0] : *N, training, nullptr, fit_only).bytes;
   if ((int64_t)ws_bytes < need) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)need); return AWB_ERR_WORKSPACE; }
   if (h->desc.kind == AWB_KIND_FLOW_ICNN && !h->fc_set) { set_error("awb_prior_set_flow_consts not called"); return AWB_ERR_INVALID; }
   return AWB_OK;
@@ -384,6 +392,64 @@ int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_g
   rc = simt_backward(h, params, g, target, loss, nullptr, false, w, st);
   if (rc) return rc;
   return simt_reduce_opt(h, params, opt_state, hy, loss_out, w, N, st);
+}
+
+// single-object ICNN and RealNVP o ICNN handles (the priors of the spatio-temporal fit)
+static int check_sliceable(awb_handle h) {
+  if (!h) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if ((h->desc.kind != AWB_KIND_ICNN && h->desc.kind != AWB_KIND_FLOW_ICNN) || h->desc.n_objects != 1) {
+    set_error("gradient rows support single-object ICNN and RealNVP o ICNN priors (kind %d, %d objects)", h->desc.kind,
+              h->desc.n_objects);
+    return AWB_ERR_UNSUPPORTED;
+  }
+  return AWB_OK;
+}
+
+int64_t awb_prior_grad_row_floats(awb_handle h) { return h ? h->lay.P + 1 : -1; }
+
+int awb_prior_slice_grads(awb_handle h, const float* params, const awb_grid_spec* g, int64_t row_begin, int64_t row_end,
+                          const float* target, const awb_loss_spec* loss, float* grad_row, void* ws, size_t ws_bytes,
+                          int32_t flags, void* stream) {
+  int rc = check_sliceable(h);
+  if (rc) return rc;
+  int64_t N;
+  const int64_t window[2] = {row_begin, row_end};
+  rc = check_common(h, g, ws, ws_bytes, true, &N, /*fit_only=*/true, window);
+  if (rc) return rc;
+  if (!params || !target || !loss || !grad_row) { set_error("null argument"); return AWB_ERR_INVALID; }
+  const int64_t n = row_end - row_begin;
+  Workspace w = carve(h, n, true, ws, true);
+  w.row0 = row_begin;
+  const float* tg = target + row_begin;
+  float* loss_slot = grad_row + h->lay.P;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (h->desc.precision == AWB_PREC_F16) {
+    const bool reuse = (flags & AWB_FIT_REUSE_PACKED) != 0;
+    const bool flow = has_flow(h);
+    int n_part = 0;
+    if (flow) { rc = flow_forward(h, params, g, w, nullptr, st); if (rc) return rc; }
+    rc = tc_fit_forward_backward(h, params, g, tg, loss, nullptr, 1, w, &n_part, st, reuse, flow ? w.X : nullptr,
+                                 flow ? w.dX : nullptr);
+    if (rc) return rc;
+    if (flow) { rc = flow_backward(h, params, g, w, st); if (rc) return rc; }
+    return simt_reduce_grads(h, grad_row, w, n, st, n_part, loss_slot);
+  }
+  rc = simt_forward(h, params, g, nullptr, nullptr, true, w, st);
+  if (rc) return rc;
+  rc = simt_backward(h, params, g, tg, loss, nullptr, false, w, st);
+  if (rc) return rc;
+  return simt_reduce_grads(h, grad_row, w, n, st, -1, loss_slot);
+}
+
+int awb_prior_rows_opt_step(awb_handle h, float* params, void* opt_state, const float* rows, int32_t n_rows,
+                            const awb_opt_hyper* hy, float* loss_out, void* ws, size_t ws_bytes, void* stream) {
+  (void)ws; (void)ws_bytes;   // the optimizer needs no scratch (see awb.h)
+  int rc = check_sliceable(h);
+  if (rc) return rc;
+  if (!params || !opt_state || !rows || !hy) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if (n_rows < 1) { set_error("n_rows must be >= 1, got %d", n_rows); return AWB_ERR_INVALID; }
+  const int64_t R = h->lay.P + 1;
+  return reduce_opt_plain(h, params, opt_state, hy, loss_out, rows, n_rows, R, rows + h->lay.P, R, (cudaStream_t)stream);
 }
 
 int awb_prior_fit_steps(awb_handle h, float* params, void* opt_state, const awb_grid_spec* g, const float* const* targets,
@@ -514,7 +580,7 @@ int awb_star_fit_step(awb_handle h, float* params, void* opt_state, const float*
   cudaStream_t st = (cudaStream_t)stream;
   int rc = star_run(h, params, x, target, n, loss, nullptr, part, lossp, true, &nc, st);
   if (rc) return rc;
-  return reduce_opt_plain(h, params, opt_state, hy, loss_out, part, nc, lossp, st);
+  return reduce_opt_plain(h, params, opt_state, hy, loss_out, part, nc, h->lay.P, lossp, 1, st);
 }
 
 int awb_opt_set_lr(awb_handle h, void* opt_state, const double* lr, void* stream) {

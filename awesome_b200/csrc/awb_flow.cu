@@ -1623,12 +1623,12 @@ static FlowP make_p(const awb_prior* h, const float* params, const awb_grid_spec
   const Layout& L = h->lay;
   FlowP p = {};
   p.g.mode = g->mode; p.g.B = g->B; p.g.H = g->H; p.g.W = g->W; p.g.C = L.C;
-  p.g.t0 = g->t0; p.g.t_step = g->t_step; p.g.grid = g->grid;
+  p.g.t0 = g->t0; p.g.t_step = g->t_step; p.g.grid = g->grid; p.g.row0 = (uint32_t)ws.row0;
   p.fc = h->fc;
   p.params = params; p.P = L.P; p.off_flow = L.off_flow; p.P_flow = L.P_flow; p.per_flow = L.per_flow;
   p.off_lin = L.off_lin;
   p.C = L.C; p.F = L.F; p.m = L.m; p.tanh_out = h->desc.flow_tanh; p.use_linear = 1; p.out_scale = h->fc.out_scale; p.inv_out_scale = 1.f / h->fc.out_scale;
-  p.N = (int64_t)g->B * g->H * g->W;
+  p.N = ws.N;
   p.X = ws.X; p.zin = nullptr; p.deformed = nullptr; p.dX = ws.dX; p.fpart = ws.fpart;
   p.chunk = split_chunk(p.N); p.O = h->desc.n_objects; p.rounds = 1; p.rounds1 = 0; p.dz_smem = 0; p.dzp_g = nullptr;
   p.tab = ws.flowtab; p.segscr = nullptr;
@@ -1718,6 +1718,7 @@ int flow_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
 
 int flow_inverse(const awb_prior* h, const float* params, const awb_grid_spec* g, float* out, cudaStream_t st) {
   Workspace none = {};
+  none.N = (int64_t)g->B * g->H * g->W;
   FlowP p = make_p(h, params, g, none);
   const int PF = (int)(h->lay.P_flow + 2 * h->lay.C);
   size_t smem = sizeof(float) * PF;

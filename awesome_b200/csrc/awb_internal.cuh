@@ -112,6 +112,10 @@ struct Workspace {
   float* flowseg; // RealNVP, C = 2, training: [S][O][F][8][144] per-warp histogram sums of the segment backward
   void* tc;       // tensor-core path scratch
   int64_t bytes;
+  // the pixel rows [row0, row0 + N) of the grid's batch this call works on: the whole batch (row0 = 0) for every entry
+  // point but awb_prior_slice_grads.  Kernels index their scratch and the target by the local row and generate (or read)
+  // coordinates at the global one.
+  int64_t row0, N;
 };
 Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only = false);
 
@@ -150,6 +154,7 @@ struct GridDev {
   int mode, B, H, W, C;
   float t0, t_step;
   const float* grid;
+  uint32_t row0;   // global index of local row 0 (Workspace::row0)
 };
 int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, float* logits_out,
                  float* deformed, bool training, const Workspace& ws, cudaStream_t st);
@@ -161,7 +166,9 @@ int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
 // partials always come from flow_backward's n_splits(N) pixel ranges.
 int simt_reduce_opt(const awb_prior* h, float* params, void* opt_state, const awb_opt_hyper* hy,
                     float* loss_out, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1);
-int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1);
+// loss_slot (optional, single object): receives the sum of the loss partials (gradient row of awb_prior_slice_grads)
+int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1,
+                      float* loss_slot = nullptr);
 int absmax_per_object(const float* x, int64_t n, int O, float* out, cudaStream_t st);   // out[o] = max |x[o][:]|
 int simt_dgrid(const awb_prior* h, const awb_grid_spec* g, float* dgrid, const Workspace& ws, cudaStream_t st);
 int optim_step(const awb_prior* h, float* params, const float* grads, void* opt_state,
@@ -169,8 +176,11 @@ int optim_step(const awb_prior* h, float* params, const float* grads, void* opt_
 int clamp_only(const awb_prior* h, float* params, cudaStream_t st);
 int plateau_step(const awb_prior* h, void* opt_state, const float* loss, int stride, const awb_opt_hyper* hy, cudaStream_t st);
 // reduce [S][P] plain (state_dict order) gradient partials + [S] loss partials, then the optimizer step
+// (partial s at partials + s * part_stride, its loss at lossp[s * loss_stride]; awb_prior_rows_opt_step: the loss is
+// column P of each gradient row)
 int reduce_opt_plain(const awb_prior* h, float* params, void* opt_state, const awb_opt_hyper* hy, float* loss_out,
-                     const float* partials, int S, const float* lossp, cudaStream_t st);
+                     const float* partials, int S, int64_t part_stride, const float* lossp, int64_t loss_stride,
+                     cudaStream_t st);
 // ---- star-shape prior, implemented in awb_star.cu
 int star_n_ctas(int64_t n);
 int star_run(const awb_prior* h, const float* params, const float* x, const float* target, int64_t n,
@@ -225,7 +235,7 @@ inline int any_flow_backward(const awb_prior* h, const float* params, const awb_
   return h->desc.kind == AWB_KIND_DIFFEO_ICNN ? diffeo_backward(h, params, g, ws, st) : flow_backward(h, params, g, ws, st);
 }
 
-// Pixel coordinate of row n, channel c (SURVEY a1).  torch.linspace semantics for
+// Pixel coordinate of local row n (global row n + g.row0), channel c (SURVEY a1).  torch.linspace semantics for
 // AWB_GRID_LINSPACE: step = 1/(n-1); first half start+i*step, second half end-(n-1-i)*step.
 __device__ __forceinline__ float lin01(int i, int n) {
   if (n <= 1) return 0.f;
@@ -234,7 +244,7 @@ __device__ __forceinline__ float lin01(int i, int n) {
 }
 __device__ __forceinline__ float coord(const GridDev& g, int64_t n, int c) {
   // 32-bit index arithmetic: N <= 2^30 pixel rows is checked at every entry point (check_common)
-  const uint32_t hw = (uint32_t)g.H * (uint32_t)g.W, nn = (uint32_t)n;
+  const uint32_t hw = (uint32_t)g.H * (uint32_t)g.W, nn = (uint32_t)n + g.row0;
   const uint32_t b = nn / hw, r = nn - b * hw;
   if (g.mode == AWB_GRID_EXPLICIT) return g.grid[((int64_t)b * g.C + c) * hw + r];
   if (c == 2) return g.t0 + (float)b * g.t_step;

@@ -438,7 +438,7 @@ struct OptP {
   float* params; float* m; float* v; OptScal* scal;
   const float* part; int64_t sSplit; int S;      // ICNN partials [S][O][G]
   const float* fpart; int64_t sFSplit; int SF;   // flow+linear partials [SF][O][PF]
-  const float* lossp;                            // [S][O]
+  const float* lossp; int64_t sLoss;             // loss partial s of object o at lossp[s * sLoss + o]
   const float* grads;                            // direct gradients (awb_optim_step) or null
   const int32_t* map; const uint8_t* clamp; const uint8_t* group;
   int64_t P, off_icnn, P_icnn, off_flow, PF, G;
@@ -470,7 +470,7 @@ __global__ void __launch_bounds__(256) k_reduce_opt(OptP a, int n_groups, int us
       // fixed-order loss sum: lane-strided then butterfly
       float l = 0.f;
       const int SL = a.S > 0 ? a.S : a.SF;
-      for (int s = lane; s < SL; s += 32) l += a.lossp[s * a.O + o];
+      for (int s = lane; s < SL; s += 32) l += a.lossp[s * a.sLoss + o];
 #pragma unroll
       for (int off = 16; off > 0; off >>= 1) l += __shfl_xor_sync(0xffffffffu, l, off);
       if (lane == 0) s_loss = l;
@@ -732,11 +732,22 @@ int absmax_per_object(const float* x, int64_t n, int O, float* out, cudaStream_t
   return AWB_OK;
 }
 
+// grads[o][i] = sum of the partials of parameter i in fixed partial order.  loss_slot (single object): thread P writes the
+// sum of the S loss partials behind the gradient -- the [P + 1] gradient row of awb_prior_slice_grads.
 __global__ void k_reduce_grads(float* grads, const float* part, int64_t sSplit, int S, int SF, const float* fpart,
                                int64_t sFSplit, const int32_t* map, int64_t P, int64_t off_icnn,
-                               int64_t P_icnn, int64_t off_flow, int64_t PF, int64_t G) {
+                               int64_t P_icnn, int64_t off_flow, int64_t PF, int64_t G, const float* lossp,
+                               float* loss_slot) {
+  grid_dep_wait();      // the partials are complete
+  grid_dep_launch();
   int o = blockIdx.y;
   int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+  if (loss_slot && i == P) {
+    float l = 0.f;
+    for (int s = 0; s < S; s++) l += lossp[s];
+    *loss_slot = l;
+    return;
+  }
   if (i >= P) return;
   float g = 0.f;
   if (i >= off_icnn && i < off_icnn + P_icnn) {
@@ -780,10 +791,10 @@ __global__ void k_dgrid(const float* dX, float* dgrid, int64_t N, int64_t HW, in
 }
 
 // ======================================================================= host launchers
-static GridDev to_dev(const awb_grid_spec* g, int C) {
+static GridDev to_dev(const awb_grid_spec* g, int C, int64_t row0) {
   GridDev d;
   d.mode = g->mode; d.B = g->B; d.H = g->H; d.W = g->W; d.C = C;
-  d.t0 = g->t0; d.t_step = g->t_step; d.grid = g->grid;
+  d.t0 = g->t0; d.t_step = g->t_step; d.grid = g->grid; d.row0 = (uint32_t)row0;
   return d;
 }
 
@@ -798,7 +809,7 @@ int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
                  float* deformed, bool training, const Workspace& ws, cudaStream_t st) {
   const Layout& L = h->lay;
   const int O = h->desc.n_objects;
-  const int64_t N = (int64_t)g->B * g->H * g->W;
+  const int64_t N = ws.N;
   AWB_CUDA(cudaMemsetAsync(ws.waug, 0, sizeof(float) * O * L.G, st));
   AWB_LAUNCH(PK_PACK, st, k_pack<<<dim3((unsigned)((L.P_icnn + 255) / 256), O), 256, 0, st>>>(params, ws.waug, h->d_map, (int)L.P_icnn,
                                                                        L.P, L.off_icnn, L.G));
@@ -810,7 +821,7 @@ int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
   }
   const int64_t sLayer = N * L.ld;            // one ZA layer
   const int64_t sZAobj = (L.L + 1) * sLayer;  // all layers of an object
-  AWB_LAUNCH(PK_INPUT, st, k_input<<<dim3((unsigned)((N + 63) / 64), O), 256, 0, st>>>(to_dev(g, L.C), x_ready, ws.X, ws.waug, ws.ZA, N,
+  AWB_LAUNCH(PK_INPUT, st, k_input<<<dim3((unsigned)((N + 63) / 64), O), 256, 0, st>>>(to_dev(g, L.C, ws.row0), x_ready, ws.X, ws.waug, ws.ZA, N,
                                                               L.h, L.C, L.ld, L.G, L.aug_in, sZAobj));
   for (int i = 0; i < L.L; i++) {
     GemmP p = {};
@@ -851,7 +862,7 @@ int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
                   cudaStream_t st) {
   const Layout& L = h->lay;
   const int O = h->desc.n_objects;
-  const int64_t N = (int64_t)g->B * g->H * g->W;
+  const int64_t N = ws.N;
   const int S = n_splits(N);
   const int64_t chunk = split_chunk(N);
   const int64_t sLayer = N * L.ld, sZAobj = (L.L + 1) * sLayer, sDobj = 2 * sLayer;
@@ -924,7 +935,7 @@ int simt_reduce_opt(const awb_prior* h, float* params, void* opt_state, const aw
   a.SF = n_splits(N);
   a.PF = L.P_flow + L.n_lin;
   a.fpart = ws.fpart; a.sFSplit = (int64_t)O * a.PF;
-  a.lossp = ws.lossp; a.grads = nullptr;
+  a.lossp = ws.lossp; a.sLoss = O; a.grads = nullptr;
   a.map = h->d_map; a.clamp = h->d_clamp; a.group = h->d_group;
   a.P = L.P; a.off_icnn = L.off_icnn; a.P_icnn = L.P_icnn; a.off_flow = L.off_flow; a.G = L.G;
   a.O = O; a.hy = *hy; a.loss_out = loss_out;
@@ -955,14 +966,15 @@ int simt_reduce_opt(const awb_prior* h, float* params, void* opt_state, const aw
 }
 
 int reduce_opt_plain(const awb_prior* h, float* params, void* opt_state, const awb_opt_hyper* hy, float* loss_out,
-                     const float* partials, int S, const float* lossp, cudaStream_t st) {
+                     const float* partials, int S, int64_t part_stride, const float* lossp, int64_t loss_stride,
+                     cudaStream_t st) {
   const Layout& L = h->lay;
   OptP a = {};
   a.params = params;
   opt_ptrs(h, opt_state, &a.m, &a.v, &a.scal);
   a.part = nullptr; a.sSplit = 0; a.S = 0;
-  a.fpart = partials; a.PF = L.P; a.sFSplit = L.P; a.SF = S;
-  a.lossp = lossp; a.grads = nullptr;
+  a.fpart = partials; a.PF = L.P; a.sFSplit = part_stride; a.SF = S;
+  a.lossp = lossp; a.sLoss = loss_stride; a.grads = nullptr;
   a.map = nullptr; a.clamp = h->d_clamp; a.group = h->d_group;
   a.P = L.P; a.off_icnn = 0; a.P_icnn = 0; a.off_flow = 0; a.G = 0;
   a.O = 1; a.hy = *hy; a.loss_out = loss_out;
@@ -971,13 +983,17 @@ int reduce_opt_plain(const awb_prior* h, float* params, void* opt_state, const a
   return AWB_OK;
 }
 
-int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials) {
+int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials,
+                      float* loss_slot) {
   const Layout& L = h->lay;
   const int O = h->desc.n_objects;
+  if (loss_slot && O != 1) { set_error("internal: a gradient row is single-object"); return AWB_ERR_INVALID; }
   int64_t PF = L.P_flow + L.n_lin;
-  AWB_LAUNCH(PK_OPT, st, k_reduce_grads<<<dim3((unsigned)((L.P + 255) / 256), O), 256, 0, st>>>(
-      grads, ws.part, (int64_t)O * L.G, n_partials > 0 ? n_partials : n_splits(N), n_splits(N), ws.fpart, (int64_t)O * PF, h->d_map, L.P, L.off_icnn,
-      L.P_icnn, L.off_flow, PF, L.G));
+  const int64_t n_thr = L.P + (loss_slot ? 1 : 0);
+  AWB_LAUNCH(PK_OPT, st, AWB_CUDA(launch_ex(k_reduce_grads, dim3((unsigned)((n_thr + 255) / 256), O), dim3(256), 0, st, true,
+      grads, (const float*)ws.part, (int64_t)O * L.G, n_partials > 0 ? n_partials : n_splits(N), n_splits(N),
+      (const float*)ws.fpart, (int64_t)O * PF, (const int32_t*)h->d_map, (int64_t)L.P, (int64_t)L.off_icnn,
+      (int64_t)L.P_icnn, (int64_t)L.off_flow, PF, (int64_t)L.G, (const float*)ws.lossp, loss_slot)));
   AWB_CUDA(cudaGetLastError());
   return AWB_OK;
 }

@@ -118,6 +118,7 @@ __device__ __forceinline__ float half_hi(uint32_t u) { return __high2float(*rein
 // Out of line on purpose: the hot loop only carries the division-free linspace path; explicit grids, the notebooks'
 // index grid and the padding rows of a last tile come here (the fused kernel's speed depends on its code footprint).
 __device__ __noinline__ void row_coords(const GridDev g, uint32_t n, int C, float& x0, float& x1, float& x2) {
+  n += g.row0;   // local -> global row
   const uint32_t hw = (uint32_t)g.H * (uint32_t)g.W;
   const uint32_t b = n / hw, r = n - b * hw;
   const uint32_t i = r / (uint32_t)g.W, j = r - i * (uint32_t)g.W;
@@ -438,7 +439,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
     const uint32_t gW = (uint32_t)p.g.W, gH = (uint32_t)p.g.H, hw = gH * gW;
     uint32_t pb, pi, pj, db, di, dj;
     {
-      const uint32_t n0 = blockIdx.x * 128u + (uint32_t)row, d = gridDim.x * 128u;
+      const uint32_t n0 = p.g.row0 + blockIdx.x * 128u + (uint32_t)row, d = gridDim.x * 128u;   // global row
       pb = n0 / hw; uint32_t r = n0 - pb * hw; pi = r / gW; pj = r - pi * gW;
       db = d / hw; r = d - db * hw; di = r / gW; dj = r - di * gW;
     }
@@ -849,7 +850,7 @@ int tc_fit_forward_backward(const awb_prior* h, const float* params, const awb_g
                             cudaStream_t st, bool reuse_packed, const float* Xrows, float* dXrows, const float* amax) {
   const Layout& Ly = h->lay;
   const int O = h->desc.n_objects, L = Ly.L, C = Ly.C;
-  const int64_t N = (int64_t)g->B * g->H * g->W;
+  const int64_t N = ws.N;
   if (!tc_supported(h)) { set_error("precision f16 supports ICNN / flow+ICNN priors with h=130, L in {1,2}"); return AWB_ERR_UNSUPPORTED; }
   const int n_tiles = (int)((N + 127) / 128);
   int sms = 148;
@@ -868,6 +869,7 @@ int tc_fit_forward_backward(const awb_prior* h, const float* params, const awb_g
                                                                                       L, Ly.P, img_stride));
   TcP p = {};
   p.g.mode = g->mode; p.g.B = g->B; p.g.H = g->H; p.g.W = g->W; p.g.C = C; p.g.t0 = g->t0; p.g.t_step = g->t_step; p.g.grid = g->grid;
+  p.g.row0 = (uint32_t)ws.row0;
   p.img = (const uint8_t*)ws.tc; p.img_stride = img_stride;
   p.target = target;
   for (int o = 0; o < O && o < 16; o++) {

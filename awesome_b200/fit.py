@@ -329,3 +329,140 @@ class FlowIdentityFitter(PriorFitter):
         L.check(self.lib.awb_flow_identity_step(self.prior.handle, self.params.data_ptr(), self.opt_state.data_ptr(),
                                                 C.byref(self._gs), C.byref(self._hyper), loss_ptr,
                                                 self.ws.data_ptr(), self.ws.numel(), L.stream_ptr()))
+
+
+# ------------------------------------------------------------------ pixel-sliced fit step (one prior on several GPUs)
+SLICE_ALIGN = 128     # one tile of the tensor path
+
+
+def slice_plan(n_rows: int, n_slices: int) -> List[tuple]:
+    """Cut the pixel rows ``[0, n_rows)`` of a step's batch into ``n_slices`` contiguous ``(begin, end)`` slices.
+
+    Boundaries lie on multiples of 128 rows (except ``n_rows`` itself) and slice sizes differ by at most 128: slice ``k``
+    gets tiles ``[k T // S, (k + 1) T // S)`` of the ``T = ceil(n_rows / 128)`` tiles, so the last slice, which holds
+    the partial tile, is one of the larger ones.  With fewer tiles than slices some slices are empty (``begin == end``);
+    their gradient row is zero.  The plan depends on ``n_rows`` and ``n_slices`` only, never on the number of ranks."""
+    if n_slices < 1:
+        raise ValueError(f"n_slices must be >= 1, got {n_slices}")
+    if n_rows < 1:
+        raise ValueError(f"n_rows must be >= 1, got {n_rows}")
+    tiles = (n_rows + SLICE_ALIGN - 1) // SLICE_ALIGN
+    cuts = [min(n_rows, (k * tiles // n_slices) * SLICE_ALIGN) for k in range(n_slices + 1)]
+    return [(cuts[k], cuts[k + 1]) for k in range(n_slices)]
+
+
+def rank_slices(n_slices: int, rank: int, world: int) -> range:
+    """The slices rank ``rank`` of ``world`` computes: ``[rank S / world, (rank + 1) S / world)``."""
+    if world < 1 or not 0 <= rank < world:
+        raise ValueError(f"bad rank {rank} of world {world}")
+    if n_slices % world:
+        raise ValueError(f"the number of slices ({n_slices}) must be a multiple of the number of ranks ({world})")
+    per = n_slices // world
+    return range(rank * per, (rank + 1) * per)
+
+
+def gather_slice_rows(mine: Sequence[int], local: torch.Tensor, rows: torch.Tensor, produce, group=None) -> torch.Tensor:
+    """One sliced step up to the optimizer: ``produce(k, local[j], j)`` writes the row of this rank's ``j``-th slice ``k``
+    into ``local``, then ``all_gather_into_tensor`` gives every rank all ``[S, R]`` rows in slice order (a copy: every rank
+    holds the same bits).  ``local`` may be ``rows`` itself (one rank: no collective)."""
+    for j, k in enumerate(mine):
+        produce(k, local[j], j)
+    if local.data_ptr() != rows.data_ptr() or local.shape != rows.shape:
+        import torch.distributed as dist
+        dist.all_gather_into_tensor(rows, local, group=group)
+    return rows
+
+
+class SlicedFitter:
+    """The fused fit step of ``PriorFitter`` computed in pixel slices, for fitting ONE prior on several GPUs.
+
+    The batch's pixel rows are cut into ``n_slices`` slices (``slice_plan``); this rank computes the gradient rows of its
+    slices (``rank_slices``), the rows of all ranks are gathered in slice order over ``group`` and every rank runs the same
+    optimizer kernel on the same rows.  The parameters after any number of steps are therefore bit-identical for every
+    ``world`` dividing ``n_slices``, and on every rank; a one-rank run computes all slices one after the other.
+
+    The loss is the full batch's (coefficients from ``loss.to_specs`` on the whole target), so the rows add up to the
+    fused step's gradient and loss up to summation order.  Single-object ICNN and RealNVP o ICNN priors."""
+
+    def __init__(self, prior: Prior, params: torch.Tensor, grid: GridSpecHost, target: torch.Tensor,
+                 loss: LossConfig, optim: OptimConfig, n_slices: int = 8, group=None):
+        L.require_cuda()
+        if prior.n_objects != 1:
+            raise ValueError("sliced fits take single-object priors")
+        if group is not None:
+            import torch.distributed as dist
+            rank, world = dist.get_rank(group), dist.get_world_size(group)
+        else:
+            rank, world = 0, 1
+        self.mine = rank_slices(int(n_slices), rank, world)        # raises unless world divides n_slices
+        self.prior, self.params, self.group = prior, params, group
+        self.n_slices = int(n_slices)
+        self.device = params.device
+        self.lib = prior.lib
+        self.target = target.detach().reshape(1, -1).contiguous().float()
+        if self.target.shape[1] != grid.n_pixels:
+            raise ValueError(f"target has {self.target.shape[1]} pixels, grid has {grid.n_pixels}")
+        if params.numel() != prior.n_params or params.dtype != torch.float32 or not params.is_contiguous():
+            raise ValueError("params must be a contiguous fp32 [1,P] arena")
+        self.grid = grid
+        self.plan = slice_plan(grid.n_pixels, self.n_slices)
+        R = prior.grad_row_floats
+        biggest = max(e - b for b, e in self.plan)
+        with torch.cuda.device(self.device):
+            self.ws = prior.new_workspace(biggest, 2, self.device)          # one slice after the other
+            self.opt_state = torch.empty(prior.opt_state_bytes(), dtype=torch.uint8, device=self.device)
+            self.rows = torch.zeros((self.n_slices, R), dtype=torch.float32, device=self.device)   # empty slices stay 0
+            self.local = self.rows if world == 1 else torch.zeros((len(self.mine), R), dtype=torch.float32,
+                                                                   device=self.device)
+            self._spec = loss.to_specs(self.target)[0]
+        self._hyper = optim.to_c()
+        self.optim = optim
+        self.steps_done = 0
+        self.reset_optimizer()
+
+    def reset_optimizer(self) -> None:
+        lrs = (C.c_double * L.AWB_MAX_GROUPS)(*self.optim.lrs())
+        with torch.cuda.device(self.device):
+            L.check(self.lib.awb_opt_state_init(self.prior.handle, self.opt_state.data_ptr(), lrs, L.stream_ptr()))
+        self.steps_done = 0
+
+    def set_target(self, target: torch.Tensor) -> None:
+        """New unaries for the same grid shape; the loss coefficients are kept (as ``PriorFitter.set_target``)."""
+        self.target.copy_(target.detach().reshape(self.target.shape))
+
+    def _produce(self, k: int, row: torch.Tensor, j: int) -> None:
+        b, e = self.plan[k]
+        if j == 0:
+            self._packed = 0            # the parameters have changed since the last slice
+        if b == e:
+            row.zero_()
+            return
+        # the weight image sits at an offset of the workspace that depends on the window's row count
+        self.prior.slice_grads(self.params, self.grid, b, e, self.target, self._spec, row, self.ws,
+                               reuse_packed=self._packed == e - b)
+        self._packed = e - b
+
+    def step(self, loss_out: Optional[torch.Tensor] = None) -> None:
+        """One sliced step; ``loss_out`` (optional, one device float) receives the step's loss.  No host sync."""
+        with torch.cuda.device(self.device):
+            rows = gather_slice_rows(self.mine, self.local, self.rows, self._produce, self.group)
+            self.prior.rows_opt_step(self.params, self.opt_state, rows, self._hyper, loss_out)
+        self.steps_done += 1
+
+    def run(self, steps: int) -> torch.Tensor:
+        """``steps`` sliced steps.  Returns the device loss history ``[steps, 1]`` (written by the optimizer kernel)."""
+        hist = torch.empty((steps, 1), dtype=torch.float32, device=self.device)
+        for s in range(steps):
+            self.step(hist[s])
+        return hist
+
+    def scalars(self, obj: int = 0) -> L.OptScalars:
+        out = L.OptScalars()
+        with torch.cuda.device(self.device):
+            L.check(self.lib.awb_opt_read_scalars(self.prior.handle, self.opt_state.data_ptr(), obj, C.byref(out),
+                                                  L.stream_ptr()))
+        return out
+
+    def raise_if_nonfinite(self) -> None:
+        if self.scalars(0).nonfinite:
+            raise ValueError("Loss is nan or inf!")

@@ -21,7 +21,7 @@ import torch
 
 from . import _lib as L
 from .core import GridSpecHost, iou_counts, target_counts
-from .fit import LossConfig, OptimConfig, PriorFitter
+from .fit import LossConfig, OptimConfig, PriorFitter, SlicedFitter
 
 
 @dataclass
@@ -54,6 +54,8 @@ class FitSchedule:
     plateau_factor: float = 0.5
     plateau_threshold: float = 1e-4      # torch default (rel)
     steps_per_graph: int = 50
+    sequence_slices: int = 0             # spatio-temporal loop: pixel slices per step across the ranks of torch.distributed
+                                         # (0 = off; used by pretrain() when a process group is initialised)
 
     @classmethod
     def from_pretrain_args(cls, kwargs: Dict[str, Any]) -> "FitSchedule":
@@ -316,7 +318,7 @@ def _plateau_hyper(s: FitSchedule, has_flow: bool):
 
 def fit_sequence(model, n_frames: int, H: int, W: int, unaries: torch.Tensor, schedule: Optional[FitSchedule] = None,
                  grid_mode: str = "linspace", first_last_unaries: Optional[torch.Tensor] = None,
-                 lr_trace: Optional[list] = None) -> torch.Tensor:
+                 lr_trace: Optional[list] = None, n_slices: Optional[int] = None, group=None) -> torch.Tensor:
     """Spatio-temporal fit (``_non_prior_based_pretrain``, ``path_connected_net.py:511-728``): ONE (x, y, t) prior for all
     frames.  ``unaries`` ``[T,H,W]``; frame ``i`` has ``t = i / (T - 1)`` (``awesome/dataset/transformator.py:54-60``).
 
@@ -327,6 +329,16 @@ def fit_sequence(model, n_frames: int, H: int, W: int, unaries: torch.Tensor, sc
       ``ceil(T / batch_size)`` frame batches (in order, or shuffled with ``dataloader_shuffle``), one fused fit step per
       batch; ``ReduceLROnPlateau.step`` ONCE PER EPOCH on the epoch-mean loss (``:719``) -- the batch steps run with the
       scheduler off and the epoch end calls ``awb_opt_plateau_step``.
+
+    ``n_slices``: the main loop runs pixel-sliced (``SlicedFitter``): the pixel rows of every batch are cut into
+    ``n_slices`` slices, spread over the ranks of ``group`` (a ``torch.distributed`` process group, ``None`` = this
+    process alone), whose gradient rows are gathered and summed in slice order before the optimizer step.  The batches,
+    their order and the number of optimizer steps are the reference's; only the summation order of a step's gradient
+    differs from the unsliced loop, and the result is bit-identical for every number of ranks dividing ``n_slices``.  The
+    prefits and the ActNorm init are not sliced: every rank runs them, and rank 0's result (arena and, with
+    ``noisy_percentage``, the unaries) is then broadcast, so all ranks start the main loop from the same bits even when
+    their random number generators differ.  With ``dataloader_shuffle`` rank 0 draws each epoch's permutation from the
+    global RNG exactly as a one-rank run does and broadcasts it.  ``None`` keeps the unsliced fused loop.
     Returns the per-step loss history ``[num_epochs * n_batches]`` (device)."""
     import ctypes as C
     import dataclasses
@@ -338,6 +350,14 @@ def fit_sequence(model, n_frames: int, H: int, W: int, unaries: torch.Tensor, sc
     un = unaries.detach().to(dev).float().reshape(T, H * W)
     if s.noisy_percentage > 0:
         un, _ = noisy_unaries(un, s.noisy_percentage)
+    sliced = n_slices is not None
+    multi_rank = sliced and group is not None
+    if multi_rank:
+        import torch.distributed as dist
+        src = dist.get_global_rank(group, 0)
+        if s.noisy_percentage > 0:
+            un = un.contiguous()
+            dist.broadcast(un, src, group=group)
     has_flow = hasattr(model, "flow_net")
     C_in = getattr(model, "in_channels", getattr(model, "in_features", 2))
     full = GridSpecHost(grid_mode, T, H, W, t0=0.0, t_step=t_step)
@@ -354,6 +374,9 @@ def fit_sequence(model, n_frames: int, H: int, W: int, unaries: torch.Tensor, sc
                                max_iter=s.prefit_convex_net_num_epochs, use_progress_bar=False)
     if has_flow:
         model._maybe_actnorm_init(full.materialize(C_in, dev)[:min(bs, T)])     # first batch the full prior ever sees
+    if multi_rank:
+        arena = model._ensure_flat()
+        dist.broadcast(arena.data, src, group=group)
     # batch steps never advance the scheduler; the epoch end does
     step_optim = dataclasses.replace(s.optim(has_flow), plateau=False)
     plateau_hy = _plateau_hyper(s, has_flow)
@@ -369,7 +392,28 @@ def fit_sequence(model, n_frames: int, H: int, W: int, unaries: torch.Tensor, sc
             f.opt_state = first.opt_state
             if f.ws.numel() == first.ws.numel():
                 f.ws = first.ws     # batches run one after the other: one scratch area
+            if sliced:              # ... and one row buffer
+                f.rows, f.local = first.rows, (first.rows if first.local is first.rows else first.local)
         return f
+
+    def make(spec: GridSpecHost, target: torch.Tensor):
+        if not sliced:
+            return share(model.make_fitter(spec, target, s.criterion, step_optim, use_graph=False))
+        prior = model._prior_for(model._ensure_flat().device)
+        return share(SlicedFitter(prior, model._ensure_flat(), spec, target, s.criterion, step_optim, n_slices=n_slices,
+                                  group=group))
+
+    def epoch_batches() -> List[torch.Tensor]:
+        """The reference's DataLoader(shuffle=True) batches of this epoch (same sampler, same global-RNG stream); with
+        several ranks rank 0 draws them and broadcasts the permutation."""
+        from torch.utils.data import DataLoader, TensorDataset
+        if not multi_rank:
+            return [idx for (idx,) in DataLoader(TensorDataset(torch.arange(T)), batch_size=bs, shuffle=True)]
+        perm = torch.empty(T, dtype=torch.int64, device=dev)
+        if dist.get_rank(group) == 0:
+            perm.copy_(torch.cat([idx for (idx,) in DataLoader(TensorDataset(torch.arange(T)), batch_size=bs, shuffle=True)]))
+        dist.broadcast(perm, src, group=group)
+        return list(perm.cpu().split(bs))
 
     def end_of_epoch(losses: List[torch.Tensor]) -> None:
         if not s.plateau:
@@ -386,8 +430,7 @@ def fit_sequence(model, n_frames: int, H: int, W: int, unaries: torch.Tensor, sc
         for b0 in range(0, T, bs):
             nb = min(bs, T - b0)
             spec = GridSpecHost(grid_mode, nb, H, W, t0=b0 * t_step, t_step=t_step)
-            fitters.append(share(model.make_fitter(spec, un[b0:b0 + nb].reshape(1, -1), s.criterion, step_optim,
-                                                   use_graph=False)))
+            fitters.append(make(spec, un[b0:b0 + nb].reshape(1, -1)))
         for _ in range(s.num_epochs):
             ep = [f.run(1)[0, 0] for f in fitters]
             hist += ep
@@ -395,18 +438,16 @@ def fit_sequence(model, n_frames: int, H: int, W: int, unaries: torch.Tensor, sc
     else:
         # shuffled batches (the reference's DataLoader(shuffle=True): same sampler, same global-RNG stream): the frames of a
         # batch are not equidistant in t, so the batch grid is gathered into a staging tensor
-        from torch.utils.data import DataLoader, TensorDataset
         gfull = full.materialize(C_in, dev)
         stage_g, stage_u, fitters_by = {}, {}, {}
         for _ in range(s.num_epochs):
             ep = []
-            for (idx,) in DataLoader(TensorDataset(torch.arange(T)), batch_size=bs, shuffle=True):
+            for idx in epoch_batches():
                 nb = int(idx.numel())
                 if nb not in fitters_by:
                     stage_g[nb] = torch.empty((nb, C_in, H, W), dtype=torch.float32, device=dev)
                     stage_u[nb] = torch.empty((1, nb * H * W), dtype=torch.float32, device=dev)
-                    fitters_by[nb] = share(model.make_fitter(GridSpecHost.from_tensor(stage_g[nb]), stage_u[nb], s.criterion,
-                                                             step_optim, use_graph=False))
+                    fitters_by[nb] = make(GridSpecHost.from_tensor(stage_g[nb]), stage_u[nb])
                 di = idx.to(dev)
                 torch.index_select(gfull, 0, di, out=stage_g[nb])
                 fitters_by[nb].set_target(torch.index_select(un, 0, di).reshape(1, -1))
@@ -597,7 +638,10 @@ def pretrain(self, train_set, test_set=None, device=None, agent=None, use_progre
             return cache.get_state()
         T = len(grids)
         H, W = grids[0].shape[-2:]
-        fit_sequence(self, T, H, W, torch.stack([u.reshape(H, W) for u in uns]), sched)
+        import torch.distributed as dist
+        sliced = sched.sequence_slices > 0 and dist.is_available() and dist.is_initialized()
+        fit_sequence(self, T, H, W, torch.stack([u.reshape(H, W) for u in uns]), sched,
+                     n_slices=sched.sequence_slices if sliced else None, group=dist.group.WORLD if sliced else None)
         return {k: v.detach().cpu().clone() for k, v in self.state_dict().items()}
     finally:
         wrapper_module.train(was_training)

@@ -194,6 +194,30 @@ int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_g
                        const float* target, const awb_loss_spec* loss, const awb_opt_hyper* hyper,
                        float* loss_out, void* workspace, size_t workspace_bytes, int32_t flags, void* stream);
 
+/* Pixel-sliced fit step (one prior fitted on several GPUs, each computing some pixel slices of every step).
+ * Single-object AWB_KIND_ICNN and AWB_KIND_FLOW_ICNN handles, both precisions; other handles: AWB_ERR_UNSUPPORTED.
+ * A gradient row holds the gradient of a slice in state_dict order followed by the slice's loss sum: P + 1 floats. */
+int64_t awb_prior_grad_row_floats(awb_handle h);
+/* Gradient row of pixel rows [row_begin, row_end) of the batch described by grid (the reference's step restricted to
+ * those pixels): forward, loss, backward, cross-CTA reduction; NO optimizer.  Coordinates (generated or read from an
+ * explicit grid) are those of the global rows.  target: the FULL batch [N] (read at row_begin); loss: coefficients of the
+ * FULL batch (1/N, class weights), so that rows add up to the step's gradient and loss.  workspace:
+ * awb_prior_workspace_bytes(h, row_end - row_begin, 2).  flags: AWB_FIT_REUSE_PACKED -- the previous call on this
+ * workspace was a slice of the same params with the same number of rows (tensor path: its fp16 weight image, whose place
+ * in the workspace depends on the row count, is reused).  An empty or out-of-range
+ * window: AWB_ERR_INVALID. */
+int awb_prior_slice_grads(awb_handle h, const float* params, const awb_grid_spec* grid, int64_t row_begin,
+                          int64_t row_end, const float* target, const awb_loss_spec* loss, float* grad_row,
+                          void* workspace, size_t workspace_bytes, int32_t flags, void* stream);
+/* Sum of n_rows gradient rows (row stride awb_prior_grad_row_floats), in a fixed order, then the optimizer step of
+ * awb_prior_fit_step (L2, clamp, non-finite skip + sticky flag, plateau per hyper); loss_out (optional, device) = summed
+ * loss.  The same rows give the same bits on every device.  workspace: unused (may be null), kept so that the optimizer
+ * can later refresh the tensor path's fp16 weight image in place without an ABI change; the next
+ * awb_prior_slice_grads must therefore re-pack (flags = 0). */
+int awb_prior_rows_opt_step(awb_handle h, float* params, void* opt_state, const float* rows, int32_t n_rows,
+                            const awb_opt_hyper* hyper, float* loss_out, void* workspace, size_t workspace_bytes,
+                            void* stream);
+
 /* n_steps fused fit steps in one call, step s fitting the DEVICE target targets[(first + s) % n_targets] ([O][N] each): the
  * reference's step loop (path_connected_net.py:939-953) without a host round trip per step.  loss_out (optional, device):
  * [n_steps][O].  Asynchronous. */
