@@ -178,7 +178,7 @@ def flow_forward(p: Params, z: torch.Tensor, prefix: str, output_fn: Optional[st
     an ``ActNorm``.  With ``actnorm_init`` the ActNorm parameters whose
     ``data_dep_init_done`` buffer is 0 are set from the batch statistics (first
     forward call) and written back into ``p``."""
-    nan = torch.tensor(float("nan"), dtype=z.dtype)
+    nan = torch.tensor(float("nan"), dtype=z.dtype, device=z.device)
     for f in range(flow_num(p, prefix)):
         a, n = f"{prefix}flows.{2 * f}.", f"{prefix}flows.{2 * f + 1}."
         b = p[a + "b"].to(z.dtype)
