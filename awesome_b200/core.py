@@ -92,7 +92,8 @@ class Prior:
         return self._h
 
     def workspace_bytes(self, n_pixels: int, training) -> int:
-        """``training``: False / True, or 2 for a fit-step-only workspace (see ``awb_prior_workspace_bytes``)."""
+        """``training``: False / True, 2 for a fit-step-only workspace, 3 for a deformation-only workspace (see
+        ``awb_prior_workspace_bytes``)."""
         b = int(self.lib.awb_prior_workspace_bytes(self._h, n_pixels, int(training)))
         if b < 0:
             raise L.AwbError(b, "workspace size query failed")
@@ -156,6 +157,28 @@ class Prior:
         L.check(self.lib.awb_prior_backward(self._h, params.data_ptr(), C.byref(gs), dlogits.data_ptr(),
                                             grads.data_ptr(), dgrid.data_ptr() if dgrid is not None else None,
                                             ws.data_ptr(), ws.numel(), L.stream_ptr()))
+        return grads, dgrid
+
+    def deformation(self, params: torch.Tensor, grid: GridSpecHost, training: bool, ws: torch.Tensor) -> torch.Tensor:
+        """``get_deformation`` alone (1x1 conv / linear and flow, no ICNN): pixel rows ``[N, C]``.  ``ws``:
+        ``workspace_bytes(N, 3)``; ``training`` keeps the coupling records for ``deformation_backward``."""
+        out = torch.empty((grid.n_pixels, self.C), dtype=torch.float32, device=params.device)
+        gs = grid.to_c()
+        L.check(self.lib.awb_prior_deformation(self._h, params.data_ptr(), C.byref(gs), out.data_ptr(), int(bool(training)),
+                                               ws.data_ptr(), ws.numel(), L.stream_ptr()))
+        return out
+
+    def deformation_backward(self, params: torch.Tensor, grid: GridSpecHost, d_deformed: torch.Tensor, ws: torch.Tensor,
+                             want_dgrid: bool) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+        """Gradients of ``deformation(training=True)`` on the same ``ws`` for the upstream ``d_deformed`` (``[N, C]``
+        fp32, contiguous): ``grads [P]`` (ICNN entries 0) and, when asked, ``dgrid [B, C, H, W]``."""
+        grads = torch.empty(self.n_params, dtype=torch.float32, device=params.device)
+        dgrid = torch.empty((grid.B, self.C, grid.H, grid.W), dtype=torch.float32, device=params.device) \
+            if want_dgrid else None
+        gs = grid.to_c()
+        L.check(self.lib.awb_prior_deformation_backward(self._h, params.data_ptr(), C.byref(gs), d_deformed.data_ptr(),
+                                                        grads.data_ptr(), dgrid.data_ptr() if dgrid is not None else None,
+                                                        ws.data_ptr(), ws.numel(), L.stream_ptr()))
         return grads, dgrid
 
     def enforce_convexity(self, params: torch.Tensor) -> None:

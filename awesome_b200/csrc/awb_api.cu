@@ -61,7 +61,8 @@ static int64_t align256(int64_t b) { return round_up(b, 256); }
 
 // fit_only: layout for awb_prior_fit_step on a tensor-path handle -- the fused kernel keeps activations on the SM, so
 // the [N][ld] activation / delta planes of the CUDA-core path are not carved (0.85 GB per 640x480 frame).
-Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only) {
+// deform_only: layout of awb_prior_deformation / _backward -- no ICNN partials, planes or tensor-path image either.
+Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only, bool deform_only) {
   const Layout& L = h->lay;
   const int64_t O = h->desc.n_objects;
   int S = n_splits(N);
@@ -75,12 +76,12 @@ Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool f
   auto take = [&](int64_t bytes) { char* r = p ? p + off : nullptr; off += align256(bytes); return r; };
   Workspace w = {};
   w.waug = (float*)take(4 * O * L.G);
-  w.part = (float*)take(training ? 4 * (int64_t)S * O * L.G : 0);
+  w.part = (float*)take(training && !deform_only ? 4 * (int64_t)S * O * L.G : 0);
   w.lossp = (float*)take(4 * ((int64_t)kMaxSplits * O + O));   // [S][O] loss partials + [O] spare scalars (max |dlogits|)
   w.fpart = (float*)take(training ? 4 * (int64_t)S * O * (L.P_flow + L.n_lin) : 0);
   w.X = (float*)take(4 * O * N * 4);
   w.dX = (float*)take(training ? 4 * O * N * 4 : 0);
-  const bool planes = !(fit_only && h->desc.precision == AWB_PREC_F16 && tc_supported(h));
+  const bool planes = !deform_only && !(fit_only && h->desc.precision == AWB_PREC_F16 && tc_supported(h));
   w.ZA = (float*)take(planes ? 4 * O * (L.L + 1) * N * L.ld : 0);
   w.D = (float*)take(training && planes ? 4 * O * 2 * N * L.ld : 0);
   w.logits = (float*)take(4 * O * N);
@@ -90,7 +91,8 @@ Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool f
   w.flowd = (training && rnvp && L.C == 3 && !flow_bwd_dz_in_smem(h, N)) ? (float*)take(4 * O * N * 4) : nullptr;
   w.flowtab = (rnvp && flow_tab_floats(h) > 0) ? (float*)take(4 * flow_tab_floats(h)) : nullptr;
   w.flowseg = (training && rnvp && flow_seg_scratch_floats(h, S) > 0) ? (float*)take(4 * flow_seg_scratch_floats(h, S)) : nullptr;
-  w.tc = (h->desc.precision == AWB_PREC_F16 && tc_supported(h)) ? (void*)take(O * (int64_t)tc_image_bytes(L.L)) : nullptr;
+  w.tc = (!deform_only && h->desc.precision == AWB_PREC_F16 && tc_supported(h)) ? (void*)take(O * (int64_t)tc_image_bytes(L.L))
+                                                                               : nullptr;
   w.bytes = off;
   w.row0 = 0; w.N = N;
   return w;
@@ -233,7 +235,7 @@ int64_t awb_prior_param_count(awb_handle h) { return h ? h->lay.P : -1; }
 
 int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t training) {
   if (!h || n_pixels < 1) return -1;
-  return carve(h, n_pixels, training != 0, nullptr, training == 2).bytes;
+  return carve(h, n_pixels, training != 0, nullptr, training == 2, training == 3).bytes;
 }
 
 int64_t awb_opt_state_bytes(awb_handle h) {
@@ -273,7 +275,7 @@ int awb_prior_set_flow_eval(awb_handle h, int32_t mode) {
 // window (optional, {row_begin, row_end}): the call works on the pixel rows [row_begin, row_end) of the batch, which must
 // be a non-empty range inside [0, N), and the workspace is sized for them
 static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, bool training, int64_t* N,
-                        bool fit_only = false, const int64_t* window = nullptr) {
+                        bool fit_only = false, const int64_t* window = nullptr, bool deform_only = false) {
   if (!h || !g || !ws) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (g->B < 1 || g->H < 1 || g->W < 1) { set_error("empty grid %dx%dx%d", g->B, g->H, g->W); return AWB_ERR_INVALID; }
   if (g->mode == AWB_GRID_EXPLICIT && !g->grid) { set_error("explicit grid needs a pointer"); return AWB_ERR_INVALID; }
@@ -285,7 +287,7 @@ static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t w
               (long long)*N);
     return AWB_ERR_INVALID;
   }
-  int64_t need = carve(h, window ? window[1] - window[0] : *N, training, nullptr, fit_only).bytes;
+  int64_t need = carve(h, window ? window[1] - window[0] : *N, training, nullptr, fit_only, deform_only).bytes;
   if ((int64_t)ws_bytes < need) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)need); return AWB_ERR_WORKSPACE; }
   if (h->desc.kind == AWB_KIND_FLOW_ICNN && !h->fc_set) { set_error("awb_prior_set_flow_consts not called"); return AWB_ERR_INVALID; }
   return AWB_OK;
@@ -326,8 +328,9 @@ int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* g
   int rc = check_common(h, g, ws, ws_bytes, true, &N);
   if (rc) return rc;
   if (!params || !dlogits || !grads) { set_error("null argument"); return AWB_ERR_INVALID; }
-  if (dgrid && (h->desc.kind != AWB_KIND_ICNN || h->desc.n_objects != 1)) {
-    set_error("dgrid is only provided for single-object ICNN priors");
+  if (dgrid && (h->desc.kind == AWB_KIND_STAR || h->desc.n_objects != 1)) {
+    set_error("dgrid is provided for single-object ICNN, RealNVP o ICNN and NormalizingFlow1D o ICNN priors only "
+              "(no caller needs it on grouped or star handles; kind %d, %d objects)", h->desc.kind, h->desc.n_objects);
     return AWB_ERR_UNSUPPORTED;
   }
   Workspace w = carve(h, N, true, ws);
@@ -346,17 +349,18 @@ int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* g
     rc = tc_fit_forward_backward(h, params, g, dlogits, up, nullptr, 1, w, &n_part, st, false, flow ? w.X : nullptr,
                                  (flow || dgrid) ? w.dX : nullptr, amax);
     if (rc) return rc;
-    if (flow) { rc = any_flow_backward(h, params, g, w, st); if (rc) return rc; }
+    // flow priors: the flow backward writes dgrid itself (dX holds the gradient at the deformed coordinates, not the grid)
+    if (flow) { rc = any_flow_backward(h, params, g, w, st, dgrid); if (rc) return rc; }
     rc = simt_reduce_grads(h, grads, w, N, st, n_part);
     if (rc) return rc;
-    if (dgrid) rc = simt_dgrid(h, g, dgrid, w, st);
+    if (dgrid && !flow) rc = simt_dgrid(h, g, dgrid, w, st);
     return rc;
   }
-  rc = simt_backward(h, params, g, nullptr, nullptr, dlogits, dgrid != nullptr, w, st);
+  rc = simt_backward(h, params, g, nullptr, nullptr, dlogits, dgrid != nullptr, w, st, dgrid);
   if (rc) return rc;
   rc = simt_reduce_grads(h, grads, w, N, st);
   if (rc) return rc;
-  if (dgrid) rc = simt_dgrid(h, g, dgrid, w, st);
+  if (dgrid && !has_flow(h)) rc = simt_dgrid(h, g, dgrid, w, st);
   return rc;
 }
 
@@ -392,6 +396,48 @@ int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_g
   rc = simt_backward(h, params, g, target, loss, nullptr, false, w, st);
   if (rc) return rc;
   return simt_reduce_opt(h, params, opt_state, hy, loss_out, w, N, st);
+}
+
+// get_deformation: single-object RealNVP o ICNN and NormalizingFlow1D o ICNN handles
+static int check_deformable(awb_handle h) {
+  if (!h) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if (h->desc.kind == AWB_KIND_ICNN) { set_error("an ICNN prior has no deformation"); return AWB_ERR_INVALID; }
+  if (!has_flow(h) || h->desc.n_objects != 1) {
+    set_error("the deformation entry points support single-object flow priors (kind %d, %d objects)", h->desc.kind,
+              h->desc.n_objects);
+    return AWB_ERR_UNSUPPORTED;
+  }
+  return AWB_OK;
+}
+
+int awb_prior_deformation(awb_handle h, const float* params, const awb_grid_spec* g, float* deformed, int32_t training,
+                          void* ws, size_t ws_bytes, void* stream) {
+  int rc = check_deformable(h);
+  if (rc) return rc;
+  int64_t N;
+  rc = check_common(h, g, ws, ws_bytes, true, &N, false, nullptr, /*deform_only=*/true);
+  if (rc) return rc;
+  if (!params || !deformed) { set_error("null argument"); return AWB_ERR_INVALID; }
+  Workspace w = carve(h, N, true, ws, false, true);
+  if (!training) w.flowz = nullptr;   // the coupling records are kept for awb_prior_deformation_backward only
+  return any_flow_forward(h, params, g, w, deformed, (cudaStream_t)stream);
+}
+
+int awb_prior_deformation_backward(awb_handle h, const float* params, const awb_grid_spec* g, const float* d_deformed,
+                                   float* grads, float* dgrid, void* ws, size_t ws_bytes, void* stream) {
+  int rc = check_deformable(h);
+  if (rc) return rc;
+  int64_t N;
+  rc = check_common(h, g, ws, ws_bytes, true, &N, false, nullptr, /*deform_only=*/true);
+  if (rc) return rc;
+  if (!params || !d_deformed || !grads) { set_error("null argument"); return AWB_ERR_INVALID; }
+  Workspace w = carve(h, N, true, ws, false, true);
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = simt_seed_dX(h, d_deformed, w, st);
+  if (rc) return rc;
+  rc = any_flow_backward(h, params, g, w, st, dgrid);
+  if (rc) return rc;
+  return simt_reduce_grads(h, grads, w, N, st, /*n_partials=*/0);   // no ICNN partials: its entries are exactly 0
 }
 
 // single-object ICNN and RealNVP o ICNN handles (the priors of the spatio-temporal fit)

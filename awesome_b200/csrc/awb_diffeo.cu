@@ -31,6 +31,7 @@ struct DiffP {
   int64_t N;
   float* X; float* zin; float* deformed; const float* dX; float* fpart;
   int64_t chunk; int O;
+  float* dgrid;   // backward, single object (optional): d / d grid, planar [B][2][H][W]
 };
 
 // arena block of one backbone: [b1 (w) | g1 | v1 (w) | b2 | g2 | v2 (w)]
@@ -103,7 +104,8 @@ __global__ void __launch_bounds__(256) k_diffeo_fwd(DiffP p) {
   if (p.deformed) { p.deformed[((int64_t)o * p.N + n) * 2] = x1; p.deformed[((int64_t)o * p.N + n) * 2 + 1] = x2; }
 }
 
-template <int NC>
+// DG: also write the coordinate gradient p.dgrid (a separate instantiation, so that the fit path's code is untouched)
+template <int NC, bool DG>
 __global__ void __launch_bounds__(256) k_diffeo_bwd(DiffP p) {
   extern __shared__ float sm[];
   const int w = p.w, es = eff_size(w), bs = bb_size(w);
@@ -186,6 +188,10 @@ __global__ void __launch_bounds__(256) k_diffeo_bwd(DiffP p) {
     glin[0] = fmaf(dz1, gx, glin[0]); glin[1] = fmaf(dz1, gy, glin[1]);
     glin[2] = fmaf(dz2, gx, glin[2]); glin[3] = fmaf(dz2, gy, glin[3]);
     glin[4] += dz1; glin[5] += dz2;
+    if (DG && lane == 0) {          // coordinate gradient W^T (dz1, dz2): every lane holds the same dz1, dz2
+      p.dgrid[planar_index(p.g, n, 0)] = fmaf(lin[0], dz1, lin[2] * dz2);
+      p.dgrid[planar_index(p.g, n, 1)] = fmaf(lin[1], dz1, lin[3] * dz2);
+    }
   }
   // ---- per-warp sums -> shared memory -> fixed-order sum over the warps
   float* mine = red + (int64_t)warp * RED;
@@ -266,7 +272,7 @@ static DiffP make_dp(const awb_prior* h, const float* params, const awb_grid_spe
   p.nc = L.F; p.w = L.m;
   p.N = (int64_t)g->B * g->H * g->W;
   p.X = ws.X; p.zin = nullptr; p.deformed = nullptr; p.dX = ws.dX; p.fpart = ws.fpart;
-  p.chunk = split_chunk(p.N); p.O = h->desc.n_objects;
+  p.chunk = split_chunk(p.N); p.O = h->desc.n_objects; p.dgrid = nullptr;
   return p;
 }
 
@@ -282,17 +288,21 @@ int diffeo_forward(const awb_prior* h, const float* params, const awb_grid_spec*
   return AWB_OK;
 }
 
-int diffeo_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws, cudaStream_t st) {
+int diffeo_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws, cudaStream_t st,
+                    float* dgrid) {
   DiffP p = make_dp(h, params, g, ws);
   p.zin = ws.flowz;
+  p.dgrid = dgrid;
   if (!p.zin) { set_error("flow backward needs a training workspace"); return AWB_ERR_WORKSPACE; }
+  if (dgrid && h->desc.n_objects != 1) { set_error("internal: dgrid needs one object"); return AWB_ERR_INVALID; }
   const int RED = p.nc * 2 * 3 * p.w + p.nc * 3 + 6;
   const size_t smem = sizeof(float) * ((size_t)p.nc * 2 * (3 * p.w + 1) + kMaxNC + 8 + 8 * kMaxNC + 8 * (size_t)RED);
   dim3 grid(n_splits(p.N), h->desc.n_objects);
 #define AWB_DIFFEO_BWD(NC_)                                                                                    \
   do {                                                                                                         \
-    AWB_CUDA(cudaFuncSetAttribute(k_diffeo_bwd<NC_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    AWB_LAUNCH(PK_FLOW_BWD, st, k_diffeo_bwd<NC_><<<grid, 256, smem, st>>>(p));                                \
+    auto kernel = p.dgrid ? k_diffeo_bwd<NC_, true> : k_diffeo_bwd<NC_, false>;                              \
+    AWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
+    AWB_LAUNCH(PK_FLOW_BWD, st, kernel<<<grid, 256, smem, st>>>(p));                                          \
   } while (0)
   if (p.nc == 2) AWB_DIFFEO_BWD(2);
   else if (p.nc == 4) AWB_DIFFEO_BWD(4);

@@ -40,6 +40,7 @@ struct FlowP {
   float* dzp_g;          // backward, C = 3, !dz_smem: [O][N][4] scratch for the partial gradient between unit passes
   float* tab;            // C = 2: [O][F][FLOW_TAB] segment tables of the coupling MLPs (k_flow_tables), or null
   float* segscr;         // C = 2 backward: [S][O][F][8 warps][FLOW_SEG_RS] per-warp histogram sums
+  float* dgrid;          // backward, single object (optional): d / d grid, planar [B][C][H][W]
 };
 
 // tanh and exp of the coupling outputs on the special-function unit: tanh(a) = 1 - 2 / (exp(2a) + 1) with ex2.approx /
@@ -803,7 +804,8 @@ __device__ __forceinline__ void flow_bwd_one(const FlowP& p, const FlowBwdShared
   }
 }
 
-template <int C>
+// DG: also write the coordinate gradient p.dgrid (a separate instantiation, so that the fit path's code is untouched)
+template <int C, bool DG>
 __global__ void __launch_bounds__(FLOW_BWD_T, 1) k_flow_bwd(FlowP p) {
   extern __shared__ __align__(16) float sp[];
   constexpr int RW = FlowSave<C>::RW;
@@ -869,6 +871,18 @@ __global__ void __launch_bounds__(FLOW_BWD_T, 1) k_flow_bwd(FlowP p) {
         const float dxc = dzg[c * dz_cs + (int)(n - r0) * dz_ps] * ((p.fc.new_max - p.fc.new_min) / (p.fc.nmax[c] - p.fc.nmin[c]));
         glw[c] = fmaf(dxc, coord(p.g, n, c), glw[c]);     // linear.weight
         glb[c] += dxc;                                     // linear.bias
+      }
+    }
+  }
+  if constexpr (DG) {       // coordinate gradient: linear.weight[c] * dxc (groups = C: weight [C,1,1,1]), one store per pixel
+    float lw[C];
+#pragma unroll
+    for (int c = 0; c < C; c++) lw[c] = par[p.P_flow + c];
+    for (int64_t n = r0 + tid; n < r1; n += T) {
+#pragma unroll
+      for (int c = 0; c < C; c++) {
+        const float dxc = dzg[c * dz_cs + (int)(n - r0) * dz_ps] * ((p.fc.new_max - p.fc.new_min) / (p.fc.nmax[c] - p.fc.nmin[c]));
+        p.dgrid[planar_index(p.g, n, c)] = lw[c] * dxc;
       }
     }
   }
@@ -1200,7 +1214,7 @@ __device__ __forceinline__ float warp_reduce_scatter(float* v, int lane) {
 // Shared memory: tables [F][FLOW_TAB] | exp(an_s) [F][4] | 64 floats | staged records [2][P][T][4] | histogram [132][T]
 // (afterwards: summed rows [F][FLOW_SEG_RS]) | running gradient [2][chunk] (DZS)
 constexpr int FLOW_SEG_RS = 144;      // scratch floats per (flow, warp): 132 histogram rows | 6 scalar sums | pad
-template <bool DZS>
+template <bool DZS, bool DG>
 __global__ void __launch_bounds__(FLOW_BWD_T, 1) k_flow_bwd_seg(FlowP p) {
   extern __shared__ __align__(16) float sp[];
   constexpr int C = 2, RW = 4, P = FLOW_PB, T = FLOW_BWD_T;      // always 256 threads: strides are immediates
@@ -1399,6 +1413,14 @@ __global__ void __launch_bounds__(FLOW_BWD_T, 1) k_flow_bwd_seg(FlowP p) {
         glw[c] = fmaf(dxc, coord(p.g, r0 + n, c), glw[c]);
         glb[c] += dxc;
       }
+    }
+  }
+  if constexpr (DG) {       // coordinate gradient: linear.weight[c] * dxc, one store per pixel and channel
+    const float lw0 = par[p.P_flow], lw1 = par[p.P_flow + 1];
+    for (int n = tid; n < len; n += T) {
+      p.dgrid[planar_index(p.g, r0 + n, 0)] = lw0 * (dzg[n * dz_ps] * ((p.fc.new_max - p.fc.new_min) / (p.fc.nmax[0] - p.fc.nmin[0])));
+      p.dgrid[planar_index(p.g, r0 + n, 1)] =
+          lw1 * (dzg[dz_cs + n * dz_ps] * ((p.fc.new_max - p.fc.new_min) / (p.fc.nmax[1] - p.fc.nmin[1])));
     }
   }
 #pragma unroll
@@ -1631,7 +1653,7 @@ static FlowP make_p(const awb_prior* h, const float* params, const awb_grid_spec
   p.N = ws.N;
   p.X = ws.X; p.zin = nullptr; p.deformed = nullptr; p.dX = ws.dX; p.fpart = ws.fpart;
   p.chunk = split_chunk(p.N); p.O = h->desc.n_objects; p.rounds = 1; p.rounds1 = 0; p.dz_smem = 0; p.dzp_g = nullptr;
-  p.tab = ws.flowtab; p.segscr = nullptr;
+  p.tab = ws.flowtab; p.segscr = nullptr; p.dgrid = nullptr;
   return p;
 }
 
@@ -1747,11 +1769,13 @@ bool flow_bwd_dz_in_smem(const awb_prior* h, int64_t N) {
 }
 
 int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
-                  cudaStream_t st, bool use_linear) {
+                  cudaStream_t st, bool use_linear, float* dgrid) {
   FlowP p = make_p(h, params, g, ws);
   p.use_linear = use_linear ? 1 : 0;
   p.zin = ws.flowz;
+  p.dgrid = dgrid;
   if (!p.zin) { set_error("flow backward needs a training workspace"); return AWB_ERR_WORKSPACE; }
+  if (dgrid && (!use_linear || h->desc.n_objects != 1)) { set_error("internal: dgrid needs one object and the 1x1 conv"); return AWB_ERR_INVALID; }
   if (h->lay.m > 32) { set_error("flow MLP width must be <= 32"); return AWB_ERR_UNSUPPORTED; }
   const int C = h->lay.C;
   for (int f = 0; f < h->lay.F; f++) {
@@ -1785,19 +1809,23 @@ int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
     smem = flow_seg_bwd_smem(h, geo.T, p.dz_smem ? geo.chunk : 0);
     p.segscr = ws.flowseg;
     if (!p.segscr) { set_error("flow backward: workspace lacks the segment scratch"); return AWB_ERR_WORKSPACE; }
-    if (p.dz_smem) {
-      AWB_CUDA(cudaFuncSetAttribute(k_flow_bwd_seg<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      AWB_LAUNCH(PK_FLOW_BWD, st, AWB_CUDA(launch_ex(k_flow_bwd_seg<true>, grid, dim3(geo.T), smem, st, true, p)));
-    } else {
-      AWB_CUDA(cudaFuncSetAttribute(k_flow_bwd_seg<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      AWB_LAUNCH(PK_FLOW_BWD, st, AWB_CUDA(launch_ex(k_flow_bwd_seg<false>, grid, dim3(geo.T), smem, st, true, p)));
-    }
-  } else if (C == 2) {
-    AWB_CUDA(cudaFuncSetAttribute(k_flow_bwd<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    AWB_LAUNCH(PK_FLOW_BWD, st, k_flow_bwd<2><<<grid, geo.T, smem, st>>>(p));
+    auto seg = [&](auto kernel) -> int {
+      AWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      AWB_LAUNCH(PK_FLOW_BWD, st, AWB_CUDA(launch_ex(kernel, grid, dim3(geo.T), smem, st, true, p)));
+      return AWB_OK;
+    };
+    int rc = p.dz_smem ? (dgrid ? seg(k_flow_bwd_seg<true, true>) : seg(k_flow_bwd_seg<true, false>))
+                       : (dgrid ? seg(k_flow_bwd_seg<false, true>) : seg(k_flow_bwd_seg<false, false>));
+    if (rc) return rc;
   } else {
-    AWB_CUDA(cudaFuncSetAttribute(k_flow_bwd<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    AWB_LAUNCH(PK_FLOW_BWD, st, k_flow_bwd<3><<<grid, geo.T, smem, st>>>(p));
+    auto unit = [&](auto kernel) -> int {
+      AWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      AWB_LAUNCH(PK_FLOW_BWD, st, kernel<<<grid, geo.T, smem, st>>>(p));
+      return AWB_OK;
+    };
+    int rc = C == 2 ? (dgrid ? unit(k_flow_bwd<2, true>) : unit(k_flow_bwd<2, false>))
+                    : (dgrid ? unit(k_flow_bwd<3, true>) : unit(k_flow_bwd<3, false>));
+    if (rc) return rc;
   }
   AWB_CUDA(cudaGetLastError());
   return AWB_OK;

@@ -117,7 +117,9 @@ struct Workspace {
   // coordinates at the global one.
   int64_t row0, N;
 };
-Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only = false);
+// deform_only: the layout of awb_prior_deformation / _backward -- flow buffers only (X, coupling records, dX, flow partials
+// and scratch), no ICNN weights, partials or activation planes
+Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only = false, bool deform_only = false);
 
 // ---- per-kernel-class timing (CUDA events on the launch stream) and launch counting ----
 enum { PK_PACK = 0, PK_INPUT, PK_GEMM_FWD, PK_OUT_LOSS, PK_GEMM_WGRAD, PK_GEMM_DGRAD, PK_IN_BWD, PK_OPT,
@@ -159,18 +161,22 @@ struct GridDev {
 int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, float* logits_out,
                  float* deformed, bool training, const Workspace& ws, cudaStream_t st);
 // loss != nullptr: fit mode (dy from loss); else dy = dlogits.
+// dgrid (optional, flow priors): the flow backward also writes d / d grid, planar [B,C,H,W]
 int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
                   const awb_loss_spec* loss, const float* dlogits, bool need_dx, const Workspace& ws,
-                  cudaStream_t st);
+                  cudaStream_t st, float* dgrid = nullptr);
 // n_partials: number of ICNN gradient partials ([S][O][G]) the producer wrote (-1: n_splits(N)); the flow
 // partials always come from flow_backward's n_splits(N) pixel ranges.
 int simt_reduce_opt(const awb_prior* h, float* params, void* opt_state, const awb_opt_hyper* hy,
                     float* loss_out, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1);
-// loss_slot (optional, single object): receives the sum of the loss partials (gradient row of awb_prior_slice_grads)
+// loss_slot (optional, single object): receives the sum of the loss partials (gradient row of awb_prior_slice_grads).
+// n_partials = 0: no ICNN partials were written (flow-only backward), the ICNN entries of grads are exactly 0.
 int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1,
                       float* loss_slot = nullptr);
 int absmax_per_object(const float* x, int64_t n, int O, float* out, cudaStream_t st);   // out[o] = max |x[o][:]|
 int simt_dgrid(const awb_prior* h, const awb_grid_spec* g, float* dgrid, const Workspace& ws, cudaStream_t st);
+// ws.dX[n] = (d_deformed[n][0..C), 0...): seeds the flow backward with a caller gradient on the deformed coordinates
+int simt_seed_dX(const awb_prior* h, const float* d_deformed, const Workspace& ws, cudaStream_t st);
 int optim_step(const awb_prior* h, float* params, const float* grads, void* opt_state,
                const awb_opt_hyper* hy, cudaStream_t st);
 int clamp_only(const awb_prior* h, float* params, cudaStream_t st);
@@ -207,8 +213,9 @@ int flow_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
                  float* deformed, cudaStream_t st, bool use_linear = true);
 int flow_inverse(const awb_prior* h, const float* params, const awb_grid_spec* g, float* out, cudaStream_t st);
 int flow_identity_loss(const awb_prior* h, const awb_grid_spec* g, const Workspace& ws, cudaStream_t st);
+// dgrid (optional, single object, use_linear): d / d grid [B,C,H,W] = linear.weight[c] * (gradient at the 1x1-conv output)
 int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
-                  cudaStream_t st, bool use_linear = true);
+                  cudaStream_t st, bool use_linear = true, float* dgrid = nullptr);
 int flow_save_floats(int C);                                     // floats saved per pixel and flow by the training forward
 bool flow_seg_capable(const awb_prior* h);                        // C = 2, m <= 32: segment-table kernels exist (awb_flow.cu)
 bool flow_seg_path(const awb_prior* h);                           // ... and are the ones this handle runs
@@ -222,7 +229,9 @@ int flow_actnorm_init(const awb_prior* h, float* params, const awb_grid_spec* g,
 // ---- NormalizingFlow1D coupling flow (ConvexDiffeomorphismNet), implemented in awb_diffeo.cu
 int diffeo_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws, float* deformed,
                    cudaStream_t st);
-int diffeo_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws, cudaStream_t st);
+// dgrid (optional, single object): d / d grid [B,2,H,W] = linear.weight^T (gradient at the linear's output)
+int diffeo_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws, cudaStream_t st,
+                    float* dgrid = nullptr);
 inline bool has_flow(const awb_prior* h) { return h->desc.kind == AWB_KIND_FLOW_ICNN || h->desc.kind == AWB_KIND_DIFFEO_ICNN; }
 // the coordinate transform in front of the ICNN, whichever flow the prior has
 inline int any_flow_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
@@ -231,8 +240,9 @@ inline int any_flow_forward(const awb_prior* h, const float* params, const awb_g
                                               : flow_forward(h, params, g, ws, deformed, st);
 }
 inline int any_flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
-                             cudaStream_t st) {
-  return h->desc.kind == AWB_KIND_DIFFEO_ICNN ? diffeo_backward(h, params, g, ws, st) : flow_backward(h, params, g, ws, st);
+                             cudaStream_t st, float* dgrid = nullptr) {
+  return h->desc.kind == AWB_KIND_DIFFEO_ICNN ? diffeo_backward(h, params, g, ws, st, dgrid)
+                                              : flow_backward(h, params, g, ws, st, true, dgrid);
 }
 
 // Pixel coordinate of local row n (global row n + g.row0), channel c (SURVEY a1).  torch.linspace semantics for
@@ -251,6 +261,12 @@ __device__ __forceinline__ float coord(const GridDev& g, int64_t n, int c) {
   const uint32_t i = r / (uint32_t)g.W, j = r - i * (uint32_t)g.W;
   if (g.mode == AWB_GRID_LINSPACE) return c == 0 ? lin01((int)j, g.W) : lin01((int)i, g.H);
   return c == 0 ? (float)j / (float)g.W : (float)i / (float)g.H;
+}
+// Index of local row n, channel c in a planar [B,C,H,W] tensor (the layout of the grid and of its gradient dgrid).
+__device__ __forceinline__ int64_t planar_index(const GridDev& g, int64_t n, int c) {
+  const uint32_t hw = (uint32_t)g.H * (uint32_t)g.W, nn = (uint32_t)n + g.row0;
+  const uint32_t b = nn / hw, r = nn - b * hw;
+  return ((int64_t)b * g.C + c) * hw + r;
 }
 
 }  // namespace awb

@@ -790,6 +790,15 @@ __global__ void k_dgrid(const float* dX, float* dgrid, int64_t N, int64_t HW, in
   for (int c = 0; c < C; c++) dgrid[(b * C + c) * HW + r] = dX[n * 4 + c];
 }
 
+// dX[n] = (d_deformed[n][0..C), 0...): a caller gradient on the deformed coordinates, in the layout the flow backward reads
+__global__ void k_seed_dX(const float* dd, float* dX, int64_t N, int C) {
+  int64_t n = (int64_t)blockIdx.x * 256 + threadIdx.x;
+  if (n >= N) return;
+  float d[3] = {0.f, 0.f, 0.f};
+  for (int c = 0; c < C; c++) d[c] = dd[n * C + c];
+  *reinterpret_cast<float4*>(dX + n * 4) = make_float4(d[0], d[1], d[2], 0.f);
+}
+
 // ======================================================================= host launchers
 static GridDev to_dev(const awb_grid_spec* g, int C, int64_t row0) {
   GridDev d;
@@ -859,7 +868,7 @@ int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
 
 int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
                   const awb_loss_spec* loss, const float* dlogits, bool need_dx, const Workspace& ws,
-                  cudaStream_t st) {
+                  cudaStream_t st, float* dgrid) {
   const Layout& L = h->lay;
   const int O = h->desc.n_objects;
   const int64_t N = ws.N;
@@ -916,7 +925,7 @@ int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
                                                                  L.h, L.ld));
   AWB_CUDA(cudaGetLastError());
   if (has_flow(h)) {
-    int rc = any_flow_backward(h, params, g, ws, st);
+    int rc = any_flow_backward(h, params, g, ws, st, dgrid);
     if (rc) return rc;
   }
   return AWB_OK;
@@ -991,9 +1000,15 @@ int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int
   int64_t PF = L.P_flow + L.n_lin;
   const int64_t n_thr = L.P + (loss_slot ? 1 : 0);
   AWB_LAUNCH(PK_OPT, st, AWB_CUDA(launch_ex(k_reduce_grads, dim3((unsigned)((n_thr + 255) / 256), O), dim3(256), 0, st, true,
-      grads, (const float*)ws.part, (int64_t)O * L.G, n_partials > 0 ? n_partials : n_splits(N), n_splits(N),
+      grads, (const float*)ws.part, (int64_t)O * L.G, n_partials >= 0 ? n_partials : n_splits(N), n_splits(N),
       (const float*)ws.fpart, (int64_t)O * PF, (const int32_t*)h->d_map, (int64_t)L.P, (int64_t)L.off_icnn,
       (int64_t)L.P_icnn, (int64_t)L.off_flow, PF, (int64_t)L.G, (const float*)ws.lossp, loss_slot)));
+  AWB_CUDA(cudaGetLastError());
+  return AWB_OK;
+}
+
+int simt_seed_dX(const awb_prior* h, const float* d_deformed, const Workspace& ws, cudaStream_t st) {
+  AWB_LAUNCH(PK_MISC, st, k_seed_dX<<<(unsigned)((ws.N + 255) / 256), 256, 0, st>>>(d_deformed, ws.dX, ws.N, h->lay.C));
   AWB_CUDA(cudaGetLastError());
   return AWB_OK;
 }

@@ -1,12 +1,15 @@
 """Shared machinery of the drop-in prior modules: one flat fp32 parameter arena per module
 (state-dict tensors are views into it), lazy creation of the native handle, and the
-autograd bridge to ``awb_prior_forward`` / ``awb_prior_backward``."""
+autograd bridges to ``awb_prior_forward`` / ``awb_prior_backward`` and to ``awb_prior_deformation`` /
+``awb_prior_deformation_backward``.  Both backwards are first-order only: a double backward raises."""
 from __future__ import annotations
 
+import functools
 from typing import List, Optional, Tuple
 
 import torch
 from torch import nn
+from torch.autograd.function import once_differentiable
 
 from .. import _lib as L
 from ..core import GridSpecHost, Prior
@@ -37,6 +40,36 @@ class Affine(nn.Module):
         return f"weight={tuple(self.weight.shape)}, bias={self.bias is not None}"
 
 
+def _first_order_only(backward):
+    """``once_differentiable`` for a backward whose upstream gradient may be a constant.  torch's decorator arms its
+    double-backward error only when the incoming gradient requires grad; for ``grad(y.sum(), x, create_graph=True)`` it does
+    not, and a gradient penalty built on the result would silently lose its second-order term.  Under ``create_graph``
+    (grad mode on during the backward) the incoming gradients are passed as aliases that require grad, so every result
+    carries a grad_fn that raises when it is differentiated."""
+    inner = once_differentiable(backward)
+
+    @functools.wraps(backward)
+    def wrapper(ctx, *grads):
+        if torch.is_grad_enabled():
+            grads = tuple(g.detach().requires_grad_() if isinstance(g, torch.Tensor) and not g.requires_grad else g
+                          for g in grads)
+        return inner(ctx, *grads)
+    return wrapper
+
+
+def _split_grads(flat: torch.Tensor, shapes) -> Tuple[torch.Tensor, ...]:
+    """Views of the arena-ordered gradient vector in the shapes of the module's parameters."""
+    outs, off = [], 0
+    flat = flat.reshape(-1)
+    for shp in shapes:
+        n = 1
+        for s in shp:
+            n *= s
+        outs.append(flat[off:off + n].view(shp))
+        off += n
+    return tuple(outs)
+
+
 class _PriorFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, module, spec, needs_grad, grid_tensor, *params):
@@ -59,6 +92,7 @@ class _PriorFunction(torch.autograd.Function):
         return logits
 
     @staticmethod
+    @_first_order_only
     def backward(ctx, dlogits):
         module, spec, prior = ctx.module, ctx.spec, ctx.prior
         if ctx.ws is None:
@@ -68,15 +102,33 @@ class _PriorFunction(torch.autograd.Function):
         if dgrid is not None and ctx.rows_input:      # pixel rows [N,C] went in as [1,C,1,N]: hand their gradient back as [N,C]
             dgrid = dgrid.reshape(dgrid.shape[1], -1).t().contiguous()
         ctx.ws = None
-        outs, off = [], 0
-        flat = grads.reshape(-1)
-        for shp in ctx.shapes:
-            n = 1
-            for s in shp:
-                n *= s
-            outs.append(flat[off:off + n].view(shp))
-            off += n
-        return (None, None, None, dgrid) + tuple(outs)
+        return (None, None, None, dgrid) + _split_grads(grads, ctx.shapes)
+
+
+class _DeformationFunction(torch.autograd.Function):
+    """``get_deformation`` of a flow prior with autograd: pixel rows ``[N, C]`` of the deformed coordinates.  The forward keeps
+    the coupling records in a private deformation-only workspace; the backward returns the flow and linear gradients (the
+    ICNN's are 0) and, when the grid requires grad, ``dgrid``."""
+
+    @staticmethod
+    def forward(ctx, module, spec, grid_tensor, *params):
+        prior = module._prior_for(params[0].device)
+        arena = module._arena
+        ws = prior.new_workspace(spec.n_pixels, 3, arena.device)
+        rows = prior.deformation(arena, spec, True, ws)
+        ctx.module, ctx.spec, ctx.ws, ctx.prior = module, spec, ws, prior
+        ctx.shapes = [p.shape for p in params]
+        return rows
+
+    @staticmethod
+    @_first_order_only
+    def backward(ctx, d_rows):
+        if ctx.ws is None:
+            raise RuntimeError("get_deformation's backward runs once per forward (its workspace is released after it)")
+        grads, dgrid = ctx.prior.deformation_backward(ctx.module._arena, ctx.spec, d_rows.contiguous().float(), ctx.ws,
+                                                      ctx.needs_input_grad[2])
+        ctx.ws = None
+        return (None, None, dgrid) + _split_grads(grads, ctx.shapes)
 
 
 class ArenaPriorModule(nn.Module):
@@ -198,6 +250,22 @@ class ArenaPriorModule(nn.Module):
         spec = GridSpecHost.from_tensor(x)
         out = self._logits(spec, x if x.requires_grad else None).reshape(x.shape[0], 1, x.shape[2], x.shape[3])
         return out[0] if squeeze else out
+
+    def _deformation_rows(self, x: torch.Tensor) -> torch.Tensor:
+        """``get_deformation`` of ``x`` (``[B,C,H,W]``) as pixel rows ``[N, C]``.  With grad mode on and a parameter or ``x``
+        requiring grad it runs through ``_DeformationFunction`` (differentiable w.r.t. the parameters and ``x``); otherwise
+        through the inference forward on the cached workspace, as it always has."""
+        arena = self._ensure_flat()
+        params = self._arena_params()
+        prior = self._prior_for(arena.device)
+        spec = GridSpecHost.from_tensor(x)
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params)):
+            with torch.cuda.device(arena.device):
+                return _DeformationFunction.apply(self, spec, x if x.requires_grad else None, *params)
+        with torch.no_grad(), torch.cuda.device(arena.device):
+            ws = prior.cached_workspace(spec.n_pixels, False, arena.device)
+            _, deformed = prior.forward(arena, spec, False, ws, want_deformed=True)
+        return deformed[0]
 
     def make_fitter(self, grid, target, loss=None, optim=None, **kw):
         """A ``PriorFitter`` running fused fit steps in place on this module's parameters."""

@@ -172,16 +172,12 @@ class ConvexDiffeomorphismNet(ArenaPriorModule):
         return self._forward_any(x, self.in_features)
 
     def get_deformation(self, x: torch.Tensor) -> torch.Tensor:
-        """``convex_diffeomorphism_net.py:180-185``: linear -> flow.  ``[B,2,H,W] -> [B,2,H,W]``."""
+        """``convex_diffeomorphism_net.py:180-185``: linear -> flow.  ``[B,2,H,W] -> [B,2,H,W]``.  Differentiable w.r.t.
+        the parameters (flow and linear; the ICNN's gradients are 0) and ``x``, first order only."""
         squeeze = x.dim() == 3
         if squeeze:
             x = x.unsqueeze(0)
-        arena = self._ensure_flat()
-        prior = self._prior_for(arena.device)
-        spec = GridSpecHost.from_tensor(x)
-        with torch.no_grad(), torch.cuda.device(arena.device):
-            ws = prior.cached_workspace(spec.n_pixels, False, arena.device)
-            _, deformed = prior.forward(arena, spec, False, ws, want_deformed=True)
+        rows = self._deformation_rows(x)
         B, C_, H, W = x.shape
-        out = deformed.reshape(B, H, W, C_).permute(0, 3, 1, 2).contiguous()
+        out = rows.reshape(B, H, W, C_).permute(0, 3, 1, 2).contiguous()
         return out[0] if squeeze else out

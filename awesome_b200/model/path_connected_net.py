@@ -277,23 +277,20 @@ class PathConnectedNet(ArenaPriorModule):
         return super().make_fitter(grid, target, loss, optim, **kw)
 
     def get_deformation(self, x: torch.Tensor) -> torch.Tensor:
-        """``path_connected_net.py:125-129``: 1x1 conv -> NormNet(flow).  ``[B,C,H,W] -> [B,C,H,W]``."""
+        """``path_connected_net.py:125-129``: 1x1 conv -> NormNet(flow).  ``[B,C,H,W] -> [B,C,H,W]``.  Differentiable
+        w.r.t. the parameters (flow and 1x1 conv; the ICNN's gradients are 0) and ``x``, first order only."""
         squeeze = x.dim() == 3
         if squeeze:
             x = x.unsqueeze(0)
         self._maybe_actnorm_init(x)
-        arena = self._ensure_flat()
-        prior = self._prior_for(arena.device)
-        spec = GridSpecHost.from_tensor(x)
-        with torch.no_grad(), torch.cuda.device(arena.device):
-            ws = prior.cached_workspace(spec.n_pixels, False, arena.device)
-            _, deformed = prior.forward(arena, spec, False, ws, want_deformed=True)
+        rows = self._deformation_rows(x)
         B, C_, H, W = x.shape
-        out = deformed.reshape(B, H, W, C_).permute(0, 3, 1, 2).contiguous()
+        out = rows.reshape(B, H, W, C_).permute(0, 3, 1, 2).contiguous()
         return out[0] if squeeze else out
 
     def inverse(self, x: torch.Tensor, *args, **kwargs) -> torch.Tensor:
-        """``path_connected_net.py:107-122``: inverse of ``get_deformation``.  ``[B,C,H,W] -> [B,C,H,W]``."""
+        """``path_connected_net.py:107-122``: inverse of ``get_deformation``.  ``[B,C,H,W] -> [B,C,H,W]``.  Not
+        differentiable: the result carries no autograd graph."""
         squeeze = x.dim() == 3
         if squeeze:
             x = x.unsqueeze(0)
@@ -317,6 +314,8 @@ class PathConnectedNet(ArenaPriorModule):
             return
         if x.dim() == 3:
             x = x.unsqueeze(0)
+        elif x.dim() == 2:                    # pixel rows [N, C], as forward takes them
+            x = x.detach().t().reshape(1, x.shape[1], 1, x.shape[0])
         self.actnorm_init(GridSpecHost.from_tensor(x), use_linear=True)
 
     def actnorm_init(self, grid: GridSpecHost, use_linear: bool = True) -> None:
@@ -400,7 +399,8 @@ class PathConnectedNet(ArenaPriorModule):
         arena = self._ensure_flat()
         x = x.to(arena.device)
         if use_deformed_grid:
-            x = self.get_deformation(x)
+            with torch.no_grad():                 # a fixed input grid of the ICNN fit: no graph, no training workspace
+                x = self.get_deformation(x)
         if mode == "circle":
             unaries = 1 - self.get_unary_circle_approximation(1 - unaries[0])[None, ...].float()
         fitter = self.convex_net.make_fitter(x, unaries.to(arena.device), LossConfig("mse"),

@@ -128,7 +128,9 @@ int awb_prior_destroy(awb_handle h);
 int64_t awb_prior_param_count(awb_handle h);
 /* Bytes of scratch the caller must provide for n_pixels rows (all objects).  training: 0 forward only,
  * 1 forward + backward / any call, 2 awb_prior_fit_step only (much smaller on tensor-path handles, whose fused
- * kernel keeps the activations on the SM). */
+ * kernel keeps the activations on the SM), 3 awb_prior_deformation / awb_prior_deformation_backward only (the flow's
+ * buffers: deformed coordinates, coupling records, their gradient and the flow's partials; no ICNN activations, about
+ * 80 MB instead of 0.85 GB for a 640x480 C = 2 frame). */
 int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t training);
 int64_t awb_opt_state_bytes(awb_handle h);
 
@@ -175,11 +177,28 @@ int awb_prior_forward(awb_handle h, const float* params, const awb_grid_spec* gr
 int awb_prior_flow_inverse(awb_handle h, const float* params, const awb_grid_spec* grid, float* out, void* stream);
 
 /* autograd backward of forward(): dlogits [O][N] -> grads [O][P] (overwritten), optional
- * dgrid [B,C,H,W] (ICNN, single object; model_input_requires_grad configs).  Must follow
- * awb_prior_forward(training=1) on the same workspace. */
+ * dgrid [B,C,H,W] = d loss / d grid (model_input_requires_grad configs, gradient penalties).  Must follow
+ * awb_prior_forward(training=1, or 3 on f16 handles) on the same workspace.
+ * dgrid is provided for single-object AWB_KIND_ICNN, AWB_KIND_FLOW_ICNN (C = 2, 3) and AWB_KIND_DIFFEO_ICNN handles, at
+ * both precisions and under every flow_eval mode; the flow backward forms it in its last pass over each pixel range
+ * (linear^T times the gradient at the 1x1 conv / linear output), so requesting it leaves grads bit-identical.  Grouped
+ * handles (n_objects > 1) and star handles: AWB_ERR_UNSUPPORTED. */
 int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* grid,
                        const float* dlogits, float* grads, float* dgrid, void* workspace,
                        size_t workspace_bytes, void* stream);
+
+/* get_deformation() alone (path_connected_net.py:125-129, convex_diffeomorphism_net.py:180-185): the 1x1 conv (linear)
+ * and the flow, no ICNN.  deformed: device [N][C] pixel rows.  training = 1 keeps the coupling records in the workspace
+ * for awb_prior_deformation_backward.  workspace: awb_prior_workspace_bytes(h, N, 3).
+ * Single-object AWB_KIND_FLOW_ICNN and AWB_KIND_DIFFEO_ICNN handles; an ICNN handle has no deformation (AWB_ERR_INVALID),
+ * any other handle: AWB_ERR_UNSUPPORTED. */
+int awb_prior_deformation(awb_handle h, const float* params, const awb_grid_spec* grid, float* deformed, int32_t training,
+                          void* workspace, size_t workspace_bytes, void* stream);
+/* Backward of awb_prior_deformation: d_deformed [N][C] (upstream gradient on the deformed coordinates) -> grads [P]
+ * (overwritten, state_dict order: the flow and linear entries, every ICNN entry exactly 0) and optional dgrid [B,C,H,W].
+ * Must follow awb_prior_deformation(training = 1) on the same workspace and params.  Same handles and errors. */
+int awb_prior_deformation_backward(awb_handle h, const float* params, const awb_grid_spec* grid, const float* d_deformed,
+                                   float* grads, float* dgrid, void* workspace, size_t workspace_bytes, void* stream);
 
 /* One fused fit step = the body of the reference's hot loops
  * (path_connected_net.py:939-953, :364-379; notebooks/how_to/convexity.ipynb cell 9):
