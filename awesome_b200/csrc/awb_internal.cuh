@@ -45,8 +45,9 @@ struct OptScal {  // per object, device resident
   int32_t pad;
   float last_loss;
   float pad2;
-  int32_t group_start[AWB_MAX_GROUPS];   // optimizer step at which a group last was inactive (torch keeps a step
-                                         // counter per parameter: a group that joins late starts its bias correction at 1)
+  int32_t group_start[AWB_MAX_GROUPS];   // steps this group sat out (not in active_groups).  torch keeps a step counter per
+                                         // parameter and does not advance it while the grad is None, so the group's own
+                                         // count -- the one its bias correction uses -- is step - group_start[g]
 };
 
 struct FlowConsts {

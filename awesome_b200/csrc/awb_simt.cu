@@ -529,7 +529,7 @@ __global__ void __launch_bounds__(256) k_reduce_opt(OptP a, int n_groups, int us
         s.step += 1;
         if (a.hy.active_groups)
           for (int g = 0; g < AWB_MAX_GROUPS; g++)
-            if (!((a.hy.active_groups >> g) & 1)) s.group_start[g] = s.step;
+            if (!((a.hy.active_groups >> g) & 1)) s.group_start[g] += 1;
         if (a.hy.plateau_enabled && use_loss) {
           const double cur = (double)s_loss;
           if (cur < s.best * (1.0 - (double)a.hy.threshold)) { s.best = cur; s.num_bad = 0; }
@@ -569,19 +569,20 @@ struct OptA {
 __global__ void __launch_bounds__(256) k_reduce_opt_aug(OptA a, int n_groups) {
   __shared__ float s_loss;
   __shared__ float4 s_part[8][32];
-  __shared__ float s_step_size[AWB_MAX_GROUPS], s_bc2s;
+  __shared__ float s_step_size[AWB_MAX_GROUPS], s_bc2s[AWB_MAX_GROUPS];
   const int o = blockIdx.y;
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t g0 = (int64_t)blockIdx.x * 128;
   // ---- before the producer of the partials has finished (programmatic dependent launch: these blocks become
   // resident as the fit kernel's CTAs retire): everything that only depends on the previous optimizer step --
   // bias corrections, index maps, the parameter and its moments.
-  if (threadIdx.x >= 128 && threadIdx.x < 128 + AWB_MAX_GROUPS) {   // bias corrections, once per block
+  if (threadIdx.x >= 128 && threadIdx.x < 128 + AWB_MAX_GROUPS) {   // bias corrections, once per block and group
     const int g = threadIdx.x - 128;
-    const int step1 = a.scal[o].step + 1;
+    int step1 = a.scal[o].step + 1 - a.scal[o].group_start[g];      // the group's own step count, as in k_reduce_opt
+    if (step1 < 1) step1 = 1;
     const double bc1 = 1.0 - pow((double)a.hy.beta1, (double)step1);
     s_step_size[g] = (float)(a.scal[o].lr[g] / bc1);
-    if (g == 0) s_bc2s = (float)sqrt(1.0 - pow((double)a.hy.beta2, (double)step1));
+    s_bc2s[g] = (float)sqrt(1.0 - pow((double)a.hy.beta2, (double)step1));
   }
   const int t = threadIdx.x;
   const bool flow_blk = (int)blockIdx.x >= a.nb_aug && a.nb_aug > 0;
@@ -664,7 +665,7 @@ __global__ void __launch_bounds__(256) k_reduce_opt_aug(OptA a, int n_groups) {
       float g = 0.f;
 #pragma unroll
       for (int ww = 0; ww < 8; ww++) g += reinterpret_cast<const float*>(&s_part[ww][0])[t];
-      opt_update(a.hy.kind, p, g, m, v, s_step_size[grp], s_bc2s, a.hy.beta1, a.hy.beta2, a.hy.eps,
+      opt_update(a.hy.kind, p, g, m, v, s_step_size[grp], s_bc2s[grp], a.hy.beta1, a.hy.beta2, a.hy.eps,
                  a.hy.weight_decay[grp]);
       if (do_clamp) p = fmaxf(p, 0.f);                     // enforce_convexity
       a.params[gi] = p; a.m[gi] = m; a.v[gi] = v;
@@ -693,6 +694,9 @@ __global__ void __launch_bounds__(256) k_reduce_opt_aug(OptA a, int n_groups) {
         s.nonfinite = 1;
       } else {
         s.step += 1;
+        if (a.hy.active_groups)
+          for (int g = 0; g < AWB_MAX_GROUPS; g++)
+            if (!((a.hy.active_groups >> g) & 1)) s.group_start[g] += 1;
         if (a.hy.plateau_enabled) {
           const double cur = (double)s_loss;
           if (cur < s.best * (1.0 - (double)a.hy.threshold)) { s.best = cur; s.num_bad = 0; }

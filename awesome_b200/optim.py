@@ -111,7 +111,8 @@ class _FusedBase(torch.optim.Optimizer):
             arena = m._ensure_flat()
             prior = m._prior_for(arena.device)
             aparams = m._arena_params()
-            if all(p.grad is None for p in aparams):
+            active = self._active_groups(m, aparams)
+            if active is None:
                 continue
             grads = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1).float()
                                for p in aparams])
@@ -131,7 +132,7 @@ class _FusedBase(torch.optim.Optimizer):
                     L.check(prior.lib.awb_opt_set_lr(prior.handle, ent["state"].data_ptr(), lr_c, L.stream_ptr()))
                 kind = L.AWB_OPT_ADAM if self._kind == "adam" else L.AWB_OPT_ADAMAX
                 hy = L.OptHyper(kind, betas[0], betas[1], eps, (C.c_float * L.AWB_MAX_GROUPS)(*wds), 0, 0, 0.0, 0.0,
-                                0.0, 0.0, 0)
+                                0.0, 0.0, active)
                 L.check(prior.lib.awb_optim_step(prior.handle, arena.data_ptr(), grads.data_ptr(),
                                                  ent["state"].data_ptr(), C.byref(hy), L.stream_ptr()))
         if self._inner is not None:
@@ -139,6 +140,25 @@ class _FusedBase(torch.optim.Optimizer):
                 g["lr"] = self.param_groups[g["_src"]]["lr"]
             self._inner.step()
         return loss
+
+    @staticmethod
+    def _active_groups(m, aparams) -> Optional[int]:
+        """``active_groups`` mask of one native step, like torch, which skips a parameter whose ``.grad`` is None (its
+        moments, weight decay and step count stay put): 0 when every native group has grads, the groups that have them
+        otherwise, None when none has.  A group is stepped as a whole, so one with only some grads raises."""
+        gids = m._optimizer_group_ids()
+        has: Dict[int, List[bool]] = {}
+        for p, g in zip(aparams, gids):
+            has.setdefault(g, []).append(p.grad is not None)
+        for p, g in zip(aparams, gids):
+            if p.grad is None and any(has[g]):
+                name = next(n for n, q in m.named_parameters() if q is p)
+                raise ValueError(f"{type(m).__name__}.{name} has no grad while other parameters of its optimizer group "
+                                 f"{g} do; the fused step updates a group as a whole")
+        on = [g for g, h in has.items() if h[0]]
+        if not on:
+            return None
+        return 0 if len(on) == len(has) else sum(1 << g for g in on)
 
     def add_param_group(self, param_group):
         super().add_param_group(param_group)

@@ -132,6 +132,8 @@ int64_t awb_prior_param_count(awb_handle h);
  * buffers: deformed coordinates, coupling records, their gradient and the flow's partials; no ICNN activations, about
  * 80 MB instead of 0.85 GB for a 640x480 C = 2 frame). */
 int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t training);
+/* Layout of the optimizer state: fp32 m[O][P], then fp32 v[O][P] (Adamax: the exp_inf u), then the per-object scalars at
+ * byte offset round_up(8 * O * P, 256), read through awb_opt_read_scalars. */
 int64_t awb_opt_state_bytes(awb_handle h);
 
 /* MinMax buffers of NormNet (awesome/transforms/min_max.py:28-32, net_factory.py:159-165)

@@ -61,6 +61,54 @@ def test_fused_optimizer_matches_torch_in_agent_loop(A, kind):
         assert float(prior.state_dict()[k].min()) >= 0.0
 
 
+@pytest.mark.parametrize("kind", ["adam", "adamax"])
+def test_fused_optimizer_skips_a_group_without_grads_like_torch(A, kind):
+    """A RealNVP prior whose flow group is frozen (grads None) on the first two steps and on step 4: torch.optim leaves
+    those parameters, their moments and their step count alone, and the flow joins late and rejoins with its own count.
+    A group in which only some tensors have a grad cannot be stepped as a whole: ValueError naming the tensor."""
+    torch.manual_seed(0)
+    H, W = 24, 32
+
+    def make():
+        torch.manual_seed(0)
+        m = A.real_nvp_path_connected_net(channels=2, hidden_units=16, flow_n_flows=4, flow_output_fn="tanh",
+                                          convex_net_hidden_layers=1)
+        sd = m.state_dict()
+        for k in sd:
+            if ".net.2." in k:                                 # zero-initialised couplings would make the flow trivial
+                sd[k] = 0.05 * torch.randn_like(sd[k])
+            elif k.endswith("data_dep_init_done"):
+                sd[k] = torch.ones_like(sd[k])
+        m.load_state_dict(sd)
+        return m.to(DEV)
+
+    prior, ref = make(), make()
+    cls = A.FusedAdam if kind == "adam" else A.FusedAdamax
+    tcls = torch.optim.Adam if kind == "adam" else torch.optim.Adamax
+    groups = lambda m: [dict(params=list(m.convex_net.parameters()), weight_decay=1e-3),
+                        dict(params=list(m.flow_net.parameters()), lr=5e-3, weight_decay=1e-2),
+                        dict(params=list(m.linear.parameters()))]
+    opt, topt = cls(groups(prior), lr=2e-3), tcls(groups(ref), lr=2e-3)
+    grid = O.grid_linspace(H, W)[None].to(DEV)
+    un = blob(H, W).to(DEV)
+    flow_on = [False, False, True, False, True, True]
+    for on in flow_on:
+        for m, o in ((prior, opt), (ref, topt)):
+            m.flow_net.requires_grad_(on)
+            o.zero_grad(set_to_none=True)
+            ((torch.sigmoid(m(grid))[0, 0] - un) ** 2).mean().backward()
+            o.step()
+            if m is ref:
+                m.enforce_convexity()
+    for (k, a), b in zip(prior.state_dict().items(), ref.state_dict().values()):
+        torch.testing.assert_close(a, b, rtol=1e-5, atol=1e-7, msg=lambda s: f"{k}: {s}")
+    opt.zero_grad(set_to_none=True)
+    ((torch.sigmoid(prior(grid))[0, 0] - un) ** 2).mean().backward()
+    prior.convex_net.out.ln.weight.grad = None
+    with pytest.raises(ValueError, match=r"convex_net\.out\.ln\.weight"):
+        opt.step()
+
+
 def test_fit_frames_warm_start_chain_and_skip(A):
     """_prior_based_pretrain semantics on a 4-frame synthetic sequence: cold first frame (num_epochs), warm
     successors (reuse_state_epochs), a frame without foreground is skipped and keeps the chain, IoU check passes."""
