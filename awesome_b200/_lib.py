@@ -78,6 +78,7 @@ SYMBOLS = [
     ("awb_prior_forward", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P, C.c_int32, _P, C.c_size_t, _P]),
     ("awb_prior_flow_inverse", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P]),
     ("awb_prior_backward", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P, _P, _P, C.c_size_t, _P]),
+    ("awb_prior_grid_grad_backward", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P, _P, _P, _P, C.c_size_t, _P]),
     ("awb_prior_deformation", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, C.c_int32, _P, C.c_size_t, _P]),
     ("awb_prior_deformation_backward", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P, _P, _P, C.c_size_t, _P]),
     ("awb_prior_fit_step", C.c_int, [_P, _P, _P, C.POINTER(GridSpec), _P, C.POINTER(LossSpec),

@@ -92,8 +92,8 @@ class Prior:
         return self._h
 
     def workspace_bytes(self, n_pixels: int, training) -> int:
-        """``training``: False / True, 2 for a fit-step-only workspace, 3 for a deformation-only workspace (see
-        ``awb_prior_workspace_bytes``)."""
+        """``training``: False / True, 2 for a fit-step-only workspace, 3 for a deformation-only workspace, 4 for a
+        training workspace that also holds the second-order pass's tangent rows (see ``awb_prior_workspace_bytes``)."""
         b = int(self.lib.awb_prior_workspace_bytes(self._h, n_pixels, int(training)))
         if b < 0:
             raise L.AwbError(b, "workspace size query failed")
@@ -158,6 +158,20 @@ class Prior:
                                             grads.data_ptr(), dgrid.data_ptr() if dgrid is not None else None,
                                             ws.data_ptr(), ws.numel(), L.stream_ptr()))
         return grads, dgrid
+
+    def grid_grad_backward(self, params: torch.Tensor, grid: GridSpecHost, dlogits: torch.Tensor, d_dgrid: torch.Tensor,
+                           ws: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Double backward of ``backward``'s dgrid (``awb_prior_grid_grad_backward``, single-object ICNN): ``dlogits``
+        (``[1, N]``) is the first backward's, ``d_dgrid`` (``[B, C, H, W]`` fp32, contiguous) the gradient on its dgrid.
+        Returns ``d_dlogits [1, N]`` and ``grads [1, P]``.  ``ws``: ``workspace_bytes(N, 4)``, after ``forward(training=1)``
+        on it."""
+        d_dlogits = torch.empty((self.n_objects, grid.n_pixels), dtype=torch.float32, device=params.device)
+        grads = torch.empty((self.n_objects, self.n_params), dtype=torch.float32, device=params.device)
+        gs = grid.to_c()
+        L.check(self.lib.awb_prior_grid_grad_backward(self._h, params.data_ptr(), C.byref(gs), dlogits.data_ptr(),
+                                                      d_dgrid.data_ptr(), d_dlogits.data_ptr(), grads.data_ptr(),
+                                                      ws.data_ptr(), ws.numel(), L.stream_ptr()))
+        return d_dlogits, grads
 
     def deformation(self, params: torch.Tensor, grid: GridSpecHost, training: bool, ws: torch.Tensor) -> torch.Tensor:
         """``get_deformation`` alone (1x1 conv / linear and flow, no ICNN): pixel rows ``[N, C]``.  ``ws``:

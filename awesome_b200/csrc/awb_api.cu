@@ -62,7 +62,7 @@ static int64_t align256(int64_t b) { return round_up(b, 256); }
 // fit_only: layout for awb_prior_fit_step on a tensor-path handle -- the fused kernel keeps activations on the SM, so
 // the [N][ld] activation / delta planes of the CUDA-core path are not carved (0.85 GB per 640x480 frame).
 // deform_only: layout of awb_prior_deformation / _backward -- no ICNN partials, planes or tensor-path image either.
-Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only, bool deform_only) {
+Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only, bool deform_only, bool tangent) {
   const Layout& L = h->lay;
   const int64_t O = h->desc.n_objects;
   int S = n_splits(N);
@@ -93,6 +93,7 @@ Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool f
   w.flowseg = (training && rnvp && flow_seg_scratch_floats(h, S) > 0) ? (float*)take(4 * flow_seg_scratch_floats(h, S)) : nullptr;
   w.tc = (!deform_only && h->desc.precision == AWB_PREC_F16 && tc_supported(h)) ? (void*)take(O * (int64_t)tc_image_bytes(L.L))
                                                                                : nullptr;
+  w.ZT = tangent ? (float*)take(4 * O * (L.L + 1) * N * L.ld) : nullptr;
   w.bytes = off;
   w.row0 = 0; w.N = N;
   return w;
@@ -235,7 +236,7 @@ int64_t awb_prior_param_count(awb_handle h) { return h ? h->lay.P : -1; }
 
 int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t training) {
   if (!h || n_pixels < 1) return -1;
-  return carve(h, n_pixels, training != 0, nullptr, training == 2, training == 3).bytes;
+  return carve(h, n_pixels, training != 0, nullptr, training == 2, training == 3, training == 4).bytes;
 }
 
 int64_t awb_opt_state_bytes(awb_handle h) {
@@ -275,7 +276,8 @@ int awb_prior_set_flow_eval(awb_handle h, int32_t mode) {
 // window (optional, {row_begin, row_end}): the call works on the pixel rows [row_begin, row_end) of the batch, which must
 // be a non-empty range inside [0, N), and the workspace is sized for them
 static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, bool training, int64_t* N,
-                        bool fit_only = false, const int64_t* window = nullptr, bool deform_only = false) {
+                        bool fit_only = false, const int64_t* window = nullptr, bool deform_only = false,
+                        bool tangent = false) {
   if (!h || !g || !ws) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (g->B < 1 || g->H < 1 || g->W < 1) { set_error("empty grid %dx%dx%d", g->B, g->H, g->W); return AWB_ERR_INVALID; }
   if (g->mode == AWB_GRID_EXPLICIT && !g->grid) { set_error("explicit grid needs a pointer"); return AWB_ERR_INVALID; }
@@ -287,7 +289,7 @@ static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t w
               (long long)*N);
     return AWB_ERR_INVALID;
   }
-  int64_t need = carve(h, window ? window[1] - window[0] : *N, training, nullptr, fit_only, deform_only).bytes;
+  int64_t need = carve(h, window ? window[1] - window[0] : *N, training, nullptr, fit_only, deform_only, tangent).bytes;
   if ((int64_t)ws_bytes < need) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)need); return AWB_ERR_WORKSPACE; }
   if (h->desc.kind == AWB_KIND_FLOW_ICNN && !h->fc_set) { set_error("awb_prior_set_flow_consts not called"); return AWB_ERR_INVALID; }
   return AWB_OK;
@@ -362,6 +364,26 @@ int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* g
   if (rc) return rc;
   if (dgrid && !has_flow(h)) rc = simt_dgrid(h, g, dgrid, w, st);
   return rc;
+}
+
+int awb_prior_grid_grad_backward(awb_handle h, const float* params, const awb_grid_spec* g, const float* dlogits,
+                                 const float* d_dgrid, float* d_dlogits, float* grads, void* ws, size_t ws_bytes,
+                                 void* stream) {
+  if (!h) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if (h->desc.kind != AWB_KIND_ICNN || h->desc.n_objects != 1) {
+    set_error("the second-order pass is provided for single-object ICNN priors only (kind %d, %d objects)", h->desc.kind,
+              h->desc.n_objects);
+    return AWB_ERR_UNSUPPORTED;
+  }
+  int64_t N;
+  int rc = check_common(h, g, ws, ws_bytes, true, &N, false, nullptr, false, /*tangent=*/true);
+  if (rc) return rc;
+  if (!params || !dlogits || !d_dgrid || !d_dlogits || !grads) { set_error("null argument"); return AWB_ERR_INVALID; }
+  Workspace w = carve(h, N, true, ws, false, false, true);
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = simt_grid_grad_backward(h, g, dlogits, d_dgrid, d_dlogits, w, st);
+  if (rc) return rc;
+  return simt_reduce_grads(h, grads, w, N, st);
 }
 
 int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_grid_spec* g, const float* target,

@@ -112,6 +112,8 @@ struct Workspace {
   float* flowtab; // RealNVP, C = 2: [O][F][2][132] segment tables of the coupling MLPs, rebuilt by every forward
   float* flowseg; // RealNVP, C = 2, training: [S][O][F][8][144] per-warp histogram sums of the segment backward
   void* tc;       // tensor-core path scratch
+  float* ZT;      // second-order pass (awb_prior_grid_grad_backward): [L+1][N][ld] tangent rows, after everything else so
+                  // that the training forward's layout is a prefix of this one
   int64_t bytes;
   // the pixel rows [row0, row0 + N) of the grid's batch this call works on: the whole batch (row0 = 0) for every entry
   // point but awb_prior_slice_grads.  Kernels index their scratch and the target by the local row and generate (or read)
@@ -119,12 +121,13 @@ struct Workspace {
   int64_t row0, N;
 };
 // deform_only: the layout of awb_prior_deformation / _backward -- flow buffers only (X, coupling records, dX, flow partials
-// and scratch), no ICNN weights, partials or activation planes
-Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only = false, bool deform_only = false);
+// and scratch), no ICNN weights, partials or activation planes.  tangent: the training layout plus the tangent rows ZT.
+Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only = false, bool deform_only = false,
+                bool tangent = false);
 
 // ---- per-kernel-class timing (CUDA events on the launch stream) and launch counting ----
 enum { PK_PACK = 0, PK_INPUT, PK_GEMM_FWD, PK_OUT_LOSS, PK_GEMM_WGRAD, PK_GEMM_DGRAD, PK_IN_BWD, PK_OPT,
-       PK_FLOW_FWD, PK_FLOW_BWD, PK_TC_FUSED, PK_MISC, PK_COUNT };
+       PK_FLOW_FWD, PK_FLOW_BWD, PK_TC_FUSED, PK_MISC, PK_TAN_FWD, PK_TAN_OUT, PK_COUNT };
 void prof_begin(int cls, cudaStream_t st);
 void prof_end(int cls, cudaStream_t st);
 #define AWB_LAUNCH(cls, st, ...)  \
@@ -174,6 +177,10 @@ int simt_reduce_opt(const awb_prior* h, float* params, void* opt_state, const aw
 // n_partials = 0: no ICNN partials were written (flow-only backward), the ICNN entries of grads are exactly 0.
 int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1,
                       float* loss_slot = nullptr);
+// second-order pass of the coordinate gradient (single-object ICNN, after simt_forward(training) on ws, ws carved with
+// tangent rows): d_dgrid [B,C,H,W] -> ydot [N] and the parameter-gradient partials that simt_reduce_grads sums
+int simt_grid_grad_backward(const awb_prior* h, const awb_grid_spec* g, const float* dlogits, const float* d_dgrid,
+                            float* ydot, const Workspace& ws, cudaStream_t st);
 int absmax_per_object(const float* x, int64_t n, int O, float* out, cudaStream_t st);   // out[o] = max |x[o][:]|
 int simt_dgrid(const awb_prior* h, const awb_grid_spec* g, float* dgrid, const Workspace& ws, cudaStream_t st);
 // ws.dX[n] = (d_deformed[n][0..C), 0...): seeds the flow backward with a caller gradient on the deformed coordinates

@@ -74,6 +74,49 @@ __global__ void __launch_bounds__(256) k_input(GridDev g, int x_ready, float* __
   }
 }
 
+// ------------------------------------------------------------------ tangent input layer (second-order pass)
+// Tangent of the forward along u_n = d R / d dgrid_n (planar [B,C,H,W], read through gu):
+// ZT0[n] = [ (W_in u) .* (z0 > 0) | u | 0 | 0-pad ] -- the bias column is the tangent of a constant -- and the rows
+// (u, 0) that the input layer's weight gradient reads.  Single object.
+__global__ void __launch_bounds__(256) k_tan_input(GridDev gu, const float* __restrict__ waug,
+                                                   const float* __restrict__ ZA0, float* __restrict__ ZT0,
+                                                   float* __restrict__ U, int64_t N, int h, int C, int ld,
+                                                   int64_t aug_in) {
+  __shared__ float us[64][4];
+  int64_t n0 = (int64_t)blockIdx.x * 64;
+  if (threadIdx.x < 64) {
+    int64_t n = n0 + threadIdx.x;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (n < N) {
+      v.x = gu.grid[planar_index(gu, n, 0)];
+      v.y = gu.grid[planar_index(gu, n, 1)];
+      v.z = C > 2 ? gu.grid[planar_index(gu, n, 2)] : 0.f;
+      *reinterpret_cast<float4*>(U + n * 4) = v;
+    }
+    us[threadIdx.x][0] = v.x; us[threadIdx.x][1] = v.y; us[threadIdx.x][2] = v.z; us[threadIdx.x][3] = 0.f;
+  }
+  __syncthreads();
+  const float* win = waug + aug_in;
+  for (int idx = threadIdx.x; idx < 64 * ld; idx += 256) {
+    int r = idx / ld, c = idx - r * ld;
+    int64_t n = n0 + r;
+    if (n >= N) break;
+    float v;
+    if (c < h) {
+      float4 w = *reinterpret_cast<const float4*>(win + c * 4);
+      float a = us[r][0] * w.x;
+      a = fmaf(us[r][1], w.y, a);
+      if (C > 2) a = fmaf(us[r][2], w.z, a);
+      v = ZA0[n * ld + c] > 0.f ? a : 0.f;
+    } else if (c < h + C) {
+      v = us[r][c - h];
+    } else {
+      v = 0.f;
+    }
+    ZT0[n * ld + c] = v;
+  }
+}
+
 // ------------------------------------------------------------------ tiled SGEMM with fused epilogues
 struct GemmP {
   const float* A; const float* B; float* Cout;
@@ -85,11 +128,13 @@ struct GemmP {
   int h, C;
   int64_t k_chunk;         // wgrad: pixel rows per split (blockIdx.x)
   int64_t sSplit;          // wgrad: stride between splits in Cout
+  const float* Mz; int64_t sMz;  // tangent fwd: ZA_out of the forward (its relu mask)
 };
 
 // MODE 0: ZA_out = relu(ZA_in * Waug^T)                 A(m,k)=A[m*lda+k]   B(k,n)=B[n*ldb+k]
 // MODE 1: delta_prev = (delta * Waug) .* (ZA_prev > 0)  A(m,k)=A[m*lda+k]   B(k,n)=B[k*ldb+n]
 // MODE 2: dWaug[split] = delta^T * ZA_prev              A(m,k)=A[k*lda+m]   B(k,n)=B[k*ldb+n]
+// MODE 3: ZT_out = (ZT_in * Waug^T) .* (ZA_out > 0)     as MODE 0: the tangent of MODE 0 along the tangent rows ZT_in
 template <int MODE>
 __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
   constexpr int BM = (MODE == 2) ? 144 : 128;
@@ -136,7 +181,7 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
       int e = tid + 256 * i;
       float v = 0.f;
       if (e < BN * BK) {
-        if (MODE == 0) {  // k contiguous in global: B(k,n) = W[n][k], rows n < h
+        if (MODE == 0 || MODE == 3) {  // k contiguous in global: B(k,n) = W[n][k], rows n < h
           int n = e / BK, k = e - n * BK;
           int64_t kk = k0 + k;
           if (n < p.N && kk < p.ldb) v = B[(int64_t)n * p.ldb + kk];
@@ -163,7 +208,7 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
     for (int i = 0; i < NB; i++) {
       int e = tid + 256 * i;
       if (e < BN * BK) {
-        if (MODE == 0) { int n = e / BK, k = e - n * BK; Bs[buf][k][n] = rb[i]; }
+        if (MODE == 0 || MODE == 3) { int n = e / BK, k = e - n * BK; Bs[buf][k][n] = rb[i]; }
         else { int k = e / BN, n = e - k * BN; Bs[buf][k][n] = rb[i]; }
       }
     }
@@ -204,9 +249,10 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
   }
 
   // ---- epilogue
-  if (MODE == 0) {
+  if (MODE == 0 || MODE == 3) {
     float* Cz = p.Cout + (int64_t)o * p.sC;
     const float* Zin = p.E0 + (int64_t)o * p.sE0;
+    const float* Zm = MODE == 3 ? p.Mz + (int64_t)o * p.sMz : nullptr;
 #pragma unroll
     for (int i = 0; i < TM; i++) {
       int64_t m = m0 + ty + 16 * i;
@@ -215,7 +261,9 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
       for (int j = 0; j < TN; j++) {
         int n = tx + 16 * j;
         if (n >= p.ldc) continue;
-        float v = (n < p.h) ? fmaxf(acc[i][j], 0.f) : Zin[m * p.ldc + n];
+        float v;
+        if (MODE == 0) v = (n < p.h) ? fmaxf(acc[i][j], 0.f) : Zin[m * p.ldc + n];
+        else v = (n < p.h) ? (Zm[m * p.ldc + n] > 0.f ? acc[i][j] : 0.f) : Zin[m * p.ldc + n];
         Cz[m * p.ldc + n] = v;
       }
     }
@@ -366,12 +414,81 @@ __global__ void __launch_bounds__(256) k_out(OutP p) {
   }
 }
 
+// ------------------------------------------------------------------ tangent output layer (second-order pass)
+// Per pixel: ydot = waug_out . ZT_L (= w_o . zdot_L + s_o . u, the derivative of the logit along u), written to ydot[n];
+// delta_L = w .* w_o .* (z_L > 0) exactly as k_out seeds it from dlogits = w; the output layer's partials sum w * ZT_L
+// (d w_o = sum w zdot_L, d s_o = sum w u, d b_o = 0).  Single object; pixel range s = blockIdx.x, fixed-order block sum.
+struct TanOutP {
+  const float* ZA;                // ZA_L (relu mask)
+  const float* ZT;                // ZT_L
+  const float* waug; int64_t aug_out;
+  const float* w;                 // [N] dlogits of the first backward
+  float* ydot;                    // [N]
+  float* D;                       // delta_L out
+  float* part; int64_t sSplit;    // partial sums [S][G]
+  int64_t N, chunk;
+  int h, ld;
+};
+
+template <int Q>
+__global__ void __launch_bounds__(256) k_tan_out(TanOutP p) {
+  extern __shared__ float sm[];   // [8][ld] gradient partials
+  const int s = blockIdx.x;
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const float* wo = p.waug + p.aug_out;
+  float wq[Q], gacc[Q];
+#pragma unroll
+  for (int q = 0; q < Q; q++) {
+    int c = lane + 32 * q;
+    wq[q] = c < p.ld ? wo[c] : 0.f;
+    gacc[q] = 0.f;
+  }
+  int64_t r0 = (int64_t)s * p.chunk;
+  int64_t r1 = r0 + p.chunk < p.N ? r0 + p.chunk : p.N;
+  for (int64_t n = r0 + w; n < r1; n += 8) {
+    float zt[Q];
+    float dot = 0.f;
+#pragma unroll
+    for (int q = 0; q < Q; q++) {
+      int c = lane + 32 * q;
+      zt[q] = c < p.ld ? p.ZT[n * p.ld + c] : 0.f;
+      dot = fmaf(zt[q], wq[q], dot);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, off);
+    if (lane == 0) p.ydot[n] = dot;
+    const float dy = p.w[n];
+    float* Dr = p.D + n * p.ld;
+#pragma unroll
+    for (int q = 0; q < Q; q++) {
+      int c = lane + 32 * q;
+      if (c < p.ld) {
+        Dr[c] = (c < p.h && p.ZA[n * p.ld + c] > 0.f) ? dy * wq[q] : 0.f;
+        gacc[q] = fmaf(dy, zt[q], gacc[q]);
+      }
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < Q; q++) {
+    int c = lane + 32 * q;
+    if (c < p.ld) sm[w * p.ld + c] = gacc[q];
+  }
+  __syncthreads();
+  for (int c = threadIdx.x; c < p.ld; c += 256) {
+    float a = 0.f;
+#pragma unroll
+    for (int ww = 0; ww < 8; ww++) a += sm[ww * p.ld + c];
+    p.part[(int64_t)s * p.sSplit + p.aug_out + c] = a;
+  }
+}
+
 // ------------------------------------------------------------------ input layer backward
-// dW_in[j][c] = sum_n delta0[n][j] x[n][c];  db_in[j] = sum_n delta0[n][j]
+// dW_in[j][c] = sum_n delta0[n][j] x[n][c];  db_in[j] = sum_n delta0[n][j] one  (one = 1; 0 against tangent rows,
+// whose bias input is the tangent of a constant: fmaf(d, 1, a) rounds like a + d, so the first-order bits are kept)
 __global__ void __launch_bounds__(256) k_in_wgrad(const float* __restrict__ D0, int64_t sD,
                                                   const float* __restrict__ X, float* __restrict__ part,
                                                   int64_t sSplit, int64_t G, int64_t aug_in, int64_t N,
-                                                  int64_t chunk, int h, int ld) {
+                                                  int64_t chunk, int h, int ld, float one) {
   int s = blockIdx.x, o = blockIdx.y, j = threadIdx.x;
   const float* D = D0 + (int64_t)o * sD;
   const float* Xo = X + (int64_t)o * N * 4;
@@ -381,7 +498,7 @@ __global__ void __launch_bounds__(256) k_in_wgrad(const float* __restrict__ D0, 
     for (int64_t n = r0; n < r1; n++) {
       float d = D[n * ld + j];
       float4 x = *reinterpret_cast<const float4*>(Xo + n * 4);
-      a0 = fmaf(d, x.x, a0); a1 = fmaf(d, x.y, a1); a2 = fmaf(d, x.z, a2); a3 += d;
+      a0 = fmaf(d, x.x, a0); a1 = fmaf(d, x.y, a1); a2 = fmaf(d, x.z, a2); a3 = fmaf(d, one, a3);
     }
     float* out = part + (int64_t)s * sSplit + (int64_t)o * G + aug_in + j * 4;
     *reinterpret_cast<float4*>(out) = make_float4(a0, a1, a2, a3);
@@ -923,7 +1040,7 @@ int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
       AWB_LAUNCH(PK_GEMM_DGRAD, st, k_gemm<1><<<dim3((unsigned)((N + 127) / 128), 1, O), 256, 0, st>>>(p));
     }
   }
-  AWB_LAUNCH(PK_IN_BWD, st, k_in_wgrad<<<dim3(S, O), 256, 0, st>>>(ws.D, sDobj, ws.X, ws.part, sSplit, L.G, L.aug_in, N, chunk, L.h, L.ld));
+  AWB_LAUNCH(PK_IN_BWD, st, k_in_wgrad<<<dim3(S, O), 256, 0, st>>>(ws.D, sDobj, ws.X, ws.part, sSplit, L.G, L.aug_in, N, chunk, L.h, L.ld, 1.f));
   if (need_dx)
     AWB_LAUNCH(PK_IN_BWD, st, k_in_dgrad<<<dim3((unsigned)((N + 7) / 8), O), 256, 0, st>>>(ws.D, sDobj, ws.waug, L.G, L.aug_in, ws.dX, N,
                                                                  L.h, L.ld));
@@ -932,6 +1049,72 @@ int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
     int rc = any_flow_backward(h, params, g, ws, st, dgrid);
     if (rc) return rc;
   }
+  return AWB_OK;
+}
+
+// Second-order pass of the ICNN's coordinate gradient (DESIGN 3b.1).  The first backward maps (w = dlogits, params) to
+// dgrid_n = w_n J_n^T; for a cotangent u on dgrid it returns ydot_n = J_n u_n (to w) and sum_n w_n d(J_n u_n)/d params.
+// The relu masks are piecewise constant, so the backprop of the tangent network seeded with w has the deltas of the
+// first backward; the weight gradients contract them with the tangent rows ZT instead of the activation rows ZA, and
+// every bias gradient is exactly 0.  Reads ZA / X / waug of the training forward, writes ZT, D, dX (as u rows) and part.
+int simt_grid_grad_backward(const awb_prior* h, const awb_grid_spec* g, const float* dlogits, const float* d_dgrid,
+                            float* ydot, const Workspace& ws, cudaStream_t st) {
+  const Layout& L = h->lay;
+  const int64_t N = ws.N;
+  const int S = n_splits(N);
+  const int64_t chunk = split_chunk(N);
+  const int64_t sLayer = N * L.ld;
+  const int64_t sSplit = L.G;    // one object
+  GridDev gu = to_dev(g, L.C, 0);
+  gu.mode = AWB_GRID_EXPLICIT; gu.grid = d_dgrid;
+  AWB_LAUNCH(PK_TAN_FWD, st, k_tan_input<<<(unsigned)((N + 63) / 64), 256, 0, st>>>(gu, ws.waug, ws.ZA, ws.ZT, ws.dX, N, L.h,
+                                                                                 L.C, L.ld, L.aug_in));
+  for (int i = 0; i < L.L; i++) {
+    GemmP p = {};
+    p.A = ws.ZT + i * sLayer; p.lda = L.ld;
+    p.B = ws.waug + L.aug_layer + (int64_t)i * L.h * L.ld; p.ldb = L.ld;
+    p.Cout = ws.ZT + (i + 1) * sLayer; p.ldc = L.ld;
+    p.M = N; p.N = L.h; p.K = L.ld;
+    p.E0 = p.A;
+    p.Mz = ws.ZA + (i + 1) * sLayer;
+    p.h = L.h; p.C = L.C;
+    AWB_LAUNCH(PK_TAN_FWD, st, k_gemm<3><<<dim3((unsigned)((N + 127) / 128), 1, 1), 256, 0, st>>>(p));
+  }
+  TanOutP q = {};
+  q.ZA = ws.ZA + L.L * sLayer; q.ZT = ws.ZT + L.L * sLayer;
+  q.waug = ws.waug; q.aug_out = L.aug_out;
+  q.w = dlogits; q.ydot = ydot;
+  q.D = ws.D + (L.L & 1) * sLayer;
+  q.part = ws.part; q.sSplit = sSplit;
+  q.N = N; q.chunk = chunk; q.h = L.h; q.ld = L.ld;
+  const size_t smem = 8 * L.ld * sizeof(float);
+  if (L.ld <= 160) AWB_LAUNCH(PK_TAN_OUT, st, k_tan_out<5><<<S, 256, smem, st>>>(q));
+  else AWB_LAUNCH(PK_TAN_OUT, st, k_tan_out<9><<<S, 256, smem, st>>>(q));
+  for (int i = L.L; i >= 1; i--) {
+    const float* delta = ws.D + (i & 1) * sLayer;
+    {  // dWaug_i = delta_i^T * ZT_{i-1}
+      GemmP p = {};
+      p.A = delta; p.lda = L.ld;
+      p.B = ws.ZT + (i - 1) * sLayer; p.ldb = L.ld;
+      p.Cout = ws.part + L.aug_layer + (int64_t)(i - 1) * L.h * L.ld; p.ldc = L.ld;
+      p.M = L.h; p.N = L.ld; p.K = (int)N;
+      p.h = L.h; p.C = L.C; p.k_chunk = chunk; p.sSplit = sSplit;
+      AWB_LAUNCH(PK_GEMM_WGRAD, st, k_gemm<2><<<dim3(S, 1, 1), 256, 0, st>>>(p));
+    }
+    {  // delta_{i-1}: the data gradient of the first backward (no coordinate gradient)
+      GemmP p = {};
+      p.A = delta; p.lda = L.ld;
+      p.B = ws.waug + L.aug_layer + (int64_t)(i - 1) * L.h * L.ld; p.ldb = L.ld;
+      p.Cout = ws.D + ((i - 1) & 1) * sLayer; p.ldc = L.ld;
+      p.M = N; p.N = L.ld; p.K = L.h;
+      p.E0 = ws.ZA + (i - 1) * sLayer;
+      p.h = L.h; p.C = L.C;
+      AWB_LAUNCH(PK_GEMM_DGRAD, st, k_gemm<1><<<dim3((unsigned)((N + 127) / 128), 1, 1), 256, 0, st>>>(p));
+    }
+  }
+  AWB_LAUNCH(PK_IN_BWD, st, k_in_wgrad<<<dim3(S, 1), 256, 0, st>>>(ws.D, 2 * sLayer, ws.dX, ws.part, sSplit, L.G, L.aug_in, N,
+                                                                    chunk, L.h, L.ld, 0.f));
+  AWB_CUDA(cudaGetLastError());
   return AWB_OK;
 }
 

@@ -1,7 +1,9 @@
 """Shared machinery of the drop-in prior modules: one flat fp32 parameter arena per module
 (state-dict tensors are views into it), lazy creation of the native handle, and the
 autograd bridges to ``awb_prior_forward`` / ``awb_prior_backward`` and to ``awb_prior_deformation`` /
-``awb_prior_deformation_backward``.  Both backwards are first-order only: a double backward raises."""
+``awb_prior_deformation_backward``.  Both backwards are first-order only: a double backward raises.  The exception is an
+ICNN prior built with ``second_order=True``: under ``create_graph`` its coordinate gradient is differentiable
+(``_GridGradFunction``, ``awb_prior_grid_grad_backward``)."""
 from __future__ import annotations
 
 import functools
@@ -57,6 +59,13 @@ def _first_order_only(backward):
     return wrapper
 
 
+def reject_second_order(kind: str, kwargs) -> None:
+    """Second derivatives are provided for the ICNN priors only: any other prior refuses the flag instead of ignoring it."""
+    if kwargs.get("second_order"):
+        raise ValueError(f"{kind} has no second-order backward (second_order=True is provided for ConvexNextNet and "
+                         "ConvexNet: the flows' couplings have non-zero second derivatives in the coordinates)")
+
+
 def _split_grads(flat: torch.Tensor, shapes) -> Tuple[torch.Tensor, ...]:
     """Views of the arena-ordered gradient vector in the shapes of the module's parameters."""
     outs, off = [], 0
@@ -70,6 +79,63 @@ def _split_grads(flat: torch.Tensor, shapes) -> Tuple[torch.Tensor, ...]:
     return tuple(outs)
 
 
+def _prior_backward(ctx, dlogits):
+    module, spec, prior = ctx.module, ctx.spec, ctx.prior
+    if ctx.ws is None:
+        raise RuntimeError("backward through an awesome_b200 prior needs a forward that ran with grad enabled")
+    want_dgrid = ctx.needs_input_grad[3]
+    grads, dgrid = prior.backward(module._arena, spec, dlogits.contiguous().float(), ctx.ws, want_dgrid)
+    if dgrid is not None and ctx.rows_input:      # pixel rows [N,C] went in as [1,C,1,N]: hand their gradient back as [N,C]
+        dgrid = dgrid.reshape(dgrid.shape[1], -1).t().contiguous()
+    if not ctx.second_order:    # second order: a retained graph may come back through here after the second-order pass
+        ctx.ws = None
+    return (None, None, None, dgrid) + _split_grads(grads, ctx.shapes)
+
+
+_prior_backward_first_order = _first_order_only(_prior_backward)
+
+
+class _GridGradFunction(torch.autograd.Function):
+    """The first backward of an ICNN prior as a differentiable function of its upstream gradient ``w`` and the
+    parameters.  Forward: ``awb_prior_backward`` (dgrid and the parameter gradients, the bits of the first-order path).
+    Backward: ``awb_prior_grid_grad_backward`` turns the gradient ``u`` on dgrid into ``J u`` for ``w`` and
+    ``sum_n w_n d(J_n u_n) / d params`` for the parameters; the grid gets nothing (the ICNN is piecewise linear in it).
+    Differentiating the parameter-gradient outputs raises."""
+
+    @staticmethod
+    def forward(ctx, module, spec, prior, ws, rows_input, dlogits, *params):
+        ctx.set_materialize_grads(False)
+        w = dlogits.contiguous().float()
+        grads, dgrid = prior.backward(module._arena, spec, w, ws, True)
+        if rows_input:
+            dgrid = dgrid.reshape(dgrid.shape[1], -1).t().contiguous()
+        ctx.module, ctx.spec, ctx.prior, ctx.ws, ctx.rows_input = module, spec, prior, ws, rows_input
+        ctx.shapes = [p.shape for p in params]
+        ctx.save_for_backward(w)
+        return (dgrid,) + tuple(g.clone() for g in _split_grads(grads, ctx.shapes))
+
+    @staticmethod
+    @_first_order_only
+    def backward(ctx, d_dgrid, *d_grads):
+        if any(g is not None for g in d_grads):
+            raise RuntimeError("awesome_b200 priors do not differentiate their parameter gradients: with "
+                               "second_order=True only the coordinate gradient of an ICNN prior (a penalty on d prior / "
+                               "d grid) has a second derivative")
+        if d_dgrid is None:
+            return (None,) * (6 + len(ctx.shapes))
+        (w,) = ctx.saved_tensors
+        module, spec, prior = ctx.module, ctx.spec, ctx.prior
+        u = (d_dgrid.t() if ctx.rows_input else d_dgrid).contiguous().float()    # planar [B,C,H,W] ([1,C,1,N] for rows)
+        u = u.reshape(spec.B, -1, spec.H, spec.W)
+        ws = ctx.ws
+        if module.precision == "f16":
+            # the first order ran on the tensor path, which keeps no activations: an exact fp32 forward provides them
+            ws = prior.new_workspace(spec.n_pixels, 4, w.device)
+            prior.forward(module._arena, spec, 1, ws)
+        d_w, grads = prior.grid_grad_backward(module._arena, spec, w, u, ws)
+        return (None, None, None, None, None, d_w) + _split_grads(grads, ctx.shapes)
+
+
 class _PriorFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, module, spec, needs_grad, grid_tensor, *params):
@@ -78,8 +144,12 @@ class _PriorFunction(torch.autograd.Function):
         path (mode 0) on the cached workspace, whatever ``requires_grad`` says."""
         prior = module._prior_for(params[0].device)
         arena = module._arena
+        second_order = needs_grad and module.second_order
         if needs_grad:
-            ws = prior.new_workspace(spec.n_pixels, True, arena.device)   # private: several forwards may precede backward
+            # private: several forwards may precede backward.  An exact second-order module also keeps room for the
+            # tangent rows of the second-order pass (the training layout is a prefix of that one).
+            ws = prior.new_workspace(spec.n_pixels, 4 if second_order and module.precision == "fp32" else True,
+                                     arena.device)
         else:
             ws = prior.cached_workspace(spec.n_pixels, False, arena.device)
         # training forward of a tensor-path module: logits from the fused tcgen05 kernel (mode 3); backward re-runs it
@@ -89,20 +159,22 @@ class _PriorFunction(torch.autograd.Function):
         ctx.module, ctx.spec, ctx.ws, ctx.prior = module, spec, (ws if needs_grad else None), prior
         ctx.shapes = [p.shape for p in params]
         ctx.rows_input = grid_tensor is not None and grid_tensor.dim() == 2
+        ctx.second_order = second_order
+        if second_order:
+            ctx.save_for_backward(*params)
         return logits
 
     @staticmethod
-    @_first_order_only
     def backward(ctx, dlogits):
-        module, spec, prior = ctx.module, ctx.spec, ctx.prior
-        if ctx.ws is None:
-            raise RuntimeError("backward through an awesome_b200 prior needs a forward that ran with grad enabled")
-        want_dgrid = ctx.needs_input_grad[3]
-        grads, dgrid = prior.backward(module._arena, spec, dlogits.contiguous().float(), ctx.ws, want_dgrid)
-        if dgrid is not None and ctx.rows_input:      # pixel rows [N,C] went in as [1,C,1,N]: hand their gradient back as [N,C]
-            dgrid = dgrid.reshape(dgrid.shape[1], -1).t().contiguous()
-        ctx.ws = None
-        return (None, None, None, dgrid) + _split_grads(grads, ctx.shapes)
+        # a backward that builds a graph (create_graph) and returns dgrid: differentiable on second-order modules
+        if ctx.second_order and torch.is_grad_enabled() and ctx.needs_input_grad[3]:
+            if ctx.ws is None:
+                raise RuntimeError("backward through an awesome_b200 prior needs a forward that ran with grad enabled")
+            # the graph built here comes back through this forward when w depends on the logits
+            outs = _GridGradFunction.apply(ctx.module, ctx.spec, ctx.prior, ctx.ws, ctx.rows_input, dlogits,
+                                           *ctx.saved_tensors)
+            return (None, None, None) + tuple(outs)
+        return _prior_backward_first_order(ctx, dlogits)
 
 
 class _DeformationFunction(torch.autograd.Function):
@@ -135,11 +207,12 @@ class ArenaPriorModule(nn.Module):
     """Base class: subclasses register their parameters (in state_dict order == arena order)
     and implement ``_make_prior(device)``."""
 
-    def __init__(self, precision: str = "fp32"):
+    def __init__(self, precision: str = "fp32", second_order: bool = False):
         super().__init__()
         if precision not in _PRECISIONS:
             raise ValueError(f"precision must be one of {list(_PRECISIONS)}, got {precision!r}")
         self.precision = precision
+        self.second_order = bool(second_order)
         self._arena: Optional[torch.Tensor] = None
         self._prior: Optional[Prior] = None
         self._prior_device = None

@@ -15,7 +15,7 @@ from torch import nn
 
 from .. import _lib as L
 from ..core import GridSpecHost, Prior
-from .base import _PRECISIONS, ArenaPriorModule
+from .base import _PRECISIONS, ArenaPriorModule, reject_second_order
 from .convex_net import ConvexNextNet
 
 
@@ -85,6 +85,7 @@ class ConvexDiffeomorphismNet(ArenaPriorModule):
     def __init__(self, n_hidden: int = 130, n_hidden_layers: int = 1, nf_layers: int = 4, nf_hidden: int = 70,
                  in_features: int = 2, diffeo_args: Optional[Dict[str, Any]] = None, precision: str = "fp32", **kwargs):
         super().__init__(precision=precision)
+        reject_second_order("ConvexDiffeomorphismNet", kwargs)
         if in_features != 2:
             raise ValueError("NormalizingFlow1D couples two variables: in_features must be 2")
         self.in_features = self.in_channels = in_features

@@ -2,7 +2,12 @@
 
 Same constructor arguments, ``state_dict`` keys/shapes and initial weights for a given
 seed as the reference (``awesome/model/convex_net.py:10-40,134-220``); the arithmetic runs
-in ``libawb.so``."""
+in ``libawb.so``.
+
+``second_order=True`` (not a reference argument; it changes neither the state_dict nor the initial weights) makes the
+coordinate gradient differentiable: ``g = grad(prior(x).sum(), x, create_graph=True)`` followed by a loss on ``g`` (a
+gradient penalty) trains the prior, as with the reference's plain-torch module.  Differentiating the parameter gradients
+still raises.  With the default, a double backward raises."""
 from __future__ import annotations
 
 import math
@@ -56,8 +61,8 @@ class OutBlock(SkipBlock):
 
 class ConvexNextNet(ArenaPriorModule):
     def __init__(self, n_hidden: int = 130, in_features: int = 2, out_features: int = 1,
-                 n_hidden_layers: int = 1, precision: str = "fp32", **kwargs):
-        super().__init__(precision=precision)
+                 n_hidden_layers: int = 1, precision: str = "fp32", second_order: bool = False, **kwargs):
+        super().__init__(precision=precision, second_order=second_order)
         if out_features != 1:
             raise ValueError("the fused prior supports out_features == 1 (as every reference config)")
         self.n_hidden, self.in_features, self.n_hidden_layers = n_hidden, in_features, n_hidden_layers
@@ -86,8 +91,9 @@ class ConvexNet(ArenaPriorModule):
     """Older naming (``convex_net.py:10-40``): same network as ``ConvexNextNet(n_hidden_layers=1)``
     with keys ``W0y, W1z, W2z, W1y, W2y``; clamps ``W1z.weight`` and ``W2z.weight``."""
 
-    def __init__(self, n_hidden: int = 130, in_channels: int = 2, precision: str = "fp32", **kwargs):
-        super().__init__(precision=precision)
+    def __init__(self, n_hidden: int = 130, in_channels: int = 2, precision: str = "fp32", second_order: bool = False,
+                 **kwargs):
+        super().__init__(precision=precision, second_order=second_order)
         in_features, out_features = in_channels, 1
         self.n_hidden, self.in_features = n_hidden, in_features
         # reference registration order: W0y, W1z, W2z, W1y, W2y

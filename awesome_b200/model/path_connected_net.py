@@ -15,7 +15,7 @@ from torch import nn
 
 from .. import _lib as L
 from ..core import GridSpecHost, Prior
-from .base import _PRECISIONS, Affine, ArenaPriorModule
+from .base import _PRECISIONS, Affine, ArenaPriorModule, reject_second_order
 from .convex_net import ConvexNextNet
 
 
@@ -181,6 +181,7 @@ class PathConnectedNet(ArenaPriorModule):
         super().__init__(precision=precision or getattr(convex_net, "precision", "fp32"))
         if not isinstance(convex_net, ConvexNextNet):
             raise TypeError("convex_net must be an awesome_b200 ConvexNextNet")
+        reject_second_order("PathConnectedNet", {"second_order": kwargs.get("second_order") or convex_net.second_order})
         if not isinstance(flow_net, NormNet) or not isinstance(flow_net.net, PixelizeNet) \
                 or not isinstance(flow_net.net.network, RealNVP) or not isinstance(flow_net.norm, (MinMax, MeanStd)):
             raise TypeError("flow_net must be NormNet(PixelizeNet(init_realnvp(...)), MinMax | MeanStd)")
@@ -484,6 +485,7 @@ def real_nvp_path_connected_net(channels: int = 2, hidden_units: int = 130, flow
     ``net_factory.real_nvp_path_connected_net`` (``net_factory.py:124-176``).  The MinMax fit on a
     [0,1] coordinate grid is min=0, max=1 per channel (SURVEY 7.2 item 6), so the 1.2 GB grid the
     reference materialises for C=3 is never built."""
+    reject_second_order("real_nvp_path_connected_net", kwargs)
     network_type = network_type or PathConnectedNet
     network_args = network_args or {}
     flow = init_realnvp(channels=channels, hidden_units=hidden_units, output_fn=flow_output_fn,

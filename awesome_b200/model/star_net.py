@@ -12,7 +12,7 @@ from torch import nn
 
 from .. import _lib as L
 from ..core import Prior
-from .base import Affine, ArenaPriorModule
+from .base import Affine, ArenaPriorModule, reject_second_order
 
 
 def _lin(i: int, o: int) -> Affine:
@@ -35,6 +35,7 @@ class _StarFunction(torch.autograd.Function):
 class StarShapedNet(ArenaPriorModule):
     def __init__(self, n_hidden: int = 150, **kwargs):
         super().__init__(precision="fp32")
+        reject_second_order("StarShapedNet", kwargs)
         self.n_hidden = n_hidden
         self.offset = nn.Parameter(torch.zeros(1, 2))
         self.offset.requires_grad = False            # the notebook unfreezes it at epoch 1000

@@ -130,7 +130,8 @@ int64_t awb_prior_param_count(awb_handle h);
  * 1 forward + backward / any call, 2 awb_prior_fit_step only (much smaller on tensor-path handles, whose fused
  * kernel keeps the activations on the SM), 3 awb_prior_deformation / awb_prior_deformation_backward only (the flow's
  * buffers: deformed coordinates, coupling records, their gradient and the flow's partials; no ICNN activations, about
- * 80 MB instead of 0.85 GB for a 640x480 C = 2 frame). */
+ * 80 MB instead of 0.85 GB for a 640x480 C = 2 frame), 4 awb_prior_forward(training = 1) followed by
+ * awb_prior_backward and awb_prior_grid_grad_backward (layout 1 plus L + 1 tangent activation planes). */
 int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t training);
 /* Layout of the optimizer state: fp32 m[O][P], then fp32 v[O][P] (Adamax: the exp_inf u), then the per-object scalars at
  * byte offset round_up(8 * O * P, 256), read through awb_opt_read_scalars. */
@@ -188,6 +189,21 @@ int awb_prior_flow_inverse(awb_handle h, const float* params, const awb_grid_spe
 int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* grid,
                        const float* dlogits, float* grads, float* dgrid, void* workspace,
                        size_t workspace_bytes, void* stream);
+
+/* Double backward of awb_prior_backward's dgrid (gradient penalties trained through the prior, DESIGN 3b.1).  The first
+ * backward maps (w = dlogits, params) to dgrid_n = w_n J_n^T with J_n = d y_n / d x_n.  For the cotangent
+ * d_dgrid = d R / d dgrid ([B,C,H,W], the layout of dgrid) this returns d_dlogits [N] = J_n u_n, the derivative of each
+ * logit along its u_n, and grads [P] (overwritten, state_dict order) = sum_n w_n d(J_n u_n) / d params; every bias
+ * entry is exactly 0.  d R / d grid is 0: the ICNN is piecewise linear in its input.  Exact fp32 kernels at both
+ * precisions; the masks, weights and activations are those of the training forward.
+ * Must follow awb_prior_forward(training = 1) on the same workspace, of awb_prior_workspace_bytes(h, N, 4) bytes (the
+ * training = 1 layout followed by L + 1 tangent activation planes).  The forward's activations are only read, so the
+ * call may be repeated; awb_prior_backward may run on the same workspace before or after it.  dlogits: the first
+ * backward's [N]; params: those of the forward.  Single-object AWB_KIND_ICNN handles; any other handle:
+ * AWB_ERR_UNSUPPORTED. */
+int awb_prior_grid_grad_backward(awb_handle h, const float* params, const awb_grid_spec* grid, const float* dlogits,
+                                 const float* d_dgrid, float* d_dlogits, float* grads, void* workspace,
+                                 size_t workspace_bytes, void* stream);
 
 /* get_deformation() alone (path_connected_net.py:125-129, convex_diffeomorphism_net.py:180-185): the 1x1 conv (linear)
  * and the flow, no ICNN.  deformed: device [N][C] pixel rows.  training = 1 keeps the coupling records in the workspace
