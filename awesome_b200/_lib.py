@@ -15,6 +15,8 @@ LIB_PATH = os.environ.get("AWB_LIB_PATH") or os.path.join(_HERE, "csrc", "libawb
 AWB_KIND_ICNN, AWB_KIND_FLOW_ICNN, AWB_KIND_STAR, AWB_KIND_DIFFEO_ICNN = 0, 1, 2, 3
 AWB_PREC_FP32, AWB_PREC_F16 = 0, 1
 AWB_GRID_EXPLICIT, AWB_GRID_LINSPACE, AWB_GRID_INDEX = 0, 1, 2
+AWB_WS_INFERENCE, AWB_WS_TRAINING, AWB_WS_FIT_STEP, AWB_WS_DEFORMATION, AWB_WS_SECOND_ORDER = 0, 1, 2, 3, 4
+AWB_FWD_EXACT, AWB_FWD_EXACT_TRAINING, AWB_FWD_TC, AWB_FWD_TC_TRAINING = 0, 1, 2, 3
 AWB_LOSS_SE_SIGMOID, AWB_LOSS_BCE_LOGITS = 0, 1
 AWB_CLS_UNARY_LT_HALF, AWB_CLS_NOT_ONE = 0, 1
 AWB_OPT_ADAM, AWB_OPT_ADAMAX = 0, 1

@@ -91,23 +91,22 @@ class Prior:
     def handle(self):
         return self._h
 
-    def workspace_bytes(self, n_pixels: int, training) -> int:
-        """``training``: False / True, 2 for a fit-step-only workspace, 3 for a deformation-only workspace, 4 for a
-        training workspace that also holds the second-order pass's tangent rows (see ``awb_prior_workspace_bytes``)."""
-        b = int(self.lib.awb_prior_workspace_bytes(self._h, n_pixels, int(training)))
+    def workspace_bytes(self, n_pixels: int, layout: int) -> int:
+        """Bytes of a workspace of ``layout`` (``L.AWB_WS_*``, see ``awb_prior_workspace_bytes``)."""
+        b = int(self.lib.awb_prior_workspace_bytes(self._h, n_pixels, layout))
         if b < 0:
             raise L.AwbError(b, "workspace size query failed")
         return b
 
-    def new_workspace(self, n_pixels: int, training, device) -> torch.Tensor:
-        return torch.empty(self.workspace_bytes(n_pixels, training), dtype=torch.uint8, device=device)
+    def new_workspace(self, n_pixels: int, layout: int, device) -> torch.Tensor:
+        return torch.empty(self.workspace_bytes(n_pixels, layout), dtype=torch.uint8, device=device)
 
-    def cached_workspace(self, n_pixels: int, training: bool, device) -> torch.Tensor:
-        key = (n_pixels, training, str(device))
+    def cached_workspace(self, n_pixels: int, layout: int, device) -> torch.Tensor:
+        key = (n_pixels, layout, str(device))
         ws = self._ws_cache.get(key)
         if ws is None:
             self._ws_cache.clear()
-            ws = self.new_workspace(n_pixels, training, device)
+            ws = self.new_workspace(n_pixels, layout, device)
             self._ws_cache[key] = ws
         return ws
 
@@ -127,9 +126,9 @@ class Prior:
         L.check(self.lib.awb_prior_set_flow_eval(self._h, int(mode)))
 
     # ---- kernels
-    def forward(self, params: torch.Tensor, grid: GridSpecHost, training, ws: torch.Tensor,
+    def forward(self, params: torch.Tensor, grid: GridSpecHost, mode: int, ws: torch.Tensor,
                 want_deformed: bool = False) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
-        """``training``: 0 / False inference, 1 / True exact training forward, 3 tensor-path training forward."""
+        """``mode``: ``L.AWB_FWD_*``; ``ws`` of the workspace layout ``awb_prior_forward`` names for it."""
         N = grid.n_pixels
         logits = torch.empty((self.n_objects, N), dtype=torch.float32, device=params.device)
         deformed = torch.empty((self.n_objects, N, self.C), dtype=torch.float32, device=params.device) \
@@ -137,16 +136,8 @@ class Prior:
         gs = grid.to_c()
         L.check(self.lib.awb_prior_forward(self._h, params.data_ptr(), C.byref(gs), logits.data_ptr(),
                                            deformed.data_ptr() if deformed is not None else None,
-                                           int(training), ws.data_ptr(), ws.numel(), L.stream_ptr()))
+                                           mode, ws.data_ptr(), ws.numel(), L.stream_ptr()))
         return logits, deformed
-
-    def forward_tensor_path(self, params: torch.Tensor, grid: GridSpecHost, ws: torch.Tensor) -> torch.Tensor:
-        """Logits through the tcgen05 forward (fp16 operands, fp32 accumulate); f16 handles only."""
-        logits = torch.empty((self.n_objects, grid.n_pixels), dtype=torch.float32, device=params.device)
-        gs = grid.to_c()
-        L.check(self.lib.awb_prior_forward(self._h, params.data_ptr(), C.byref(gs), logits.data_ptr(), None, 2,
-                                           ws.data_ptr(), ws.numel(), L.stream_ptr()))
-        return logits
 
     def backward(self, params: torch.Tensor, grid: GridSpecHost, dlogits: torch.Tensor, ws: torch.Tensor,
                  want_dgrid: bool) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
@@ -163,8 +154,8 @@ class Prior:
                            ws: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
         """Double backward of ``backward``'s dgrid (``awb_prior_grid_grad_backward``, single-object ICNN): ``dlogits``
         (``[1, N]``) is the first backward's, ``d_dgrid`` (``[B, C, H, W]`` fp32, contiguous) the gradient on its dgrid.
-        Returns ``d_dlogits [1, N]`` and ``grads [1, P]``.  ``ws``: ``workspace_bytes(N, 4)``, after ``forward(training=1)``
-        on it."""
+        Returns ``d_dlogits [1, N]`` and ``grads [1, P]``.  ``ws``: layout ``AWB_WS_SECOND_ORDER``, after
+        ``forward(AWB_FWD_EXACT_TRAINING)`` on it."""
         d_dlogits = torch.empty((self.n_objects, grid.n_pixels), dtype=torch.float32, device=params.device)
         grads = torch.empty((self.n_objects, self.n_params), dtype=torch.float32, device=params.device)
         gs = grid.to_c()
@@ -175,7 +166,7 @@ class Prior:
 
     def deformation(self, params: torch.Tensor, grid: GridSpecHost, training: bool, ws: torch.Tensor) -> torch.Tensor:
         """``get_deformation`` alone (1x1 conv / linear and flow, no ICNN): pixel rows ``[N, C]``.  ``ws``:
-        ``workspace_bytes(N, 3)``; ``training`` keeps the coupling records for ``deformation_backward``."""
+        layout ``AWB_WS_DEFORMATION``; ``training`` keeps the coupling records for ``deformation_backward``."""
         out = torch.empty((grid.n_pixels, self.C), dtype=torch.float32, device=params.device)
         gs = grid.to_c()
         L.check(self.lib.awb_prior_deformation(self._h, params.data_ptr(), C.byref(gs), out.data_ptr(), int(bool(training)),
@@ -208,8 +199,8 @@ class Prior:
                     loss, grad_row: torch.Tensor, ws: torch.Tensor, reuse_packed: bool = False) -> None:
         """Gradient row of pixel rows ``[row_begin, row_end)`` of the batch into ``grad_row`` (``[P + 1]`` fp32, device).
         ``target`` is the FULL batch ``[N]``; ``loss`` the ``LossSpec`` of the full batch.  ``ws``:
-        ``workspace_bytes(row_end - row_begin, 2)``.  ``reuse_packed``: the previous call on ``ws`` was a slice of the
-        same parameters."""
+        layout ``AWB_WS_FIT_STEP`` for ``row_end - row_begin`` pixels.  ``reuse_packed``: the previous call on ``ws`` was
+        a slice of the same parameters."""
         gs = grid.to_c()
         L.check(self.lib.awb_prior_slice_grads(self._h, params.data_ptr(), C.byref(gs), int(row_begin), int(row_end),
                                                target.data_ptr(), C.byref(loss), grad_row.data_ptr(), ws.data_ptr(),

@@ -59,10 +59,12 @@ static Layout make_layout(const awb_desc& d) {
 
 static int64_t align256(int64_t b) { return round_up(b, 256); }
 
-// fit_only: layout for awb_prior_fit_step on a tensor-path handle -- the fused kernel keeps activations on the SM, so
-// the [N][ld] activation / delta planes of the CUDA-core path are not carved (0.85 GB per 640x480 frame).
-// deform_only: layout of awb_prior_deformation / _backward -- no ICNN partials, planes or tensor-path image either.
-Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only, bool deform_only, bool tangent) {
+// fit_only: on a tensor-path handle the fused kernel keeps activations on the SM, so the [N][ld] activation / delta
+// planes of the CUDA-core path are not carved (0.85 GB per 640x480 frame).
+// deform_only: no ICNN partials, planes or tensor-path image either.
+Workspace carve(const awb_prior* h, int64_t N, int layout, void* base) {
+  const bool training = layout != AWB_WS_INFERENCE, fit_only = layout == AWB_WS_FIT_STEP,
+             deform_only = layout == AWB_WS_DEFORMATION, tangent = layout == AWB_WS_SECOND_ORDER;
   const Layout& L = h->lay;
   const int64_t O = h->desc.n_objects;
   int S = n_splits(N);
@@ -234,9 +236,9 @@ int awb_prior_destroy(awb_handle h) {
 
 int64_t awb_prior_param_count(awb_handle h) { return h ? h->lay.P : -1; }
 
-int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t training) {
-  if (!h || n_pixels < 1) return -1;
-  return carve(h, n_pixels, training != 0, nullptr, training == 2, training == 3, training == 4).bytes;
+int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t layout) {
+  if (!h || n_pixels < 1 || layout < AWB_WS_INFERENCE || layout > AWB_WS_SECOND_ORDER) return -1;
+  return carve(h, n_pixels, layout, nullptr).bytes;
 }
 
 int64_t awb_opt_state_bytes(awb_handle h) {
@@ -273,40 +275,42 @@ int awb_prior_set_flow_eval(awb_handle h, int32_t mode) {
   return AWB_OK;
 }
 
-// window (optional, {row_begin, row_end}): the call works on the pixel rows [row_begin, row_end) of the batch, which must
-// be a non-empty range inside [0, N), and the workspace is sized for them
-static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, bool training, int64_t* N,
-                        bool fit_only = false, const int64_t* window = nullptr, bool deform_only = false,
-                        bool tangent = false) {
+// Validates the arguments every workspace entry point shares and carves the workspace, of layout `layout` (AWB_WS_*),
+// into *out.  window (optional, {row_begin, row_end}): the call works on the pixel rows [row_begin, row_end) of the
+// batch, which must be a non-empty range inside [0, N), and the workspace is sized for them; out->row0 = row_begin.
+static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, int layout,
+                        const int64_t* window, Workspace* out) {
   if (!h || !g || !ws) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (g->B < 1 || g->H < 1 || g->W < 1) { set_error("empty grid %dx%dx%d", g->B, g->H, g->W); return AWB_ERR_INVALID; }
   if (g->mode == AWB_GRID_EXPLICIT && !g->grid) { set_error("explicit grid needs a pointer"); return AWB_ERR_INVALID; }
   if (g->mode < 0 || g->mode > 2) { set_error("unknown grid mode %d", g->mode); return AWB_ERR_INVALID; }
-  *N = (int64_t)g->B * g->H * g->W;
-  if (*N > (int64_t)1 << 30) { set_error("too many pixel rows"); return AWB_ERR_UNSUPPORTED; }
-  if (window && (window[0] < 0 || window[0] >= window[1] || window[1] > *N)) {
+  const int64_t N = (int64_t)g->B * g->H * g->W;
+  if (N > (int64_t)1 << 30) { set_error("too many pixel rows"); return AWB_ERR_UNSUPPORTED; }
+  if (window && (window[0] < 0 || window[0] >= window[1] || window[1] > N)) {
     set_error("pixel-row window [%lld, %lld) is empty or outside [0, %lld)", (long long)window[0], (long long)window[1],
-              (long long)*N);
+              (long long)N);
     return AWB_ERR_INVALID;
   }
-  int64_t need = carve(h, window ? window[1] - window[0] : *N, training, nullptr, fit_only, deform_only, tangent).bytes;
-  if ((int64_t)ws_bytes < need) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)need); return AWB_ERR_WORKSPACE; }
+  const Workspace w = carve(h, window ? window[1] - window[0] : N, layout, ws);
+  if ((int64_t)ws_bytes < w.bytes) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)w.bytes); return AWB_ERR_WORKSPACE; }
   if (h->desc.kind == AWB_KIND_FLOW_ICNN && !h->fc_set) { set_error("awb_prior_set_flow_consts not called"); return AWB_ERR_INVALID; }
+  *out = w;
+  out->row0 = window ? window[0] : 0;
   return AWB_OK;
 }
 
 int awb_prior_forward(awb_handle h, const float* params, const awb_grid_spec* g, float* logits, float* deformed,
-                      int32_t training, void* ws, size_t ws_bytes, void* stream) {
-  int64_t N;
-  int rc = check_common(h, g, ws, ws_bytes, training == 1 || training == 3, &N);
+                      int32_t mode, void* ws, size_t ws_bytes, void* stream) {
+  if (mode < AWB_FWD_EXACT || mode > AWB_FWD_TC_TRAINING) { set_error("unknown forward mode %d", mode); return AWB_ERR_INVALID; }
+  const bool training = mode == AWB_FWD_EXACT_TRAINING || mode == AWB_FWD_TC_TRAINING;
+  Workspace w;
+  int rc = check_common(h, g, ws, ws_bytes, training ? AWB_WS_TRAINING : AWB_WS_INFERENCE, nullptr, &w);
   if (rc) return rc;
   if (!params) { set_error("null params"); return AWB_ERR_INVALID; }
-  Workspace w = carve(h, N, training == 1, ws);
-  if (training == 2 || training == 3) {   // tensor-path logits (fp16 operands); the default forward stays exact fp32
+  if (mode == AWB_FWD_TC || mode == AWB_FWD_TC_TRAINING) {   // tensor-path logits (fp16 operands); the default forward stays exact fp32
     if (h->desc.precision != AWB_PREC_F16) { set_error("tensor-path forward needs an f16 handle"); return AWB_ERR_INVALID; }
     if (!logits) { set_error("null logits"); return AWB_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
-    if (training == 3) w = carve(h, N, true, ws);
     if (has_flow(h)) {
       rc = any_flow_forward(h, params, g, w, deformed, st);   // keeps X (and the coupling inputs when training)
       if (rc) return rc;
@@ -314,7 +318,7 @@ int awb_prior_forward(awb_handle h, const float* params, const awb_grid_spec* g,
     return tc_fit_forward_backward(h, params, g, nullptr, nullptr, logits, 0, w, nullptr, st, false,
                                    has_flow(h) ? w.X : nullptr, nullptr);
   }
-  return simt_forward(h, params, g, logits, deformed, training != 0, w, (cudaStream_t)stream);
+  return simt_forward(h, params, g, logits, deformed, training, w, (cudaStream_t)stream);
 }
 
 int awb_prior_flow_inverse(awb_handle h, const float* params, const awb_grid_spec* g, float* out, void* stream) {
@@ -326,8 +330,8 @@ int awb_prior_flow_inverse(awb_handle h, const float* params, const awb_grid_spe
 
 int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* g, const float* dlogits, float* grads,
                        float* dgrid, void* ws, size_t ws_bytes, void* stream) {
-  int64_t N;
-  int rc = check_common(h, g, ws, ws_bytes, true, &N);
+  Workspace w;
+  int rc = check_common(h, g, ws, ws_bytes, AWB_WS_TRAINING, nullptr, &w);
   if (rc) return rc;
   if (!params || !dlogits || !grads) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (dgrid && (h->desc.kind == AWB_KIND_STAR || h->desc.n_objects != 1)) {
@@ -335,11 +339,12 @@ int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* g
               "(no caller needs it on grouped or star handles; kind %d, %d objects)", h->desc.kind, h->desc.n_objects);
     return AWB_ERR_UNSUPPORTED;
   }
-  Workspace w = carve(h, N, true, ws);
+  const int64_t N = w.N;
   cudaStream_t st = (cudaStream_t)stream;
   if (h->desc.precision == AWB_PREC_F16) {
     // tensor path: one fused kernel recomputes the forward and runs the backward on the upstream gradient
-    // (must follow awb_prior_forward(training = 3) on the same workspace: the flow's X / coupling inputs live there)
+    // (must follow awb_prior_forward(AWB_FWD_TC_TRAINING) on the same workspace: the flow's X / coupling inputs live
+    // there)
     const int O = h->desc.n_objects;
     awb_loss_spec up[16];
     for (int o = 0; o < O && o < 16; o++) { up[o].kind = AWB_LOSS_UPSTREAM; up[o].cls_rule = AWB_CLS_UNARY_LT_HALF; up[o].coef_fg = 1.f; up[o].coef_bg = 1.f; }
@@ -375,49 +380,53 @@ int awb_prior_grid_grad_backward(awb_handle h, const float* params, const awb_gr
               h->desc.n_objects);
     return AWB_ERR_UNSUPPORTED;
   }
-  int64_t N;
-  int rc = check_common(h, g, ws, ws_bytes, true, &N, false, nullptr, false, /*tangent=*/true);
+  Workspace w;
+  int rc = check_common(h, g, ws, ws_bytes, AWB_WS_SECOND_ORDER, nullptr, &w);
   if (rc) return rc;
   if (!params || !dlogits || !d_dgrid || !d_dlogits || !grads) { set_error("null argument"); return AWB_ERR_INVALID; }
-  Workspace w = carve(h, N, true, ws, false, false, true);
   cudaStream_t st = (cudaStream_t)stream;
   rc = simt_grid_grad_backward(h, g, dlogits, d_dgrid, d_dlogits, w, st);
   if (rc) return rc;
-  return simt_reduce_grads(h, grads, w, N, st);
+  return simt_reduce_grads(h, grads, w, w.N, st);
+}
+
+// Forward, loss and backward of a fit step on the rows of w (AWB_WS_FIT_STEP), up to the gradient and loss partials that
+// the caller reduces.  f16 handles: the flow on CUDA cores (K = C is too thin for tensor cores) around the tensor-path
+// ICNN -- the flow writes the deformed coordinates X, the fused kernel returns d loss / d X, the flow backward consumes
+// it.  reuse: the fused kernel reuses the packed fp16 weight image left in w.  *n_part: the number of ICNN partials
+// written, -1 (n_splits(N)) on the exact fp32 path.
+static int fit_gradients(awb_handle h, const float* params, const awb_grid_spec* g, const float* target,
+                         const awb_loss_spec* loss, bool reuse, const Workspace& w, cudaStream_t st, int* n_part) {
+  int rc;
+  if (h->desc.precision == AWB_PREC_F16) {
+    const bool flow = has_flow(h);
+    if (flow) { rc = any_flow_forward(h, params, g, w, nullptr, st); if (rc) return rc; }
+    *n_part = 0;
+    rc = tc_fit_forward_backward(h, params, g, target, loss, nullptr, 1, w, n_part, st, reuse, flow ? w.X : nullptr,
+                                 flow ? w.dX : nullptr);
+    if (rc) return rc;
+    return flow ? any_flow_backward(h, params, g, w, st) : AWB_OK;
+  }
+  *n_part = -1;
+  rc = simt_forward(h, params, g, nullptr, nullptr, true, w, st);
+  if (rc) return rc;
+  return simt_backward(h, params, g, target, loss, nullptr, false, w, st);
 }
 
 int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_grid_spec* g, const float* target,
                        const awb_loss_spec* loss, const awb_opt_hyper* hy, float* loss_out, void* ws, size_t ws_bytes,
                        int32_t flags, void* stream) {
-  int64_t N;
-  int rc = check_common(h, g, ws, ws_bytes, true, &N, /*fit_only=*/true);
+  Workspace w;
+  int rc = check_common(h, g, ws, ws_bytes, AWB_WS_FIT_STEP, nullptr, &w);
   if (rc) return rc;
   if (!params || !opt_state || !target || !loss || !hy) { set_error("null argument"); return AWB_ERR_INVALID; }
-  Workspace w = carve(h, N, true, ws, true);
+  // simt_reduce_opt refreshes a flow prior's fp16 weight image only when its optimizer owns every group
+  const bool reuse = (flags & AWB_FIT_REUSE_PACKED) != 0 && (!has_flow(h) || hy->active_groups == 0);
   cudaStream_t st = (cudaStream_t)stream;
-  if (h->desc.precision == AWB_PREC_F16) {
-    int n_part = 0;
-    if (has_flow(h)) {
-      // RealNVP on CUDA cores (K = C is too thin for tensor cores) around the tensor-path ICNN: the flow writes the
-      // deformed coordinates X, the fused kernel returns d loss / d X, the flow backward consumes it.
-      rc = any_flow_forward(h, params, g, w, nullptr, st);
-      if (rc) return rc;
-      rc = tc_fit_forward_backward(h, params, g, target, loss, nullptr, 1, w, &n_part, st,
-                                   (flags & AWB_FIT_REUSE_PACKED) != 0 && hy->active_groups == 0, w.X, w.dX);
-      if (rc) return rc;
-      rc = any_flow_backward(h, params, g, w, st);
-      if (rc) return rc;
-      return simt_reduce_opt(h, params, opt_state, hy, loss_out, w, N, st, n_part);
-    }
-    rc = tc_fit_forward_backward(h, params, g, target, loss, nullptr, 1, w, &n_part, st, (flags & AWB_FIT_REUSE_PACKED) != 0);
-    if (rc) return rc;
-    return simt_reduce_opt(h, params, opt_state, hy, loss_out, w, N, st, n_part);
-  }
-  rc = simt_forward(h, params, g, nullptr, nullptr, true, w, st);
+  int n_part;
+  rc = fit_gradients(h, params, g, target, loss, reuse, w, st, &n_part);
   if (rc) return rc;
-  rc = simt_backward(h, params, g, target, loss, nullptr, false, w, st);
-  if (rc) return rc;
-  return simt_reduce_opt(h, params, opt_state, hy, loss_out, w, N, st);
+  return simt_reduce_opt(h, params, opt_state, hy, loss_out, w, w.N, st, n_part);
 }
 
 // get_deformation: single-object RealNVP o ICNN and NormalizingFlow1D o ICNN handles
@@ -436,11 +445,10 @@ int awb_prior_deformation(awb_handle h, const float* params, const awb_grid_spec
                           void* ws, size_t ws_bytes, void* stream) {
   int rc = check_deformable(h);
   if (rc) return rc;
-  int64_t N;
-  rc = check_common(h, g, ws, ws_bytes, true, &N, false, nullptr, /*deform_only=*/true);
+  Workspace w;
+  rc = check_common(h, g, ws, ws_bytes, AWB_WS_DEFORMATION, nullptr, &w);
   if (rc) return rc;
   if (!params || !deformed) { set_error("null argument"); return AWB_ERR_INVALID; }
-  Workspace w = carve(h, N, true, ws, false, true);
   if (!training) w.flowz = nullptr;   // the coupling records are kept for awb_prior_deformation_backward only
   return any_flow_forward(h, params, g, w, deformed, (cudaStream_t)stream);
 }
@@ -449,17 +457,16 @@ int awb_prior_deformation_backward(awb_handle h, const float* params, const awb_
                                    float* grads, float* dgrid, void* ws, size_t ws_bytes, void* stream) {
   int rc = check_deformable(h);
   if (rc) return rc;
-  int64_t N;
-  rc = check_common(h, g, ws, ws_bytes, true, &N, false, nullptr, /*deform_only=*/true);
+  Workspace w;
+  rc = check_common(h, g, ws, ws_bytes, AWB_WS_DEFORMATION, nullptr, &w);
   if (rc) return rc;
   if (!params || !d_deformed || !grads) { set_error("null argument"); return AWB_ERR_INVALID; }
-  Workspace w = carve(h, N, true, ws, false, true);
   cudaStream_t st = (cudaStream_t)stream;
   rc = simt_seed_dX(h, d_deformed, w, st);
   if (rc) return rc;
   rc = any_flow_backward(h, params, g, w, st, dgrid);
   if (rc) return rc;
-  return simt_reduce_grads(h, grads, w, N, st, /*n_partials=*/0);   // no ICNN partials: its entries are exactly 0
+  return simt_reduce_grads(h, grads, w, w.N, st, /*n_partials=*/0);   // no ICNN partials: its entries are exactly 0
 }
 
 // single-object ICNN and RealNVP o ICNN handles (the priors of the spatio-temporal fit)
@@ -480,33 +487,16 @@ int awb_prior_slice_grads(awb_handle h, const float* params, const awb_grid_spec
                           int32_t flags, void* stream) {
   int rc = check_sliceable(h);
   if (rc) return rc;
-  int64_t N;
+  Workspace w;
   const int64_t window[2] = {row_begin, row_end};
-  rc = check_common(h, g, ws, ws_bytes, true, &N, /*fit_only=*/true, window);
+  rc = check_common(h, g, ws, ws_bytes, AWB_WS_FIT_STEP, window, &w);
   if (rc) return rc;
   if (!params || !target || !loss || !grad_row) { set_error("null argument"); return AWB_ERR_INVALID; }
-  const int64_t n = row_end - row_begin;
-  Workspace w = carve(h, n, true, ws, true);
-  w.row0 = row_begin;
-  const float* tg = target + row_begin;
-  float* loss_slot = grad_row + h->lay.P;
   cudaStream_t st = (cudaStream_t)stream;
-  if (h->desc.precision == AWB_PREC_F16) {
-    const bool reuse = (flags & AWB_FIT_REUSE_PACKED) != 0;
-    const bool flow = has_flow(h);
-    int n_part = 0;
-    if (flow) { rc = flow_forward(h, params, g, w, nullptr, st); if (rc) return rc; }
-    rc = tc_fit_forward_backward(h, params, g, tg, loss, nullptr, 1, w, &n_part, st, reuse, flow ? w.X : nullptr,
-                                 flow ? w.dX : nullptr);
-    if (rc) return rc;
-    if (flow) { rc = flow_backward(h, params, g, w, st); if (rc) return rc; }
-    return simt_reduce_grads(h, grad_row, w, n, st, n_part, loss_slot);
-  }
-  rc = simt_forward(h, params, g, nullptr, nullptr, true, w, st);
+  int n_part;
+  rc = fit_gradients(h, params, g, target + row_begin, loss, (flags & AWB_FIT_REUSE_PACKED) != 0, w, st, &n_part);
   if (rc) return rc;
-  rc = simt_backward(h, params, g, tg, loss, nullptr, false, w, st);
-  if (rc) return rc;
-  return simt_reduce_grads(h, grad_row, w, n, st, -1, loss_slot);
+  return simt_reduce_grads(h, grad_row, w, w.N, st, n_part, grad_row + h->lay.P);   // the loss sum goes to column P
 }
 
 int awb_prior_rows_opt_step(awb_handle h, float* params, void* opt_state, const float* rows, int32_t n_rows,
@@ -540,9 +530,10 @@ int awb_prior_fit_host_frames(awb_handle h, float* params, void* opt_state, cons
                               const float* const* host_targets, int32_t n_host, int32_t n_steps, const awb_loss_spec* loss,
                               const awb_opt_hyper* hy, float* loss_host, float* staging, void* ws, size_t ws_bytes,
                               int32_t flags, void* stream) {
-  int64_t N;
-  int rc = check_common(h, g, ws, ws_bytes, true, &N, /*fit_only=*/true);
+  Workspace w;   // awb_prior_fit_step carves it again for every step
+  int rc = check_common(h, g, ws, ws_bytes, AWB_WS_FIT_STEP, nullptr, &w);
   if (rc) return rc;
+  const int64_t N = w.N;
   if (!params || !opt_state || !host_targets || !loss || !hy || !staging) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (n_host < 1 || n_steps < 0) { set_error("n_host must be >= 1 and n_steps >= 0"); return AWB_ERR_INVALID; }
   for (int i = 0; i < n_host; i++)
@@ -588,12 +579,11 @@ int awb_prior_fit_host_frames(awb_handle h, float* params, void* opt_state, cons
 
 int awb_flow_identity_step(awb_handle h, float* params, void* opt_state, const awb_grid_spec* g,
                            const awb_opt_hyper* hy, float* loss_out, void* ws, size_t ws_bytes, void* stream) {
-  int64_t N;
-  int rc = check_common(h, g, ws, ws_bytes, true, &N);
+  Workspace w;
+  int rc = check_common(h, g, ws, ws_bytes, AWB_WS_TRAINING, nullptr, &w);
   if (rc) return rc;
   if (!params || !opt_state || !hy) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (h->desc.kind != AWB_KIND_FLOW_ICNN) { set_error("not a flow prior"); return AWB_ERR_INVALID; }
-  Workspace w = carve(h, N, true, ws);
   cudaStream_t st = (cudaStream_t)stream;
   rc = flow_forward(h, params, g, w, nullptr, st, /*use_linear=*/false);
   if (rc) return rc;
@@ -603,7 +593,7 @@ int awb_flow_identity_step(awb_handle h, float* params, void* opt_state, const a
   if (rc) return rc;
   awb_opt_hyper hh = *hy;
   hh.active_groups = 1;   // flow_net only
-  return simt_reduce_opt(h, params, opt_state, &hh, loss_out, w, N, st);
+  return simt_reduce_opt(h, params, opt_state, &hh, loss_out, w, w.N, st);
 }
 
 int awb_optim_step(awb_handle h, float* params, const float* grads, void* opt_state, const awb_opt_hyper* hy,
@@ -678,11 +668,10 @@ int awb_opt_read_scalars(awb_handle h, const void* opt_state, int32_t obj, awb_o
 
 int awb_prior_actnorm_init(awb_handle h, float* params, const awb_grid_spec* g, void* ws, size_t ws_bytes,
                            void* stream) {
-  int64_t N;
-  int rc = check_common(h, g, ws, ws_bytes, false, &N);
+  Workspace w;
+  int rc = check_common(h, g, ws, ws_bytes, AWB_WS_INFERENCE, nullptr, &w);
   if (rc) return rc;
   if (h->desc.kind != AWB_KIND_FLOW_ICNN) { set_error("not a flow prior"); return AWB_ERR_INVALID; }
-  Workspace w = carve(h, N, false, ws);
   return flow_actnorm_init(h, params, g, w, (cudaStream_t)stream);
 }
 

@@ -120,10 +120,10 @@ struct Workspace {
   // coordinates at the global one.
   int64_t row0, N;
 };
-// deform_only: the layout of awb_prior_deformation / _backward -- flow buffers only (X, coupling records, dX, flow partials
-// and scratch), no ICNN weights, partials or activation planes.  tangent: the training layout plus the tangent rows ZT.
-Workspace carve(const awb_prior* h, int64_t N, bool training, void* base, bool fit_only = false, bool deform_only = false,
-                bool tangent = false);
+// Regions of workspace layout `layout` (AWB_WS_*, validated by the caller) for N pixel rows at base (null: sizes only).
+// AWB_WS_DEFORMATION: flow buffers only (X, coupling records, dX, flow partials and scratch), no ICNN weights, partials
+// or activation planes.  AWB_WS_SECOND_ORDER: the training layout plus the tangent rows ZT.
+Workspace carve(const awb_prior* h, int64_t N, int layout, void* base);
 
 // ---- per-kernel-class timing (CUDA events on the launch stream) and launch counting ----
 enum { PK_PACK = 0, PK_INPUT, PK_GEMM_FWD, PK_OUT_LOSS, PK_GEMM_WGRAD, PK_GEMM_DGRAD, PK_IN_BWD, PK_OPT,

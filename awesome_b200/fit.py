@@ -133,7 +133,7 @@ class PriorFitter:
             raise ValueError("params must be a contiguous fp32 [O,P] arena")
         self.lib = prior.lib
         with torch.cuda.device(self.device):
-            self.ws = prior.new_workspace(grid.n_pixels, 2, self.device)     # fit-step-only layout
+            self.ws = prior.new_workspace(grid.n_pixels, L.AWB_WS_FIT_STEP, self.device)
             self.opt_state = torch.empty(prior.opt_state_bytes(), dtype=torch.uint8, device=self.device)
             self._specs_list = loss.to_specs(self.target)
         self._specs = (L.LossSpec * O)(*self._specs_list)
@@ -310,7 +310,7 @@ class FlowIdentityFitter(PriorFitter):
         self.device = params.device
         self.lib = prior.lib
         with torch.cuda.device(self.device):
-            self.ws = prior.new_workspace(grid.n_pixels, True, self.device)
+            self.ws = prior.new_workspace(grid.n_pixels, L.AWB_WS_TRAINING, self.device)
             self.opt_state = torch.empty(prior.opt_state_bytes(), dtype=torch.uint8, device=self.device)
         self._hyper = optim.to_c()
         self._gs = grid.to_c()
@@ -409,7 +409,7 @@ class SlicedFitter:
         R = prior.grad_row_floats
         biggest = max(e - b for b, e in self.plan)
         with torch.cuda.device(self.device):
-            self.ws = prior.new_workspace(biggest, 2, self.device)          # one slice after the other
+            self.ws = prior.new_workspace(biggest, L.AWB_WS_FIT_STEP, self.device)   # one slice after the other
             self.opt_state = torch.empty(prior.opt_state_bytes(), dtype=torch.uint8, device=self.device)
             self.rows = torch.zeros((self.n_slices, R), dtype=torch.float32, device=self.device)   # empty slices stay 0
             self.local = self.rows if world == 1 else torch.zeros((len(self.mine), R), dtype=torch.float32,

@@ -130,8 +130,8 @@ class _GridGradFunction(torch.autograd.Function):
         ws = ctx.ws
         if module.precision == "f16":
             # the first order ran on the tensor path, which keeps no activations: an exact fp32 forward provides them
-            ws = prior.new_workspace(spec.n_pixels, 4, w.device)
-            prior.forward(module._arena, spec, 1, ws)
+            ws = prior.new_workspace(spec.n_pixels, L.AWB_WS_SECOND_ORDER, w.device)
+            prior.forward(module._arena, spec, L.AWB_FWD_EXACT_TRAINING, ws)
         d_w, grads = prior.grid_grad_backward(module._arena, spec, w, u, ws)
         return (None, None, None, None, None, d_w) + _split_grads(grads, ctx.shapes)
 
@@ -141,20 +141,21 @@ class _PriorFunction(torch.autograd.Function):
     def forward(ctx, module, spec, needs_grad, grid_tensor, *params):
         """``needs_grad`` is decided by the caller (grad mode is always off inside ``Function.forward`` and
         ``ctx.needs_input_grad`` ignores ``torch.no_grad()``): a forward under ``no_grad`` takes the exact fp32 inference
-        path (mode 0) on the cached workspace, whatever ``requires_grad`` says."""
+        path (``AWB_FWD_EXACT``) on the cached workspace, whatever ``requires_grad`` says."""
         prior = module._prior_for(params[0].device)
         arena = module._arena
         second_order = needs_grad and module.second_order
         if needs_grad:
             # private: several forwards may precede backward.  An exact second-order module also keeps room for the
             # tangent rows of the second-order pass (the training layout is a prefix of that one).
-            ws = prior.new_workspace(spec.n_pixels, 4 if second_order and module.precision == "fp32" else True,
-                                     arena.device)
-        else:
-            ws = prior.cached_workspace(spec.n_pixels, False, arena.device)
-        # training forward of a tensor-path module: logits from the fused tcgen05 kernel (mode 3); backward re-runs it
-        # with the upstream gradient.  Inference (no grad) always takes the exact fp32 path.
-        mode = (3 if module.precision == "f16" else 1) if needs_grad else 0
+            layout = L.AWB_WS_SECOND_ORDER if second_order and module.precision == "fp32" else L.AWB_WS_TRAINING
+            ws = prior.new_workspace(spec.n_pixels, layout, arena.device)
+            # training forward of a tensor-path module: logits from the fused tcgen05 kernel; backward re-runs it with
+            # the upstream gradient
+            mode = L.AWB_FWD_TC_TRAINING if module.precision == "f16" else L.AWB_FWD_EXACT_TRAINING
+        else:   # inference (no grad) always takes the exact fp32 path
+            ws = prior.cached_workspace(spec.n_pixels, L.AWB_WS_INFERENCE, arena.device)
+            mode = L.AWB_FWD_EXACT
         logits, _ = prior.forward(arena, spec, mode, ws)
         ctx.module, ctx.spec, ctx.ws, ctx.prior = module, spec, (ws if needs_grad else None), prior
         ctx.shapes = [p.shape for p in params]
@@ -186,7 +187,7 @@ class _DeformationFunction(torch.autograd.Function):
     def forward(ctx, module, spec, grid_tensor, *params):
         prior = module._prior_for(params[0].device)
         arena = module._arena
-        ws = prior.new_workspace(spec.n_pixels, 3, arena.device)
+        ws = prior.new_workspace(spec.n_pixels, L.AWB_WS_DEFORMATION, arena.device)
         rows = prior.deformation(arena, spec, True, ws)
         ctx.module, ctx.spec, ctx.ws, ctx.prior = module, spec, ws, prior
         ctx.shapes = [p.shape for p in params]
@@ -336,8 +337,8 @@ class ArenaPriorModule(nn.Module):
             with torch.cuda.device(arena.device):
                 return _DeformationFunction.apply(self, spec, x if x.requires_grad else None, *params)
         with torch.no_grad(), torch.cuda.device(arena.device):
-            ws = prior.cached_workspace(spec.n_pixels, False, arena.device)
-            _, deformed = prior.forward(arena, spec, False, ws, want_deformed=True)
+            ws = prior.cached_workspace(spec.n_pixels, L.AWB_WS_INFERENCE, arena.device)
+            _, deformed = prior.forward(arena, spec, L.AWB_FWD_EXACT, ws, want_deformed=True)
         return deformed[0]
 
     def make_fitter(self, grid, target, loss=None, optim=None, **kw):

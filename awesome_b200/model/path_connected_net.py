@@ -329,7 +329,7 @@ class PathConnectedNet(ArenaPriorModule):
                 self.linear.bias.fill_(0)
         gs = grid.to_c()
         with torch.no_grad(), torch.cuda.device(arena.device):
-            ws = prior.cached_workspace(grid.n_pixels, False, arena.device)
+            ws = prior.cached_workspace(grid.n_pixels, L.AWB_WS_INFERENCE, arena.device)
             L.check(prior.lib.awb_prior_actnorm_init(prior.handle, arena.data_ptr(), C.byref(gs), ws.data_ptr(),
                                                      ws.numel(), L.stream_ptr()))
             if not use_linear:

@@ -124,15 +124,30 @@ const char* awb_last_error(void);
 int awb_prior_create(const awb_desc* desc, awb_handle* out);
 int awb_prior_destroy(awb_handle h);
 
+/* workspace layouts (awb_prior_workspace_bytes) */
+#define AWB_WS_INFERENCE 0    /* awb_prior_forward(AWB_FWD_EXACT or AWB_FWD_TC), awb_prior_actnorm_init */
+#define AWB_WS_TRAINING 1     /* a training forward + awb_prior_backward; large enough for every awb_prior_* entry
+                                 point except awb_prior_grid_grad_backward */
+#define AWB_WS_FIT_STEP 2     /* awb_prior_fit_step / _fit_steps / _fit_host_frames / _slice_grads only: much smaller on
+                                 tensor-path handles, whose fused kernel keeps the activations on the SM */
+#define AWB_WS_DEFORMATION 3  /* awb_prior_deformation / _deformation_backward only: the flow's buffers (deformed
+                                 coordinates, coupling records, their gradient and the flow's partials), no ICNN
+                                 activations; about 80 MB instead of 0.85 GB for a 640x480 C = 2 frame */
+#define AWB_WS_SECOND_ORDER 4 /* awb_prior_forward(AWB_FWD_EXACT_TRAINING) followed by awb_prior_backward and
+                                 awb_prior_grid_grad_backward: AWB_WS_TRAINING (a prefix of this layout) plus L + 1
+                                 tangent activation planes */
+
+/* forward modes (awb_prior_forward) */
+#define AWB_FWD_EXACT 0          /* exact fp32 inference; workspace AWB_WS_INFERENCE */
+#define AWB_FWD_EXACT_TRAINING 1 /* exact fp32, keeps its activations for awb_prior_backward; AWB_WS_TRAINING */
+#define AWB_FWD_TC 2             /* tensor-path logits only (f16 handles); AWB_WS_INFERENCE */
+#define AWB_FWD_TC_TRAINING 3    /* tensor-path training forward (f16 handles); AWB_WS_TRAINING */
+
 /* Number of trainable fp32 parameters per object, in state_dict order (SURVEY 8b). */
 int64_t awb_prior_param_count(awb_handle h);
-/* Bytes of scratch the caller must provide for n_pixels rows (all objects).  training: 0 forward only,
- * 1 forward + backward / any call, 2 awb_prior_fit_step only (much smaller on tensor-path handles, whose fused
- * kernel keeps the activations on the SM), 3 awb_prior_deformation / awb_prior_deformation_backward only (the flow's
- * buffers: deformed coordinates, coupling records, their gradient and the flow's partials; no ICNN activations, about
- * 80 MB instead of 0.85 GB for a 640x480 C = 2 frame), 4 awb_prior_forward(training = 1) followed by
- * awb_prior_backward and awb_prior_grid_grad_backward (layout 1 plus L + 1 tangent activation planes). */
-int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t training);
+/* Bytes of scratch the caller must provide for n_pixels rows (all objects) in workspace layout `layout` (AWB_WS_*);
+ * -1 for a null handle, n_pixels < 1 or an unknown layout. */
+int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t layout);
 /* Layout of the optimizer state: fp32 m[O][P], then fp32 v[O][P] (Adamax: the exp_inf u), then the per-object scalars at
  * byte offset round_up(8 * O * P, 256), read through awb_opt_read_scalars. */
 int64_t awb_opt_state_bytes(awb_handle h);
@@ -159,19 +174,18 @@ int awb_prior_set_flow_output_scale(awb_handle h, float scale);
 int awb_prior_set_flow_eval(awb_handle h, int32_t mode);
 
 /* forward(grid) -> raw logits [O][N]  (ConvexNextNet.forward convex_net.py:205-214;
- * PathConnectedNet.forward path_connected_net.py:79-85).  Leaves activations in the
- * workspace for awb_prior_backward when training != 0.  deformed (optional, [O][N][C])
- * receives get_deformation() (path_connected_net.py:125-129).
- * training: 0 inference (exact fp32), 1 exact fp32 forward that keeps its activations for awb_prior_backward,
- * 2 tensor-path logits only (f16 handles), 3 tensor-path training forward (f16 handles).  Tensor-path logits are computed
+ * PathConnectedNet.forward path_connected_net.py:79-85).  mode: AWB_FWD_*, each with the workspace layout named at
+ * its definition; an unknown mode is AWB_ERR_INVALID.  The training modes leave what awb_prior_backward needs in the
+ * workspace.  deformed (optional, [O][N][C]) receives get_deformation() (path_connected_net.py:125-129).
+ * The tensor-path modes need an f16 handle.  Their logits are computed
  * with fp16 operands (fp32 accumulation): |logit - exact| <= 3e-2 * max(1, |exact|) per pixel and <= 1e-3 normwise on the
  * weights of a finished 4000-step 640x480 fit (measured 2.2e-2 / 7.0e-4, 69 of 307200 mask pixels differ:
- * tests/test_gpu_full_schedule.py); masks / reported logits use mode 0.
- * Mode 3: logits from the tcgen05
+ * tests/test_gpu_full_schedule.py); masks / reported logits use AWB_FWD_EXACT.
+ * AWB_FWD_TC_TRAINING: logits from the tcgen05
  * kernel, nothing kept but the flow's deformed coordinates -- awb_prior_backward then re-runs the fused
  * forward+backward kernel with the upstream gradient (joint UNet + prior step, torch_agent.py:470-492). */
 int awb_prior_forward(awb_handle h, const float* params, const awb_grid_spec* grid, float* logits,
-                      float* deformed, int32_t training, void* workspace, size_t workspace_bytes,
+                      float* deformed, int32_t mode, void* workspace, size_t workspace_bytes,
                       void* stream);
 
 /* PathConnectedNet.inverse (path_connected_net.py:86-122): maps get_deformation() outputs back to grid coordinates
@@ -181,7 +195,7 @@ int awb_prior_flow_inverse(awb_handle h, const float* params, const awb_grid_spe
 
 /* autograd backward of forward(): dlogits [O][N] -> grads [O][P] (overwritten), optional
  * dgrid [B,C,H,W] = d loss / d grid (model_input_requires_grad configs, gradient penalties).  Must follow
- * awb_prior_forward(training=1, or 3 on f16 handles) on the same workspace.
+ * awb_prior_forward(AWB_FWD_EXACT_TRAINING, or AWB_FWD_TC_TRAINING on f16 handles) on the same workspace.
  * dgrid is provided for single-object AWB_KIND_ICNN, AWB_KIND_FLOW_ICNN (C = 2, 3) and AWB_KIND_DIFFEO_ICNN handles, at
  * both precisions and under every flow_eval mode; the flow backward forms it in its last pass over each pixel range
  * (linear^T times the gradient at the 1x1 conv / linear output), so requesting it leaves grads bit-identical.  Grouped
@@ -196,8 +210,8 @@ int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* g
  * logit along its u_n, and grads [P] (overwritten, state_dict order) = sum_n w_n d(J_n u_n) / d params; every bias
  * entry is exactly 0.  d R / d grid is 0: the ICNN is piecewise linear in its input.  Exact fp32 kernels at both
  * precisions; the masks, weights and activations are those of the training forward.
- * Must follow awb_prior_forward(training = 1) on the same workspace, of awb_prior_workspace_bytes(h, N, 4) bytes (the
- * training = 1 layout followed by L + 1 tangent activation planes).  The forward's activations are only read, so the
+ * Must follow awb_prior_forward(AWB_FWD_EXACT_TRAINING) on the same workspace, of layout AWB_WS_SECOND_ORDER (the
+ * AWB_WS_TRAINING layout followed by L + 1 tangent activation planes).  The forward's activations are only read, so the
  * call may be repeated; awb_prior_backward may run on the same workspace before or after it.  dlogits: the first
  * backward's [N]; params: those of the forward.  Single-object AWB_KIND_ICNN handles; any other handle:
  * AWB_ERR_UNSUPPORTED. */
@@ -206,15 +220,15 @@ int awb_prior_grid_grad_backward(awb_handle h, const float* params, const awb_gr
                                  size_t workspace_bytes, void* stream);
 
 /* get_deformation() alone (path_connected_net.py:125-129, convex_diffeomorphism_net.py:180-185): the 1x1 conv (linear)
- * and the flow, no ICNN.  deformed: device [N][C] pixel rows.  training = 1 keeps the coupling records in the workspace
- * for awb_prior_deformation_backward.  workspace: awb_prior_workspace_bytes(h, N, 3).
+ * and the flow, no ICNN.  deformed: device [N][C] pixel rows.  training != 0 keeps the coupling records in the workspace
+ * for awb_prior_deformation_backward.  workspace: layout AWB_WS_DEFORMATION.
  * Single-object AWB_KIND_FLOW_ICNN and AWB_KIND_DIFFEO_ICNN handles; an ICNN handle has no deformation (AWB_ERR_INVALID),
  * any other handle: AWB_ERR_UNSUPPORTED. */
 int awb_prior_deformation(awb_handle h, const float* params, const awb_grid_spec* grid, float* deformed, int32_t training,
                           void* workspace, size_t workspace_bytes, void* stream);
 /* Backward of awb_prior_deformation: d_deformed [N][C] (upstream gradient on the deformed coordinates) -> grads [P]
  * (overwritten, state_dict order: the flow and linear entries, every ICNN entry exactly 0) and optional dgrid [B,C,H,W].
- * Must follow awb_prior_deformation(training = 1) on the same workspace and params.  Same handles and errors. */
+ * Must follow awb_prior_deformation(training != 0) on the same workspace and params.  Same handles and errors. */
 int awb_prior_deformation_backward(awb_handle h, const float* params, const awb_grid_spec* grid, const float* d_deformed,
                                    float* grads, float* dgrid, void* workspace, size_t workspace_bytes, void* stream);
 
@@ -239,7 +253,7 @@ int64_t awb_prior_grad_row_floats(awb_handle h);
  * those pixels): forward, loss, backward, cross-CTA reduction; NO optimizer.  Coordinates (generated or read from an
  * explicit grid) are those of the global rows.  target: the FULL batch [N] (read at row_begin); loss: coefficients of the
  * FULL batch (1/N, class weights), so that rows add up to the step's gradient and loss.  workspace:
- * awb_prior_workspace_bytes(h, row_end - row_begin, 2).  flags: AWB_FIT_REUSE_PACKED -- the previous call on this
+ * layout AWB_WS_FIT_STEP for row_end - row_begin pixels.  flags: AWB_FIT_REUSE_PACKED -- the previous call on this
  * workspace was a slice of the same params with the same number of rows (tensor path: its fp16 weight image, whose place
  * in the workspace depends on the row count, is reused).  An empty or out-of-range
  * window: AWB_ERR_INVALID. */

@@ -398,7 +398,8 @@ def test_get_deformation_gradients_against_float64(A, case):
         arena = m._ensure_flat()
         prior = m._prior_for(arena.device)
         spec = A.GridSpecHost.from_tensor(x4)
-        _, d_fwd = prior.forward(arena, spec, False, prior.new_workspace(n, False, DEV), want_deformed=True)
+        ws = prior.new_workspace(n, A._lib.AWB_WS_INFERENCE, DEV)
+        _, d_fwd = prior.forward(arena, spec, A._lib.AWB_FWD_EXACT, ws, want_deformed=True)
     assert torch.equal(rows_of(d_ng), d_fwd[0])
     m.zero_grad()
     x = x4.clone().requires_grad_(True)
@@ -481,17 +482,17 @@ def test_c_abi_errors(A):
     grouped = A.Prior(L.AWB_KIND_FLOW_ICNN, 2, 130, 2, n_flows=4, flow_hidden=32, flow_tanh=True, n_objects=2)
     m._push_consts(grouped)
     params2 = torch.stack([m._ensure_flat().detach()] * 2).contiguous()
-    ws = grouped.new_workspace(N, True, DEV)
+    ws = grouped.new_workspace(N, L.AWB_WS_TRAINING, DEV)
     rc = lib.awb_prior_backward(grouped.handle, params2.data_ptr(), C.byref(gs), torch.zeros(2, N, device=DEV).data_ptr(),
                                 torch.empty_like(params2).data_ptr(), dgrid.data_ptr(), ws.data_ptr(), ws.numel(),
                                 L.stream_ptr())
     assert rc == -2
     assert b"grouped" in lib.awb_last_error()
-    assert deform_rcs(grouped, params2, grouped.new_workspace(N, 3, DEV)) == (-2, -2)
+    assert deform_rcs(grouped, params2, grouped.new_workspace(N, L.AWB_WS_DEFORMATION, DEV)) == (-2, -2)
     # an ICNN handle has no deformation
     icnn = A.Prior(L.AWB_KIND_ICNN, 2, 130, 2)
     p_icnn = torch.zeros(icnn.n_params, device=DEV)
-    assert deform_rcs(icnn, p_icnn, icnn.new_workspace(N, 3, DEV)) == (-1, -1)
+    assert deform_rcs(icnn, p_icnn, icnn.new_workspace(N, L.AWB_WS_DEFORMATION, DEV)) == (-1, -1)
     assert b"no deformation" in lib.awb_last_error()
     # the star prior: unsupported
     star = A.Prior(L.AWB_KIND_STAR, 2, 32, 0)
@@ -500,8 +501,8 @@ def test_c_abi_errors(A):
     # a workspace one byte short of the deformation layout
     single = m._prior_for(torch.device(DEV))
     arena = m._ensure_flat()
-    need = single.workspace_bytes(N, 3)
-    assert 0 < need < single.workspace_bytes(N, 2)          # the deformation layout carries no ICNN activations
+    need = single.workspace_bytes(N, L.AWB_WS_DEFORMATION)
+    assert 0 < need < single.workspace_bytes(N, L.AWB_WS_FIT_STEP)   # the deformation layout carries no ICNN activations
     assert deform_rcs(single, arena, torch.empty(need - 1, dtype=torch.uint8, device=DEV)) == (-4, -4)
     assert deform_rcs(single, arena, torch.empty(need, dtype=torch.uint8, device=DEV)) == (0, 0)
     torch.cuda.synchronize()

@@ -207,13 +207,13 @@ def test_c2_per_frame_cold_4000_then_warm_400(A, golden, precision):
         direct = _compare(f"c2 frame {k} {precision}", fg, ref_fg, un < 0.5, fr["iou_vs_unaries"])
         assert direct > 0.99
         if precision == "f16" and k == 0:
-            # The stated bound of the tensor-path logits (awb_prior_forward training = 2 / 3; include/awb.h): on the weights of
-            # a finished 4000-step fit at 640x480, against the exact fp32 forward of the same weights.
+            # The stated bound of the tensor-path logits (awb_prior_forward AWB_FWD_TC / _TC_TRAINING; include/awb.h): on
+            # the weights of a finished 4000-step fit at 640x480, against the exact fp32 forward of the same weights.
             prior = m._prior_for(torch.device(DEV))
             with torch.no_grad():
                 exact = m(x).reshape(-1)
-                ws = prior.new_workspace(spec.n_pixels, True, torch.device(DEV))
-                tp = prior.forward_tensor_path(m._ensure_flat(), spec, ws).reshape(-1)
+                ws = prior.new_workspace(spec.n_pixels, A._lib.AWB_WS_TRAINING, torch.device(DEV))
+                tp = prior.forward(m._ensure_flat(), spec, A._lib.AWB_FWD_TC, ws)[0].reshape(-1)
             per_px = float(((tp - exact).abs() / exact.abs().clamp(min=1.0)).max())
             normwise = float((tp - exact).norm() / exact.norm())
             flips = int(((tp < 0) != (exact < 0)).sum())

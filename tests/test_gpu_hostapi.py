@@ -427,7 +427,7 @@ def test_no_grad_forward_is_exact_fp32_on_cached_workspace(A):
     with torch.no_grad():
         y32, y16 = m32(x), m16(x)
         ws = m16._prior._ws_cache
-        assert len(ws) == 1 and list(ws.keys())[0][1] is False          # inference workspace, cached
+        assert len(ws) == 1 and list(ws.keys())[0][1] == A._lib.AWB_WS_INFERENCE   # inference workspace, cached
         y16b = m16(x)
         assert len(m16._prior._ws_cache) == 1
     assert torch.equal(y32, y16) and torch.equal(y16, y16b)               # bit-identical: same fp32 kernels
@@ -435,6 +435,14 @@ def test_no_grad_forward_is_exact_fp32_on_cached_workspace(A):
     y_train = m16(x)                                                     # grad enabled: tensor-path logits, differentiable
     assert y_train.requires_grad
     assert float((y_train - y32).abs().max()) < 2e-2
+    # a workspace layout or forward mode outside the named ones is refused, not mapped to a neighbouring one
+    L, prior = A._lib, m16._prior
+    for layout in (L.AWB_WS_INFERENCE - 1, L.AWB_WS_SECOND_ORDER + 1):
+        assert prior.lib.awb_prior_workspace_bytes(prior.handle, 40 * 56, layout) == -1
+    ws = prior.new_workspace(40 * 56, L.AWB_WS_SECOND_ORDER, DEV)
+    with pytest.raises(L.AwbError, match="unknown forward mode 4") as err:
+        prior.forward(m16._ensure_flat(), A.GridSpecHost("linspace", 1, 40, 56), L.AWB_FWD_TC_TRAINING + 1, ws)
+    assert err.value.code == -1                                          # AWB_ERR_INVALID
 
 
 def test_pixel_row_input_gradient_shape_and_values(A):

@@ -59,16 +59,16 @@ def test_generated_grids_equal_explicit(A, golden):
     m = model_from(A, g2["init"], 2)
     H, W = g2["H"], g2["W"]
     prior = m._prior_for(torch.device(DEV))
-    ws = prior.new_workspace(H * W, False, DEV)
-    y_gen, _ = prior.forward(m._ensure_flat(), A.GridSpecHost("linspace", 1, H, W), False, ws)
+    ws = prior.new_workspace(H * W, A._lib.AWB_WS_INFERENCE, DEV)
+    y_gen, _ = prior.forward(m._ensure_flat(), A.GridSpecHost("linspace", 1, H, W), A._lib.AWB_FWD_EXACT, ws)
     y_exp = m(g2["grid"].to(DEV)).reshape(1, -1)
     assert torch.equal(y_gen, y_exp), "in-kernel linspace grid differs from torch.linspace"
     g1 = golden("icnn_c1.pt")
     m1 = model_from(A, g1["init"], 1)
     H, W = g1["H"], g1["W"]
     prior = m1._prior_for(torch.device(DEV))
-    ws = prior.new_workspace(H * W, False, DEV)
-    y_gen, _ = prior.forward(m1._ensure_flat(), A.GridSpecHost("index", 1, H, W), False, ws)
+    ws = prior.new_workspace(H * W, A._lib.AWB_WS_INFERENCE, DEV)
+    y_gen, _ = prior.forward(m1._ensure_flat(), A.GridSpecHost("index", 1, H, W), A._lib.AWB_FWD_EXACT, ws)
     assert torch.equal(y_gen, m1(g1["grid"].to(DEV)).reshape(1, -1))
 
 

@@ -297,13 +297,14 @@ def split_params(flat, names, ref_grads):
     return out
 
 
-def run_kernels(A, case, prior, params, spec, target, training):
+def run_kernels(A, case, prior, params, spec, target, mode):
     """Logits, deformation, autograd gradients (``awb_prior_backward`` with dlogits of the same loss) and the loss and
     gradient of one fused step (Adam's first ``exp_avg`` is 0.1 g)."""
     N = spec.n_pixels
     Oo, P = params.shape
-    ws = prior.new_workspace(N, True, DEV)
-    logits, deformed = prior.forward(params, spec, training, ws, want_deformed=case["kind"] == "flow" and training == 1)
+    ws = prior.new_workspace(N, A._lib.AWB_WS_TRAINING, DEV)
+    want_deformed = case["kind"] == "flow" and mode == A._lib.AWB_FWD_EXACT_TRAINING
+    logits, deformed = prior.forward(params, spec, mode, ws, want_deformed=want_deformed)
     s = torch.sigmoid(logits.double())
     dlog = (2.0 * (s - target.double()) * s * (1 - s) / N).float().contiguous()
     g_ag, _ = prior.backward(params, spec, dlog, ws, False)
@@ -386,7 +387,7 @@ def test_exact_path_against_float64(A, case):
     prior, params = make_handle(A, case, models)
     spec = grid_spec(A, case)
     target = make_target(case)
-    logits, deformed, g_ag, loss, g_fs = run_kernels(A, case, prior, params, spec, target, 1)
+    logits, deformed, g_ag, loss, g_fs = run_kernels(A, case, prior, params, spec, target, A._lib.AWB_FWD_EXACT_TRAINING)
     rows = O.pixelize(torch_grid("linspace", case["B"], case["H"], case["W"], case["C"]))
     worst = dict(fwd=0.0, loss=0.0, grad=0.0, sens=float("inf"))
     for o, m in enumerate(models):
@@ -460,7 +461,7 @@ def test_tensor_path_against_float64(A, case):
     prior, params = make_handle(A, case, models)
     spec = grid_spec(A, case)
     target = make_target(case)
-    logits, _, g_ag, loss, g_fs = run_kernels(A, case, prior, params, spec, target, 3)
+    logits, _, g_ag, loss, g_fs = run_kernels(A, case, prior, params, spec, target, A._lib.AWB_FWD_TC_TRAINING)
     rows = O.pixelize(torch_grid("linspace", case["B"], case["H"], case["W"], case["C"]))
     for o, m in enumerate(models):
         ref = reference(m, case["kind"], rows, target[o], r["bwd.last"])
@@ -509,10 +510,10 @@ def test_generated_grid_equals_explicit_grid(A, kind, precision, C_, B, H, W):
     models = make_models(A, case, seed=5)
     prior, params = make_handle(A, case, models)
     target = make_target(case)
-    training = 3 if precision == "f16" else 1
+    fwd = A._lib.AWB_FWD_TC_TRAINING if precision == "f16" else A._lib.AWB_FWD_EXACT_TRAINING
     for mode in ("linspace", "index"):
-        gen = run_kernels(A, case, prior, params, grid_spec(A, case, mode), target, training)
-        exp = run_kernels(A, case, prior, params, A.GridSpecHost.from_tensor(torch_grid(mode, B, H, W, C_)), target, training)
+        gen = run_kernels(A, case, prior, params, grid_spec(A, case, mode), target, fwd)
+        exp = run_kernels(A, case, prior, params, A.GridSpecHost.from_tensor(torch_grid(mode, B, H, W, C_)), target, fwd)
         for name, a, b in zip(("logits", "deformation", "autograd gradients", "fused-step loss", "fused-step gradients"), gen, exp):
             if a is None:
                 continue
@@ -533,7 +534,7 @@ def test_slice_windows_generated_grid_equals_explicit_grid(A, kind, precision):
     prior, params = make_handle(A, case, models)
     target = make_target(case)
     spec_loss = A.LossConfig("mse").to_specs(target)[0]
-    ws = prior.new_workspace(max(e - b for b, e in SLICE_WINDOWS), 2, DEV)
+    ws = prior.new_workspace(max(e - b for b, e in SLICE_WINDOWS), A._lib.AWB_WS_FIT_STEP, DEV)
     for mode in ("linspace", "index"):
         rows = {}
         for key, spec in (("generated", grid_spec(A, case, mode)),
@@ -601,8 +602,9 @@ def test_tensor_path_tile_walk_equals_explicit_grid(A, C_, L, B, H, W, O_):
     models = make_models(A, case, seed=9)
     prior, params = make_handle(A, case, models)
     target = make_target(case)
-    gen = run_kernels(A, case, prior, params, grid_spec(A, case, "linspace"), target, 3)
-    exp = run_kernels(A, case, prior, params, A.GridSpecHost.from_tensor(torch_grid("linspace", B, H, W, C_)), target, 3)
+    fwd = A._lib.AWB_FWD_TC_TRAINING
+    gen = run_kernels(A, case, prior, params, grid_spec(A, case, "linspace"), target, fwd)
+    exp = run_kernels(A, case, prior, params, A.GridSpecHost.from_tensor(torch_grid("linspace", B, H, W, C_)), target, fwd)
     for name, a, b in zip(("logits", "deformation", "autograd gradients", "fused-step loss", "fused-step gradients"), gen, exp):
         if a is None:
             continue
@@ -627,7 +629,7 @@ def test_slice_window_tile_walk_equals_explicit_grid(A, C_):
     prior, params = make_handle(A, case, models)
     target = make_target(case)
     spec_loss = A.LossConfig("mse").to_specs(target)[0]
-    ws = prior.new_workspace(max(e - b for b, e in WALK_WINDOWS), 2, DEV)
+    ws = prior.new_workspace(max(e - b for b, e in WALK_WINDOWS), A._lib.AWB_WS_FIT_STEP, DEV)
     rows = {}
     for key, spec in (("generated", grid_spec(A, case, "linspace")),
                       ("explicit", A.GridSpecHost.from_tensor(torch_grid("linspace", B, H, W, C_)))):

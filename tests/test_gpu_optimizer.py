@@ -421,7 +421,7 @@ def test_fit_step_per_formula(A, case, opt):
     spec = A.GridSpecHost("linspace", 1, H, W, t0=0.1, t_step=0.2)
     target = torch.stack([_blob(H, W, o).reshape(-1) for o in range(O_)]).to(DEV).contiguous()
     st = _new_state(A, prior)
-    ws = prior.new_workspace(spec.n_pixels, 2, DEV)
+    ws = prior.new_workspace(spec.n_pixels, A._lib.AWB_WS_FIT_STEP, DEV)
     hy = _hyper(A, opt)
     for k in range(2):
         lr = _lrs(A, prior, st)
@@ -435,8 +435,8 @@ def test_fit_step_per_formula(A, case, opt):
             p0, m0 = before[0].double(), before[1].double()
             wd = torch.tensor(list(hy.weight_decay), dtype=torch.float64, device=DEV)[group.long()]
             g_k = (m0 + (after[1].double() - m0) / (1 - hy.beta1)) - wd * p0
-            wsb = prior.new_workspace(spec.n_pixels, True, DEV)
-            logits, _ = prior.forward(before[0], spec, 1, wsb)
+            wsb = prior.new_workspace(spec.n_pixels, A._lib.AWB_WS_TRAINING, DEV)
+            logits, _ = prior.forward(before[0], spec, A._lib.AWB_FWD_EXACT_TRAINING, wsb)
             s = torch.sigmoid(logits.double())
             dlog = (2.0 * (s - target.double()) * s * (1 - s) / spec.n_pixels).float().contiguous()
             g_b, _ = prior.backward(before[0], spec, dlog, wsb, False)
@@ -466,7 +466,7 @@ def test_flow_identity_then_fit_bias_corrects_each_group_from_its_own_step(A, pr
     spec = A.GridSpecHost("linspace", 1, H, W)
     target = _blob(H, W).reshape(1, -1).to(DEV).contiguous()
     st = _new_state(A, prior)
-    wsi = prior.new_workspace(spec.n_pixels, True, DEV)
+    wsi = prior.new_workspace(spec.n_pixels, A._lib.AWB_WS_TRAINING, DEV)
     hy = _hyper(A, "adamax")
     gs = spec.to_c()
     for _ in range(k):
@@ -482,14 +482,15 @@ def test_flow_identity_then_fit_bias_corrects_each_group_from_its_own_step(A, pr
     row = torch.empty(1, prior.grad_row_floats, device=DEV)
     prior.slice_grads(p_rows, spec, 0, spec.n_pixels, target.reshape(-1),
                       A._lib.LossSpec(A._lib.AWB_LOSS_SE_SIGMOID, A._lib.AWB_CLS_UNARY_LT_HALF, 1.0 / spec.n_pixels,
-                                      1.0 / spec.n_pixels), row[0], prior.new_workspace(spec.n_pixels, 2, DEV))
+                                      1.0 / spec.n_pixels), row[0],
+                      prior.new_workspace(spec.n_pixels, A._lib.AWB_WS_FIT_STEP, DEV))
     before = _snap(p_rows, prior, st_rows)
     prior.rows_opt_step(p_rows, st_rows, row, hy)
     torch.cuda.synchronize()
     check_step(hy, lr, own, before, _snap(p_rows, prior, st_rows), group, clamp, g=row[:, :-1].double(), what="rows")
     # fused fit step (k_reduce_opt_aug) on the original
     before = _snap(params, prior, st)
-    _fit_step(A, prior, params, st, spec, target, hy, prior.new_workspace(spec.n_pixels, 2, DEV))
+    _fit_step(A, prior, params, st, spec, target, hy, prior.new_workspace(spec.n_pixels, A._lib.AWB_WS_FIT_STEP, DEV))
     torch.cuda.synchronize()
     check_step(hy, lr, own, before, _snap(params, prior, st), group, clamp, what="fit_step")
 
@@ -568,7 +569,7 @@ def test_reused_weight_image_matches_a_fresh_pack(A, kind, L_, O_):
     gs = spec.to_c()
     p_a, st_a = params.clone(), _new_state(A, prior)
     p_b, st_b = params.clone(), st_a.clone()
-    ws_a, ws_b = prior.new_workspace(spec.n_pixels, 2, DEV), prior.new_workspace(spec.n_pixels, 2, DEV)
+    ws_a, ws_b = (prior.new_workspace(spec.n_pixels, L.AWB_WS_FIT_STEP, DEV) for _ in range(2))
     loss_a = torch.zeros(8, O_, device=DEV)
     loss_b = torch.zeros(8, O_, device=DEV)
     ptrs = (C.c_void_p * 3)(*[t.data_ptr() for t in targets])

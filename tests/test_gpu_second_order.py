@@ -293,10 +293,10 @@ def test_c_abi_errors(A):
     for precision in ("fp32", "f16"):
         prior = A.Prior(L.AWB_KIND_ICNN, 2, 130, 2, precision=L.AWB_PREC_FP32 if precision == "fp32" else L.AWB_PREC_F16)
         params = make(A, "icnn", 2, 130, 2, seed=8)._ensure_flat()
-        need = prior.workspace_bytes(N, 4)
-        assert need > prior.workspace_bytes(N, 1)
+        need = prior.workspace_bytes(N, L.AWB_WS_SECOND_ORDER)
+        assert need > prior.workspace_bytes(N, L.AWB_WS_TRAINING)
         ws = torch.empty(need, dtype=torch.uint8, device=DEV)
-        prior.forward(params, spec, 1, ws)
+        prior.forward(params, spec, L.AWB_FWD_EXACT_TRAINING, ws)
         assert rc(prior, params, torch.empty(need - 1, dtype=torch.uint8, device=DEV)) == -4
         assert rc(prior, params, ws) == 0
     torch.cuda.synchronize()

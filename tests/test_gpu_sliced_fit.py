@@ -56,7 +56,7 @@ def _target(B, H, W):
 
 def _rows(A, prior, params, grid, target, spec, windows):
     """Gradient rows of the given windows, one workspace reused window after window."""
-    ws = prior.new_workspace(max(e - b for b, e in windows), 2, DEV)
+    ws = prior.new_workspace(max(e - b for b, e in windows), A._lib.AWB_WS_FIT_STEP, DEV)
     rows = torch.empty((len(windows), prior.grad_row_floats), dtype=torch.float32, device=DEV)
     for k, (b, e) in enumerate(windows):
         prior.slice_grads(params, grid, b, e, target, spec, rows[k], ws)
@@ -84,8 +84,9 @@ def test_rows_add_up_to_the_full_batch_step(A, kind, C_, precision, mode):
     rows = _rows(A, prior, params, grid, target, spec, windows)
     total = rows.double().sum(0).cpu()
     # full-batch reference: forward (exact fp32, or the tensor path's training forward), dlogits in torch, backward
-    ws = prior.new_workspace(N, True, DEV)
-    logits, _ = prior.forward(params, grid, 3 if precision == "f16" else 1, ws)
+    ws = prior.new_workspace(N, A._lib.AWB_WS_TRAINING, DEV)
+    mode = A._lib.AWB_FWD_TC_TRAINING if precision == "f16" else A._lib.AWB_FWD_EXACT_TRAINING
+    logits, _ = prior.forward(params, grid, mode, ws)
     y = logits.detach().double()
     s = torch.sigmoid(y)
     t = target.double()
@@ -136,7 +137,7 @@ def _simulated_world(A, prior, params0, grid, target, spec, hyper, S, world, ste
         lrs = (C.c_double * 4)(*[2e-3] * 4)
         A._lib.check(prior.lib.awb_opt_state_init(prior.handle, st.data_ptr(), lrs, A._lib.stream_ptr()))
         states.append(st)
-    ws = prior.new_workspace(max(e - b for b, e in plan), 2, DEV)
+    ws = prior.new_workspace(max(e - b for b, e in plan), A._lib.AWB_WS_FIT_STEP, DEV)
     losses = [torch.empty(steps, device=DEV) for _ in range(world)]
     for s in range(steps):
         merged = []
@@ -234,7 +235,7 @@ def test_error_paths(A):
     target = _target(B, H, W)
     spec = A.LossConfig("mse").to_specs(target)[0]
     row = torch.zeros(prior.grad_row_floats, device=DEV)
-    ws = prior.new_workspace(N, 2, DEV)
+    ws = prior.new_workspace(N, L.AWB_WS_FIT_STEP, DEV)
     assert prior.grad_row_floats == prior.n_params + 1
     assert _status(A, prior, params, grid, 0, N, target, spec, row, ws) == 0
     assert _status(A, prior, params, grid, 0, N + 1, target, spec, row, ws) == -1           # past the batch
@@ -243,18 +244,18 @@ def test_error_paths(A):
     assert _status(A, prior, params, grid, 9, 3, target, spec, row, ws) == -1               # reversed
     assert _status(A, prior, params, grid, 0, -1, target, spec, row, ws) == -1              # negative end
     assert _status(A, prior, params, grid, -64, -1, target, spec, row, ws) == -1            # entirely before the batch
-    small = prior.workspace_bytes(128, 2)
+    small = prior.workspace_bytes(128, L.AWB_WS_FIT_STEP)
     assert _status(A, prior, params, grid, 0, N, target, spec, row, ws, nbytes=small) == -4  # short workspace
     assert _status(A, prior, params, grid, 0, 128, target, spec, row, ws, nbytes=small) == 0  # ... enough for its window
     # several objects, NormalizingFlow1D: unsupported
     multi = A.Prior(L.AWB_KIND_ICNN, 2, 130, 2, n_objects=2)
     pm = torch.zeros(2 * multi.n_params, device=DEV)
     assert _status(A, multi, pm, grid, 0, N, target, spec, torch.zeros(multi.n_params + 1, device=DEV),
-                   multi.new_workspace(N, 2, DEV)) == -2
+                   multi.new_workspace(N, L.AWB_WS_FIT_STEP, DEV)) == -2
     diffeo = A.Prior(L.AWB_KIND_DIFFEO_ICNN, 2, 130, 2, n_flows=2, flow_hidden=16)
     pd = torch.zeros(diffeo.n_params, device=DEV)
     assert _status(A, diffeo, pd, grid, 0, N, target, spec, torch.zeros(diffeo.n_params + 1, device=DEV),
-                   diffeo.new_workspace(N, 2, DEV)) == -2
+                   diffeo.new_workspace(N, L.AWB_WS_FIT_STEP, DEV)) == -2
     st = torch.empty(diffeo.opt_state_bytes(), dtype=torch.uint8, device=DEV)
     rows = torch.zeros((2, diffeo.n_params + 1), device=DEV)
     assert diffeo.lib.awb_prior_rows_opt_step(diffeo.handle, pd.data_ptr(), st.data_ptr(), rows.data_ptr(), 2,

@@ -100,8 +100,8 @@ def test_tensor_forward_logits(A):
     m16.load_state_dict(m32.state_dict())
     m16.to(DEV)
     prior = m16._prior_for(torch.device(DEV))
-    ws = prior.new_workspace(H * W, False, DEV)
-    y16 = prior.forward_tensor_path(m16._ensure_flat(), grid, ws).reshape(-1)
+    ws = prior.new_workspace(H * W, A._lib.AWB_WS_INFERENCE, DEV)
+    y16 = prior.forward(m16._ensure_flat(), grid, A._lib.AWB_FWD_TC, ws)[0].reshape(-1)
     y32 = m32(grid.materialize(2, DEV)).reshape(-1)
     assert float((y16 - y32).norm() / y32.norm()) < 1e-3
     per_px = ((y16 - y32).abs() / y32.abs().clamp(min=1.0)).max()

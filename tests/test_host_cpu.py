@@ -28,6 +28,19 @@ def test_header_symbols_exported():
     assert b"sm_100a" in lib.awb_version()
 
 
+def test_header_constants_match_binding():
+    from awesome_b200 import _lib
+    header = open(os.path.join(ROOT, "include", "awb.h")).read()
+    defined = {name: int(value) for name, value in
+               re.findall(r"^#define\s+(AWB_[A-Z0-9_]+)\s+\(?(-?\d+)\)?(?:\s|$)", header, re.M)}
+    assert {"AWB_WS_INFERENCE", "AWB_WS_SECOND_ORDER", "AWB_FWD_EXACT", "AWB_FWD_TC_TRAINING"} <= set(defined)
+    for name, value in defined.items():
+        if name.startswith(("AWB_WS_", "AWB_FWD_")):
+            assert hasattr(_lib, name), f"{name} is not mirrored in _lib.py"
+        if hasattr(_lib, name):
+            assert getattr(_lib, name) == value, f"{name}: header {value}, _lib.py {getattr(_lib, name)}"
+
+
 def test_state_dict_contract_matches_reference_fixture(golden):
     import awesome_b200 as A
     g = golden("icnn_c1.pt")

@@ -63,10 +63,10 @@ class _Float64Prior:
         g = spec.grid.double()
         return g.permute(0, 2, 3, 1).reshape(-1, g.shape[1]).clone().requires_grad_(True)
 
-    def new_workspace(self, n_pixels, training, device):
-        return {"training": training}
+    def new_workspace(self, n_pixels, layout, device):
+        return {"layout": layout}
 
-    def forward(self, arena, spec, training, ws, want_deformed=False):
+    def forward(self, arena, spec, mode, ws, want_deformed=False):
         with torch.no_grad():
             y = O.icnn_forward(self._params(arena), self._rows(spec)).reshape(1, -1)
         return y.float(), None
@@ -81,7 +81,8 @@ class _Float64Prior:
 
     @torch.enable_grad()
     def grid_grad_backward(self, arena, spec, w, u, ws):
-        assert ws["training"] == 4 and u.is_contiguous() and u.shape == (spec.B, len(spec.grid[0]), spec.H, spec.W)
+        assert ws["layout"] == A._lib.AWB_WS_SECOND_ORDER
+        assert u.is_contiguous() and u.shape == (spec.B, len(spec.grid[0]), spec.H, spec.W)
         p, x = self._params(arena), self._rows(spec)
         y = O.icnn_forward(p, x)
         J = torch.autograd.grad(y.sum(), x, create_graph=True)[0]
