@@ -103,6 +103,8 @@ SYMBOLS = [
     ("awb_star_workspace_bytes", C.c_int64, [_P, C.c_int64]),
     ("awb_star_fit_step", C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.POINTER(LossSpec), C.POINTER(OptHyper), _P, _P,
                                     C.c_size_t, _P]),
+    ("awb_star_backward_workspace_bytes", C.c_int64, [_P, C.c_int64]),
+    ("awb_star_backward", C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_size_t, _P]),
     ("awb_opt_set_lr", C.c_int, [_P, _P, C.POINTER(C.c_double), _P]),
     ("awb_opt_plateau_step", C.c_int, [_P, _P, _P, C.c_int32, C.POINTER(OptHyper), _P]),
     ("awb_opt_read_scalars", C.c_int, [_P, _P, C.c_int32, C.POINTER(OptScalars), _P]),

@@ -641,6 +641,20 @@ int awb_star_fit_step(awb_handle h, float* params, void* opt_state, const float*
   return reduce_opt_plain(h, params, opt_state, hy, loss_out, part, nc, h->lay.P, lossp, 1, st);
 }
 
+int64_t awb_star_backward_workspace_bytes(awb_handle h, int64_t n) {
+  if (!h || n < 1 || h->desc.kind != AWB_KIND_STAR) return -1;
+  return round_up(4 * (int64_t)star_bwd_ctas(n, nullptr) * h->lay.P, 256);
+}
+
+int awb_star_backward(awb_handle h, const float* params, const float* x, int64_t n, const float* dlogits, float* grads,
+                      float* dx, void* ws, size_t ws_bytes, void* stream) {
+  if (!h || !params || !x || !dlogits || !grads || !ws || n < 1) { set_error("bad argument"); return AWB_ERR_INVALID; }
+  if (h->desc.kind != AWB_KIND_STAR) { set_error("not a star prior"); return AWB_ERR_INVALID; }
+  const int64_t need = awb_star_backward_workspace_bytes(h, n);
+  if ((int64_t)ws_bytes < need) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)need); return AWB_ERR_WORKSPACE; }
+  return star_backward(h, params, x, dlogits, n, grads, dx, (float*)ws, (cudaStream_t)stream);
+}
+
 int awb_opt_set_lr(awb_handle h, void* opt_state, const double* lr, void* stream) {
   if (!h || !opt_state || !lr) { set_error("null argument"); return AWB_ERR_INVALID; }
   return opt_set_lr(h, opt_state, lr, (cudaStream_t)stream);

@@ -127,7 +127,7 @@ Workspace carve(const awb_prior* h, int64_t N, int layout, void* base);
 
 // ---- per-kernel-class timing (CUDA events on the launch stream) and launch counting ----
 enum { PK_PACK = 0, PK_INPUT, PK_GEMM_FWD, PK_OUT_LOSS, PK_GEMM_WGRAD, PK_GEMM_DGRAD, PK_IN_BWD, PK_OPT,
-       PK_FLOW_FWD, PK_FLOW_BWD, PK_TC_FUSED, PK_MISC, PK_TAN_FWD, PK_TAN_OUT, PK_COUNT };
+       PK_FLOW_FWD, PK_FLOW_BWD, PK_TC_FUSED, PK_MISC, PK_TAN_FWD, PK_TAN_OUT, PK_STAR_BWD, PK_COUNT };
 void prof_begin(int cls, cudaStream_t st);
 void prof_end(int cls, cudaStream_t st);
 #define AWB_LAUNCH(cls, st, ...)  \
@@ -195,10 +195,18 @@ int plateau_step(const awb_prior* h, void* opt_state, const float* loss, int str
 int reduce_opt_plain(const awb_prior* h, float* params, void* opt_state, const awb_opt_hyper* hy, float* loss_out,
                      const float* partials, int S, int64_t part_stride, const float* lossp, int64_t loss_stride,
                      cudaStream_t st);
+// grads[P] = sum of S plain (state_dict order) gradient partials, partial s at partials + s * part_stride, in partial order
+// (k_reduce_grads, single object)
+int reduce_grads_plain(const awb_prior* h, float* grads, const float* partials, int S, int64_t part_stride, cudaStream_t st);
 // ---- star-shape prior, implemented in awb_star.cu
 int star_n_ctas(int64_t n);
 int star_run(const awb_prior* h, const float* params, const float* x, const float* target, int64_t n,
              const awb_loss_spec* loss, float* logits, float* part, float* lossp, bool fit, int* n_ctas, cudaStream_t st);
+// backward of the star forward for the upstream gradient dy [n]: grads [P] (overwritten), dx [n][2] (optional); part:
+// star_bwd_ctas(n) partials of P floats.  *chunk (optional): points per CTA.
+int star_bwd_ctas(int64_t n, int64_t* chunk);
+int star_backward(const awb_prior* h, const float* params, const float* x, const float* dy, int64_t n, float* grads,
+                  float* dx, float* part, cudaStream_t st);
 int opt_state_init(const awb_prior* h, void* opt_state, const double* lr, cudaStream_t st);
 int opt_set_lr(const awb_prior* h, void* opt_state, const double* lr, cudaStream_t st);
 

@@ -1194,6 +1194,15 @@ int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int
   return AWB_OK;
 }
 
+int reduce_grads_plain(const awb_prior* h, float* grads, const float* partials, int S, int64_t part_stride, cudaStream_t st) {
+  const int64_t P = h->lay.P;   // no augmented ICNN partials: every entry is read from the plain partials
+  AWB_LAUNCH(PK_OPT, st, AWB_CUDA(launch_ex(k_reduce_grads, dim3((unsigned)((P + 255) / 256), 1), dim3(256), 0, st, true,
+      grads, (const float*)nullptr, (int64_t)0, 0, S, partials, part_stride, (const int32_t*)nullptr, P, (int64_t)0,
+      (int64_t)0, (int64_t)0, P, (int64_t)0, (const float*)nullptr, (float*)nullptr)));
+  AWB_CUDA(cudaGetLastError());
+  return AWB_OK;
+}
+
 int simt_seed_dX(const awb_prior* h, const float* d_deformed, const Workspace& ws, cudaStream_t st) {
   AWB_LAUNCH(PK_MISC, st, k_seed_dX<<<(unsigned)((ws.N + 255) / 256), 256, 0, st>>>(d_deformed, ws.dX, ws.N, h->lay.C));
   AWB_CUDA(cudaGetLastError());

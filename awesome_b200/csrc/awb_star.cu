@@ -170,4 +170,306 @@ int star_run(const awb_prior* h, const float* params, const float* x, const floa
   return AWB_OK;
 }
 
+// ---- backward for an upstream gradient per point (awb_star_backward): the autograd path of StarShapedNet.
+// k_star walks its points one at a time with block barriers in between, which is fine for the notebook's 1000 samples
+// but serial at a full frame (307 200 points = ~2000 points per CTA).  k_star_bwd works on a tile of kStarT points per
+// iteration instead.  Each warp owns kStarTM points of the tile and each lane the hidden units l + 32 u (u < NU), so
+//   bpre = W1 a + W1_r r + b1 + b1_r   and   da = W1^T db + dyr w2
+// are register-blocked [kStarTM x NU] products over W1 in shared memory, and the tile's a and db (shared memory, [T][HP])
+// feed dW1 += db^T a once per tile, a [HP x T] x [T x HP] contraction whose accumulator stays in registers for the whole
+// CTA (thread (jt, kt) owns dW1[jt + 16 a][kt + 16 b]).  Every product is fp32 FMA in k_star's order of operations; the
+// sums over points run in point order within the CTA and per-CTA partials are reduced in CTA order (no atomics).
+constexpr int kStarT = 64;                       // points per tile
+constexpr int kStarWarps = 8;                    // 256 threads
+constexpr int kStarTM = kStarT / kStarWarps;     // points per warp in the two W1 products
+enum { SP_W0X = 0, SP_W0Y, SP_B0, SP_W1R, SP_B1, SP_W2, SP_W2R, SP_N };           // per-unit parameters (sPar rows)
+enum { SG_W0X = 0, SG_W0Y, SG_B0, SG_B1, SG_W1R, SG_W2, SG_W2R, SG_N };           // per-unit gradient sums (sAcc rows)
+enum { PT_PX = 0, PT_PY, PT_R, PT_Q, PT_UX, PT_UY, PT_DY, PT_DYR, PT_N };         // per-point values (sPt rows)
+
+struct StarBwdP {
+  const float* params; int64_t P; int h;
+  const float* x;        // [n][2]
+  const float* dy;       // [n]
+  int64_t n, chunk;      // chunk: points per CTA, a multiple of kStarT
+  float* part;           // [S][P]
+  float* dx;             // [n][2] or null
+};
+
+template <int NU>
+constexpr size_t star_bwd_smem() {
+  return sizeof(float) * ((size_t)32 * NU * (32 * NU + 4) + 2 * kStarT * 32 * NU + (size_t)(kStarWarps * SG_N + SP_N) * 32 * NU +
+                          PT_N * kStarT);
+}
+
+__device__ __forceinline__ float warp_sum(float v) {
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+  return v;
+}
+
+template <int NU>
+__global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
+  constexpr int HP = 32 * NU, LDW = HP + 4, T = kStarT, TM = kStarTM;
+  extern __shared__ __align__(16) float sm[];
+  float* sW1 = sm;                          // [HP][LDW] W1, zero outside [h][h]
+  float* sA = sW1 + HP * LDW;               // [T][HP] a of the tile's points (0 for units >= h)
+  float* sDB = sA + T * HP;                 // [T][HP] db
+  float* sAcc = sDB + T * HP;               // [warp][SG_N][HP] per-unit gradient sums over each warp's points
+  float* sPar = sAcc + kStarWarps * SG_N * HP;   // [SP_N][HP], zero for units >= h
+  float* sPt = sPar + SP_N * HP;            // [PT_N][T]
+  __shared__ float red[kStarWarps][3];
+  const int tid = threadIdx.x, w = tid >> 5, l = tid & 31, h = p.h;
+  const float* par = p.params;
+  const int o_W0 = 2, o_b0 = 2 + 2 * h, o_W1 = 2 + 3 * h, o_b1 = o_W1 + h * h, o_W2 = o_b1 + h, o_b2 = o_W2 + h,
+            o_W1r = o_b2 + 1, o_b1r = o_W1r + h, o_W2r = o_b1r + h, o_b2r = o_W2r + h;
+  for (int i = tid; i < HP * LDW; i += blockDim.x) {
+    const int j = i / LDW, k = i - j * LDW;
+    sW1[i] = (j < h && k < h) ? par[o_W1 + j * h + k] : 0.f;
+  }
+  for (int i = tid; i < kStarWarps * SG_N * HP; i += blockDim.x) sAcc[i] = 0.f;
+  for (int j = tid; j < HP; j += blockDim.x) {
+    const bool in = j < h;
+    sPar[SP_W0X * HP + j] = in ? par[o_W0 + 2 * j] : 0.f;
+    sPar[SP_W0Y * HP + j] = in ? par[o_W0 + 2 * j + 1] : 0.f;
+    sPar[SP_B0 * HP + j] = in ? par[o_b0 + j] : 0.f;
+    sPar[SP_W1R * HP + j] = in ? par[o_W1r + j] : 0.f;
+    sPar[SP_B1 * HP + j] = in ? par[o_b1 + j] + par[o_b1r + j] : 0.f;
+    sPar[SP_W2 * HP + j] = in ? par[o_W2 + j] : 0.f;
+    sPar[SP_W2R * HP + j] = in ? par[o_W2r + j] : 0.f;
+  }
+  const float off0 = par[0], off1 = par[1], bias2 = par[o_b2] + par[o_b2r];
+  const int Kp = (h + 3) & ~3;              // W1 products run over round_up(h, 4): the padding adds exact zeros
+  const int jt = tid >> 4, kt = tid & 15;
+  float dW[2 * NU][2 * NU];
+#pragma unroll
+  for (int a = 0; a < 2 * NU; a++)
+#pragma unroll
+    for (int b = 0; b < 2 * NU; b++) dW[a][b] = 0.f;
+  float g_ox = 0.f, g_oy = 0.f, g_b2 = 0.f;   // lanes < TM: sums over the points they finish
+  __syncthreads();
+  const int64_t c0 = (int64_t)blockIdx.x * p.chunk, c1 = c0 + p.chunk < p.n ? c0 + p.chunk : p.n;
+  for (int64_t t0 = c0; t0 < c1; t0 += T) {
+    // remainder tile: only the last tile of the last CTA has nv < T (n % kStarT != 0); its padding points sit at r = 0
+    // with dy = 0 and add exact zeros to every sum
+    const int nv = (int)(c1 - t0 < T ? c1 - t0 : T);
+    if (tid < T) {
+      float px = 0.f, py = 0.f, dy = 0.f;
+      if (tid < nv) {
+        const int64_t n = t0 + tid;
+        px = p.x[2 * n] + off0; py = p.x[2 * n + 1] + off1; dy = p.dy[n];
+      }
+      const float r = sqrtf(px * px + py * py), q = 0.01f + r;
+      sPt[PT_PX * T + tid] = px; sPt[PT_PY * T + tid] = py; sPt[PT_R * T + tid] = r; sPt[PT_Q * T + tid] = q;
+      sPt[PT_UX * T + tid] = px / q; sPt[PT_UY * T + tid] = py / q; sPt[PT_DY * T + tid] = dy; sPt[PT_DYR * T + tid] = dy * r;
+    }
+    __syncthreads();
+    // a = relu(W0 u + b0) of the warp's points
+#pragma unroll
+    for (int i = 0; i < TM; i++) {
+      const int t = w * TM + i;
+      const float ux = sPt[PT_UX * T + t], uy = sPt[PT_UY * T + t];
+#pragma unroll
+      for (int u = 0; u < NU; u++) {
+        const int j = l + 32 * u;
+        const float apre = fmaf(sPar[SP_W0X * HP + j], ux, fmaf(sPar[SP_W0Y * HP + j], uy, sPar[SP_B0 * HP + j]));
+        sA[t * HP + j] = fmaxf(apre, 0.f);
+      }
+    }
+    __syncwarp();
+    // bpre = W1_r r + b1 + b1_r + W1 a
+    float acc[TM][NU];
+#pragma unroll
+    for (int i = 0; i < TM; i++)
+#pragma unroll
+      for (int u = 0; u < NU; u++)
+        acc[i][u] = fmaf(sPar[SP_W1R * HP + l + 32 * u], sPt[PT_R * T + w * TM + i], sPar[SP_B1 * HP + l + 32 * u]);
+    for (int k = 0; k < Kp; k += 4) {
+      float4 wv[NU];
+#pragma unroll
+      for (int u = 0; u < NU; u++) wv[u] = *reinterpret_cast<const float4*>(sW1 + (l + 32 * u) * LDW + k);
+#pragma unroll
+      for (int i = 0; i < TM; i++) {
+        const float4 a4 = *reinterpret_cast<const float4*>(sA + (w * TM + i) * HP + k);
+#pragma unroll
+        for (int u = 0; u < NU; u++) {
+          acc[i][u] = fmaf(wv[u].x, a4.x, acc[i][u]); acc[i][u] = fmaf(wv[u].y, a4.y, acc[i][u]);
+          acc[i][u] = fmaf(wv[u].z, a4.z, acc[i][u]); acc[i][u] = fmaf(wv[u].w, a4.w, acc[i][u]);
+        }
+      }
+    }
+    // b, db; s and drb = sum_j db_j w1r_j per point; the per-unit sums of dyr a, dyr b, db, db r
+    float s[TM], drb[TM];
+#pragma unroll
+    for (int i = 0; i < TM; i++) { s[i] = 0.f; drb[i] = 0.f; }
+#pragma unroll
+    for (int u = 0; u < NU; u++) {
+      const int j = l + 32 * u;
+      const float w2 = sPar[SP_W2 * HP + j], w2r = sPar[SP_W2R * HP + j], w1r = sPar[SP_W1R * HP + j];
+      float* ga = sAcc + w * SG_N * HP + j;
+      float g_w2 = ga[SG_W2 * HP], g_w2r = ga[SG_W2R * HP], g_b1 = ga[SG_B1 * HP], g_w1r = ga[SG_W1R * HP];
+#pragma unroll
+      for (int i = 0; i < TM; i++) {
+        const int t = w * TM + i;
+        const float a = sA[t * HP + j], b = fmaxf(acc[i][u], 0.f);
+        const float dyr = sPt[PT_DYR * T + t], r = sPt[PT_R * T + t];
+        s[i] += fmaf(w2, a, w2r * b);
+        const float db = acc[i][u] > 0.f ? dyr * w2r : 0.f;
+        sDB[t * HP + j] = db;
+        drb[i] = fmaf(db, w1r, drb[i]);
+        g_w2 = fmaf(dyr, a, g_w2); g_w2r = fmaf(dyr, b, g_w2r);
+        g_b1 += db; g_w1r = fmaf(db, r, g_w1r);
+      }
+      ga[SG_W2 * HP] = g_w2; ga[SG_W2R * HP] = g_w2r; ga[SG_B1 * HP] = g_b1; ga[SG_W1R * HP] = g_w1r;
+    }
+    float s_me = 0.f, drb_me = 0.f;   // lane i < TM keeps point w * TM + i
+#pragma unroll
+    for (int i = 0; i < TM; i++) {
+      const float si = warp_sum(s[i]), di = warp_sum(drb[i]);
+      if (l == i) { s_me = si; drb_me = di; }
+    }
+    __syncwarp();
+    // da = dyr w2 + W1^T db; dapre; the per-unit sums of dapre ux, dapre uy, dapre; du = W0^T dapre per point
+#pragma unroll
+    for (int i = 0; i < TM; i++)
+#pragma unroll
+      for (int u = 0; u < NU; u++) acc[i][u] = sPt[PT_DYR * T + w * TM + i] * sPar[SP_W2 * HP + l + 32 * u];
+    for (int j = 0; j < Kp; j += 4) {
+      float wv[4][NU];
+#pragma unroll
+      for (int c = 0; c < 4; c++)
+#pragma unroll
+        for (int u = 0; u < NU; u++) wv[c][u] = sW1[(j + c) * LDW + l + 32 * u];
+#pragma unroll
+      for (int i = 0; i < TM; i++) {
+        const float4 d4 = *reinterpret_cast<const float4*>(sDB + (w * TM + i) * HP + j);
+#pragma unroll
+        for (int u = 0; u < NU; u++) {
+          acc[i][u] = fmaf(d4.x, wv[0][u], acc[i][u]); acc[i][u] = fmaf(d4.y, wv[1][u], acc[i][u]);
+          acc[i][u] = fmaf(d4.z, wv[2][u], acc[i][u]); acc[i][u] = fmaf(d4.w, wv[3][u], acc[i][u]);
+        }
+      }
+    }
+    float dux[TM], duy[TM];
+#pragma unroll
+    for (int i = 0; i < TM; i++) { dux[i] = 0.f; duy[i] = 0.f; }
+#pragma unroll
+    for (int u = 0; u < NU; u++) {
+      const int k = l + 32 * u;
+      const float w0x = sPar[SP_W0X * HP + k], w0y = sPar[SP_W0Y * HP + k];
+      float* ga = sAcc + w * SG_N * HP + k;
+      float g_w0x = ga[SG_W0X * HP], g_w0y = ga[SG_W0Y * HP], g_b0 = ga[SG_B0 * HP];
+#pragma unroll
+      for (int i = 0; i < TM; i++) {
+        const int t = w * TM + i;
+        const float dapre = sA[t * HP + k] > 0.f ? acc[i][u] : 0.f;   // a > 0 exactly where its pre-activation is
+        g_w0x = fmaf(dapre, sPt[PT_UX * T + t], g_w0x); g_w0y = fmaf(dapre, sPt[PT_UY * T + t], g_w0y); g_b0 += dapre;
+        dux[i] = fmaf(dapre, w0x, dux[i]); duy[i] = fmaf(dapre, w0y, duy[i]);
+      }
+      ga[SG_W0X * HP] = g_w0x; ga[SG_W0Y * HP] = g_w0y; ga[SG_B0 * HP] = g_b0;
+    }
+    float dux_me = 0.f, duy_me = 0.f;
+#pragma unroll
+    for (int i = 0; i < TM; i++) {
+      const float xi = warp_sum(dux[i]), yi = warp_sum(duy[i]);
+      if (l == i) { dux_me = xi; duy_me = yi; }
+    }
+    // the point gradient, written once by the lane that finishes the point; the offset's gradient is its sum
+    if (l < TM && w * TM + l < nv) {
+      const int t = w * TM + l;
+      const float px = sPt[PT_PX * T + t], py = sPt[PT_PY * T + t], r = sPt[PT_R * T + t], q = sPt[PT_Q * T + t];
+      const float dy = sPt[PT_DY * T + t];
+      g_b2 += sPt[PT_DYR * T + t];
+      // r = 0 (the point at -offset): no contribution through r, as in k_star; the u path (du/dx = I / 0.01) is kept
+      float gx = dux_me / q, gy = duy_me / q;
+      if (r > 0.f) {
+        const float dr = fmaf(dy, s_me + bias2, drb_me) - (dux_me * px + duy_me * py) / (q * q);
+        gx = dux_me / q + dr * (px / r);
+        gy = duy_me / q + dr * (py / r);
+      }
+      g_ox += gx; g_oy += gy;
+      if (p.dx) { const int64_t n = t0 + t; p.dx[2 * n] = gx; p.dx[2 * n + 1] = gy; }
+    }
+    __syncthreads();
+    // dW1 += db^T a over the tile's points, in point order
+    for (int t = 0; t < nv; t++) {
+      float dbv[2 * NU], av[2 * NU];
+#pragma unroll
+      for (int a = 0; a < 2 * NU; a++) { dbv[a] = sDB[t * HP + jt + 16 * a]; av[a] = sA[t * HP + kt + 16 * a]; }
+#pragma unroll
+      for (int a = 0; a < 2 * NU; a++)
+#pragma unroll
+        for (int b = 0; b < 2 * NU; b++) dW[a][b] = fmaf(dbv[a], av[b], dW[a][b]);
+    }
+    __syncthreads();     // the next tile rewrites sPt, sA and sDB
+  }
+  // this CTA's partial, state_dict order; every sum over warps or lanes in a fixed order
+  float* out = p.part + (int64_t)blockIdx.x * p.P;
+  for (int j = tid; j < h; j += blockDim.x) {
+    float g[SG_N];
+#pragma unroll
+    for (int q = 0; q < SG_N; q++) {
+      g[q] = 0.f;
+      for (int v = 0; v < kStarWarps; v++) g[q] += sAcc[(v * SG_N + q) * HP + j];
+    }
+    out[o_W0 + 2 * j] = g[SG_W0X]; out[o_W0 + 2 * j + 1] = g[SG_W0Y]; out[o_b0 + j] = g[SG_B0];
+    out[o_b1 + j] = g[SG_B1]; out[o_b1r + j] = g[SG_B1]; out[o_W1r + j] = g[SG_W1R];
+    out[o_W2 + j] = g[SG_W2]; out[o_W2r + j] = g[SG_W2R];
+  }
+#pragma unroll
+  for (int a = 0; a < 2 * NU; a++)
+#pragma unroll
+    for (int b = 0; b < 2 * NU; b++) {
+      const int j = jt + 16 * a, k = kt + 16 * b;
+      if (j < h && k < h) out[o_W1 + j * h + k] = dW[a][b];
+    }
+  g_ox = warp_sum(g_ox); g_oy = warp_sum(g_oy); g_b2 = warp_sum(g_b2);
+  if (l == 0) { red[w][0] = g_ox; red[w][1] = g_oy; red[w][2] = g_b2; }
+  __syncthreads();
+  if (tid == 0) {
+    float ox = 0.f, oy = 0.f, b2 = 0.f;
+    for (int v = 0; v < kStarWarps; v++) { ox += red[v][0]; oy += red[v][1]; b2 += red[v][2]; }
+    out[0] = ox; out[1] = oy; out[o_b2] = b2; out[o_b2r] = b2;
+  }
+}
+
+// Launch geometry of k_star_bwd.  Size-dependent branches (tests/test_gpu_star_autograd.py covers both sides of each):
+//  - tiles per CTA: ceil(n / kStarT) tiles are dealt to at most kMaxSplits CTAs in runs of ceil(tiles / kMaxSplits):
+//    one tile per CTA while n <= kMaxSplits * kStarT = 9472, several above;
+//  - CTA count S = ceil(tiles / tiles per CTA) (<= kMaxSplits; no CTA is empty);
+//  - remainder tile: n % kStarT != 0 leaves the last tile of the last CTA partial.
+int star_bwd_ctas(int64_t n, int64_t* chunk) {
+  const int64_t tiles = (n + kStarT - 1) / kStarT, per = (tiles + kMaxSplits - 1) / kMaxSplits;
+  if (chunk) *chunk = per * kStarT;
+  return (int)((tiles + per - 1) / per);
+}
+
+template <int NU>
+static int star_bwd_launch(const StarBwdP& p, int S, cudaStream_t st) {
+  constexpr size_t smem = star_bwd_smem<NU>();
+  static_assert(smem <= 227 * 1024, "k_star_bwd shared memory");
+  AWB_CUDA(cudaFuncSetAttribute(k_star_bwd<NU>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  AWB_LAUNCH(PK_STAR_BWD, st, k_star_bwd<NU><<<S, kStarWarps * 32, smem, st>>>(p));
+  AWB_CUDA(cudaGetLastError());
+  return AWB_OK;
+}
+
+int star_backward(const awb_prior* h, const float* params, const float* x, const float* dy, int64_t n, float* grads,
+                  float* dx, float* part, cudaStream_t st) {
+  const int hh = h->lay.h;
+  if (hh > 160) { set_error("star prior supports n_hidden <= 160, got %d", hh); return AWB_ERR_UNSUPPORTED; }
+  StarBwdP p = {};
+  p.params = params; p.P = h->lay.P; p.h = hh; p.x = x; p.dy = dy; p.n = n; p.part = part; p.dx = dx;
+  const int S = star_bwd_ctas(n, &p.chunk);
+  int rc;
+  switch ((hh + 31) / 32) {
+    case 1: rc = star_bwd_launch<1>(p, S, st); break;
+    case 2: rc = star_bwd_launch<2>(p, S, st); break;
+    case 3: rc = star_bwd_launch<3>(p, S, st); break;
+    case 4: rc = star_bwd_launch<4>(p, S, st); break;
+    default: rc = star_bwd_launch<5>(p, S, st); break;
+  }
+  if (rc) return rc;
+  return reduce_grads_plain(h, grads, part, S, h->lay.P, st);
+}
+
 }  // namespace awb

@@ -1,7 +1,12 @@
 """Star-shape prior (SURVEY a16): drop-in for the notebook class ``myNet``
 (``notebooks/icml_teaser_code/star_shaped/star.ipynb`` cell 2) -- same constructor argument, parameter names
 (``offset, W0, W1, W2, W1_r, W2_r``), initial weights for a given seed and ``forward(x[n,2]) -> [n,1]`` -- with the
-training loop of cell 3 as fused native steps (``StarFitter``)."""
+training loop of cell 3 as fused native steps (``StarFitter``).
+
+``forward`` is differentiable w.r.t. the parameters and the points (``awb_star_forward`` / ``awb_star_backward``), so
+the notebook's own loop (``loss = mse(sigmoid(net(x)), t); loss.backward(); optimizer.step()``), a custom loss or a
+gradient w.r.t. ``x`` work as with the plain-torch class.  First order only: a double backward raises.  A point at
+exactly ``-offset`` gets ``dx = 0`` (torch's ``sqrt`` backward gives NaN there; see ``include/awb.h``)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -12,7 +17,7 @@ from torch import nn
 
 from .. import _lib as L
 from ..core import Prior
-from .base import Affine, ArenaPriorModule, reject_second_order
+from .base import Affine, ArenaPriorModule, _first_order_only, _split_grads, reject_second_order
 
 
 def _lin(i: int, o: int) -> Affine:
@@ -21,15 +26,37 @@ def _lin(i: int, o: int) -> Affine:
 
 
 class _StarFunction(torch.autograd.Function):
+    """``apply(module, x, *params)``: the parameters are inputs so that autograd routes their gradients.  The forward is
+    ``awb_star_forward`` whether or not a graph is built (same bits); the backward is ``awb_star_backward``."""
+
     @staticmethod
-    def forward(ctx, module, x):
+    def forward(ctx, module, x, *params):
         prior = module._prior_for(x.device)
-        arena = module._ensure_flat()
+        arena = module._arena
         xs = x.detach().contiguous().float()
         out = torch.empty(xs.shape[0], dtype=torch.float32, device=x.device)
         L.check(prior.lib.awb_star_forward(prior.handle, arena.data_ptr(), xs.data_ptr(), xs.shape[0], out.data_ptr(),
                                            L.stream_ptr()))
+        ctx.module, ctx.prior, ctx.x_dtype = module, prior, x.dtype
+        ctx.shapes = [p.shape for p in params]
+        ctx.save_for_backward(xs, *params)    # params: autograd refuses a backward after they were modified in place
         return out.reshape(-1, 1)
+
+    @staticmethod
+    @_first_order_only
+    def backward(ctx, dy):
+        xs = ctx.saved_tensors[0]
+        prior, arena, n = ctx.prior, ctx.module._arena, xs.shape[0]
+        dy = dy.detach().reshape(-1).contiguous().float()
+        grads = torch.empty(arena.numel(), dtype=torch.float32, device=xs.device)
+        dx = torch.empty_like(xs) if ctx.needs_input_grad[1] else None
+        ws = torch.empty(int(prior.lib.awb_star_backward_workspace_bytes(prior.handle, n)), dtype=torch.uint8,
+                         device=xs.device)
+        L.check(prior.lib.awb_star_backward(prior.handle, arena.data_ptr(), xs.data_ptr(), n, dy.data_ptr(),
+                                            grads.data_ptr(), dx.data_ptr() if dx is not None else None, ws.data_ptr(),
+                                            ws.numel(), L.stream_ptr()))
+        pgrads = tuple(g if need else None for g, need in zip(_split_grads(grads, ctx.shapes), ctx.needs_input_grad[2:]))
+        return (None, dx.to(ctx.x_dtype) if dx is not None else None) + pgrads
 
 
 class StarShapedNet(ArenaPriorModule):
@@ -50,13 +77,15 @@ class StarShapedNet(ArenaPriorModule):
         return Prior(L.AWB_KIND_STAR, 2, self.n_hidden, 0)
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        """Inference forward (native).  Training goes through ``make_fitter`` (the notebook's loop, fused)."""
+        """Native forward, differentiable w.r.t. the parameters and ``x``.  ``make_fitter`` runs the notebook's loop as
+        fused steps."""
         if x.dim() != 2 or x.shape[1] != 2:
             raise ValueError(f"expected [n,2] points, got {tuple(x.shape)}")
         if not x.is_cuda:
             raise L.AwbLibraryError("awesome_b200 priors run on CUDA only (no CPU fallback)")
+        self._ensure_flat()
         with torch.cuda.device(x.device):
-            return _StarFunction.apply(self, x)
+            return _StarFunction.apply(self, x, *self._arena_params())
 
     def enforce_convexity(self) -> None:
         """The notebook's projection: ``W2_r.weight <- relu(W2_r.weight)`` (cell 3)."""

@@ -334,6 +334,21 @@ int awb_star_fit_step(awb_handle h, float* params, void* opt_state, const float*
                       const awb_loss_spec* loss, const awb_opt_hyper* hyper, float* loss_out, void* workspace,
                       size_t workspace_bytes, void* stream);
 
+/* Autograd backward of awb_star_forward: for the upstream gradient dlogits [n] (d loss / d logits) and the forward's
+ * params and x, grads [P] (overwritten, state_dict order) = sum_n dlogits_n d y_n / d params, and dx [n][2] (optional,
+ * null = not wanted) = dlogits_n d y_n / d x_n.  The forward adds the bias pairs W1.bias + W1_r.bias and
+ * W2.bias + W2_r.bias, so both biases of a pair receive the same gradient.  The offset's gradient is the sum of the point
+ * gradients and is computed whether dx is wanted or not; dx only adds its store, so grads do not depend on it.
+ * A point at exactly -offset (r = ||x + offset|| = 0) contributes nothing through r, as in awb_star_fit_step; its path
+ * through u = (x + offset) / (0.01 + r) is kept (d u / d x = I / 0.01 there).  Every term of the gradient carries a
+ * factor r, so such a point adds exactly 0 to grads and gets dx = 0, where torch's sqrt backward gives NaN.  Exact fp32;
+ * per-CTA partials summed in a fixed order: repeated calls give the same bits.  workspace: at least
+ * awb_star_backward_workspace_bytes(h, n) bytes.  A non-star handle, n < 1 or a null required pointer: AWB_ERR_INVALID;
+ * a smaller workspace: AWB_ERR_WORKSPACE.  The workspace query returns -1 for those handles and sizes. */
+int64_t awb_star_backward_workspace_bytes(awb_handle h, int64_t n);
+int awb_star_backward(awb_handle h, const float* params, const float* x, int64_t n, const float* dlogits, float* grads,
+                      float* dx, void* workspace, size_t workspace_bytes, void* stream);
+
 /* counts[O][4] (int64 device): {fg&fg, pred_fg, target_fg, n} for masks thresholded at 0.5 with
  * fg = value < 0.5 (MIOU(average="binary", invert=True): awesome/measures/miou.py:29-48;
  * in-loop check path_connected_net.py:964-982). pred_is_logit: threshold logits at 0. */
