@@ -47,6 +47,9 @@ static Layout make_layout(const awb_desc& d) {
     L.off_lin = L.off_flow + L.P_flow;
     L.n_lin = (int64_t)d.C * d.C + d.C;
     L.P = L.off_lin + L.n_lin;
+  } else if (d.kind == AWB_KIND_STAR) {   // plain state_dict-order arena, no augmented space
+    L.P = (int64_t)d.h * d.h + 8 * (int64_t)d.h + 4;
+    L.P_icnn = 0; L.off_flow = 0; L.P_flow = 0; L.off_lin = L.P;
   } else {
     L.off_flow = L.P_icnn; L.P_flow = 0; L.off_lin = L.P_icnn; L.P = L.P_icnn;
   }
@@ -135,11 +138,6 @@ int awb_prior_create(const awb_desc* d, awb_handle* out) {
   if (d->kind == AWB_KIND_ICNN || d->kind == AWB_KIND_STAR) { h->desc.F = 0; h->desc.m = 0; }
   if (d->kind == AWB_KIND_STAR) h->desc.L = 0;
   h->lay = make_layout(h->desc);
-  if (d->kind == AWB_KIND_STAR) {   // plain state_dict-order arena, no augmented space
-    const int64_t hh = d->h;
-    h->lay.P = hh * hh + 8 * hh + 4;
-    h->lay.P_icnn = 0; h->lay.off_flow = 0; h->lay.P_flow = 0; h->lay.off_lin = h->lay.P;
-  }
   h->fc_set = false;
   h->fc.out_scale = 1.f;
   h->flow_eval = 0;
@@ -169,7 +167,7 @@ int awb_prior_create(const awb_desc* d, awb_handle* out) {
     const int64_t o_W2r = 2 + 3 * (int64_t)hh + (int64_t)hh * hh + hh + hh + 1 + hh + hh;
     for (int k = 0; k < hh; k++) clamp[o_W2r + k] = 1;                  // W2_r.weight >= 0 (cell 3)
   }
-  if (i != L.P_icnn) { set_error("internal: layout mismatch"); delete h; return AWB_ERR_INVALID; }
+  if (i != L.P_icnn) { set_error("internal: layout mismatch"); awb_prior_destroy(h); return AWB_ERR_INVALID; }
   for (int64_t k = L.off_flow; k < L.off_flow + L.P_flow; k++) group[k] = 0;
   for (int64_t k = L.off_lin; k < L.P; k++) group[k] = 2;
   if (d->kind == AWB_KIND_DIFFEO_ICNN) {
@@ -185,22 +183,17 @@ int awb_prior_create(const awb_desc* d, awb_handle* out) {
   std::vector<int32_t> imap(L.G, -1);
   for (int64_t k = 0; k < L.P_icnn; k++) imap[map[k]] = (int32_t)k;
   cudaError_t e;
+  auto fail = [&](const char* what) { awb_prior_destroy(h); return cuda_fail(e, what); };   // frees what was allocated
   if ((e = cudaMalloc(&h->d_imap, sizeof(int32_t) * L.G)) != cudaSuccess ||
-      (e = cudaMemcpy(h->d_imap, imap.data(), sizeof(int32_t) * L.G, cudaMemcpyHostToDevice)) != cudaSuccess) {
-    cudaFree(h->d_imap);
-    delete h;
-    return cuda_fail(e, "awb_prior_create (inverse map)");
-  }
+      (e = cudaMemcpy(h->d_imap, imap.data(), sizeof(int32_t) * L.G, cudaMemcpyHostToDevice)) != cudaSuccess)
+    return fail("awb_prior_create (inverse map)");
   if ((e = cudaGetDevice(&h->device)) != cudaSuccess ||
       (e = cudaMalloc(&h->d_map, sizeof(int32_t) * L.P_icnn)) != cudaSuccess ||
       (e = cudaMalloc(&h->d_clamp, L.P)) != cudaSuccess || (e = cudaMalloc(&h->d_group, L.P)) != cudaSuccess ||
       (e = cudaMemcpy(h->d_map, map.data(), sizeof(int32_t) * L.P_icnn, cudaMemcpyHostToDevice)) != cudaSuccess ||
       (e = cudaMemcpy(h->d_clamp, clamp.data(), L.P, cudaMemcpyHostToDevice)) != cudaSuccess ||
-      (e = cudaMemcpy(h->d_group, group.data(), L.P, cudaMemcpyHostToDevice)) != cudaSuccess) {
-    cudaFree(h->d_map); cudaFree(h->d_clamp); cudaFree(h->d_group);
-    delete h;
-    return cuda_fail(e, "awb_prior_create");
-  }
+      (e = cudaMemcpy(h->d_group, group.data(), L.P, cudaMemcpyHostToDevice)) != cudaSuccess)
+    return fail("awb_prior_create");
   if (d->kind != AWB_KIND_STAR && tc_supported(h)) {
     std::vector<int32_t> tmap(tc_map_elems(L.L)), a2i(L.G);
     tc_build_map_host(L, tmap.data());
@@ -208,14 +201,10 @@ int awb_prior_create(const awb_desc* d, awb_handle* out) {
     if ((e = cudaMalloc(&h->d_tcmap, sizeof(int32_t) * tmap.size())) != cudaSuccess ||
         (e = cudaMemcpy(h->d_tcmap, tmap.data(), sizeof(int32_t) * tmap.size(), cudaMemcpyHostToDevice)) != cudaSuccess ||
         (e = cudaMalloc(&h->d_aug2img, sizeof(int32_t) * L.G)) != cudaSuccess ||
-        (e = cudaMemcpy(h->d_aug2img, a2i.data(), sizeof(int32_t) * L.G, cudaMemcpyHostToDevice)) != cudaSuccess) {
-      cudaFree(h->d_map); cudaFree(h->d_clamp); cudaFree(h->d_group); cudaFree(h->d_tcmap); cudaFree(h->d_imap); cudaFree(h->d_aug2img);
-      delete h;
-      return cuda_fail(e, "awb_prior_create (tensor path)");
-    }
+        (e = cudaMemcpy(h->d_aug2img, a2i.data(), sizeof(int32_t) * L.G, cudaMemcpyHostToDevice)) != cudaSuccess)
+      return fail("awb_prior_create (tensor path)");
   } else if (d->precision == AWB_PREC_F16) {
-    cudaFree(h->d_map); cudaFree(h->d_clamp); cudaFree(h->d_group); cudaFree(h->d_imap);
-    delete h;
+    awb_prior_destroy(h);
     set_error("precision f16 (tcgen05 path) supports priors with ICNN width h=130 and L in {1,2}; use fp32 for this shape");
     return AWB_ERR_UNSUPPORTED;
   }
@@ -299,26 +288,70 @@ static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t w
   return AWB_OK;
 }
 
+// One pass of an ICNN prior on the rows of a workspace.  dy comes from the loss on target (fit step: forward and
+// backward), from dlogits (backward of an earlier training forward on the same workspace, which holds the flow's outputs
+// and, on the exact path, the ICNN's activations) or from nowhere (forward only).
+struct Pass {
+  bool tensor;                                      // the fused tcgen05 kernel, else the exact fp32 kernels
+  const float* target; const awb_loss_spec* loss;   // dy from the loss on target ...
+  const float* dlogits;                             // ... or dy = dlogits
+  float *logits, *deformed, *dgrid;                 // optional outputs (a plain ICNN leaves dgrid in ws.dX)
+  bool training;                                    // exact forward only: keep the activations for a later backward
+  bool reuse;                                       // tensor path: the packed fp16 weight image in ws is current
+};
+
+// Flow forward, ICNN on the chosen path, flow backward.  The flow always runs on CUDA cores (K = C is too thin for
+// tensor cores): it writes the deformed coordinates X that the ICNN reads and consumes the d / d X the ICNN returns.
+// *n_part: the number of ICNN gradient partials written.
+static int run_pass(awb_handle h, const float* params, const awb_grid_spec* g, const Workspace& w, const Pass& p,
+                    cudaStream_t st, int* n_part) {
+  const bool flow = has_flow(h), forward = !p.dlogits, backward = p.target || p.dlogits;
+  const bool need_dx = backward && (flow || p.dgrid);
+  int rc;
+  if (flow && forward) {
+    rc = any_flow_forward(h, params, g, w, p.deformed, st);   // keeps X (and the coupling inputs when training)
+    if (rc) return rc;
+  }
+  if (p.tensor) {
+    // backward from dlogits: the fused kernel recomputes the forward and reads dy as the target of an upstream "loss"
+    const int O = h->desc.n_objects;
+    awb_loss_spec up[16];
+    float* amax = nullptr;
+    if (p.dlogits) {
+      for (int o = 0; o < O && o < 16; o++) { up[o].kind = AWB_LOSS_UPSTREAM; up[o].cls_rule = AWB_CLS_UNARY_LT_HALF; up[o].coef_fg = 1.f; up[o].coef_bg = 1.f; }
+      amax = w.lossp + (int64_t)kMaxSplits * O;       // spare floats behind the loss partials (lossp is [S][O], S <= 148 ... see carve)
+      rc = absmax_per_object(p.dlogits, w.N, O, amax, st);
+      if (rc) return rc;
+    }
+    *n_part = 0;
+    rc = tc_fit_forward_backward(h, params, g, p.dlogits ? p.dlogits : p.target, p.dlogits ? up : p.loss, p.logits,
+                                 backward ? 1 : 0, w, n_part, st, p.reuse, flow ? w.X : nullptr,
+                                 need_dx ? w.dX : nullptr, amax);
+  } else {
+    *n_part = n_splits(w.N);
+    rc = forward ? simt_forward(h, params, g, p.logits, p.training || backward, flow, w, st) : AWB_OK;
+    if (!rc && backward) rc = simt_backward(h, p.target, p.loss, p.dlogits, need_dx, w, st);
+  }
+  if (rc) return rc;
+  // flow priors: the flow backward writes dgrid itself (dX holds the gradient at the deformed coordinates, not the grid)
+  return flow && backward ? any_flow_backward(h, params, g, w, st, p.dgrid) : AWB_OK;
+}
+
 int awb_prior_forward(awb_handle h, const float* params, const awb_grid_spec* g, float* logits, float* deformed,
                       int32_t mode, void* ws, size_t ws_bytes, void* stream) {
   if (mode < AWB_FWD_EXACT || mode > AWB_FWD_TC_TRAINING) { set_error("unknown forward mode %d", mode); return AWB_ERR_INVALID; }
   const bool training = mode == AWB_FWD_EXACT_TRAINING || mode == AWB_FWD_TC_TRAINING;
+  const bool tensor = mode == AWB_FWD_TC || mode == AWB_FWD_TC_TRAINING;   // the default forward stays exact fp32
   Workspace w;
   int rc = check_common(h, g, ws, ws_bytes, training ? AWB_WS_TRAINING : AWB_WS_INFERENCE, nullptr, &w);
   if (rc) return rc;
   if (!params) { set_error("null params"); return AWB_ERR_INVALID; }
-  if (mode == AWB_FWD_TC || mode == AWB_FWD_TC_TRAINING) {   // tensor-path logits (fp16 operands); the default forward stays exact fp32
-    if (h->desc.precision != AWB_PREC_F16) { set_error("tensor-path forward needs an f16 handle"); return AWB_ERR_INVALID; }
-    if (!logits) { set_error("null logits"); return AWB_ERR_INVALID; }
-    cudaStream_t st = (cudaStream_t)stream;
-    if (has_flow(h)) {
-      rc = any_flow_forward(h, params, g, w, deformed, st);   // keeps X (and the coupling inputs when training)
-      if (rc) return rc;
-    }
-    return tc_fit_forward_backward(h, params, g, nullptr, nullptr, logits, 0, w, nullptr, st, false,
-                                   has_flow(h) ? w.X : nullptr, nullptr);
-  }
-  return simt_forward(h, params, g, logits, deformed, training, w, (cudaStream_t)stream);
+  if (tensor && h->desc.precision != AWB_PREC_F16) { set_error("tensor-path forward needs an f16 handle"); return AWB_ERR_INVALID; }
+  if (tensor && !logits) { set_error("null logits"); return AWB_ERR_INVALID; }
+  Pass p = {};
+  p.tensor = tensor; p.logits = logits; p.deformed = deformed; p.training = training;
+  int n_part;
+  return run_pass(h, params, g, w, p, (cudaStream_t)stream, &n_part);
 }
 
 int awb_prior_flow_inverse(awb_handle h, const float* params, const awb_grid_spec* g, float* out, void* stream) {
@@ -339,36 +372,17 @@ int awb_prior_backward(awb_handle h, const float* params, const awb_grid_spec* g
               "(no caller needs it on grouped or star handles; kind %d, %d objects)", h->desc.kind, h->desc.n_objects);
     return AWB_ERR_UNSUPPORTED;
   }
-  const int64_t N = w.N;
   cudaStream_t st = (cudaStream_t)stream;
-  if (h->desc.precision == AWB_PREC_F16) {
-    // tensor path: one fused kernel recomputes the forward and runs the backward on the upstream gradient
-    // (must follow awb_prior_forward(AWB_FWD_TC_TRAINING) on the same workspace: the flow's X / coupling inputs live
-    // there)
-    const int O = h->desc.n_objects;
-    awb_loss_spec up[16];
-    for (int o = 0; o < O && o < 16; o++) { up[o].kind = AWB_LOSS_UPSTREAM; up[o].cls_rule = AWB_CLS_UNARY_LT_HALF; up[o].coef_fg = 1.f; up[o].coef_bg = 1.f; }
-    float* amax = w.lossp + (int64_t)kMaxSplits * O;       // spare floats behind the loss partials (lossp is [S][O], S <= 148 ... see carve)
-    rc = absmax_per_object(dlogits, N, O, amax, st);
-    if (rc) return rc;
-    int n_part = 0;
-    const bool flow = has_flow(h);
-    rc = tc_fit_forward_backward(h, params, g, dlogits, up, nullptr, 1, w, &n_part, st, false, flow ? w.X : nullptr,
-                                 (flow || dgrid) ? w.dX : nullptr, amax);
-    if (rc) return rc;
-    // flow priors: the flow backward writes dgrid itself (dX holds the gradient at the deformed coordinates, not the grid)
-    if (flow) { rc = any_flow_backward(h, params, g, w, st, dgrid); if (rc) return rc; }
-    rc = simt_reduce_grads(h, grads, w, N, st, n_part);
-    if (rc) return rc;
-    if (dgrid && !flow) rc = simt_dgrid(h, g, dgrid, w, st);
-    return rc;
-  }
-  rc = simt_backward(h, params, g, nullptr, nullptr, dlogits, dgrid != nullptr, w, st, dgrid);
+  // the path follows the handle, not the forward: an f16 handle's backward is the fused tensor-path kernel even after an
+  // exact training forward
+  Pass p = {};
+  p.tensor = h->desc.precision == AWB_PREC_F16; p.dlogits = dlogits; p.dgrid = dgrid;
+  int n_part;
+  rc = run_pass(h, params, g, w, p, st, &n_part);
   if (rc) return rc;
-  rc = simt_reduce_grads(h, grads, w, N, st);
+  rc = simt_reduce_grads(h, grads, w, w.N, st, n_part);
   if (rc) return rc;
-  if (dgrid && !has_flow(h)) rc = simt_dgrid(h, g, dgrid, w, st);
-  return rc;
+  return dgrid && !has_flow(h) ? simt_dgrid(h, g, dgrid, w, st) : AWB_OK;   // plain ICNN: dX is d / d grid
 }
 
 int awb_prior_grid_grad_backward(awb_handle h, const float* params, const awb_grid_spec* g, const float* dlogits,
@@ -387,30 +401,7 @@ int awb_prior_grid_grad_backward(awb_handle h, const float* params, const awb_gr
   cudaStream_t st = (cudaStream_t)stream;
   rc = simt_grid_grad_backward(h, g, dlogits, d_dgrid, d_dlogits, w, st);
   if (rc) return rc;
-  return simt_reduce_grads(h, grads, w, w.N, st);
-}
-
-// Forward, loss and backward of a fit step on the rows of w (AWB_WS_FIT_STEP), up to the gradient and loss partials that
-// the caller reduces.  f16 handles: the flow on CUDA cores (K = C is too thin for tensor cores) around the tensor-path
-// ICNN -- the flow writes the deformed coordinates X, the fused kernel returns d loss / d X, the flow backward consumes
-// it.  reuse: the fused kernel reuses the packed fp16 weight image left in w.  *n_part: the number of ICNN partials
-// written, -1 (n_splits(N)) on the exact fp32 path.
-static int fit_gradients(awb_handle h, const float* params, const awb_grid_spec* g, const float* target,
-                         const awb_loss_spec* loss, bool reuse, const Workspace& w, cudaStream_t st, int* n_part) {
-  int rc;
-  if (h->desc.precision == AWB_PREC_F16) {
-    const bool flow = has_flow(h);
-    if (flow) { rc = any_flow_forward(h, params, g, w, nullptr, st); if (rc) return rc; }
-    *n_part = 0;
-    rc = tc_fit_forward_backward(h, params, g, target, loss, nullptr, 1, w, n_part, st, reuse, flow ? w.X : nullptr,
-                                 flow ? w.dX : nullptr);
-    if (rc) return rc;
-    return flow ? any_flow_backward(h, params, g, w, st) : AWB_OK;
-  }
-  *n_part = -1;
-  rc = simt_forward(h, params, g, nullptr, nullptr, true, w, st);
-  if (rc) return rc;
-  return simt_backward(h, params, g, target, loss, nullptr, false, w, st);
+  return simt_reduce_grads(h, grads, w, w.N, st, n_splits(w.N));
 }
 
 int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_grid_spec* g, const float* target,
@@ -421,10 +412,12 @@ int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_g
   if (rc) return rc;
   if (!params || !opt_state || !target || !loss || !hy) { set_error("null argument"); return AWB_ERR_INVALID; }
   // simt_reduce_opt refreshes a flow prior's fp16 weight image only when its optimizer owns every group
-  const bool reuse = (flags & AWB_FIT_REUSE_PACKED) != 0 && (!has_flow(h) || hy->active_groups == 0);
+  Pass p = {};
+  p.tensor = h->desc.precision == AWB_PREC_F16; p.target = target; p.loss = loss;
+  p.reuse = (flags & AWB_FIT_REUSE_PACKED) != 0 && (!has_flow(h) || hy->active_groups == 0);
   cudaStream_t st = (cudaStream_t)stream;
   int n_part;
-  rc = fit_gradients(h, params, g, target, loss, reuse, w, st, &n_part);
+  rc = run_pass(h, params, g, w, p, st, &n_part);
   if (rc) return rc;
   return simt_reduce_opt(h, params, opt_state, hy, loss_out, w, w.N, st, n_part);
 }
@@ -492,9 +485,12 @@ int awb_prior_slice_grads(awb_handle h, const float* params, const awb_grid_spec
   rc = check_common(h, g, ws, ws_bytes, AWB_WS_FIT_STEP, window, &w);
   if (rc) return rc;
   if (!params || !target || !loss || !grad_row) { set_error("null argument"); return AWB_ERR_INVALID; }
+  Pass p = {};
+  p.tensor = h->desc.precision == AWB_PREC_F16; p.target = target + row_begin; p.loss = loss;
+  p.reuse = (flags & AWB_FIT_REUSE_PACKED) != 0;
   cudaStream_t st = (cudaStream_t)stream;
   int n_part;
-  rc = fit_gradients(h, params, g, target + row_begin, loss, (flags & AWB_FIT_REUSE_PACKED) != 0, w, st, &n_part);
+  rc = run_pass(h, params, g, w, p, st, &n_part);
   if (rc) return rc;
   return simt_reduce_grads(h, grad_row, w, w.N, st, n_part, grad_row + h->lay.P);   // the loss sum goes to column P
 }
@@ -593,7 +589,7 @@ int awb_flow_identity_step(awb_handle h, float* params, void* opt_state, const a
   if (rc) return rc;
   awb_opt_hyper hh = *hy;
   hh.active_groups = 1;   // flow_net only
-  return simt_reduce_opt(h, params, opt_state, &hh, loss_out, w, w.N, st);
+  return simt_reduce_opt(h, params, opt_state, &hh, loss_out, w, w.N, st, n_splits(w.N));
 }
 
 int awb_optim_step(awb_handle h, float* params, const float* grads, void* opt_state, const awb_opt_hyper* hy,

@@ -6,6 +6,9 @@
 
 #include "../../include/awb.h"
 
+// awb_loss_spec.kind of the tensor path's backward: `target` carries d loss / d logits (awb_prior_backward)
+#define AWB_LOSS_UPSTREAM 2
+
 namespace awb {
 
 constexpr int kMaxSplits = 148;  // pixel ranges for cross-pixel reductions = one per SM
@@ -162,20 +165,21 @@ struct GridDev {
   const float* grid;
   uint32_t row0;   // global index of local row 0 (Workspace::row0)
 };
-int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, float* logits_out,
-                 float* deformed, bool training, const Workspace& ws, cudaStream_t st);
-// loss != nullptr: fit mode (dy from loss); else dy = dlogits.
-// dgrid (optional, flow priors): the flow backward also writes d / d grid, planar [B,C,H,W]
-int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
-                  const awb_loss_spec* loss, const float* dlogits, bool need_dx, const Workspace& ws,
-                  cudaStream_t st, float* dgrid = nullptr);
-// n_partials: number of ICNN gradient partials ([S][O][G]) the producer wrote (-1: n_splits(N)); the flow
-// partials always come from flow_backward's n_splits(N) pixel ranges.
+// The exact fp32 ICNN passes; a flow prior's flow runs around them (awb_api.cu run_pass).  x_ready: the flow forward
+// has written the ICNN's input rows ws.X (otherwise k_input generates them from the grid).
+int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, float* logits_out, bool training,
+                 bool x_ready, const Workspace& ws, cudaStream_t st);
+// loss != nullptr: fit mode (dy from loss); else dy = dlogits.  need_dx: write d / d X into ws.dX (a flow backward or
+// dgrid reads it).
+int simt_backward(const awb_prior* h, const float* target, const awb_loss_spec* loss, const float* dlogits, bool need_dx,
+                  const Workspace& ws, cudaStream_t st);
+// n_partials: number of ICNN gradient partials ([S][O][G]) the producer wrote; the flow partials always come from
+// flow_backward's n_splits(N) pixel ranges.
 int simt_reduce_opt(const awb_prior* h, float* params, void* opt_state, const awb_opt_hyper* hy,
-                    float* loss_out, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1);
+                    float* loss_out, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials);
 // loss_slot (optional, single object): receives the sum of the loss partials (gradient row of awb_prior_slice_grads).
 // n_partials = 0: no ICNN partials were written (flow-only backward), the ICNN entries of grads are exactly 0.
-int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials = -1,
+int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int64_t N, cudaStream_t st, int n_partials,
                       float* loss_slot = nullptr);
 // second-order pass of the coordinate gradient (single-object ICNN, after simt_forward(training) on ws, ws carved with
 // tangent rows): d_dgrid [B,C,H,W] -> ydot [N] and the parameter-gradient partials that simt_reduce_grads sums
@@ -220,8 +224,8 @@ int64_t tc_vec_offset_bytes(int L);                       // byte offset of the 
 // mode 0: forward only (logits), mode 1: forward + loss + backward partials (part / lossp, *n_splits_out CTAs)
 int tc_fit_forward_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
                             const awb_loss_spec* loss, float* logits, int mode, const Workspace& ws,
-                            int* n_splits_out, cudaStream_t st, bool reuse_packed = false,
-                            const float* Xrows = nullptr, float* dXrows = nullptr, const float* amax = nullptr);
+                            int* n_splits_out, cudaStream_t st, bool reuse_packed, const float* Xrows, float* dXrows,
+                            const float* amax);
 int tc_trace_read(unsigned long long* host, int max_ctas);   // debug timeline (AWB_TC_TRACE=1): 256 stamps per CTA
 
 // ---- flows, implemented in awb_flow.cu ----

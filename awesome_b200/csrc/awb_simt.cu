@@ -935,23 +935,17 @@ static void opt_ptrs(const awb_prior* h, void* opt_state, float** m, float** v, 
   *sc = (OptScal*)((char*)opt_state + round_up(2 * n * 4, 256));
 }
 
-int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, float* logits_out,
-                 float* deformed, bool training, const Workspace& ws, cudaStream_t st) {
+int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, float* logits_out, bool training,
+                 bool x_ready, const Workspace& ws, cudaStream_t st) {
   const Layout& L = h->lay;
   const int O = h->desc.n_objects;
   const int64_t N = ws.N;
   AWB_CUDA(cudaMemsetAsync(ws.waug, 0, sizeof(float) * O * L.G, st));
   AWB_LAUNCH(PK_PACK, st, k_pack<<<dim3((unsigned)((L.P_icnn + 255) / 256), O), 256, 0, st>>>(params, ws.waug, h->d_map, (int)L.P_icnn,
                                                                        L.P, L.off_icnn, L.G));
-  int x_ready = 0;
-  if (has_flow(h)) {
-    int rc = any_flow_forward(h, params, g, ws, deformed, st);
-    if (rc) return rc;
-    x_ready = 1;
-  }
   const int64_t sLayer = N * L.ld;            // one ZA layer
   const int64_t sZAobj = (L.L + 1) * sLayer;  // all layers of an object
-  AWB_LAUNCH(PK_INPUT, st, k_input<<<dim3((unsigned)((N + 63) / 64), O), 256, 0, st>>>(to_dev(g, L.C, ws.row0), x_ready, ws.X, ws.waug, ws.ZA, N,
+  AWB_LAUNCH(PK_INPUT, st, k_input<<<dim3((unsigned)((N + 63) / 64), O), 256, 0, st>>>(to_dev(g, L.C, ws.row0), (int)x_ready, ws.X, ws.waug, ws.ZA, N,
                                                               L.h, L.C, L.ld, L.G, L.aug_in, sZAobj));
   for (int i = 0; i < L.L; i++) {
     GemmP p = {};
@@ -963,17 +957,7 @@ int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
     p.h = L.h; p.C = L.C;
     AWB_LAUNCH(PK_GEMM_FWD, st, k_gemm<0><<<dim3((unsigned)((N + 127) / 128), 1, O), 256, 0, st>>>(p));
   }
-  if (!training) {
-    OutP q = {};
-    q.ZA = ws.ZA + L.L * sLayer; q.sZA = sZAobj;
-    q.waug = ws.waug; q.G = L.G; q.aug_out = L.aug_out;
-    q.logits = logits_out; q.train = 0; q.N = N; q.chunk = split_chunk(N);
-    q.h = L.h; q.C = L.C; q.ld = L.ld; q.O = O;
-    size_t smem = (8 * L.ld + 8) * sizeof(float);
-    if (L.ld <= 160) AWB_LAUNCH(PK_OUT_LOSS, st, k_out<5><<<dim3(n_splits(N), O), 256, smem, st>>>(q));
-    else AWB_LAUNCH(PK_OUT_LOSS, st, k_out<9><<<dim3(n_splits(N), O), 256, smem, st>>>(q));
-  } else if (logits_out) {
-    // training forward: logits are produced by the same kernel that starts the backward
+  if (!training || logits_out) {   // a training forward without logits leaves k_out to the backward
     OutP q = {};
     q.ZA = ws.ZA + L.L * sLayer; q.sZA = sZAobj;
     q.waug = ws.waug; q.G = L.G; q.aug_out = L.aug_out;
@@ -987,9 +971,8 @@ int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
   return AWB_OK;
 }
 
-int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
-                  const awb_loss_spec* loss, const float* dlogits, bool need_dx, const Workspace& ws,
-                  cudaStream_t st, float* dgrid) {
+int simt_backward(const awb_prior* h, const float* target, const awb_loss_spec* loss, const float* dlogits, bool need_dx,
+                  const Workspace& ws, cudaStream_t st) {
   const Layout& L = h->lay;
   const int O = h->desc.n_objects;
   const int64_t N = ws.N;
@@ -997,7 +980,6 @@ int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
   const int64_t chunk = split_chunk(N);
   const int64_t sLayer = N * L.ld, sZAobj = (L.L + 1) * sLayer, sDobj = 2 * sLayer;
   const int64_t sSplit = (int64_t)O * L.G;
-  if (has_flow(h)) need_dx = true;
 
   OutP q = {};
   q.ZA = ws.ZA + L.L * sLayer; q.sZA = sZAobj;
@@ -1045,10 +1027,6 @@ int simt_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
     AWB_LAUNCH(PK_IN_BWD, st, k_in_dgrad<<<dim3((unsigned)((N + 7) / 8), O), 256, 0, st>>>(ws.D, sDobj, ws.waug, L.G, L.aug_in, ws.dX, N,
                                                                  L.h, L.ld));
   AWB_CUDA(cudaGetLastError());
-  if (has_flow(h)) {
-    int rc = any_flow_backward(h, params, g, ws, st, dgrid);
-    if (rc) return rc;
-  }
   return AWB_OK;
 }
 
@@ -1127,7 +1105,7 @@ int simt_reduce_opt(const awb_prior* h, float* params, void* opt_state, const aw
   OptP a = {};
   a.params = params;
   opt_ptrs(h, opt_state, &a.m, &a.v, &a.scal);
-  a.part = ws.part; a.sSplit = (int64_t)O * L.G; a.S = n_partials > 0 ? n_partials : n_splits(N);
+  a.part = ws.part; a.sSplit = (int64_t)O * L.G; a.S = n_partials;
   a.SF = n_splits(N);
   a.PF = L.P_flow + L.n_lin;
   a.fpart = ws.fpart; a.sFSplit = (int64_t)O * a.PF;
@@ -1187,7 +1165,7 @@ int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int
   int64_t PF = L.P_flow + L.n_lin;
   const int64_t n_thr = L.P + (loss_slot ? 1 : 0);
   AWB_LAUNCH(PK_OPT, st, AWB_CUDA(launch_ex(k_reduce_grads, dim3((unsigned)((n_thr + 255) / 256), O), dim3(256), 0, st, true,
-      grads, (const float*)ws.part, (int64_t)O * L.G, n_partials >= 0 ? n_partials : n_splits(N), n_splits(N),
+      grads, (const float*)ws.part, (int64_t)O * L.G, n_partials, n_splits(N),
       (const float*)ws.fpart, (int64_t)O * PF, (const int32_t*)h->d_map, (int64_t)L.P, (int64_t)L.off_icnn,
       (int64_t)L.P_icnn, (int64_t)L.off_flow, PF, (int64_t)L.G, (const float*)ws.lossp, loss_slot)));
   AWB_CUDA(cudaGetLastError());

@@ -54,7 +54,6 @@ extern "C" {
 /* per-pixel loss kinds (SURVEY 8a row a10) */
 #define AWB_LOSS_SE_SIGMOID 0 /* (t - sigmoid(y))^2: awesome/measures/se.py:21-23 on WrapperModule.process_prior_output */
 #define AWB_LOSS_BCE_LOGITS 1 /* BCEWithLogitsLoss: notebooks/how_to/path-connectedness.ipynb cell 9 */
-#define AWB_LOSS_UPSTREAM 2   /* internal: `target` carries d loss / d logits from autograd (awb_prior_backward on the tensor path) */
 #define AWB_CLS_UNARY_LT_HALF 0 /* fg = target < 0.5: awesome/measures/unaries_weighted_loss.py:35-69 */
 #define AWB_CLS_NOT_ONE 1       /* fg = target != 1: how-to notebooks, cell 9 */
 
