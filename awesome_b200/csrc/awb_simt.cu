@@ -135,11 +135,16 @@ struct GemmP {
 // MODE 1: delta_prev = (delta * Waug) .* (ZA_prev > 0)  A(m,k)=A[m*lda+k]   B(k,n)=B[k*ldb+n]
 // MODE 2: dWaug[split] = delta^T * ZA_prev              A(m,k)=A[k*lda+m]   B(k,n)=B[k*ldb+n]
 // MODE 3: ZT_out = (ZT_in * Waug^T) .* (ZA_out > 0)     as MODE 0: the tangent of MODE 0 along the tangent rows ZT_in
+// A CTA writes a tile of kGemmTile output columns (and, in MODE 2, of kGemmTile output rows) chosen by blockIdx.y:
+// rows wider than one tile (ld > 144, from h = 141) take several CTAs.  MODE 2 folds its row and column tiles into
+// blockIdx.y (row tile major); blockIdx.x is the pixel block / split and blockIdx.z the object in every mode.
+constexpr int kGemmTile = 144;
+
 template <int MODE>
 __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
-  constexpr int BM = (MODE == 2) ? 144 : 128;
+  constexpr int BM = (MODE == 2) ? kGemmTile : 128;
   constexpr int TM = BM / 16;
-  constexpr int BN = 144, TN = 9, BK = 8;
+  constexpr int BN = kGemmTile, TN = 9, BK = 8;
   constexpr int NA = (BM * BK + 255) / 256, NB = (BN * BK + 255) / 256;
   __shared__ float As[2][BK][BM + 4];
   __shared__ float Bs[2][BK][BN + 4];
@@ -148,14 +153,25 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
   const int o = blockIdx.z;
   const float* A = p.A + (int64_t)o * p.sA;
   const float* B = p.B + (int64_t)o * p.sB;
-  int64_t m0 = 0, k_begin = 0, k_end = p.K;
+  int64_t m0 = 0, k_begin = 0, k_end = p.K;   // m0: first pixel row (modes 0, 1, 3) or first weight row (mode 2)
+  int n0 = (int)blockIdx.y * BN;              // first output column
   if (MODE == 2) {
+    const int col_tiles = (p.N + BN - 1) / BN;
+    const int mt = (int)blockIdx.y / col_tiles;
+    m0 = (int64_t)mt * BM;
+    n0 = ((int)blockIdx.y - mt * col_tiles) * BN;
     k_begin = (int64_t)blockIdx.x * p.k_chunk;
     k_end = k_begin + p.k_chunk < p.K ? k_begin + p.k_chunk : (int64_t)p.K;
     if (k_end < k_begin) k_end = k_begin;
   } else {
     m0 = (int64_t)blockIdx.x * BM;
   }
+  // operands and outputs seen from the tile's first column (and, in mode 2, first weight row): the loops below index them
+  // as the single-tile kernel does, against limits shifted by the offset
+  const int n_lim = ((MODE == 0 || MODE == 3) ? p.N : p.ldb) - n0;    // valid B columns of the tile
+  B += (MODE == 0 || MODE == 3) ? (int64_t)n0 * p.ldb : (int64_t)n0;
+  const int a_lim = p.lda - (MODE == 2 ? (int)m0 : 0);               // mode 2: valid A columns of the tile
+  if (MODE == 2) A += m0;
 
   float ra[NA], rb[NB];
   auto gload = [&](int64_t k0) {
@@ -167,7 +183,7 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
         if (MODE == 2) {  // m contiguous in global
           int k = e / BM, m = e - k * BM;
           int64_t kk = k0 + k;
-          if (kk < k_end && m < p.lda) v = A[kk * p.lda + m];
+          if (kk < k_end && m < a_lim) v = A[kk * p.lda + m];
         } else {          // k contiguous in global
           int m = e / BK, k = e - m * BK;
           int64_t kk = k0 + k;
@@ -184,12 +200,12 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
         if (MODE == 0 || MODE == 3) {  // k contiguous in global: B(k,n) = W[n][k], rows n < h
           int n = e / BK, k = e - n * BK;
           int64_t kk = k0 + k;
-          if (n < p.N && kk < p.ldb) v = B[(int64_t)n * p.ldb + kk];
+          if (n < n_lim && kk < p.ldb) v = B[(int64_t)n * p.ldb + kk];
         } else {          // n contiguous in global
           int k = e / BN, n = e - k * BN;
           int64_t kk = k0 + k;
           bool ok = (MODE == 1) ? (kk < p.K) : (kk < k_end);
-          if (ok && n < p.ldb) v = B[kk * p.ldb + n];
+          if (ok && n < n_lim) v = B[kk * p.ldb + n];
         }
       }
       rb[i] = v;
@@ -248,11 +264,12 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
     buf ^= 1;
   }
 
-  // ---- epilogue
+  // ---- epilogue (column n of the tile is output column n0 + n)
+  const int c_lim = p.ldc - n0, h_lim = p.h - n0;
   if (MODE == 0 || MODE == 3) {
-    float* Cz = p.Cout + (int64_t)o * p.sC;
-    const float* Zin = p.E0 + (int64_t)o * p.sE0;
-    const float* Zm = MODE == 3 ? p.Mz + (int64_t)o * p.sMz : nullptr;
+    float* Cz = p.Cout + (int64_t)o * p.sC + n0;
+    const float* Zin = p.E0 + (int64_t)o * p.sE0 + n0;
+    const float* Zm = MODE == 3 ? p.Mz + (int64_t)o * p.sMz + n0 : nullptr;
 #pragma unroll
     for (int i = 0; i < TM; i++) {
       int64_t m = m0 + ty + 16 * i;
@@ -260,16 +277,16 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
 #pragma unroll
       for (int j = 0; j < TN; j++) {
         int n = tx + 16 * j;
-        if (n >= p.ldc) continue;
+        if (n >= c_lim) continue;
         float v;
-        if (MODE == 0) v = (n < p.h) ? fmaxf(acc[i][j], 0.f) : Zin[m * p.ldc + n];
-        else v = (n < p.h) ? (Zm[m * p.ldc + n] > 0.f ? acc[i][j] : 0.f) : Zin[m * p.ldc + n];
+        if (MODE == 0) v = (n < h_lim) ? fmaxf(acc[i][j], 0.f) : Zin[m * p.ldc + n];
+        else v = (n < h_lim) ? (Zm[m * p.ldc + n] > 0.f ? acc[i][j] : 0.f) : Zin[m * p.ldc + n];
         Cz[m * p.ldc + n] = v;
       }
     }
   } else if (MODE == 1) {
-    float* Cd = p.Cout + (int64_t)o * p.sC;
-    const float* Zp = p.E0 + (int64_t)o * p.sE0;
+    float* Cd = p.Cout + (int64_t)o * p.sC + n0;
+    const float* Zp = p.E0 + (int64_t)o * p.sE0 + n0;
     float* dX = p.E1 ? p.E1 + (int64_t)o * p.sE1 : nullptr;
 #pragma unroll
     for (int i = 0; i < TM; i++) {
@@ -278,26 +295,27 @@ __global__ void __launch_bounds__(256) k_gemm(GemmP p) {
 #pragma unroll
       for (int j = 0; j < TN; j++) {
         int n = tx + 16 * j;
-        if (n >= p.ldc) continue;
+        if (n >= c_lim) continue;
         float v = 0.f;
-        if (n < p.h) {
+        if (n < h_lim) {
           v = Zp[m * p.ldc + n] > 0.f ? acc[i][j] : 0.f;
-        } else if (dX && n < p.h + p.C) {
-          dX[m * 4 + (n - p.h)] += acc[i][j];   // one thread per (m, n): no race
+        } else if (dX && n < h_lim + p.C) {
+          dX[m * 4 + (n - h_lim)] += acc[i][j];   // one thread per (m, n): no race
         }
         Cd[m * p.ldc + n] = v;
       }
     }
   } else {
-    float* Cw = p.Cout + (int64_t)blockIdx.x * p.sSplit + (int64_t)o * p.sC;
+    float* Cw = p.Cout + (int64_t)blockIdx.x * p.sSplit + (int64_t)o * p.sC + m0 * p.ldc + n0;
+    const int m_lim = p.h - (int)m0;
 #pragma unroll
     for (int i = 0; i < TM; i++) {
       int m = ty + 16 * i;
-      if (m >= p.h) continue;
+      if (m >= m_lim) continue;
 #pragma unroll
       for (int j = 0; j < TN; j++) {
         int n = tx + 16 * j;
-        if (n >= p.ldc) continue;
+        if (n >= c_lim) continue;
         Cw[(int64_t)m * p.ldc + n] = acc[i][j];
       }
     }
@@ -928,6 +946,10 @@ static GridDev to_dev(const awb_grid_spec* g, int C, int64_t row0) {
   return d;
 }
 
+// k_gemm's blockIdx.y extent: column tiles over ld (modes 0, 1, 3); row tiles over h times column tiles (mode 2)
+static unsigned gemm_col_tiles(const Layout& L) { return (unsigned)((L.ld + kGemmTile - 1) / kGemmTile); }
+static unsigned gemm_wgrad_tiles(const Layout& L) { return (unsigned)((L.h + kGemmTile - 1) / kGemmTile) * gemm_col_tiles(L); }
+
 static void opt_ptrs(const awb_prior* h, void* opt_state, float** m, float** v, OptScal** sc) {
   int64_t n = h->lay.P * h->desc.n_objects;
   *m = (float*)opt_state;
@@ -955,7 +977,7 @@ int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
     p.M = N; p.N = L.h; p.K = L.ld;
     p.E0 = p.A; p.sE0 = sZAobj;
     p.h = L.h; p.C = L.C;
-    AWB_LAUNCH(PK_GEMM_FWD, st, k_gemm<0><<<dim3((unsigned)((N + 127) / 128), 1, O), 256, 0, st>>>(p));
+    AWB_LAUNCH(PK_GEMM_FWD, st, k_gemm<0><<<dim3((unsigned)((N + 127) / 128), gemm_col_tiles(L), O), 256, 0, st>>>(p));
   }
   if (!training || logits_out) {   // a training forward without logits leaves k_out to the backward
     OutP q = {};
@@ -1008,7 +1030,7 @@ int simt_backward(const awb_prior* h, const float* target, const awb_loss_spec* 
       p.Cout = ws.part + L.aug_layer + (int64_t)(i - 1) * L.h * L.ld; p.sC = L.G; p.ldc = L.ld;
       p.M = L.h; p.N = L.ld; p.K = (int)N;
       p.h = L.h; p.C = L.C; p.k_chunk = chunk; p.sSplit = sSplit;
-      AWB_LAUNCH(PK_GEMM_WGRAD, st, k_gemm<2><<<dim3(S, 1, O), 256, 0, st>>>(p));
+      AWB_LAUNCH(PK_GEMM_WGRAD, st, k_gemm<2><<<dim3(S, gemm_wgrad_tiles(L), O), 256, 0, st>>>(p));
     }
     {  // data gradient + relu backward
       GemmP p = {};
@@ -1019,7 +1041,7 @@ int simt_backward(const awb_prior* h, const float* target, const awb_loss_spec* 
       p.E0 = za_prev; p.sE0 = sZAobj;
       p.E1 = need_dx ? ws.dX : nullptr; p.sE1 = N * 4;
       p.h = L.h; p.C = L.C;
-      AWB_LAUNCH(PK_GEMM_DGRAD, st, k_gemm<1><<<dim3((unsigned)((N + 127) / 128), 1, O), 256, 0, st>>>(p));
+      AWB_LAUNCH(PK_GEMM_DGRAD, st, k_gemm<1><<<dim3((unsigned)((N + 127) / 128), gemm_col_tiles(L), O), 256, 0, st>>>(p));
     }
   }
   AWB_LAUNCH(PK_IN_BWD, st, k_in_wgrad<<<dim3(S, O), 256, 0, st>>>(ws.D, sDobj, ws.X, ws.part, sSplit, L.G, L.aug_in, N, chunk, L.h, L.ld, 1.f));
@@ -1056,7 +1078,7 @@ int simt_grid_grad_backward(const awb_prior* h, const awb_grid_spec* g, const fl
     p.E0 = p.A;
     p.Mz = ws.ZA + (i + 1) * sLayer;
     p.h = L.h; p.C = L.C;
-    AWB_LAUNCH(PK_TAN_FWD, st, k_gemm<3><<<dim3((unsigned)((N + 127) / 128), 1, 1), 256, 0, st>>>(p));
+    AWB_LAUNCH(PK_TAN_FWD, st, k_gemm<3><<<dim3((unsigned)((N + 127) / 128), gemm_col_tiles(L), 1), 256, 0, st>>>(p));
   }
   TanOutP q = {};
   q.ZA = ws.ZA + L.L * sLayer; q.ZT = ws.ZT + L.L * sLayer;
@@ -1077,7 +1099,7 @@ int simt_grid_grad_backward(const awb_prior* h, const awb_grid_spec* g, const fl
       p.Cout = ws.part + L.aug_layer + (int64_t)(i - 1) * L.h * L.ld; p.ldc = L.ld;
       p.M = L.h; p.N = L.ld; p.K = (int)N;
       p.h = L.h; p.C = L.C; p.k_chunk = chunk; p.sSplit = sSplit;
-      AWB_LAUNCH(PK_GEMM_WGRAD, st, k_gemm<2><<<dim3(S, 1, 1), 256, 0, st>>>(p));
+      AWB_LAUNCH(PK_GEMM_WGRAD, st, k_gemm<2><<<dim3(S, gemm_wgrad_tiles(L), 1), 256, 0, st>>>(p));
     }
     {  // delta_{i-1}: the data gradient of the first backward (no coordinate gradient)
       GemmP p = {};
@@ -1087,7 +1109,7 @@ int simt_grid_grad_backward(const awb_prior* h, const awb_grid_spec* g, const fl
       p.M = N; p.N = L.ld; p.K = L.h;
       p.E0 = ws.ZA + (i - 1) * sLayer;
       p.h = L.h; p.C = L.C;
-      AWB_LAUNCH(PK_GEMM_DGRAD, st, k_gemm<1><<<dim3((unsigned)((N + 127) / 128), 1, 1), 256, 0, st>>>(p));
+      AWB_LAUNCH(PK_GEMM_DGRAD, st, k_gemm<1><<<dim3((unsigned)((N + 127) / 128), gemm_col_tiles(L), 1), 256, 0, st>>>(p));
     }
   }
   AWB_LAUNCH(PK_IN_BWD, st, k_in_wgrad<<<dim3(S, 1), 256, 0, st>>>(ws.D, 2 * sLayer, ws.dX, ws.part, sSplit, L.G, L.aug_in, N,

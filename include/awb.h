@@ -66,8 +66,9 @@ typedef struct awb_prior* awb_handle;
 typedef struct awb_desc {
   int32_t kind;      /* AWB_KIND_* */
   int32_t C;         /* coordinate channels: 2 (x,y) or 3 (x,y,t) */
-  int32_t h;         /* ICNN hidden width (n_hidden, default 130) */
-  int32_t L;         /* number of SkipBlocks (n_hidden_layers) */
+  int32_t h;         /* ICNN hidden width (n_hidden, default 130), 8..256: every width runs on the exact fp32 path;
+                        AWB_PREC_F16 takes its tensor path at h = 130, L in {1, 2} only */
+  int32_t L;         /* number of SkipBlocks (n_hidden_layers), 0..8 */
   int32_t F;         /* number of RealNVP flows (0 for AWB_KIND_ICNN) */
   int32_t m;         /* flow MLP hidden width */
   int32_t flow_tanh; /* 1: output_fn == "tanh" */

@@ -122,6 +122,10 @@ def deform64(kind, p, rows, scale=None):
 
 
 def logits64(kind, p, rows, scale=None):
+    if kind == "icnn":
+        return O.icnn_forward(p, rows).reshape(-1)
+    if kind == "convexnet":
+        return O.convexnet_forward(p, rows).reshape(-1)
     return O.icnn_forward(p, deform64(kind, p, rows, scale), "convex_net.").reshape(-1)
 
 
@@ -166,11 +170,11 @@ def kink_rows(kind, m, rows, scale=None, deformation_only=False):
     return out
 
 
-def away_from_kinks(kind, m, rows, w, scale=None, deformation_only=False):
+def away_from_kinks(kind, m, rows, w, scale=None, deformation_only=False, max_fraction=KINK_MAX_FRACTION):
     """``w`` with the upstream gradient of the kink pixels set to 0, and the excluded fraction."""
     near = kink_rows(kind, m, rows, scale, deformation_only)
     frac = float(near.float().mean())
-    assert frac <= KINK_MAX_FRACTION, frac
+    assert frac <= max_fraction, frac
     B, C_, H, W = w.shape
     w = w.permute(0, 2, 3, 1).reshape(-1, C_).clone()
     w[near] = 0

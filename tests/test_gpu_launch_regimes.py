@@ -3,7 +3,8 @@
 Every fit-path kernel picks its launch geometry, and sometimes its code path, from the problem size on the host
 (``awb_flow.cu``, ``awb_tc_fit.cu``, ``awb_internal.cuh``).  Each case below is a shape on ONE side of such a branch:
 the shared-memory / global-memory variants of the RealNVP backward (``k_flow_bwd<3>``, ``k_flow_bwd<2>``,
-``k_flow_bwd_seg``), empty and ragged pixel ranges, full / remainder rounds, and the tile and CTA edges of the tensor path.
+``k_flow_bwd_seg``), empty and ragged pixel ranges, full / remainder rounds, the tile and CTA edges of the tensor path, and
+the ICNN widths and depths of the exact path (``k_gemm``'s 144-column output tiles, ``k_out``'s columns per lane).
 ``regime()`` restates the host formulas; every case names the branch it is meant to hit and the test asserts that the
 restatement agrees, so a case fails loudly if the constants move instead of quietly covering something else.
 
@@ -62,6 +63,7 @@ FLOW_RED_FLOATS = 16 * 128 + 16 * 16
 FLOW_TAB, FLOW_SEG_ROWS, FLOW_SEG_RS = 456, 132, 144
 DZ_SMEM_LIMIT = 200 * 1024    # flow_bwd_dz_in_smem
 SEG_SMEM_LIMIT = 220 * 1024   # flow_backward's limit for flow_seg_bwd_smem
+GEMM_TILE = 144               # awb_simt.cu kGemmTile: output columns (MODE 2: also rows) of one k_gemm CTA
 
 
 def cdiv(a, b):
@@ -145,6 +147,14 @@ def tc_geometry(n, O, sms):
     return dict(n_tiles=n_tiles, grid=min(n_tiles, max(sms // O, 1)), rem=n % 128)
 
 
+def exact_geometry(C_, h):
+    """awb_api.cu ``make_layout`` and the awb_simt.cu launchers: the augmented row width ``ld``, k_gemm's output column
+    tiles (forward, dgrad, tangent) and weight-gradient row tiles, and the per-lane columns ``Q`` of k_out / k_tan_out."""
+    ld = round_up(h + C_ + 1, 8)
+    return {"ld": ld, "gemm.col_tiles": cdiv(ld, GEMM_TILE), "gemm.row_tiles": cdiv(h, GEMM_TILE),
+            "out.Q": 5 if ld <= 160 else 9}
+
+
 def regime(case, sms):
     """Flat dict of everything the host decides for this case (keys ``fwd.*``, ``bwd.*``, ``tc.*``)."""
     n = case["B"] * case["H"] * case["W"]
@@ -156,6 +166,8 @@ def regime(case, sms):
         out.update({f"bwd.{k}": v for k, v in flow_bwd_geometry(case["C"], case["F"], n, seg).items()})
     else:
         out.update({f"bwd.{k}": v for k, v in flow_bwd_geometry(2, 0, n, False).items() if k in ("S", "chunk", "empty", "last")})
+    if case["precision"] == "fp32":
+        out.update(exact_geometry(case["C"], case.get("h", 130)))
     if case["precision"] == "f16":
         out.update({f"tc.{k}": v for k, v in tc_geometry(n, case.get("O", 1), sms).items()})
     return out
@@ -173,11 +185,12 @@ def check_regime(case):
 def make_models(A, case, seed=0):
     """``O`` priors of the case's configuration with non-trivial couplings and ActNorm, in state_dict order."""
     models = []
+    h = case.get("h", 130)
     for o in range(case.get("O", 1)):
         torch.manual_seed(seed + 17 * o)
         if case["kind"] == "flow":
             m = A.real_nvp_path_connected_net(channels=case["C"], hidden_units=32, flow_n_flows=case["F"], flow_output_fn="tanh",
-                                              norm="minmax", convex_net_hidden_units=130, convex_net_hidden_layers=case["L"],
+                                              norm="minmax", convex_net_hidden_units=h, convex_net_hidden_layers=case["L"],
                                               precision=case["precision"])
             sd = m.state_dict()
             for k in sd:
@@ -188,8 +201,11 @@ def make_models(A, case, seed=0):
                 elif k.endswith("data_dep_init_done"):
                     sd[k] = torch.ones_like(sd[k])
             m.load_state_dict(sd)
+        elif case["kind"] == "convexnet":
+            assert case["L"] == 1
+            m = A.ConvexNet(n_hidden=h, in_channels=case["C"], precision=case["precision"])
         else:
-            m = A.ConvexNextNet(in_features=case["C"], n_hidden_layers=case["L"], precision=case["precision"])
+            m = A.ConvexNextNet(n_hidden=h, in_features=case["C"], n_hidden_layers=case["L"], precision=case["precision"])
         models.append(m.to(DEV))
     return models
 
@@ -198,13 +214,14 @@ def make_handle(A, case, models):
     """One native handle for the ``O`` objects (grouped launch) and the ``[O, P]`` parameter arena."""
     L = A._lib
     prec = L.AWB_PREC_F16 if case["precision"] == "f16" else L.AWB_PREC_FP32
+    h = case.get("h", 130)
     if case["kind"] == "flow":
-        prior = A.Prior(L.AWB_KIND_FLOW_ICNN, case["C"], 130, case["L"], n_flows=case["F"], flow_hidden=32, flow_tanh=True,
+        prior = A.Prior(L.AWB_KIND_FLOW_ICNN, case["C"], h, case["L"], n_flows=case["F"], flow_hidden=32, flow_tanh=True,
                         n_objects=len(models), precision=prec)
         models[0].flow_eval = case.get("flow_eval", 0)
         models[0]._push_consts(prior)
     else:
-        prior = A.Prior(L.AWB_KIND_ICNN, case["C"], 130, case["L"], n_objects=len(models), precision=prec)
+        prior = A.Prior(L.AWB_KIND_ICNN, case["C"], h, case["L"], n_objects=len(models), precision=prec)
     params = torch.stack([m._ensure_flat().detach() for m in models]).contiguous()
     assert params.shape[1] == prior.n_params
     return prior, params
@@ -248,7 +265,8 @@ def reference(model, kind, rows, target, last, chunk_rows=1 << 18):
     """float64 oracle of one object on pixel rows ``[N, C]``: logits, deformation, loss (SE of the sigmoid, mean), every
     parameter gradient, and the gradient with the rows ``last = (r0, r1)`` removed from the loss (same 1/N).  Rows are
     processed in chunks (one of them exactly ``last``); the gradients of the chunks are added in float64."""
-    names = [k for k, _ in model.named_parameters()]
+    by_id = {id(q): k for k, q in model.named_parameters()}
+    names = [by_id[id(q)] for q in model._arena_params()]      # flat arena order (ConvexNet's is not its state_dict's)
     p = {k: v.detach().to(DEV, torch.float64).clone() for k, v in model.state_dict().items()}
     for k in names:
         p[k].requires_grad_(True)
@@ -265,7 +283,7 @@ def reference(model, kind, rows, target, last, chunk_rows=1 << 18):
             y = O.icnn_forward(p, xd, "convex_net.").reshape(-1)
             deformed.append(xd.detach())
         else:
-            y = O.icnn_forward(p, O.pixelize(x)).reshape(-1)
+            y = (O.convexnet_forward if kind == "convexnet" else O.icnn_forward)(p, O.pixelize(x)).reshape(-1)
         l = ((target[a:b].double() - torch.sigmoid(y)) ** 2).sum() / N
         gs = torch.autograd.grad(l, [p[k] for k in names])
         for acc, g in zip(grads, gs):
@@ -318,8 +336,8 @@ def run_kernels(A, case, prior, params, spec, target, mode):
 
 
 # --------------------------------------------------------------------------------------------- exact fp32 path: the cases
-def _case(id_, branch, kind, C_, F, B, H, W, expect, O_=1, flow_eval=1, L=2):
-    return dict(id=id_, branch=branch, kind=kind, C=C_, F=F, L=L, B=B, H=H, W=W, O=O_, flow_eval=flow_eval,
+def _case(id_, branch, kind, C_, F, B, H, W, expect, O_=1, flow_eval=1, L=2, h=130):
+    return dict(id=id_, branch=branch, kind=kind, C=C_, F=F, L=L, h=h, B=B, H=H, W=W, O=O_, flow_eval=flow_eval,
                 precision="fp32", expect=expect)
 
 
@@ -375,6 +393,42 @@ FP32_CASES.append(_case("c3-r1-remainder", "R = 2 plus one remainder round, C = 
                         {"bwd.R": 2, "bwd.rounds1": 1, "bwd.dz_smem": True}))
 FP32_CASES.append(_case("icnn-c3-n37889", "ICNN alone: empty trailing ranges of the exact path's reductions", "icnn", 3, 0, 1,
                         1, 37889, {"bwd.empty": 4}, L=1))
+# ICNN widths and depths of the exact path: the augmented row ld = round_up(h + C + 1, 8) against k_gemm's 144-column output
+# tile (skip and bias columns past column 144 from h = 141 / 142), its 144-row weight-gradient tile (from h = 145) and
+# k_out's 5 / 9 columns per lane.  Three frames of 17 x 29 unless noted: 6 pixel ranges, ragged last pixel block.
+WIDTH_CASES = [
+    _case("c2-h8-L1", "smallest width, two pixel ranges", "icnn", 2, 0, 1, 1, 257,
+          {"ld": 16, "gemm.col_tiles": 1, "bwd.S": 2}, L=1, h=8),
+    _case("c3-h37-L0", "no hidden layer (no k_gemm)", "icnn", 3, 0, 3, 17, 29, {"ld": 48, "out.Q": 5}, L=0, h=37),
+    _case("c3-h130-L0", "no hidden layer at the default width", "icnn", 3, 0, 3, 17, 29, {"ld": 136}, L=0, h=130),
+    _case("c2-h141-L2", "last row of one column tile", "icnn", 2, 0, 3, 17, 29, {"ld": 144, "gemm.col_tiles": 1}, h=141),
+    _case("c3-h140-L2", "last row of one column tile, C = 3", "icnn", 3, 0, 3, 17, 29, {"ld": 144, "gemm.col_tiles": 1},
+          h=140),
+    _case("c2-h142-L1", "first two-tile row: bias column 145 in the second tile", "icnn", 2, 0, 3, 17, 29,
+          {"ld": 152, "gemm.col_tiles": 2, "gemm.row_tiles": 1}, L=1, h=142),
+    _case("c3-h141-L2", "first two-tile row, C = 3: skip columns 141..143, bias column 144", "icnn", 3, 0, 3, 17, 29,
+          {"ld": 152, "gemm.col_tiles": 2, "gemm.row_tiles": 1}, h=141),
+    _case("c2-h144-L2", "last weight gradient of one row tile", "icnn", 2, 0, 3, 17, 29,
+          {"ld": 152, "gemm.col_tiles": 2, "gemm.row_tiles": 1}, h=144),
+    _case("c2-h145-L2", "first weight gradient of two row tiles", "icnn", 2, 0, 3, 17, 29,
+          {"ld": 152, "gemm.col_tiles": 2, "gemm.row_tiles": 2}, h=145),
+    _case("c2-h157-L1", "k_out<5> at its widest row", "icnn", 2, 0, 3, 17, 29, {"ld": 160, "out.Q": 5}, L=1, h=157),
+    _case("c2-h158-L1", "k_out<9> at its narrowest row", "icnn", 2, 0, 3, 17, 29, {"ld": 168, "out.Q": 9}, L=1, h=158),
+    _case("c2-h130-L8", "deepest, default width", "icnn", 2, 0, 3, 17, 29, {"ld": 136, "gemm.col_tiles": 1}, L=8),
+    _case("c3-h200-L8", "deepest, two tiles, empty trailing pixel ranges", "icnn", 3, 0, 1, 1, 37889,
+          {"ld": 208, "gemm.col_tiles": 2, "gemm.row_tiles": 2, "bwd.empty": 4}, L=8, h=200),
+    _case("c2-h256-L8", "widest and deepest", "icnn", 2, 0, 3, 17, 29,
+          {"ld": 264, "gemm.col_tiles": 2, "gemm.row_tiles": 2, "out.Q": 9}, L=8, h=256),
+    _case("c3-h256-L2-frame", "widest on a 640x480 frame", "icnn", 3, 0, 1, 480, 640,
+          {"ld": 264, "gemm.col_tiles": 2, "gemm.row_tiles": 2, "bwd.S": 148}, h=256),
+    _case("c2-h200-L2-o4", "4 grouped objects: grid.z over objects with grid.y > 1", "icnn", 2, 0, 3, 17, 29,
+          {"ld": 208, "gemm.col_tiles": 2, "gemm.row_tiles": 2}, O_=4, h=200),
+    _case("flow-c3-h200-L2", "RealNVP prior (F = 18) on a two-tile ICNN", "flow", 3, 18, 3, 17, 29,
+          {"ld": 208, "gemm.col_tiles": 2, "bwd.kernel": "k_flow_bwd<3>"}, h=200),
+    _case("convexnet-h200", "ConvexNet naming, two tiles", "convexnet", 2, 0, 3, 17, 29, {"ld": 208, "gemm.col_tiles": 2},
+          L=1, h=200),
+]
+FP32_CASES += WIDTH_CASES
 
 
 @pytest.mark.parametrize("case", FP32_CASES, ids=[c["id"] for c in FP32_CASES])

@@ -150,6 +150,9 @@ EXACT = [
     _c("L3-c3-n257-eik", "icnn", 3, 130, 3, 1, 1, 257, "eikonal"),
     _c("h37-L2-c2-b2-eik", "icnn", 2, 37, 2, 2, 120, 160, "eikonal"),
     _c("h37-L3-c3-calib-bce", "icnn", 3, 37, 3, 1, 480, 640, "bce"),
+    # rows wider than one k_gemm tile (ld = 208, 264 > 144): the tangent forward, dgrad and wgrad in two column tiles
+    _c("h200-L2-c3-b2-eik", "icnn", 3, 200, 2, 2, 96, 160, "eikonal"),
+    _c("h256-L1-c2-rows-bce", "icnn", 2, 256, 1, 1, 1, 2000, "bce", rows=True),
     _c("convexnet-bce", "convexnet", 2, 130, 1, 1, 240, 320, "bce"),
     _c("convexnet-rows-sq", "convexnet", 2, 130, 1, 1, 1, 37888, "sq", rows=True),
 ]
