@@ -83,6 +83,8 @@ SYMBOLS = [
     ("awb_prior_grid_grad_backward", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P, _P, _P, _P, C.c_size_t, _P]),
     ("awb_prior_deformation", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, C.c_int32, _P, C.c_size_t, _P]),
     ("awb_prior_deformation_backward", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P, _P, _P, C.c_size_t, _P]),
+    ("awb_prior_inverse", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, C.c_int32, _P, C.c_size_t, _P]),
+    ("awb_prior_inverse_backward", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, _P, _P, _P, C.c_size_t, _P]),
     ("awb_prior_fit_step", C.c_int, [_P, _P, _P, C.POINTER(GridSpec), _P, C.POINTER(LossSpec),
                                      C.POINTER(OptHyper), _P, _P, C.c_size_t, C.c_int32, _P]),
     ("awb_prior_fit_steps", C.c_int, [_P, _P, _P, C.POINTER(GridSpec), C.POINTER(_P), C.c_int32, C.c_int32, C.c_int32,

@@ -186,6 +186,28 @@ class Prior:
                                                         ws.data_ptr(), ws.numel(), L.stream_ptr()))
         return grads, dgrid
 
+    def inverse(self, params: torch.Tensor, grid: GridSpecHost, training: bool, ws: torch.Tensor) -> torch.Tensor:
+        """``PathConnectedNet.inverse`` of the explicit ``grid``: pixel rows ``[N, C]``.  ``ws``: layout
+        ``AWB_WS_DEFORMATION``; ``training`` keeps the coupling records for ``inverse_backward``."""
+        out = torch.empty((grid.n_pixels, self.C), dtype=torch.float32, device=params.device)
+        gs = grid.to_c()
+        L.check(self.lib.awb_prior_inverse(self._h, params.data_ptr(), C.byref(gs), out.data_ptr(), int(bool(training)),
+                                           ws.data_ptr(), ws.numel(), L.stream_ptr()))
+        return out
+
+    def inverse_backward(self, params: torch.Tensor, grid: GridSpecHost, d_out: torch.Tensor, ws: torch.Tensor,
+                         want_dgrid: bool) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+        """Gradients of ``inverse(training=True)`` on the same ``ws`` for the upstream ``d_out`` (``[N, C]`` fp32,
+        contiguous): ``grads [P]`` (ICNN entries 0) and, when asked, ``dgrid [B, C, H, W]``."""
+        grads = torch.empty(self.n_params, dtype=torch.float32, device=params.device)
+        dgrid = torch.empty((grid.B, self.C, grid.H, grid.W), dtype=torch.float32, device=params.device) \
+            if want_dgrid else None
+        gs = grid.to_c()
+        L.check(self.lib.awb_prior_inverse_backward(self._h, params.data_ptr(), C.byref(gs), d_out.data_ptr(),
+                                                    grads.data_ptr(), dgrid.data_ptr() if dgrid is not None else None,
+                                                    ws.data_ptr(), ws.numel(), L.stream_ptr()))
+        return grads, dgrid
+
     def enforce_convexity(self, params: torch.Tensor) -> None:
         L.check(self.lib.awb_prior_enforce_convexity(self._h, params.data_ptr(), L.stream_ptr()))
 

@@ -462,6 +462,40 @@ int awb_prior_deformation_backward(awb_handle h, const float* params, const awb_
   return simt_reduce_grads(h, grads, w, w.N, st, /*n_partials=*/0);   // no ICNN partials: its entries are exactly 0
 }
 
+// PathConnectedNet.inverse with autograd: single-object RealNVP o ICNN handles, explicit grid; carves layout
+// AWB_WS_DEFORMATION
+static int check_inverse(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, Workspace* w) {
+  if (!h || !g) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if (h->desc.kind != AWB_KIND_FLOW_ICNN) { set_error("needs a flow prior with its constants set"); return AWB_ERR_INVALID; }
+  if (h->desc.n_objects != 1) {
+    set_error("the inverse entry points support single-object flow priors (%d objects)", h->desc.n_objects);
+    return AWB_ERR_UNSUPPORTED;
+  }
+  if (g->mode != AWB_GRID_EXPLICIT) { set_error("inverse takes an explicit [B,C,H,W] tensor"); return AWB_ERR_INVALID; }
+  return check_common(h, g, ws, ws_bytes, AWB_WS_DEFORMATION, nullptr, w);
+}
+
+int awb_prior_inverse(awb_handle h, const float* params, const awb_grid_spec* g, float* out, int32_t training,
+                      void* ws, size_t ws_bytes, void* stream) {
+  Workspace w;
+  int rc = check_inverse(h, g, ws, ws_bytes, &w);
+  if (rc) return rc;
+  if (!params || !out) { set_error("null argument"); return AWB_ERR_INVALID; }
+  return flow_inverse(h, params, g, out, (cudaStream_t)stream, training ? &w : nullptr);
+}
+
+int awb_prior_inverse_backward(awb_handle h, const float* params, const awb_grid_spec* g, const float* d_out,
+                               float* grads, float* dgrid, void* ws, size_t ws_bytes, void* stream) {
+  Workspace w;
+  int rc = check_inverse(h, g, ws, ws_bytes, &w);
+  if (rc) return rc;
+  if (!params || !d_out || !grads) { set_error("null argument"); return AWB_ERR_INVALID; }
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = flow_inverse_backward(h, params, g, w, d_out, dgrid, st);
+  if (rc) return rc;
+  return simt_reduce_grads(h, grads, w, w.N, st, /*n_partials=*/0);   // no ICNN partials: its entries are exactly 0
+}
+
 // single-object ICNN and RealNVP o ICNN handles (the priors of the spatio-temporal fit)
 static int check_sliceable(awb_handle h) {
   if (!h) { set_error("null argument"); return AWB_ERR_INVALID; }

@@ -378,8 +378,12 @@ __global__ void __launch_bounds__(256) k_flow_fwd(FlowP p) {
 // ---------------------------------------------------------------- inverse (PathConnectedNet.inverse, path_connected_net.py:107-122)
 // x (a get_deformation output) -> MinMax -> flows in reverse order, each inverted (ActNorm: (z - t) exp(-s);
 // coupling: zm + (1 - b)(z - t(zm)) exp(-s(zm)), normflows MaskedAffineFlow.inverse) -> inverse MinMax -> inverse 1x1 conv.
-template <int C>
-__global__ void __launch_bounds__(256) k_flow_inv(FlowP p, float* out) {
+// REC (training inverse, k_flow_inv_rec): also keeps what k_flow_inv_bwd needs, with the same arithmetic.  Per pixel and
+// flow, in the record format of the forward (FlowSave) at slot F - 1 - f (the order the inverse visits the flows, so that
+// the backward walks the slots like k_flow_bwd does): the coupling's input u (after the ActNorm inverse) and its s, t after
+// the output function.  Per pixel, in p.X: the coordinates in front of the inverse 1x1 conv.
+template <int C, bool REC>
+__device__ __forceinline__ void flow_inv_body(const FlowP& p, float* out) {
   extern __shared__ float sp[];   // [P_flow + 2C]
   const int o = blockIdx.y;
   const float* par = p.params + (int64_t)o * p.P + p.off_flow;
@@ -418,21 +422,39 @@ __global__ void __launch_bounds__(256) k_flow_inv(FlowP p, float* out) {
         to[c] = fmaf(w[half + m * C + m + c * m + k], ht, to[c]);
       }
     }
+    float u[3] = {0.f, 0.f, 0.f}, sv[2] = {0.f, 0.f}, tv[2] = {0.f, 0.f};
+    int nu = 0;
 #pragma unroll
     for (int c = 0; c < C; c++) {
       float s_ = p.tanh_out ? p.out_scale * tanhf(so[c]) : so[c];
       float t_ = p.tanh_out ? p.out_scale * tanhf(to[c]) : to[c];
       if (!isfinite(s_)) s_ = NAN;
       if (!isfinite(t_)) t_ = NAN;
+      if constexpr (REC) {
+        u[c] = z[c];
+        if (!b[c]) { if (nu == 0) { sv[0] = s_; tv[0] = t_; } else { sv[1] = s_; tv[1] = t_; } nu++; }
+      }
       if (!b[c]) z[c] = (z[c] - t_) * expf(-s_);
     }
+    if constexpr (REC) {
+      float4* rec = reinterpret_cast<float4*>(p.zin + (((int64_t)o * p.F + (p.F - 1 - f)) * p.N + n) * FlowSave<C>::RW);
+      if (C == 2) rec[0] = make_float4(u[0], u[1], sv[0], tv[0]);
+      else { rec[0] = make_float4(u[0], u[1], u[2], sv[0]); rec[1] = make_float4(sv[1], tv[0], tv[1], 0.f); }
+    }
   }
+  float xs[3] = {0.f, 0.f, 0.f};
 #pragma unroll
   for (int c = 0; c < C; c++) {
     float x = mm_fwd(z[c], p.fc.new_min, p.fc.new_max, p.fc.nmin[c], p.fc.nmax[c]);
+    xs[c] = x;
     out[((int64_t)o * p.N + n) * C + c] = (1.0f / lin[c]) * (x - lin[C + c]);
   }
+  if constexpr (REC) *reinterpret_cast<float4*>(p.X + ((int64_t)o * p.N + n) * 4) = make_float4(xs[0], xs[1], xs[2], 1.f);
 }
+template <int C>
+__global__ void __launch_bounds__(256) k_flow_inv(FlowP p, float* out) { flow_inv_body<C, false>(p, out); }
+template <int C>
+__global__ void __launch_bounds__(256) k_flow_inv_rec(FlowP p, float* out) { flow_inv_body<C, true>(p, out); }
 
 // ---------------------------------------------------------------- backward
 // ONE kernel, no per-pixel record through global memory.  A CTA owns a pixel range and walks the flows in reverse; the
@@ -563,8 +585,13 @@ __device__ __forceinline__ void prefetch_round(const FlowP& p, float* stage_buf,
   }
 }
 
-// one flow with NM masked components (mask pattern mb) over the CTA's pixel range
-template <int C, int NM>
+// one flow with NM masked components (mask pattern mb) over the CTA's pixel range.
+// INV: backward of the flow's inverse (k_flow_inv_bwd): dzg holds the gradient at the coupling's output and receives the
+// gradient at the ActNorm inverse's input; the records (u, s, t of k_flow_inv_rec) sit at slot F - 1 - f.  With
+// g = dzg, e = exp(-s) on a transformed component: du = g e, dt = -g e, ds = -g (u - t) e; on a masked one du = g + the MLP
+// path.  ActNorm inverse u = (z - a_t) exp(-a_s): dz = du exp(-a_s), d a_t = -du exp(-a_s), d a_s = -du u.  The MLP part
+// (unit loop, reduction, conversion) is the forward's.
+template <int C, int NM, bool INV = false>
 __device__ __forceinline__ void flow_bwd_one(const FlowP& p, const FlowBwdShared& sh, int f, int mb, int o, int64_t r0, int64_t r1,
                                              float* dzg, int dz_cs, int dz_ps, FlowStep& pre, int& buf) {
   using Cf = FlowBwdCfg<C, NM>;
@@ -573,7 +600,7 @@ __device__ __forceinline__ void flow_bwd_one(const FlowP& p, const FlowBwdShared
   const int T = blockDim.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = T >> 5;
   const int m = p.m, half = 2 * m * C + m + C;
   const float* wf = sh.wrec + f * FlowBwdPack<C>::flow_stride();
-  const float* zrec = p.zin + (((int64_t)o * p.F + f) * p.N) * RW;
+  const float* zrec = p.zin + (((int64_t)o * p.F + (INV ? p.F - 1 - f : f)) * p.N) * RW;
   // roles: mi[i] = i-th masked component, ui[j] = j-th transformed component (ascending)
   int mi[NM], ui[NU];
   {
@@ -583,11 +610,19 @@ __device__ __forceinline__ void flow_bwd_one(const FlowP& p, const FlowBwdShared
       if ((mb >> c) & 1) { if (a < NM) mi[a] = c; a++; } else { if (b < NU) ui[b] = c; b++; }
     }
   }
-  float ea_m[NM], ea_u[NU];
+  float ea_m[NM], ea_u[NU];      // exp(ActNorm.s); INV: exp(-ActNorm.s)
+  if constexpr (INV) {
+    const float* an_s = p.params + (int64_t)o * p.P + p.off_flow + (int64_t)f * p.per_flow + 2 * half;
 #pragma unroll
-  for (int i = 0; i < NM; i++) ea_m[i] = wf[32 * RKB + mi[i]];
+    for (int i = 0; i < NM; i++) ea_m[i] = expf(-an_s[mi[i]]);
 #pragma unroll
-  for (int j = 0; j < NU; j++) ea_u[j] = wf[32 * RKB + ui[j]];
+    for (int j = 0; j < NU; j++) ea_u[j] = expf(-an_s[ui[j]]);
+  } else {
+#pragma unroll
+    for (int i = 0; i < NM; i++) ea_m[i] = wf[32 * RKB + mi[i]];
+#pragma unroll
+    for (int j = 0; j < NU; j++) ea_u[j] = wf[32 * RKB + ui[j]];
+  }
   // per-thread scalar sums: d ActNorm.s / .t of the masked and of the transformed components, d s.b2 / d t.b2
   float sas_m[NM], sat_m[NM], sas_u[NU], sat_u[NU], sb2s[NU], sb2t[NU];
 #pragma unroll
@@ -634,23 +669,41 @@ __device__ __forceinline__ void flow_bwd_one(const FlowP& p, const FlowBwdShared
         for (int i = 0; i < NM; i++) {          // masked components pass through the coupling
           const float zc = pick<C>(z, mi[i]), dzc = pick<C>(dz, mi[i]);
           zm[q][i] = zc;
-          if (last_pass) { sas_m[i] = fmaf(dzc * zc, ea_m[i], sas_m[i]); sat_m[i] += dzc; }
+          if constexpr (!INV) {
+            if (last_pass) { sas_m[i] = fmaf(dzc * zc, ea_m[i], sas_m[i]); sat_m[i] += dzc; }
+          }
         }
 #pragma unroll
-        for (int j = 0; j < NU; j++) {          // transformed components: z' = z exp(s) + t
+        for (int j = 0; j < NU; j++) {          // transformed components: z' = z exp(s) + t  (INV: (u - t) exp(-s))
           const float zc = pick<C>(z, ui[j]), dzc = pick<C>(dz, ui[j]);
-          const float dzp = dzc * ea_u[j];
-          const float e = (p.tanh_out && p.out_scale == 1.f) ? exp_sfu(s[j]) : expf(s[j]);      // the same function as the forward
-          const float isc = p.inv_out_scale;
-          const float dsv = dzp * zc * e;
-          ds[q][j] = p.tanh_out ? dsv * p.out_scale * (1.f - (s[j] * isc) * (s[j] * isc)) : dsv;     // d (c tanh a) / da = c (1 - tanh^2)
-          dt[q][j] = p.tanh_out ? dzp * p.out_scale * (1.f - (t[j] * isc) * (t[j] * isc)) : dzp;
-          dzo_u[q][j] = dzp * e;
-          if (last_pass) {
-            sas_u[j] = fmaf(dzc * fmaf(zc, e, t[j]), ea_u[j], sas_u[j]);
-            sat_u[j] += dzc;
-            sb2s[j] += ds[q][j];
-            sb2t[j] += dt[q][j];
+          if constexpr (INV) {
+            const float isc = p.inv_out_scale;
+            const float e = expf(-s[j]);              // the function of the inverse
+            const float du = dzc * e;
+            const float dsv = -dzc * ((zc - t[j]) * e);
+            ds[q][j] = p.tanh_out ? dsv * p.out_scale * (1.f - (s[j] * isc) * (s[j] * isc)) : dsv;
+            dt[q][j] = p.tanh_out ? -du * p.out_scale * (1.f - (t[j] * isc) * (t[j] * isc)) : -du;
+            dzo_u[q][j] = du * ea_u[j];
+            if (last_pass) {
+              sas_u[j] = fmaf(-du, zc, sas_u[j]);
+              sat_u[j] = fmaf(-du, ea_u[j], sat_u[j]);
+              sb2s[j] += ds[q][j];
+              sb2t[j] += dt[q][j];
+            }
+          } else {
+            const float dzp = dzc * ea_u[j];
+            const float e = (p.tanh_out && p.out_scale == 1.f) ? exp_sfu(s[j]) : expf(s[j]);      // the same function as the forward
+            const float isc = p.inv_out_scale;
+            const float dsv = dzp * zc * e;
+            ds[q][j] = p.tanh_out ? dsv * p.out_scale * (1.f - (s[j] * isc) * (s[j] * isc)) : dsv;     // d (c tanh a) / da = c (1 - tanh^2)
+            dt[q][j] = p.tanh_out ? dzp * p.out_scale * (1.f - (t[j] * isc) * (t[j] * isc)) : dzp;
+            dzo_u[q][j] = dzp * e;
+            if (last_pass) {
+              sas_u[j] = fmaf(dzc * fmaf(zc, e, t[j]), ea_u[j], sas_u[j]);
+              sat_u[j] += dzc;
+              sb2s[j] += ds[q][j];
+              sb2t[j] += dt[q][j];
+            }
           }
 #pragma unroll
           for (int i = 0; i < NM; i++) { us[q][j * NM + i] = ds[q][j] * zm[q][i]; ut[q][j * NM + i] = dt[q][j] * zm[q][i]; Ds[q][j * NM + i] = 0.f; Dt[q][j * NM + i] = 0.f; }
@@ -698,6 +751,12 @@ __device__ __forceinline__ void flow_bwd_one(const FlowP& p, const FlowBwdShared
           for (int u = 0; u < NU; u++) g = fmaf(ds[q][u], Ds[q][u * NM + i], fmaf(dt[q][u], Dt[q][u * NM + i], g));
           if (NPASS > 1 && pass > 0) g += sh.dzp[mi[i] * sh.dzp_cs + n * sh.dzp_ps];
           if (!last_pass) sh.dzp[mi[i] * sh.dzp_cs + n * sh.dzp_ps] = g;
+          else if constexpr (INV) {      // du = g_out + MLP path, then the ActNorm inverse
+            const float du = dzg[mi[i] * dz_cs + n * dz_ps] + g;
+            sas_m[i] = fmaf(-du, zm[q][i], sas_m[i]);
+            sat_m[i] = fmaf(-du, ea_m[i], sat_m[i]);
+            dzg[mi[i] * dz_cs + n * dz_ps] = du * ea_m[i];
+          }
           else dzg[mi[i] * dz_cs + n * dz_ps] = fmaf(dzg[mi[i] * dz_cs + n * dz_ps], ea_m[i], g);      // dz * exp(ActNorm.s) + MLP path
         }
         if (last_pass) {
@@ -902,6 +961,105 @@ __global__ void __launch_bounds__(FLOW_BWD_T, 1) k_flow_bwd(FlowP p) {
     float a = 0.f;
     for (int w = 0; w < nwarps; w++) a += red2[w * 16 + tid];
     outb[p.P_flow + tid] = p.use_linear ? a : 0.f;
+  }
+}
+
+// ---------------------------------------------------------------- backward of the inverse (PathConnectedNet.inverse)
+// The layout of k_flow_bwd (pixel-range CTAs, running gradient in shared memory or in place in p.dX, fixed-order partials)
+// for x -> MinMax -> F x {ActNorm^-1, coupling^-1} (f = F-1 .. 0) -> MinMax^-1 -> conv^-1 (k_flow_inv_rec's records): the
+// flows are walked in the order f = 0 .. F-1.  Upstream d_out [O][N][C]; out = (v - b) / w gives dv = d_out / w,
+// db = -d_out / w, dw = -d_out out / w.  DX: d / d x (the input grid, planar [B][C][H][W]) into p.dgrid.
+template <int C, bool DX>
+__global__ void __launch_bounds__(FLOW_BWD_T, 1) k_flow_inv_bwd(FlowP p, const float* __restrict__ d_out) {
+  extern __shared__ __align__(16) float sp[];
+  constexpr int RW = FlowSave<C>::RW;
+  const int o = blockIdx.y, tid = threadIdx.x, T = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = T >> 5;
+  const float* par = p.params + (int64_t)o * p.P + p.off_flow;
+  const int PF = (int)p.P_flow + 2 * C;
+  const int64_t r0 = (int64_t)blockIdx.x * p.chunk, r1 = r0 + p.chunk < p.N ? r0 + p.chunk : p.N;
+  FlowBwdShared sh;
+  sh.wrec = sp;
+  sh.red = sp + p.F * FlowBwdPack<C>::flow_stride();
+  sh.stage = sh.red + 2 * FLOW_RED_FLOATS;
+  float* after = sh.stage + 2 * FLOW_PB * (RW / 4) * FLOW_BWD_T * 4;
+  float* dzs = p.dz_smem ? after : nullptr;
+  sh.dzp = p.dz_smem ? after + C * p.chunk : p.dzp_g + ((int64_t)o * p.N + r0) * 4;   // C = 3 only (two unit passes)
+  sh.dzp_cs = p.dz_smem ? (int)p.chunk : 1; sh.dzp_ps = p.dz_smem ? 1 : 4;
+  stage_flow_bwd<C>(par, p.F, p.m, p.per_flow, sp, p.fc);
+  float* outb = p.fpart + ((int64_t)blockIdx.x * p.O + o) * PF;
+  if (r0 >= p.N) {          // empty range (rounded-up chunk): its partial is all zeros
+    for (int i = tid; i < PF; i += T) outb[i] = 0.f;
+    return;
+  }
+  FlowStep pre = {p.F - 1, 0, -1};      // record slots F-1 .. 0 = flows 0 .. F-1
+  int buf = 0;
+  if (p.rounds > 0) {
+    pre.r = 0;
+    prefetch_round<C, FLOW_PB>(p, sh.stage, pre, o, r0, (int)(r1 - r0));
+    asm volatile("cp.async.commit_group;" ::: "memory");
+  } else {
+    pre.f = -1;
+  }
+  float lw[C];
+#pragma unroll
+  for (int c = 0; c < C; c++) lw[c] = par[p.P_flow + c];
+  float* dzg = p.dz_smem ? dzs : p.dX + ((int64_t)o * p.N + r0) * 4;
+  const int dz_cs = p.dz_smem ? (int)p.chunk : 1, dz_ps = p.dz_smem ? 1 : 4;
+  for (int64_t n = r0 + tid; n < r1; n += T) {
+#pragma unroll
+    for (int c = 0; c < C; c++)
+      dzg[c * dz_cs + (int)(n - r0) * dz_ps] = (1.0f / lw[c]) * d_out[((int64_t)o * p.N + n) * C + c] *
+                                               ((p.fc.nmax[c] - p.fc.nmin[c]) / (p.fc.new_max - p.fc.new_min));
+  }
+  __syncthreads();          // staged weights; the dz slots are thread-private: pixel n is always handled by thread (n - r0) % T
+  for (int f = 0; f < p.F; f++) {
+    int mb = 0;
+#pragma unroll
+    for (int c = 0; c < C; c++) mb |= p.fc.masks[f * C + c] != 0 ? 1 << c : 0;
+    const int nm = __popc(mb);
+    if (nm == 1) flow_bwd_one<C, 1, true>(p, sh, f, mb, o, r0, r1, dzg, dz_cs, dz_ps, pre, buf);
+    if constexpr (C == 3) {
+      if (nm == 2) flow_bwd_one<C, 2, true>(p, sh, f, mb, o, r0, r1, dzg, dz_cs, dz_ps, pre, buf);
+    }
+  }
+  // inverse 1x1 conv: out = (1 / w) (v - b) with v = p.X (k_flow_inv_rec)
+  float glw[C], glb[C];
+#pragma unroll
+  for (int c = 0; c < C; c++) { glw[c] = 0.f; glb[c] = 0.f; }
+  for (int64_t n = r0 + tid; n < r1; n += T) {
+    const float4 v = *reinterpret_cast<const float4*>(p.X + ((int64_t)o * p.N + n) * 4);
+    const float v3[3] = {v.x, v.y, v.z};
+#pragma unroll
+    for (int c = 0; c < C; c++) {
+      const float dv = (1.0f / lw[c]) * d_out[((int64_t)o * p.N + n) * C + c];
+      glw[c] = fmaf(-dv, (1.0f / lw[c]) * (v3[c] - par[p.P_flow + C + c]), glw[c]);
+      glb[c] -= dv;
+    }
+  }
+  if constexpr (DX) {       // input MinMax: one store per pixel and channel
+    for (int64_t n = r0 + tid; n < r1; n += T) {
+#pragma unroll
+      for (int c = 0; c < C; c++)
+        p.dgrid[planar_index(p.g, n, c)] =
+            dzg[c * dz_cs + (int)(n - r0) * dz_ps] * ((p.fc.new_max - p.fc.new_min) / (p.fc.nmax[c] - p.fc.nmin[c]));
+    }
+  }
+  __syncthreads();          // the last flow's conversion threads are done with the scratch
+  float* red2 = sh.red + 16 * 128;
+#pragma unroll
+  for (int c = 0; c < C; c++) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+      glw[c] += __shfl_xor_sync(0xffffffffu, glw[c], off);
+      glb[c] += __shfl_xor_sync(0xffffffffu, glb[c], off);
+    }
+    if (lane == 0) { red2[warp * 16 + c] = glw[c]; red2[warp * 16 + C + c] = glb[c]; }
+  }
+  __syncthreads();
+  if (tid < 2 * C) {
+    float a = 0.f;
+    for (int w = 0; w < nwarps; w++) a += red2[w * 16 + tid];
+    outb[p.P_flow + tid] = a;
   }
 }
 
@@ -1738,14 +1896,25 @@ int flow_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
   return AWB_OK;
 }
 
-int flow_inverse(const awb_prior* h, const float* params, const awb_grid_spec* g, float* out, cudaStream_t st) {
+int flow_inverse(const awb_prior* h, const float* params, const awb_grid_spec* g, float* out, cudaStream_t st,
+                 const Workspace* rec) {
   Workspace none = {};
   none.N = (int64_t)g->B * g->H * g->W;
-  FlowP p = make_p(h, params, g, none);
+  FlowP p = make_p(h, params, g, rec ? *rec : none);
   const int PF = (int)(h->lay.P_flow + 2 * h->lay.C);
   size_t smem = sizeof(float) * PF;
   dim3 grid((unsigned)((p.N + 255) / 256), h->desc.n_objects);
-  if (h->lay.C == 2) {
+  if (rec) {
+    p.zin = rec->flowz;
+    if (!p.zin) { set_error("training inverse needs a deformation workspace"); return AWB_ERR_WORKSPACE; }
+    if (h->lay.C == 2) {
+      AWB_CUDA(cudaFuncSetAttribute(k_flow_inv_rec<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      AWB_LAUNCH(PK_FLOW_FWD, st, k_flow_inv_rec<2><<<grid, 256, smem, st>>>(p, out));
+    } else {
+      AWB_CUDA(cudaFuncSetAttribute(k_flow_inv_rec<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      AWB_LAUNCH(PK_FLOW_FWD, st, k_flow_inv_rec<3><<<grid, 256, smem, st>>>(p, out));
+    }
+  } else if (h->lay.C == 2) {
     AWB_CUDA(cudaFuncSetAttribute(k_flow_inv<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     AWB_LAUNCH(PK_FLOW_FWD, st, k_flow_inv<2><<<grid, 256, smem, st>>>(p, out));
   } else {
@@ -1768,14 +1937,12 @@ bool flow_bwd_dz_in_smem(const awb_prior* h, int64_t N) {
   return flow_bwd_smem_base(h) + dz <= 200 * 1024;
 }
 
-int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
-                  cudaStream_t st, bool use_linear, float* dgrid) {
-  FlowP p = make_p(h, params, g, ws);
-  p.use_linear = use_linear ? 1 : 0;
+// What the unit-loop backward kernels (k_flow_bwd, k_flow_inv_bwd) take: records, width and masks checked, their launch
+// geometry.  T threads; full rounds of FLOW_PB pixels per thread, then the remainder of the range in rounds of one pixel
+// per thread (2080 rows = 2 x 1024 + 32: a third full round for 32 pixels would cost its warp 50 %).
+static int flow_bwd_setup(const awb_prior* h, const Workspace& ws, FlowP& p, FlowGeo& geo, size_t& smem) {
   p.zin = ws.flowz;
-  p.dgrid = dgrid;
   if (!p.zin) { set_error("flow backward needs a training workspace"); return AWB_ERR_WORKSPACE; }
-  if (dgrid && (!use_linear || h->desc.n_objects != 1)) { set_error("internal: dgrid needs one object and the 1x1 conv"); return AWB_ERR_INVALID; }
   if (h->lay.m > 32) { set_error("flow MLP width must be <= 32"); return AWB_ERR_UNSUPPORTED; }
   const int C = h->lay.C;
   for (int f = 0; f < h->lay.F; f++) {
@@ -1786,9 +1953,6 @@ int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
       return AWB_ERR_UNSUPPORTED;
     }
   }
-  // T threads; full rounds of FLOW_PB pixels per thread, then the remainder of the range in rounds of one pixel per thread
-  // (2080 rows = 2 x 1024 + 32: a third full round for 32 pixels would cost its warp 50 %)
-  FlowGeo geo;
   geo.S = n_splits(p.N); geo.chunk = split_chunk(p.N);
   geo.T = (int)(geo.chunk < FLOW_BWD_T ? round_up(geo.chunk, 32) : FLOW_BWD_T);
   geo.R = (int)(geo.chunk / ((int64_t)FLOW_PB * geo.T));
@@ -1797,7 +1961,20 @@ int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
   p.dz_smem = flow_bwd_dz_in_smem(h, p.N) ? 1 : 0;
   p.dzp_g = ws.flowd;
   if (!p.dz_smem && C == 3 && !p.dzp_g) { set_error("flow backward: workspace lacks the pass scratch"); return AWB_ERR_WORKSPACE; }
-  size_t smem = flow_bwd_smem_base(h) + (p.dz_smem ? sizeof(float) * (size_t)geo.chunk * C * (C == 3 ? 2 : 1) : 0);
+  smem = flow_bwd_smem_base(h) + (p.dz_smem ? sizeof(float) * (size_t)geo.chunk * C * (C == 3 ? 2 : 1) : 0);
+  return AWB_OK;
+}
+
+int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
+                  cudaStream_t st, bool use_linear, float* dgrid) {
+  FlowP p = make_p(h, params, g, ws);
+  p.use_linear = use_linear ? 1 : 0;
+  p.dgrid = dgrid;
+  if (dgrid && (!use_linear || h->desc.n_objects != 1)) { set_error("internal: dgrid needs one object and the 1x1 conv"); return AWB_ERR_INVALID; }
+  const int C = h->lay.C;
+  FlowGeo geo;
+  size_t smem;
+  if (int rc = flow_bwd_setup(h, ws, p, geo, smem)) return rc;
   dim3 grid(geo.S, h->desc.n_objects);
   if (flow_seg_path(h) && p.tab) {
     geo.T = FLOW_BWD_T;          // the segment kernel always runs 256 threads (idle ones for tiny ranges)
@@ -1827,6 +2004,26 @@ int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* 
                     : (dgrid ? unit(k_flow_bwd<3, true>) : unit(k_flow_bwd<3, false>));
     if (rc) return rc;
   }
+  AWB_CUDA(cudaGetLastError());
+  return AWB_OK;
+}
+
+int flow_inverse_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
+                          const float* d_out, float* dgrid, cudaStream_t st) {
+  FlowP p = make_p(h, params, g, ws);
+  p.dgrid = dgrid;
+  FlowGeo geo;
+  size_t smem;
+  if (int rc = flow_bwd_setup(h, ws, p, geo, smem)) return rc;
+  dim3 grid(geo.S, h->desc.n_objects);
+  auto unit = [&](auto kernel) -> int {
+    AWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    AWB_LAUNCH(PK_FLOW_BWD, st, kernel<<<grid, geo.T, smem, st>>>(p, d_out));
+    return AWB_OK;
+  };
+  int rc = h->lay.C == 2 ? (dgrid ? unit(k_flow_inv_bwd<2, true>) : unit(k_flow_inv_bwd<2, false>))
+                         : (dgrid ? unit(k_flow_inv_bwd<3, true>) : unit(k_flow_inv_bwd<3, false>));
+  if (rc) return rc;
   AWB_CUDA(cudaGetLastError());
   return AWB_OK;
 }

@@ -231,7 +231,14 @@ int tc_trace_read(unsigned long long* host, int max_ctas);   // debug timeline (
 // ---- flows, implemented in awb_flow.cu ----
 int flow_forward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
                  float* deformed, cudaStream_t st, bool use_linear = true);
-int flow_inverse(const awb_prior* h, const float* params, const awb_grid_spec* g, float* out, cudaStream_t st);
+// rec (optional, single object, layout AWB_WS_DEFORMATION): training inverse, keeps in rec->flowz / rec->X what
+// flow_inverse_backward reads; out is the same either way
+int flow_inverse(const awb_prior* h, const float* params, const awb_grid_spec* g, float* out, cudaStream_t st,
+                 const Workspace* rec = nullptr);
+// backward of flow_inverse(rec = &ws): d_out [N][C] -> flow and 1x1-conv partials in ws.fpart (n_splits(N) pixel
+// ranges), dgrid (optional) = d / d grid [B,C,H,W]
+int flow_inverse_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,
+                          const float* d_out, float* dgrid, cudaStream_t st);
 int flow_identity_loss(const awb_prior* h, const awb_grid_spec* g, const Workspace& ws, cudaStream_t st);
 // dgrid (optional, single object, use_linear): d / d grid [B,C,H,W] = linear.weight[c] * (gradient at the 1x1-conv output)
 int flow_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const Workspace& ws,

@@ -1,7 +1,8 @@
 """Shared machinery of the drop-in prior modules: one flat fp32 parameter arena per module
 (state-dict tensors are views into it), lazy creation of the native handle, and the
-autograd bridges to ``awb_prior_forward`` / ``awb_prior_backward`` and to ``awb_prior_deformation`` /
-``awb_prior_deformation_backward``.  Both backwards are first-order only: a double backward raises.  The exception is an
+autograd bridges to ``awb_prior_forward`` / ``awb_prior_backward``, to ``awb_prior_deformation`` /
+``awb_prior_deformation_backward`` and to ``awb_prior_inverse`` / ``awb_prior_inverse_backward``.  The backwards are
+first-order only: a double backward raises.  The exception is an
 ICNN prior built with ``second_order=True``: under ``create_graph`` its coordinate gradient is differentiable
 (``_GridGradFunction``, ``awb_prior_grid_grad_backward``)."""
 from __future__ import annotations
@@ -200,6 +201,32 @@ class _DeformationFunction(torch.autograd.Function):
             raise RuntimeError("get_deformation's backward runs once per forward (its workspace is released after it)")
         grads, dgrid = ctx.prior.deformation_backward(ctx.module._arena, ctx.spec, d_rows.contiguous().float(), ctx.ws,
                                                       ctx.needs_input_grad[2])
+        ctx.ws = None
+        return (None, None, dgrid) + _split_grads(grads, ctx.shapes)
+
+
+class _InverseFunction(torch.autograd.Function):
+    """``PathConnectedNet.inverse`` with autograd: pixel rows ``[N, C]`` of the points mapped back through the flow.  The
+    forward keeps the coupling records in a private deformation-only workspace; the backward returns the flow and 1x1-conv
+    gradients (the ICNN's are 0) and, when ``x`` requires grad, ``dgrid``."""
+
+    @staticmethod
+    def forward(ctx, module, spec, x, *params):
+        prior = module._prior_for(params[0].device)
+        arena = module._arena
+        ws = prior.new_workspace(spec.n_pixels, L.AWB_WS_DEFORMATION, arena.device)
+        rows = prior.inverse(arena, spec, True, ws)
+        ctx.module, ctx.spec, ctx.ws, ctx.prior = module, spec, ws, prior
+        ctx.shapes = [p.shape for p in params]
+        return rows
+
+    @staticmethod
+    @_first_order_only
+    def backward(ctx, d_rows):
+        if ctx.ws is None:
+            raise RuntimeError("inverse's backward runs once per forward (its workspace is released after it)")
+        grads, dgrid = ctx.prior.inverse_backward(ctx.module._arena, ctx.spec, d_rows.contiguous().float(), ctx.ws,
+                                                  ctx.needs_input_grad[2])
         ctx.ws = None
         return (None, None, dgrid) + _split_grads(grads, ctx.shapes)
 

@@ -15,7 +15,7 @@ from torch import nn
 
 from .. import _lib as L
 from ..core import GridSpecHost, Prior
-from .base import _PRECISIONS, Affine, ArenaPriorModule, reject_second_order
+from .base import _PRECISIONS, Affine, ArenaPriorModule, _InverseFunction, reject_second_order
 from .convex_net import ConvexNextNet
 
 
@@ -290,20 +290,27 @@ class PathConnectedNet(ArenaPriorModule):
         return out[0] if squeeze else out
 
     def inverse(self, x: torch.Tensor, *args, **kwargs) -> torch.Tensor:
-        """``path_connected_net.py:107-122``: inverse of ``get_deformation``.  ``[B,C,H,W] -> [B,C,H,W]``.  Not
-        differentiable: the result carries no autograd graph."""
+        """``path_connected_net.py:107-122``: inverse of ``get_deformation``.  ``[B,C,H,W] -> [B,C,H,W]``.  With grad
+        mode on and ``x`` or a parameter requiring grad it is differentiable w.r.t. the parameters (flow and 1x1 conv; the
+        ICNN's gradients are 0) and ``x``, first order only; otherwise the result carries no autograd graph."""
         squeeze = x.dim() == 3
         if squeeze:
             x = x.unsqueeze(0)
         arena = self._ensure_flat()
         prior = self._prior_for(arena.device)
-        spec = GridSpecHost.from_tensor(x.to(arena.device))
-        gs = spec.to_c()
+        x = x.to(arena.device)
+        spec = GridSpecHost.from_tensor(x)
         B, C_, H, W = x.shape
-        out = torch.empty((spec.n_pixels, C_), dtype=torch.float32, device=arena.device)
-        with torch.no_grad(), torch.cuda.device(arena.device):
-            L.check(prior.lib.awb_prior_flow_inverse(prior.handle, arena.data_ptr(), C.byref(gs), out.data_ptr(),
-                                                     L.stream_ptr()))
+        params = self._arena_params()
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params)):
+            with torch.cuda.device(arena.device):
+                out = _InverseFunction.apply(self, spec, x if x.requires_grad else None, *params)
+        else:
+            gs = spec.to_c()
+            out = torch.empty((spec.n_pixels, C_), dtype=torch.float32, device=arena.device)
+            with torch.no_grad(), torch.cuda.device(arena.device):
+                L.check(prior.lib.awb_prior_flow_inverse(prior.handle, arena.data_ptr(), C.byref(gs), out.data_ptr(),
+                                                         L.stream_ptr()))
         out = out.reshape(B, H, W, C_).permute(0, 3, 1, 2).contiguous()
         return out[0] if squeeze else out
 

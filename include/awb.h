@@ -130,7 +130,8 @@ int awb_prior_destroy(awb_handle h);
                                  point except awb_prior_grid_grad_backward */
 #define AWB_WS_FIT_STEP 2     /* awb_prior_fit_step / _fit_steps / _fit_host_frames / _slice_grads only: much smaller on
                                  tensor-path handles, whose fused kernel keeps the activations on the SM */
-#define AWB_WS_DEFORMATION 3  /* awb_prior_deformation / _deformation_backward only: the flow's buffers (deformed
+#define AWB_WS_DEFORMATION 3  /* awb_prior_deformation / _deformation_backward and awb_prior_inverse /
+                                 _inverse_backward only: the flow's buffers (deformed
                                  coordinates, coupling records, their gradient and the flow's partials), no ICNN
                                  activations; about 80 MB instead of 0.85 GB for a 640x480 C = 2 frame */
 #define AWB_WS_SECOND_ORDER 4 /* awb_prior_forward(AWB_FWD_EXACT_TRAINING) followed by awb_prior_backward and
@@ -231,6 +232,23 @@ int awb_prior_deformation(awb_handle h, const float* params, const awb_grid_spec
  * Must follow awb_prior_deformation(training != 0) on the same workspace and params.  Same handles and errors. */
 int awb_prior_deformation_backward(awb_handle h, const float* params, const awb_grid_spec* grid, const float* d_deformed,
                                    float* grads, float* dgrid, void* workspace, size_t workspace_bytes, void* stream);
+
+/* PathConnectedNet.inverse with a backward.  grid: the points to map back, explicit [B,C,H,W] (AWB_GRID_EXPLICIT);
+ * out: device [N][C] pixel rows, bit-identical to awb_prior_flow_inverse.  training != 0 also keeps, per pixel and flow,
+ * the coupling's input and its s, t (and per pixel the 1x1 conv's input) in the workspace for
+ * awb_prior_inverse_backward.  workspace: layout AWB_WS_DEFORMATION.  Single-object AWB_KIND_FLOW_ICNN handles with the
+ * flow constants set, at both precisions (the flow is exact fp32 either way).  Other kinds or a non-explicit grid:
+ * AWB_ERR_INVALID; grouped handles: AWB_ERR_UNSUPPORTED. */
+int awb_prior_inverse(awb_handle h, const float* params, const awb_grid_spec* grid, float* out, int32_t training,
+                      void* workspace, size_t workspace_bytes, void* stream);
+/* Backward of awb_prior_inverse(training != 0) on the same workspace, grid and params: d_out [N][C] -> grads [P]
+ * (overwritten, state_dict order: the flow and 1x1 conv entries, every ICNN entry exactly 0) and optional
+ * dgrid [B,C,H,W] = d / d grid.  Fixed-order reductions, no atomics: repeated calls give the same bits, and requesting
+ * dgrid leaves grads bit-identical.  The coupling MLPs are evaluated with unit loops whatever awb_prior_set_flow_eval
+ * says.  Flow MLP width > 32 or a coupling mask with all or no component masked: AWB_ERR_UNSUPPORTED.  Same handles and
+ * errors as awb_prior_inverse. */
+int awb_prior_inverse_backward(awb_handle h, const float* params, const awb_grid_spec* grid, const float* d_out,
+                               float* grads, float* dgrid, void* workspace, size_t workspace_bytes, void* stream);
 
 /* One fused fit step = the body of the reference's hot loops
  * (path_connected_net.py:939-953, :364-379; notebooks/how_to/convexity.ipynb cell 9):
