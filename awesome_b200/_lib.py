@@ -46,7 +46,8 @@ class GridSpec(C.Structure):
 
 
 class LossSpec(C.Structure):
-    _fields_ = [("kind", C.c_int32), ("cls_rule", C.c_int32), ("coef_fg", C.c_float), ("coef_bg", C.c_float)]
+    _fields_ = [("kind", C.c_int32), ("cls_rule", C.c_int32), ("coef_fg", C.c_float), ("coef_bg", C.c_float),
+                ("weight", C.c_void_p), ("ignore_enabled", C.c_int32), ("ignore_value", C.c_float)]
 
 
 class OptHyper(C.Structure):
@@ -113,6 +114,7 @@ SYMBOLS = [
     ("awb_prior_actnorm_init", C.c_int, [_P, _P, C.POINTER(GridSpec), _P, C.c_size_t, _P]),
     ("awb_mask_iou_counts", C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P]),
     ("awb_target_counts", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P]),
+    ("awb_target_counts_ignore", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, _P]),
     ("awb_image_process", C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P]),
     ("awb_image_edge_map", C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P]),
     ("awb_debug_umma_probe", C.c_int, [_P, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32,

@@ -220,7 +220,8 @@ class Prior:
     def slice_grads(self, params: torch.Tensor, grid: GridSpecHost, row_begin: int, row_end: int, target: torch.Tensor,
                     loss, grad_row: torch.Tensor, ws: torch.Tensor, reuse_packed: bool = False) -> None:
         """Gradient row of pixel rows ``[row_begin, row_end)`` of the batch into ``grad_row`` (``[P + 1]`` fp32, device).
-        ``target`` is the FULL batch ``[N]``; ``loss`` the ``LossSpec`` of the full batch.  ``ws``:
+        ``target`` is the FULL batch ``[N]``; ``loss`` the ``LossSpec`` of the full batch (its weight map, when set, too
+        covers the full batch and is read at the global rows).  ``ws``:
         layout ``AWB_WS_FIT_STEP`` for ``row_end - row_begin`` pixels.  ``reuse_packed``: the previous call on ``ws`` was
         a slice of the same parameters."""
         gs = grid.to_c()
@@ -255,13 +256,19 @@ def iou_counts(pred: torch.Tensor, target: torch.Tensor, pred_is_logit: bool, n_
     return counts
 
 
-def target_counts(target: torch.Tensor, cls_rule: int, n_objects: int = 1) -> torch.Tensor:
-    """``[O,2]`` int64 counts {fg, bg} of the target under ``cls_rule`` (``n_objects`` targets back to back)."""
+def target_counts(target: torch.Tensor, cls_rule: int, n_objects: int = 1,
+                  ignore_value: Optional[float] = None) -> torch.Tensor:
+    """``[O,2]`` int64 counts {fg, bg} of the target under ``cls_rule`` (``n_objects`` targets back to back).
+    ``ignore_value``: pixels whose target equals it count in neither class (``awb_target_counts_ignore``)."""
     L.require_cuda()
     lib = L.load()
     t = target.detach()
     O = n_objects
     t = t.reshape(O, -1).contiguous().float()
     counts = torch.empty((O, 2), dtype=torch.int64, device=t.device)
-    L.check(lib.awb_target_counts(t.data_ptr(), t.shape[1], O, cls_rule, counts.data_ptr(), L.stream_ptr()))
+    if ignore_value is None:
+        L.check(lib.awb_target_counts(t.data_ptr(), t.shape[1], O, cls_rule, counts.data_ptr(), L.stream_ptr()))
+    else:
+        L.check(lib.awb_target_counts_ignore(t.data_ptr(), t.shape[1], O, cls_rule, 1, float(ignore_value),
+                                             counts.data_ptr(), L.stream_ptr()))
     return counts

@@ -288,6 +288,22 @@ static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t w
   return AWB_OK;
 }
 
+static bool loss_weighted(const awb_loss_spec* loss, int O) {
+  for (int o = 0; o < O; o++)
+    if (loss_is_weighted(loss[o])) return true;
+  return false;
+}
+
+// The per-pixel part of the loss specs of a fit step: an ignore label must be a number (NaN never equals a target).
+static int check_loss(const awb_loss_spec* loss, int O) {
+  for (int o = 0; o < O; o++)
+    if (loss[o].ignore_enabled && !isfinite(loss[o].ignore_value)) {
+      set_error("loss[%d]: ignore_value must be finite", o);
+      return AWB_ERR_INVALID;
+    }
+  return AWB_OK;
+}
+
 // One pass of an ICNN prior on the rows of a workspace.  dy comes from the loss on target (fit step: forward and
 // backward), from dlogits (backward of an earlier training forward on the same workspace, which holds the flow's outputs
 // and, on the exact path, the ICNN's activations) or from nowhere (forward only).
@@ -315,18 +331,23 @@ static int run_pass(awb_handle h, const float* params, const awb_grid_spec* g, c
   if (p.tensor) {
     // backward from dlogits: the fused kernel recomputes the forward and reads dy as the target of an upstream "loss"
     const int O = h->desc.n_objects;
-    awb_loss_spec up[16];
+    awb_loss_spec up[16] = {};
     float* amax = nullptr;
+    float* wamax = nullptr;
     if (p.dlogits) {
       for (int o = 0; o < O && o < 16; o++) { up[o].kind = AWB_LOSS_UPSTREAM; up[o].cls_rule = AWB_CLS_UNARY_LT_HALF; up[o].coef_fg = 1.f; up[o].coef_bg = 1.f; }
       amax = w.lossp + (int64_t)kMaxSplits * O;       // spare floats behind the loss partials (lossp is [S][O], S <= 148 ... see carve)
       rc = absmax_per_object(p.dlogits, w.N, O, amax, st);
       if (rc) return rc;
+    } else if (p.target && loss_weighted(p.loss, O)) {
+      wamax = w.lossp + (int64_t)kMaxSplits * O;      // the same spare floats: max |w| over the kept pixels
+      rc = weight_absmax_per_object(p.loss, p.target, w.N, O, wamax, st);
+      if (rc) return rc;
     }
     *n_part = 0;
     rc = tc_fit_forward_backward(h, params, g, p.dlogits ? p.dlogits : p.target, p.dlogits ? up : p.loss, p.logits,
                                  backward ? 1 : 0, w, n_part, st, p.reuse, flow ? w.X : nullptr,
-                                 need_dx ? w.dX : nullptr, amax);
+                                 need_dx ? w.dX : nullptr, amax, wamax);
   } else {
     *n_part = n_splits(w.N);
     rc = forward ? simt_forward(h, params, g, p.logits, p.training || backward, flow, w, st) : AWB_OK;
@@ -411,6 +432,7 @@ int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_g
   int rc = check_common(h, g, ws, ws_bytes, AWB_WS_FIT_STEP, nullptr, &w);
   if (rc) return rc;
   if (!params || !opt_state || !target || !loss || !hy) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if ((rc = check_loss(loss, h->desc.n_objects))) return rc;
   // simt_reduce_opt refreshes a flow prior's fp16 weight image only when its optimizer owns every group
   Pass p = {};
   p.tensor = h->desc.precision == AWB_PREC_F16; p.target = target; p.loss = loss;
@@ -519,8 +541,11 @@ int awb_prior_slice_grads(awb_handle h, const float* params, const awb_grid_spec
   rc = check_common(h, g, ws, ws_bytes, AWB_WS_FIT_STEP, window, &w);
   if (rc) return rc;
   if (!params || !target || !loss || !grad_row) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if ((rc = check_loss(loss, 1))) return rc;
+  awb_loss_spec ls = *loss;              // the weight map, like the target, is the full batch's: read at the global row
+  if (ls.weight) ls.weight += row_begin;
   Pass p = {};
-  p.tensor = h->desc.precision == AWB_PREC_F16; p.target = target + row_begin; p.loss = loss;
+  p.tensor = h->desc.precision == AWB_PREC_F16; p.target = target + row_begin; p.loss = &ls;
   p.reuse = (flags & AWB_FIT_REUSE_PACKED) != 0;
   cudaStream_t st = (cudaStream_t)stream;
   int n_part;
@@ -659,6 +684,7 @@ int awb_star_fit_step(awb_handle h, float* params, void* opt_state, const float*
                       void* stream) {
   if (!h || !params || !opt_state || !x || !target || !loss || !hy || !ws || n < 1) { set_error("bad argument"); return AWB_ERR_INVALID; }
   if (h->desc.kind != AWB_KIND_STAR) { set_error("not a star prior"); return AWB_ERR_INVALID; }
+  if (loss_is_weighted(*loss)) { set_error("the star fit step takes no weight map or ignore label"); return AWB_ERR_UNSUPPORTED; }
   const int64_t need = awb_star_workspace_bytes(h, n);
   if ((int64_t)ws_bytes < need) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)need); return AWB_ERR_WORKSPACE; }
   const int S = star_n_ctas(n);

@@ -53,6 +53,24 @@ struct OptScal {  // per object, device resident
                                          // count -- the one its bias correction uses -- is step - group_start[g]
 };
 
+// The loss coefficients of awb_loss_spec as the kernels carry them (its first four fields), and the per-pixel part of
+// it: weight map and ignore label.  The kernel parameter blocks keep the coefficients where they always were and append
+// the per-pixel part at their end, so the unweighted instantiations compile to the same instructions as before.
+struct LossCoef {
+  int32_t kind, cls_rule;
+  float coef_fg, coef_bg;
+};
+struct LossPix {
+  const float* weight;   // [N] of the object, indexed by local row (null: 1)
+  int32_t ignore;        // drop pixels whose target == ignore_value
+  float ignore_value;
+};
+inline LossCoef loss_coef(const awb_loss_spec& s) { return LossCoef{s.kind, s.cls_rule, s.coef_fg, s.coef_bg}; }
+inline LossPix loss_pix(const awb_loss_spec& s) { return LossPix{s.weight, s.ignore_enabled ? 1 : 0, s.ignore_value}; }
+inline bool loss_is_weighted(const awb_loss_spec& s) { return s.weight || s.ignore_enabled; }
+// keep_n of awb_loss_spec: the pixel takes part in the loss
+__host__ __device__ __forceinline__ bool loss_keep(const LossPix& e, float t) { return !e.ignore || t != e.ignore_value; }
+
 struct FlowConsts {
   float nmin[4], nmax[4];
   float new_min, new_max;
@@ -186,6 +204,9 @@ int simt_reduce_grads(const awb_prior* h, float* grads, const Workspace& ws, int
 int simt_grid_grad_backward(const awb_prior* h, const awb_grid_spec* g, const float* dlogits, const float* d_dgrid,
                             float* ydot, const Workspace& ws, cudaStream_t st);
 int absmax_per_object(const float* x, int64_t n, int O, float* out, cudaStream_t st);   // out[o] = max |x[o][:]|
+// out[o] = max |w_o[n]| over the kept pixels n of object o (loss[o].weight, target [O][n]); 1 for an object without a map
+// and 0 when it keeps no pixel.  The tensor path's fp16 loss scale of a weighted loss.
+int weight_absmax_per_object(const awb_loss_spec* loss, const float* target, int64_t n, int O, float* out, cudaStream_t st);
 int simt_dgrid(const awb_prior* h, const awb_grid_spec* g, float* dgrid, const Workspace& ws, cudaStream_t st);
 // ws.dX[n] = (d_deformed[n][0..C), 0...): seeds the flow backward with a caller gradient on the deformed coordinates
 int simt_seed_dX(const awb_prior* h, const float* d_deformed, const Workspace& ws, cudaStream_t st);
@@ -225,7 +246,9 @@ int64_t tc_vec_offset_bytes(int L);                       // byte offset of the 
 int tc_fit_forward_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
                             const awb_loss_spec* loss, float* logits, int mode, const Workspace& ws,
                             int* n_splits_out, cudaStream_t st, bool reuse_packed, const float* Xrows, float* dXrows,
-                            const float* amax);
+                            const float* amax, const float* wamax = nullptr);
+// wamax (device [O], weight_absmax_per_object): set exactly when a loss spec has a weight map or an ignore label; the
+// fused kernel then takes its weighted epilogue and scales its fp16 deltas by max |w coef| instead of max |coef|.
 int tc_trace_read(unsigned long long* host, int max_ctas);   // debug timeline (AWB_TC_TRACE=1): 256 stamps per CTA
 
 // ---- flows, implemented in awb_flow.cu ----

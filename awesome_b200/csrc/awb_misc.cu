@@ -3,6 +3,8 @@
 // awesome/model/path_connected_net.py:964-982) and fg/bg pixel counts for the weighted
 // losses (torch.unique(target >= 0.5, return_counts=True),
 // awesome/measures/unaries_weighted_loss.py:38-40).  Exact integer arithmetic.
+#include <math.h>
+
 #include "awb_internal.cuh"
 
 namespace awb {
@@ -36,12 +38,15 @@ __global__ void __launch_bounds__(256) k_iou_counts(const float* __restrict__ pr
   if (threadIdx.x == 3 && blockIdx.x == 0) counts[o * 4 + 3] = (unsigned long long)N;
 }
 
+// IGN: pixels whose target equals ignore_value count in neither class (awb_target_counts_ignore)
+template <bool IGN>
 __global__ void __launch_bounds__(256) k_target_counts(const float* __restrict__ target, int64_t N, int cls_rule,
-                                                       unsigned long long* counts) {
+                                                       unsigned long long* counts, float ignore_value) {
   int o = blockIdx.y;
   const float* t = target + (int64_t)o * N;
   unsigned fg = 0, bg = 0;
   for (int64_t n = (int64_t)blockIdx.x * 256 + threadIdx.x; n < N; n += (int64_t)gridDim.x * 256) {
+    if (IGN && t[n] == ignore_value) continue;
     bool f = cls_rule == AWB_CLS_UNARY_LT_HALF ? (t[n] < 0.5f) : (t[n] != 1.0f);
     fg += f; bg += !f;
   }
@@ -82,7 +87,22 @@ int awb_target_counts(const float* target, int64_t N, int32_t O, int32_t cls_rul
   cudaStream_t st = (cudaStream_t)stream;
   AWB_CUDA(cudaMemsetAsync(counts, 0, sizeof(long long) * 2 * O, st));
   int blocks = (int)((N + 255) / 256 < 592 ? (N + 255) / 256 : 592);
-  k_target_counts<<<dim3(blocks, O), 256, 0, st>>>(target, N, cls_rule, (unsigned long long*)counts);
+  k_target_counts<false><<<dim3(blocks, O), 256, 0, st>>>(target, N, cls_rule, (unsigned long long*)counts, 0.f);
+  AWB_CUDA(cudaGetLastError());
+  return AWB_OK;
+}
+
+int awb_target_counts_ignore(const float* target, int64_t N, int32_t O, int32_t cls_rule, int32_t ignore_enabled,
+                             float ignore_value, long long* counts, void* stream) {
+  if (!target || !counts || N < 1 || O < 1) { set_error("bad argument"); return AWB_ERR_INVALID; }
+  if (ignore_enabled && !isfinite(ignore_value)) { set_error("ignore_value must be finite"); return AWB_ERR_INVALID; }
+  cudaStream_t st = (cudaStream_t)stream;
+  AWB_CUDA(cudaMemsetAsync(counts, 0, sizeof(long long) * 2 * O, st));
+  int blocks = (int)((N + 255) / 256 < 592 ? (N + 255) / 256 : 592);
+  if (ignore_enabled)
+    k_target_counts<true><<<dim3(blocks, O), 256, 0, st>>>(target, N, cls_rule, (unsigned long long*)counts, ignore_value);
+  else
+    k_target_counts<false><<<dim3(blocks, O), 256, 0, st>>>(target, N, cls_rule, (unsigned long long*)counts, 0.f);
   AWB_CUDA(cudaGetLastError());
   return AWB_OK;
 }

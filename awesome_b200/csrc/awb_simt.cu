@@ -331,16 +331,19 @@ struct OutP {
   int train;                      // 0 forward only, 1 loss-driven (fit), 2 upstream dlogits
   const float* target;            // [O][N]
   const float* dlogits;           // [O][N]
-  awb_loss_spec loss[16];
+  LossCoef loss[16];
   float* D; int64_t sD;           // delta_L out
   float* dX; int64_t sdX;         // optional: coordinate gradient init
   float* part; int64_t sSplit;    // partial sums [S][O][G]
   float* lossp;                   // [S][O]
   int64_t N, chunk;
   int h, C, ld, O;
+  LossPix pix[16];                // WL: weight map and ignore label per object
 };
 
-template <int Q>
+// WL: the loss carries per-pixel weights and / or an ignore label (awb_loss_spec); the other instantiation is the plain
+// loss and does not read pix
+template <int Q, bool WL>
 __global__ void __launch_bounds__(256) k_out(OutP p) {
   extern __shared__ float sm[];   // [8][ld] gradient partials + [8] loss
   const int s = blockIdx.x, o = blockIdx.y;
@@ -357,7 +360,8 @@ __global__ void __launch_bounds__(256) k_out(OutP p) {
   float lacc = 0.f;
   int64_t r0 = (int64_t)s * p.chunk;
   int64_t r1 = r0 + p.chunk < p.N ? r0 + p.chunk : p.N;
-  awb_loss_spec ls = p.loss[p.train == 1 ? o : 0];
+  LossCoef ls = p.loss[p.train == 1 ? o : 0];
+  const LossPix lp = p.pix[WL ? o : 0];
   for (int64_t n = r0 + w; n < r1; n += 8) {
     float z[Q];
     float dot = 0.f;
@@ -377,6 +381,7 @@ __global__ void __launch_bounds__(256) k_out(OutP p) {
       float t = p.target[(int64_t)o * p.N + n];
       bool fg = ls.cls_rule == AWB_CLS_UNARY_LT_HALF ? (t < 0.5f) : (t != 1.0f);
       float coef = fg ? ls.coef_fg : ls.coef_bg;
+      if (WL && lp.weight) coef *= lp.weight[(int64_t)n];   // w * coef: a weight of 1 leaves every bit of the loss
       float sg = 1.f / (1.f + expf(-y));
       float l;
       if (ls.kind == AWB_LOSS_SE_SIGMOID) {
@@ -387,7 +392,13 @@ __global__ void __launch_bounds__(256) k_out(OutP p) {
         l = fmaxf(y, 0.f) - y * t + log1pf(expf(-fabsf(y)));
         dy = coef * (sg - t);
       }
-      lacc += coef * l;
+      if (WL) {   // select, do not multiply: a NaN logit, target or weight of an ignored pixel cannot leak in
+        const bool keep = loss_keep(lp, t);
+        dy = keep ? dy : 0.f;
+        lacc = fmaf(keep ? coef : 0.f, keep ? l : 0.f, lacc);   // the contraction of the plain loss's lacc += coef * l
+      } else {
+        lacc += coef * l;
+      }
     } else {
       dy = p.dlogits[(int64_t)o * p.N + n];
     }
@@ -865,6 +876,38 @@ __global__ void k_absmax(const float* __restrict__ x, int64_t n, float* out) {
   }
 }
 
+// max |w[i]| over the kept pixels of object blockIdx.y, grid-stride over blockIdx.x, combined with an integer atomicMax on
+// the bits of a non-negative float (fmaxf drops a NaN weight; a kept NaN weight makes the loss itself non-finite)
+struct WAbsP {
+  LossPix pix[16];
+  const float* t;   // [O][n]
+  int64_t n;
+  float* out;       // [O], zeroed
+};
+__global__ void __launch_bounds__(256) k_weight_absmax(WAbsP p) {
+  const int o = blockIdx.y;
+  const LossPix pix = p.pix[o];
+  const float* t = p.t + (int64_t)o * p.n;
+  float m = 0.f;
+  for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < p.n; i += (int64_t)gridDim.x * 256)
+    if (loss_keep(pix, t[i])) m = fmaxf(m, pix.weight ? fabsf(pix.weight[i]) : 1.f);
+  for (int off = 16; off > 0; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, off));
+  if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<int*>(p.out + o), __float_as_int(m));
+}
+
+int weight_absmax_per_object(const awb_loss_spec* loss, const float* target, int64_t n, int O, float* out,
+                             cudaStream_t st) {
+  AWB_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * O, st));
+  WAbsP p = {};
+  for (int o = 0; o < O && o < 16; o++) p.pix[o] = loss_pix(loss[o]);
+  p.t = target; p.n = n; p.out = out;
+  const int per_obj = kMaxSplits / O > 0 ? kMaxSplits / O : 1;
+  const int blocks = (int)((n + 2047) / 2048 < per_obj ? (n + 2047) / 2048 : per_obj);
+  AWB_LAUNCH(PK_MISC, st, k_weight_absmax<<<dim3(blocks, O), 256, 0, st>>>(p));
+  AWB_CUDA(cudaGetLastError());
+  return AWB_OK;
+}
+
 int absmax_per_object(const float* x, int64_t n, int O, float* out, cudaStream_t st) {
   AWB_LAUNCH(PK_MISC, st, k_absmax<<<O, 1024, 0, st>>>(x, n, out));
   AWB_CUDA(cudaGetLastError());
@@ -986,8 +1029,8 @@ int simt_forward(const awb_prior* h, const float* params, const awb_grid_spec* g
     q.logits = logits_out; q.train = 0; q.N = N; q.chunk = split_chunk(N);
     q.h = L.h; q.C = L.C; q.ld = L.ld; q.O = O;
     size_t smem = (8 * L.ld + 8) * sizeof(float);
-    if (L.ld <= 160) AWB_LAUNCH(PK_OUT_LOSS, st, k_out<5><<<dim3(n_splits(N), O), 256, smem, st>>>(q));
-    else AWB_LAUNCH(PK_OUT_LOSS, st, k_out<9><<<dim3(n_splits(N), O), 256, smem, st>>>(q));
+    if (L.ld <= 160) AWB_LAUNCH(PK_OUT_LOSS, st, k_out<5, false><<<dim3(n_splits(N), O), 256, smem, st>>>(q));
+    else AWB_LAUNCH(PK_OUT_LOSS, st, k_out<9, false><<<dim3(n_splits(N), O), 256, smem, st>>>(q));
   }
   AWB_CUDA(cudaGetLastError());
   return AWB_OK;
@@ -1009,14 +1052,25 @@ int simt_backward(const awb_prior* h, const float* target, const awb_loss_spec* 
   q.logits = loss ? ws.logits : nullptr;
   q.train = loss ? 1 : 2;
   q.target = target; q.dlogits = dlogits;
-  if (loss) for (int o = 0; o < O && o < 16; o++) q.loss[o] = loss[o];
+  bool wl = false;
+  if (loss)
+    for (int o = 0; o < O && o < 16; o++) {
+      q.loss[o] = loss_coef(loss[o]);
+      q.pix[o] = loss_pix(loss[o]);
+      wl = wl || loss_is_weighted(loss[o]);
+    }
   q.D = ws.D + (L.L & 1) * sLayer; q.sD = sDobj;      // delta_i lives in D[i & 1]
   q.dX = need_dx ? ws.dX : nullptr; q.sdX = N * 4;
   q.part = ws.part; q.sSplit = sSplit; q.lossp = ws.lossp;
   q.N = N; q.chunk = chunk; q.h = L.h; q.C = L.C; q.ld = L.ld; q.O = O;
   size_t smem = (8 * L.ld + 8) * sizeof(float);
-  if (L.ld <= 160) AWB_LAUNCH(PK_OUT_LOSS, st, k_out<5><<<dim3(S, O), 256, smem, st>>>(q));
-  else AWB_LAUNCH(PK_OUT_LOSS, st, k_out<9><<<dim3(S, O), 256, smem, st>>>(q));
+  if (wl) {
+    if (L.ld <= 160) AWB_LAUNCH(PK_OUT_LOSS, st, k_out<5, true><<<dim3(S, O), 256, smem, st>>>(q));
+    else AWB_LAUNCH(PK_OUT_LOSS, st, k_out<9, true><<<dim3(S, O), 256, smem, st>>>(q));
+  } else {
+    if (L.ld <= 160) AWB_LAUNCH(PK_OUT_LOSS, st, k_out<5, false><<<dim3(S, O), 256, smem, st>>>(q));
+    else AWB_LAUNCH(PK_OUT_LOSS, st, k_out<9, false><<<dim3(S, O), 256, smem, st>>>(q));
+  }
 
   for (int i = L.L; i >= 1; i--) {
     const float* delta = ws.D + (i & 1) * sLayer;

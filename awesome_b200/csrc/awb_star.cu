@@ -18,7 +18,7 @@ struct StarP {
   const float* x;        // [n][2]
   const float* target;   // [n] (fit)
   int64_t n, chunk;
-  awb_loss_spec loss;
+  LossCoef loss;
   float* logits;         // [n] or null
   float* part;           // [S][P] (fit)
   float* lossp;          // [S]
@@ -155,7 +155,7 @@ int star_run(const awb_prior* h, const float* params, const float* x, const floa
   p.params = params; p.P = h->lay.P; p.h = hh; p.x = x; p.target = target; p.n = n;
   const int S = fit ? star_n_ctas(n) : (int)((n + 15) / 16 < 1184 ? (n + 15) / 16 : 1184);
   p.chunk = (n + S - 1) / S;
-  if (loss) p.loss = *loss;
+  if (loss) p.loss = loss_coef(*loss);
   p.logits = logits; p.part = part; p.lossp = lossp;
   const size_t smem = sizeof(float) * ((size_t)(fit ? 2 : 1) * hh * (hh + 1) + 2 * hh);
   if (fit) {

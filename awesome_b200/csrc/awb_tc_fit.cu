@@ -77,7 +77,7 @@ struct TcP {
   GridDev g;
   const uint8_t* img; int64_t img_stride;
   const float* target;
-  awb_loss_spec loss[16];
+  LossCoef loss[16];
   float scale[16];
   float* part; int64_t sSplit, G, aug_in, aug_layer, aug_out;
   float* lossp; int O;
@@ -88,6 +88,11 @@ struct TcP {
   const float* amax;   // optional device [O]: max |dlogits| per object; sets the fp16 loss scale of the upstream-gradient mode
   const float* X;   // optional [O][N][4]: coordinates produced by the flow (x, y, t, 1) instead of the generated grid
   float* dX;        // optional [O][N][4]: gradient w.r.t. those coordinates (consumed by the flow backward)
+  // WL only: weight map and ignore label per object; the fp16 loss scale then comes from max |w| over the kept pixels
+  // (wamax, device [O]) times max |coef| (coef_max)
+  LossPix pix[16];
+  float coef_max[16];
+  const float* wamax;
 };
 
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
@@ -157,9 +162,10 @@ __device__ __forceinline__ float warp_reduce_scatter16(float* v, int lane) {
 }
 
 // FIT: forward + loss + backward + partials (else forward only, logits out); DX: the coordinates come from a flow and
-// their gradient goes back to it.  Compile-time so that the forward-only and the plain ICNN instantiations carry
+// their gradient goes back to it; WL (with FIT): per-pixel loss weights and / or an ignore label, the weight fetched
+// with the target.  Compile-time so that the forward-only and the plain ICNN instantiations carry
 // neither the branches nor the live ranges (delta_0 words, coordinate-gradient sums) of the others.
-template <int L, int C, bool FIT, bool DX>
+template <int L, int C, bool FIT, bool DX, bool WL>
 __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   constexpr int NT = L + 2;
@@ -392,10 +398,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
     float accC[L + 1];                            // cg 2: corner sums, lane-distributed (value = lane & 15)
 #pragma unroll
     for (int i = 0; i <= L; i++) accC[i] = 0.f;
-    const awb_loss_spec ls = p.loss[o];
-    // loss scale: host-chosen power of two, or (upstream-gradient mode) derived from the device-side max |dlogits|
+    const LossCoef ls = p.loss[o];
+    // loss scale: host-chosen power of two, or (upstream-gradient mode) derived from the device-side max |dlogits|,
+    // or (weighted loss) from max |w coef| over the kept pixels
     float S = p.scale[o];
     if (p.amax) { const float am = p.amax[o]; S = (am > 0.f && isfinite(am)) ? exp2f(rintf(log2f(64.f / am))) : 1.f; }
+    LossPix lp = {};
+    if constexpr (WL) {
+      lp = p.pix[o];
+      const float am = p.wamax[o] * p.coef_max[o];
+      S = (am > 0.f && isfinite(am)) ? exp2f(rintf(log2f(64.f / am))) : 1.f;
+    }
     constexpr bool has_dx = DX;
     float adx0 = 0.f, adx1 = 0.f, adx2 = 0.f;     // last group: d loss / d (x, y, t) of this row (scaled by S)
     // the input-layer part of it comes from the tensor pipe one round trip later: the row's sums and pixel wait for it
@@ -432,7 +445,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
       if (cg == 0) st16(stx + buf * TX_B + row * 16, pack2(a0, a1), pack2(C > 2 ? a2 : 1.f, C > 2 ? 1.f : 0.f), 0u, 0u);
     };
     // coordinates / target of a tile (rows past N replicate the last pixel and carry no loss)
-    float x0n = 0.f, x1n = 0.f, x2n = 0.f, tgtn = 0.f;
+    float x0n = 0.f, x1n = 0.f, x2n = 0.f, tgtn = 0.f, wgtn = 1.f;
     bool liven = false;
     // Pixel position (frame, row, column) of this thread's row in the next tile to fetch, advanced tile by tile by
     // the decomposed tile stride: no integer divisions inside the tile loop.
@@ -465,6 +478,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
       pb += db;
       tgtn = 0.f;
       if (fit && liven) tgtn = p.target[(int64_t)o * p.N + n];
+      if constexpr (WL) wgtn = (liven && lp.weight) ? lp.weight[n] : 1.f;
     };
     auto chunk16_f32 = [&](const uint8_t* tile, float* c6) {   // columns 128..133 of a stored tile row
       const uint4 cz = *reinterpret_cast<const uint4*>(tile + 16 * 2048 + row * 16);
@@ -482,7 +496,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
       const int tile = blockIdx.x + it * gridDim.x;
       const int64_t n = (int64_t)tile * 128 + row;
       const bool live = liven;
-      const float x0 = x0n, x1 = x1n, x2 = x2n, tgt = tgtn;
+      const float x0 = x0n, x1 = x1n, x2 = x2n, tgt = tgtn, wgt = wgtn;
       const bool more = it + 1 < n_my;
       // aug values of chunk 16 columns 130..135: (x, y, [t,] 1, 0..)
       const uint32_t ax01 = pack2(x0, x1), ax2o = pack2(C > 2 ? x2 : 1.f, C > 2 ? 1.f : 0.f);
@@ -561,7 +575,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
       float dys = 0.f, lossv = 0.f;
       if (live) {
         const bool fg = ls.cls_rule == AWB_CLS_UNARY_LT_HALF ? (tgt < 0.5f) : (tgt != 1.0f);
-        const float coef = fg ? ls.coef_fg : ls.coef_bg;
+        const float coef = WL ? (fg ? ls.coef_fg : ls.coef_bg) * wgt : (fg ? ls.coef_fg : ls.coef_bg);
         const float sg = __fdividef(1.f, 1.f + __expf(-y));
         float l, dl;
         if (ls.kind == AWB_LOSS_SE_SIGMOID) { float d = tgt - sg; l = d * d; dl = -2.f * d * sg * (1.f - sg); }
@@ -569,6 +583,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_icnn_fit_tc(TcP p) {
         else { l = bce_logits(y, tgt); dl = sg - tgt; }
         dys = coef * dl * S;
         lossv = coef * l;
+        if (WL && !loss_keep(lp, tgt)) { dys = 0.f; lossv = 0.f; }      // select: a NaN there cannot leak in
       }
       // delta_L = dy * w_o .* (z_L > 0) on packed fp16 pairs
       float dL128 = 0.f, dL129 = 0.f;
@@ -847,7 +862,8 @@ int tc_trace_read(unsigned long long* host, int max_ctas) {
 
 int tc_fit_forward_backward(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
                             const awb_loss_spec* loss, float* logits, int mode, const Workspace& ws, int* n_splits_out,
-                            cudaStream_t st, bool reuse_packed, const float* Xrows, float* dXrows, const float* amax) {
+                            cudaStream_t st, bool reuse_packed, const float* Xrows, float* dXrows, const float* amax,
+                            const float* wamax) {
   const Layout& Ly = h->lay;
   const int O = h->desc.n_objects, L = Ly.L, C = Ly.C;
   const int64_t N = ws.N;
@@ -874,16 +890,18 @@ int tc_fit_forward_backward(const awb_prior* h, const float* params, const awb_g
   p.target = target;
   for (int o = 0; o < O && o < 16; o++) {
     if (loss) {
-      p.loss[o] = loss[o];
+      p.loss[o] = loss_coef(loss[o]);
       float mx = fmaxf(fabsf(loss[o].coef_fg), fabsf(loss[o].coef_bg));
       p.scale[o] = mx > 0.f ? exp2f(rintf(log2f(64.f / mx))) : 1.f;   // keeps fp16 deltas in range (loss scaling)
+      p.pix[o] = loss_pix(loss[o]);
+      p.coef_max[o] = mx;
     } else {
       p.scale[o] = 1.f;
     }
   }
   p.part = ws.part; p.sSplit = (int64_t)O * Ly.G; p.G = Ly.G; p.aug_in = Ly.aug_in; p.aug_layer = Ly.aug_layer; p.aug_out = Ly.aug_out;
   p.lossp = ws.lossp; p.O = O; p.logits = logits; p.N = N; p.n_tiles = n_tiles; p.mode = mode;
-  p.X = Xrows; p.dX = dXrows; p.amax = amax;
+  p.X = Xrows; p.dX = dXrows; p.amax = amax; p.wamax = wamax;
   p.trace = nullptr;
   if (const char* tr = getenv("AWB_TC_TRACE")) {
     p.trace_serial = atoi(tr) == 2;
@@ -892,16 +910,18 @@ int tc_fit_forward_backward(const awb_prior* h, const float* params, const awb_g
   }
   const size_t smem = smem_bytes(L);
   dim3 gd(grid, O);
-#define AWB_TC_LAUNCH3(LL, CC, FF, DD)                                                                             \
+#define AWB_TC_LAUNCH3(LL, CC, FF, DD, WW)                                                                             \
   do {                                                                                                             \
-    AWB_CUDA(cudaFuncSetAttribute(k_icnn_fit_tc<LL, CC, FF, DD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    AWB_LAUNCH(PK_TC_FUSED, st, AWB_CUDA(launch_ex(k_icnn_fit_tc<LL, CC, FF, DD>, gd, dim3(NTHREADS), smem, st, true, p))); \
+    AWB_CUDA(cudaFuncSetAttribute(k_icnn_fit_tc<LL, CC, FF, DD, WW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    AWB_LAUNCH(PK_TC_FUSED, st, AWB_CUDA(launch_ex(k_icnn_fit_tc<LL, CC, FF, DD, WW>, gd, dim3(NTHREADS), smem, st, true, p))); \
   } while (0)
-#define AWB_TC_LAUNCH(LL, CC)                                    \
-  do {                                                           \
-    if (mode == 0) AWB_TC_LAUNCH3(LL, CC, false, false);         \
-    else if (dXrows) AWB_TC_LAUNCH3(LL, CC, true, true);         \
-    else AWB_TC_LAUNCH3(LL, CC, true, false);                    \
+#define AWB_TC_LAUNCH(LL, CC)                                              \
+  do {                                                                     \
+    if (mode == 0) AWB_TC_LAUNCH3(LL, CC, false, false, false);            \
+    else if (wamax && dXrows) AWB_TC_LAUNCH3(LL, CC, true, true, true);    \
+    else if (wamax) AWB_TC_LAUNCH3(LL, CC, true, false, true);             \
+    else if (dXrows) AWB_TC_LAUNCH3(LL, CC, true, true, false);            \
+    else AWB_TC_LAUNCH3(LL, CC, true, false, false);                       \
   } while (0)
   if (L == 1 && C == 2) AWB_TC_LAUNCH(1, 2);
   else if (L == 1 && C == 3) AWB_TC_LAUNCH(1, 3);

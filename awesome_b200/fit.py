@@ -17,60 +17,113 @@ from . import _lib as L
 from .core import GridSpecHost, Prior, target_counts
 
 
+def class_weight(mode: str, fg: float, bg: float, ratio: float = 1.0) -> float:
+    """``UnariesWeightedLoss._compute_weight`` / ``WeightedLoss`` (``unaries_weighted_loss.py:35-69``): the weight of the
+    foreground pixels for ``fg`` foreground and ``bg`` background pixels, in the reference's fp32 arithmetic."""
+    cc = torch.tensor(bg, dtype=torch.float32) / torch.tensor(fg, dtype=torch.float32)
+    if mode == "ratio":
+        w = (cc - 1) * ratio + 1
+    elif mode == "sssdms":
+        w = torch.round(cc / 10) + 1
+    elif mode == "equal":
+        w = cc
+    else:
+        raise ValueError(f"Mode {mode} is not supported")
+    return float(w)
+
+
 @dataclass
 class LossConfig:
     """Which per-pixel loss the fit minimises (SURVEY a10).
 
     kind "mse": ``UnariesWeightedLoss(SE("mean"), mode=...)`` on ``sigmoid(y)``
     (``path_connected_net.py:768``; modes of ``unaries_weighted_loss.py:35-69``).
+    kind "bce": ``UnariesWeightedLoss(BCELoss(), mode=...)`` on ``sigmoid(y)`` (computed from the logits).
     kind "fgbg_se" / "fgbg_bce_logits": the how-to notebooks' fg/bg-weighted means.
+
+    ``weight``: optional per-pixel weights (confidence maps, sparse-label weights), ``[O,N]``, ``[N]`` (one map for every
+    object) or ``[B,1,H,W]``; each pixel's loss term is multiplied by its weight.  ``ignore_value``: pixels whose target
+    equals it (the reference's ``noneclass``, e.g. 2 for FBMS weak labels) are dropped -- they add nothing to the loss or
+    its gradients and are left out of the class counts and of the mean's N, as ``WeightedLoss(..., noneclass=k)`` does.
     """
     kind: str = "mse"
-    mode: str = "none"        # none | ratio | sssdms | equal   (kind == "mse")
+    mode: str = "none"        # none | ratio | sssdms | equal   (kinds "mse", "bce")
     ratio: float = 1.0
     fg_weight: float = 0.4    # fgbg_* kinds
+    weight: Optional[torch.Tensor] = field(default=None, compare=False, repr=False)
+    ignore_value: Optional[float] = None
 
     @classmethod
     def from_reference(cls, criterion) -> "LossConfig":
         """Map a reference loss object onto the fused per-pixel loss (duck-typed by class name / attributes):
-        ``UnariesWeightedLoss(SE, mode=...)`` (``awesome/measures/unaries_weighted_loss.py:35-69``),
-        ``SE`` (``se.py``), ``torch.nn.MSELoss`` -> "mse"; ``BCEWithLogitsLoss`` -> fg/bg BCE with equal weights."""
+        ``UnariesWeightedLoss(SE | BCELoss, mode=...)`` (``awesome/measures/unaries_weighted_loss.py:35-69``),
+        ``WeightedLoss(SE | BCELoss, mode=..., noneclass=k)`` (``awesome/measures/weighted_loss.py:41-92``: pixels of
+        class ``k`` dropped), ``SE`` (``se.py``), ``torch.nn.MSELoss`` -> "mse"."""
         name = type(criterion).__name__
-        if name == "UnariesWeightedLoss" and type(getattr(criterion, "criterion", None)).__name__ == "BCELoss":
-            if (getattr(criterion, "mode", "none") or "none") != "none":
-                raise ValueError("weighted BCE fits are not fused; use mode='none'")
-            return cls("bce")
-        if name == "UnariesWeightedLoss":
-            return cls("mse", mode=getattr(criterion, "mode", "none") or "none", ratio=float(getattr(criterion, "ratio", 1.0) or 1.0))
+        if name in ("UnariesWeightedLoss", "WeightedLoss"):
+            inner = type(getattr(criterion, "criterion", None)).__name__
+            if inner not in ("BCELoss", "SE", "MSELoss", "NoneType"):
+                raise ValueError(f"{name}({inner}) has no fused equivalent; pass an awesome_b200.LossConfig")
+            none = getattr(criterion, "noneclass", None) if name == "WeightedLoss" else None
+            return cls("bce" if inner == "BCELoss" else "mse", mode=getattr(criterion, "mode", "none") or "none",
+                       ratio=float(getattr(criterion, "ratio", 1.0) or 1.0),
+                       ignore_value=None if none is None else float(none))
         if name in ("SE", "MSELoss"):
             return cls("mse")
         raise ValueError(f"criterion {name} has no fused equivalent; pass an awesome_b200.LossConfig")
 
-    def to_specs(self, target: torch.Tensor) -> List[L.LossSpec]:
-        """target ``[O,N]``.  Folds 1/N, class weights and fg/bg means into two coefficients per object."""
+    @property
+    def weighted(self) -> bool:
+        return self.weight is not None or self.ignore_value is not None
+
+    def weight_map(self, O: int, N: int, device) -> Optional[torch.Tensor]:
+        """``weight`` as a contiguous fp32 ``[O,N]`` or ``[1,N]`` (shared by every object) tensor on ``device``."""
+        if self.weight is None:
+            return None
+        w = self.weight.detach()
+        if w.numel() == O * N:
+            w = w.reshape(O, N)
+        elif w.numel() == N:
+            w = w.reshape(1, N)
+        else:
+            raise ValueError(f"weight has {w.numel()} elements; expected {O}x{N} ([O,N]) or {N} ([N], [B,1,H,W])")
+        return w.to(device=device, dtype=torch.float32).contiguous()
+
+    def to_specs(self, target: torch.Tensor, weight: Optional[torch.Tensor] = None) -> List[L.LossSpec]:
+        """target ``[O,N]``.  Folds 1/N, class weights and fg/bg means into two coefficients per object.  With
+        ``ignore_value`` the class counts and N are those of the kept pixels (``awb_target_counts_ignore``).
+        ``weight``: the ``weight_map`` the specs point to; the caller keeps it alive while the specs are in use.  When
+        omitted, the map is built here and held by the returned specs (attribute ``_weight``)."""
         O, N = target.shape
+        if self.weight is not None and weight is None:
+            weight = self.weight_map(O, N, target.device)
+        specs = self._coefs(target)
+        if self.weighted:
+            for o, sp in enumerate(specs):
+                if weight is not None:
+                    sp.weight = weight[o if weight.shape[0] == O else 0].data_ptr()
+                    sp._weight = weight
+                if self.ignore_value is not None:
+                    sp.ignore_enabled, sp.ignore_value = 1, float(self.ignore_value)
+        return specs
+
+    def _coefs(self, target: torch.Tensor) -> List[L.LossSpec]:
+        O, N = target.shape
+        ign = self.ignore_value
         specs = []
-        if self.kind == "mse":
-            if self.mode == "none":
-                return [L.LossSpec(L.AWB_LOSS_SE_SIGMOID, L.AWB_CLS_UNARY_LT_HALF, 1.0 / N, 1.0 / N) for _ in range(O)]
-            cnt = target_counts(target, L.AWB_CLS_UNARY_LT_HALF, O).cpu()
+        if self.kind in ("mse", "bce"):
+            k = L.AWB_LOSS_SE_SIGMOID if self.kind == "mse" else L.AWB_LOSS_BCE_LOGITS
+            if self.mode == "none" and ign is None:
+                return [L.LossSpec(k, L.AWB_CLS_UNARY_LT_HALF, 1.0 / N, 1.0 / N) for _ in range(O)]
+            cnt = target_counts(target, L.AWB_CLS_UNARY_LT_HALF, O, ignore_value=ign).cpu()
             for o in range(O):
                 fg, bg = float(cnt[o, 0]), float(cnt[o, 1])
-                cc = torch.tensor(bg, dtype=torch.float32) / torch.tensor(fg, dtype=torch.float32)
-                if self.mode == "ratio":
-                    w = (cc - 1) * self.ratio + 1
-                elif self.mode == "sssdms":
-                    w = torch.round(cc / 10) + 1
-                elif self.mode == "equal":
-                    w = cc
-                else:
-                    raise ValueError(f"Mode {self.mode} is not supported")
-                specs.append(L.LossSpec(L.AWB_LOSS_SE_SIGMOID, L.AWB_CLS_UNARY_LT_HALF, float(w) / N, 1.0 / N))
+                n = N if ign is None else max(fg + bg, 1.0)      # the mean over the kept pixels
+                w = 1.0 if self.mode == "none" else class_weight(self.mode, fg, bg, self.ratio)
+                specs.append(L.LossSpec(k, L.AWB_CLS_UNARY_LT_HALF, w / n, 1.0 / n))
             return specs
-        if self.kind == "bce":     # UnariesWeightedLoss(nn.BCELoss(), mode="none") on sigmoid(y), soft targets allowed
-            return [L.LossSpec(L.AWB_LOSS_BCE_LOGITS, L.AWB_CLS_UNARY_LT_HALF, 1.0 / N, 1.0 / N) for _ in range(O)]
         if self.kind in ("fgbg_se", "fgbg_bce_logits"):
-            cnt = target_counts(target, L.AWB_CLS_NOT_ONE, O).cpu()
+            cnt = target_counts(target, L.AWB_CLS_NOT_ONE, O, ignore_value=ign).cpu()
             k = L.AWB_LOSS_SE_SIGMOID if self.kind == "fgbg_se" else L.AWB_LOSS_BCE_LOGITS
             for o in range(O):
                 fg, bg = float(cnt[o, 0]), float(cnt[o, 1])
@@ -135,7 +188,10 @@ class PriorFitter:
         with torch.cuda.device(self.device):
             self.ws = prior.new_workspace(grid.n_pixels, L.AWB_WS_FIT_STEP, self.device)
             self.opt_state = torch.empty(prior.opt_state_bytes(), dtype=torch.uint8, device=self.device)
-            self._specs_list = loss.to_specs(self.target)
+            # the fitter's own copy of the weight map: the specs (and the graphs captured from them) point into it
+            w = loss.weight_map(O, self.target.shape[1], self.device)
+            self._weight = w.clone() if w is not None else None
+            self._specs_list = loss.to_specs(self.target, self._weight)
         self._specs = (L.LossSpec * O)(*self._specs_list)
         self._hyper = optim.to_c()
         self._gs = grid.to_c()
@@ -157,17 +213,25 @@ class PriorFitter:
         self.steps_done = 0
 
     def set_target(self, target: torch.Tensor, loss: Optional[LossConfig] = None) -> None:
-        """New unaries for the same shapes (next frame): reuses workspace, graph and state buffers."""
+        """New unaries for the same shapes (next frame): reuses workspace, graph and state buffers.  A new weight map
+        of the same shape is copied into the fitter's map; a map of another shape, or one appearing or going away,
+        changes the pointers the captured graphs were recorded with, so they are captured again."""
         self.target.copy_(target.detach().reshape(self.target.shape))
         if loss is not None:
+            O, N = self.target.shape
             with torch.cuda.device(self.device):
-                specs = loss.to_specs(self.target)
-            changed = any((a.kind, a.cls_rule, a.coef_fg, a.coef_bg) != (b.kind, b.cls_rule, b.coef_fg, b.coef_bg)
-                          for a, b in zip(specs, self._specs_list))
+                w = loss.weight_map(O, N, self.device)
+                if w is not None and self._weight is not None and w.shape == self._weight.shape:
+                    self._weight.copy_(w)
+                else:
+                    self._weight = w.clone() if w is not None else None
+                specs = loss.to_specs(self.target, self._weight)
+            key = lambda a: (a.kind, a.cls_rule, a.coef_fg, a.coef_bg, a.weight, a.ignore_enabled, a.ignore_value)
+            changed = any(key(a) != key(b) for a, b in zip(specs, self._specs_list))
             if changed:
                 self._specs_list = specs
                 self._specs = (L.LossSpec * len(specs))(*specs)
-                self._graph = None      # coefficients are baked into the captured launches
+                self._graph = None      # coefficients and the weight pointers are baked into the captured launches
 
     def _step(self, k: int, reuse: bool = False) -> None:
         """One fused step.  ``reuse``: this call directly follows another ``_step`` of this fitter inside the
@@ -414,7 +478,7 @@ class SlicedFitter:
             self.rows = torch.zeros((self.n_slices, R), dtype=torch.float32, device=self.device)   # empty slices stay 0
             self.local = self.rows if world == 1 else torch.zeros((len(self.mine), R), dtype=torch.float32,
                                                                    device=self.device)
-            self._spec = loss.to_specs(self.target)[0]
+            self._spec = loss.to_specs(self.target)[0]        # holds its weight map (if any) alive
         self._hyper = optim.to_c()
         self.optim = optim
         self.steps_done = 0
@@ -427,7 +491,8 @@ class SlicedFitter:
         self.steps_done = 0
 
     def set_target(self, target: torch.Tensor) -> None:
-        """New unaries for the same grid shape; the loss coefficients are kept (as ``PriorFitter.set_target``)."""
+        """New unaries for the same grid shape; the loss coefficients and the weight map are kept (as
+        ``PriorFitter.set_target`` without a loss)."""
         self.target.copy_(target.detach().reshape(self.target.shape))
 
     def _produce(self, k: int, row: torch.Tensor, j: int) -> None:

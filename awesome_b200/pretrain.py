@@ -13,6 +13,7 @@ frame once per fit, not once per step.  ``pretrain`` / ``pretrain_load_state`` g
 and wrapper module the reference hands in."""
 from __future__ import annotations
 
+import dataclasses
 import logging
 from dataclasses import dataclass, field
 from typing import Any, Callable, Dict, Iterable, List, Optional, Sequence
@@ -106,11 +107,17 @@ def mask_iou(pred_prob: torch.Tensor, target_prob: torch.Tensor) -> float:
 def fit_frames(model, grids: Sequence, unaries: Sequence[torch.Tensor], schedule: Optional[FitSchedule] = None,
                on_frame: Optional[Callable[[FrameResult], None]] = None, frame_indices: Optional[Sequence[int]] = None,
                warm_start_hook: Optional[Callable[[Any, torch.Tensor, Any], None]] = None,
-               keep_masks: bool = False, initial_previous: Optional[torch.Tensor] = None) -> List[FrameResult]:
+               keep_masks: bool = False, initial_previous: Optional[torch.Tensor] = None,
+               weights: Optional[Sequence[Optional[torch.Tensor]]] = None) -> List[FrameResult]:
     """Fit ``model`` (ConvexNextNet or PathConnectedNet drop-in) to every frame in turn.  ``grids[i]`` is a
     ``[1,C,H,W]`` tensor or ``GridSpecHost``; ``unaries[i]`` the frame's soft segmentation (any shape with H*W
-    elements; convention fg = 0, bg = 1 like the reference).  The model ends holding the last proper state."""
+    elements; convention fg = 0, bg = 1 like the reference).  The model ends holding the last proper state.
+
+    ``weights[i]`` (optional, H*W elements): per-pixel loss weights of frame ``i`` (e.g. the segmentation net's
+    confidence), in place of ``schedule.criterion.weight``.  With ``criterion.ignore_value`` set (weak labels: fg 0,
+    bg 1, none 2), the none-class pixels are left out of the loss, of the no-foreground skip and of the IoU check."""
     s = schedule or FitSchedule()
+    ign = s.criterion.ignore_value
     arena = model._ensure_flat()
     dev = arena.device
     has_flow = hasattr(model, "flow_net")
@@ -124,7 +131,8 @@ def fit_frames(model, grids: Sequence, unaries: Sequence[torch.Tensor], schedule
         res = FrameResult(index=idx)
         un = un.detach().to(dev).float().reshape(1, -1)
         spec = _as_grid(grid, dev)
-        cnt = target_counts(un, L.AWB_CLS_UNARY_LT_HALF).cpu()[0]
+        crit = s.criterion if weights is None else dataclasses.replace(s.criterion, weight=weights[k])
+        cnt = target_counts(un, L.AWB_CLS_UNARY_LT_HALF, ignore_value=ign).cpu()[0]
         if int(cnt[0]) == 0 or int(cnt[1]) == 0:       # torch.unique(unaries >= 0.5) has one value (:848-855)
             logging.warning("Unaries of segmentation model contain no foreground. Skipping image. %s", idx)
             res.skipped = True
@@ -151,10 +159,10 @@ def fit_frames(model, grids: Sequence, unaries: Sequence[torch.Tensor], schedule
             model._maybe_actnorm_init(spec.materialize(model.in_channels, dev))
         key = (spec.mode, spec.B, spec.H, spec.W, spec.t0, spec.t_step, id(spec.grid))
         if fitter is None or fitter_key != key:
-            fitter = model.make_fitter(spec, un, s.criterion, s.optim(flow_group), steps_per_graph=s.steps_per_graph)
+            fitter = model.make_fitter(spec, un, crit, s.optim(flow_group), steps_per_graph=s.steps_per_graph)
             fitter_key = key
         else:
-            fitter.set_target(un, s.criterion)
+            fitter.set_target(un, crit)
         proper = False
         while not proper and res.retries <= s.proper_prior_fit_retrys:
             epochs = s.reuse_state_epochs if (warm and res.retries == 0) else s.num_epochs
@@ -165,7 +173,8 @@ def fit_frames(model, grids: Sequence, unaries: Sequence[torch.Tensor], schedule
             res.final_loss = float(hist[-1, 0]) if epochs > 0 else float("nan")
             with torch.no_grad():
                 prob = torch.sigmoid(model(spec.materialize(getattr(model, "in_channels", getattr(model, "in_features", 2)), dev)))
-            res.iou = mask_iou(prob.reshape(1, -1), un)
+            res.iou = mask_iou(prob.reshape(1, -1), un) if ign is None else \
+                mask_iou(prob.reshape(1, -1)[un != ign][None], un[un != ign][None])     # over the labelled pixels
             if keep_masks:
                 res.mask_fg = (prob.reshape(-1) <= 0.5)
             proper = res.iou >= s.proper_prior_fit_threshold

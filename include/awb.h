@@ -83,12 +83,29 @@ typedef struct awb_grid_spec {
   const float* grid; /* AWB_GRID_EXPLICIT: device [B,C,H,W] */
 } awb_grid_spec;
 
-/* loss = sum_n coef(t_n) * l(y_n, t_n); coef = fg(t_n) ? coef_fg : coef_bg.  The caller folds
- * any 1/N, class weights (ratio / sssdms / equal) or fg/bg means into the two coefficients. */
+/* loss = sum_n keep_n * w_n * coef(t_n) * l(y_n, t_n); coef = fg(t_n) ? coef_fg : coef_bg.  The caller folds
+ * any 1/N, class weights (ratio / sssdms / equal) or fg/bg means into the two coefficients (awb_target_counts_ignore
+ * gives the class counts over the kept pixels).
+ *   w_n    = weight[n] when weight is set (per-pixel confidence, sparse-label weights), else 1;
+ *   keep_n = (t_n != ignore_value) when ignore_enabled != 0 (weak labels: none class, occluders, unknown bands), else 1.
+ * An ignored pixel adds exactly 0 to the loss and to every gradient whatever its logit, target or weight (the kernels
+ * select, they do not multiply); a non-finite weight on a kept pixel makes the loss non-finite, which skips the step and
+ * raises the sticky flag like a non-finite target.  A zero-initialised tail (weight = null, ignore_enabled = 0) is the
+ * unweighted loss, computed by the same kernels as before these fields existed.  One spec per object: weight is that
+ * object's map, device [N] over the pixel rows of the call's grid.  The fused fit steps (awb_prior_fit_step, _fit_steps,
+ * _fit_host_frames, _slice_grads) honour weight and ignore; awb_prior_fit_steps and awb_prior_fit_host_frames apply
+ * the same map to every target they rotate through, and awb_prior_slice_grads reads it at the global row, like the
+ * target.  awb_star_fit_step returns AWB_ERR_UNSUPPORTED for either (awb_flow_identity_step has no loss spec: its loss
+ * is the flow's own identity regression).  ignore_enabled with a non-finite ignore_value: AWB_ERR_INVALID.  On the
+ * tensor path a weighted loss scales its fp16 deltas by max |w coef| over the kept pixels (one extra reduction over
+ * target and weight per step) instead of max |coef|. */
 typedef struct awb_loss_spec {
   int32_t kind;     /* AWB_LOSS_* */
   int32_t cls_rule; /* AWB_CLS_* */
   float coef_fg, coef_bg;
+  const float* weight;    /* optional device [N] per-pixel weights of this object (null: all 1) */
+  int32_t ignore_enabled; /* 1: pixels whose target equals ignore_value are dropped */
+  float ignore_value;     /* a finite number (the reference's `noneclass`, e.g. 2 for FBMS weak labels) */
 } awb_loss_spec;
 
 typedef struct awb_opt_hyper {
@@ -375,6 +392,11 @@ int awb_mask_iou_counts(const float* pred, const float* target, int64_t n_pixels
 /* target statistics for the weighted losses: counts[O][2] = {fg, bg} under cls_rule. */
 int awb_target_counts(const float* target, int64_t n_pixels, int32_t n_objects, int32_t cls_rule,
                       long long* counts, void* stream);
+/* The same counts over the kept pixels only: a pixel whose target equals ignore_value is in neither class (the
+ * reference's none-class filter before WeightedLoss computes its class weights, awesome/measures/weighted_loss.py).
+ * ignore_enabled == 0 gives awb_target_counts; a non-finite ignore_value: AWB_ERR_INVALID. */
+int awb_target_counts_ignore(const float* target, int64_t n_pixels, int32_t n_objects, int32_t cls_rule,
+                             int32_t ignore_enabled, float ignore_value, long long* counts, void* stream);
 
 /* Test hook: one CTA computes D[128][N] = A * B with tcgen05.mma (kind::f16, fp32 accumulate in TMEM) from raw
  * shared-memory tile images and caller-supplied descriptor fields {start offset, LBO, SBO, start advance per
