@@ -80,6 +80,14 @@ Workspace carve(const awb_prior* h, int64_t N, int layout, void* base) {
   int64_t off = 0;
   auto take = [&](int64_t bytes) { char* r = p ? p + off : nullptr; off += align256(bytes); return r; };
   Workspace w = {};
+  w.row0 = 0; w.N = N;
+  if (h->desc.kind == AWB_KIND_STAR) {   // AWB_WS_FIT_STEP only (check_common): the fit kernel's per-CTA partials
+    const int Ss = star_bwd_ctas(N, nullptr);
+    w.part = (float*)take(4 * (int64_t)Ss * L.P);
+    w.lossp = (float*)take(4 * (int64_t)Ss);
+    w.bytes = off;
+    return w;
+  }
   w.waug = (float*)take(4 * O * L.G);
   w.part = (float*)take(training && !deform_only ? 4 * (int64_t)S * O * L.G : 0);
   w.lossp = (float*)take(4 * ((int64_t)kMaxSplits * O + O));   // [S][O] loss partials + [O] spare scalars (max |dlogits|)
@@ -227,6 +235,7 @@ int64_t awb_prior_param_count(awb_handle h) { return h ? h->lay.P : -1; }
 
 int64_t awb_prior_workspace_bytes(awb_handle h, int64_t n_pixels, int32_t layout) {
   if (!h || n_pixels < 1 || layout < AWB_WS_INFERENCE || layout > AWB_WS_SECOND_ORDER) return -1;
+  if (h->desc.kind == AWB_KIND_STAR && layout != AWB_WS_FIT_STEP) return -1;   // the star prior has only the fit step
   return carve(h, n_pixels, layout, nullptr).bytes;
 }
 
@@ -264,11 +273,20 @@ int awb_prior_set_flow_eval(awb_handle h, int32_t mode) {
   return AWB_OK;
 }
 
+// A star handle reaches the generic entry points only through the whole-batch fit step (awb_prior_fit_step, _fit_steps,
+// _fit_host_frames); every other one refuses it here, before anything reads its layout as an ICNN's.
+static int refuse_star() {
+  set_error("the star prior runs awb_star_forward / awb_star_backward on points and awb_prior_fit_step (or _fit_steps, "
+            "_fit_host_frames) on an explicit grid; this entry point does not take star handles");
+  return AWB_ERR_UNSUPPORTED;
+}
+
 // Validates the arguments every workspace entry point shares and carves the workspace, of layout `layout` (AWB_WS_*),
 // into *out.  window (optional, {row_begin, row_end}): the call works on the pixel rows [row_begin, row_end) of the
 // batch, which must be a non-empty range inside [0, N), and the workspace is sized for them; out->row0 = row_begin.
 static int check_common(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, int layout,
                         const int64_t* window, Workspace* out) {
+  if (h && h->desc.kind == AWB_KIND_STAR && (layout != AWB_WS_FIT_STEP || window)) return refuse_star();
   if (!h || !g || !ws) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (g->B < 1 || g->H < 1 || g->W < 1) { set_error("empty grid %dx%dx%d", g->B, g->H, g->W); return AWB_ERR_INVALID; }
   if (g->mode == AWB_GRID_EXPLICIT && !g->grid) { set_error("explicit grid needs a pointer"); return AWB_ERR_INVALID; }
@@ -376,6 +394,7 @@ int awb_prior_forward(awb_handle h, const float* params, const awb_grid_spec* g,
 }
 
 int awb_prior_flow_inverse(awb_handle h, const float* params, const awb_grid_spec* g, float* out, void* stream) {
+  if (h && h->desc.kind == AWB_KIND_STAR) return refuse_star();
   if (!h || !params || !g || !out) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (h->desc.kind != AWB_KIND_FLOW_ICNN || !h->fc_set) { set_error("needs a flow prior with its constants set"); return AWB_ERR_INVALID; }
   if (g->mode != AWB_GRID_EXPLICIT || !g->grid || g->B < 1 || g->H < 1 || g->W < 1) { set_error("inverse takes an explicit [B,C,H,W] tensor"); return AWB_ERR_INVALID; }
@@ -410,6 +429,7 @@ int awb_prior_grid_grad_backward(awb_handle h, const float* params, const awb_gr
                                  const float* d_dgrid, float* d_dlogits, float* grads, void* ws, size_t ws_bytes,
                                  void* stream) {
   if (!h) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if (h->desc.kind == AWB_KIND_STAR) return refuse_star();
   if (h->desc.kind != AWB_KIND_ICNN || h->desc.n_objects != 1) {
     set_error("the second-order pass is provided for single-object ICNN priors only (kind %d, %d objects)", h->desc.kind,
               h->desc.n_objects);
@@ -433,11 +453,18 @@ int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_g
   if (rc) return rc;
   if (!params || !opt_state || !target || !loss || !hy) { set_error("null argument"); return AWB_ERR_INVALID; }
   if ((rc = check_loss(loss, h->desc.n_objects))) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (h->desc.kind == AWB_KIND_STAR) {   // k_star_bwd<NU, WL> over the grid's rows; no packed image, so flags do not apply
+    if (g->mode != AWB_GRID_EXPLICIT) { set_error("a star fit step takes an explicit [B,2,H,W] grid"); return AWB_ERR_INVALID; }
+    int S = 0;
+    rc = star_fit(h, params, g, target, *loss, w, &S, st);
+    if (rc) return rc;
+    return reduce_opt_plain(h, params, opt_state, hy, loss_out, w.part, S, h->lay.P, w.lossp, 1, st);
+  }
   // simt_reduce_opt refreshes a flow prior's fp16 weight image only when its optimizer owns every group
   Pass p = {};
   p.tensor = h->desc.precision == AWB_PREC_F16; p.target = target; p.loss = loss;
   p.reuse = (flags & AWB_FIT_REUSE_PACKED) != 0 && (!has_flow(h) || hy->active_groups == 0);
-  cudaStream_t st = (cudaStream_t)stream;
   int n_part;
   rc = run_pass(h, params, g, w, p, st, &n_part);
   if (rc) return rc;
@@ -447,6 +474,7 @@ int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_g
 // get_deformation: single-object RealNVP o ICNN and NormalizingFlow1D o ICNN handles
 static int check_deformable(awb_handle h) {
   if (!h) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if (h->desc.kind == AWB_KIND_STAR) return refuse_star();
   if (h->desc.kind == AWB_KIND_ICNN) { set_error("an ICNN prior has no deformation"); return AWB_ERR_INVALID; }
   if (!has_flow(h) || h->desc.n_objects != 1) {
     set_error("the deformation entry points support single-object flow priors (kind %d, %d objects)", h->desc.kind,
@@ -487,6 +515,7 @@ int awb_prior_deformation_backward(awb_handle h, const float* params, const awb_
 // PathConnectedNet.inverse with autograd: single-object RealNVP o ICNN handles, explicit grid; carves layout
 // AWB_WS_DEFORMATION
 static int check_inverse(awb_handle h, const awb_grid_spec* g, void* ws, size_t ws_bytes, Workspace* w) {
+  if (h && h->desc.kind == AWB_KIND_STAR) return refuse_star();
   if (!h || !g) { set_error("null argument"); return AWB_ERR_INVALID; }
   if (h->desc.kind != AWB_KIND_FLOW_ICNN) { set_error("needs a flow prior with its constants set"); return AWB_ERR_INVALID; }
   if (h->desc.n_objects != 1) {
@@ -521,6 +550,7 @@ int awb_prior_inverse_backward(awb_handle h, const float* params, const awb_grid
 // single-object ICNN and RealNVP o ICNN handles (the priors of the spatio-temporal fit)
 static int check_sliceable(awb_handle h) {
   if (!h) { set_error("null argument"); return AWB_ERR_INVALID; }
+  if (h->desc.kind == AWB_KIND_STAR) return refuse_star();
   if ((h->desc.kind != AWB_KIND_ICNN && h->desc.kind != AWB_KIND_FLOW_ICNN) || h->desc.n_objects != 1) {
     set_error("gradient rows support single-object ICNN and RealNVP o ICNN priors (kind %d, %d objects)", h->desc.kind,
               h->desc.n_objects);
@@ -684,7 +714,11 @@ int awb_star_fit_step(awb_handle h, float* params, void* opt_state, const float*
                       void* stream) {
   if (!h || !params || !opt_state || !x || !target || !loss || !hy || !ws || n < 1) { set_error("bad argument"); return AWB_ERR_INVALID; }
   if (h->desc.kind != AWB_KIND_STAR) { set_error("not a star prior"); return AWB_ERR_INVALID; }
-  if (loss_is_weighted(*loss)) { set_error("the star fit step takes no weight map or ignore label"); return AWB_ERR_UNSUPPORTED; }
+  if (loss_is_weighted(*loss)) {
+    set_error("awb_star_fit_step takes no weight map or ignore label; awb_prior_fit_step with an explicit [1,2,1,n] grid "
+              "of the sampled points takes both");
+    return AWB_ERR_UNSUPPORTED;
+  }
   const int64_t need = awb_star_workspace_bytes(h, n);
   if ((int64_t)ws_bytes < need) { set_error("workspace too small: %lld < %lld", (long long)ws_bytes, (long long)need); return AWB_ERR_WORKSPACE; }
   const int S = star_n_ctas(n);

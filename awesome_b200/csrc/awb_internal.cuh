@@ -148,7 +148,8 @@ Workspace carve(const awb_prior* h, int64_t N, int layout, void* base);
 
 // ---- per-kernel-class timing (CUDA events on the launch stream) and launch counting ----
 enum { PK_PACK = 0, PK_INPUT, PK_GEMM_FWD, PK_OUT_LOSS, PK_GEMM_WGRAD, PK_GEMM_DGRAD, PK_IN_BWD, PK_OPT,
-       PK_FLOW_FWD, PK_FLOW_BWD, PK_TC_FUSED, PK_MISC, PK_TAN_FWD, PK_TAN_OUT, PK_STAR_BWD, PK_COUNT };
+       PK_FLOW_FWD, PK_FLOW_BWD, PK_TC_FUSED, PK_MISC, PK_TAN_FWD, PK_TAN_OUT, PK_STAR_BWD, PK_STAR_FIT,
+       PK_COUNT };
 void prof_begin(int cls, cudaStream_t st);
 void prof_end(int cls, cudaStream_t st);
 #define AWB_LAUNCH(cls, st, ...)  \
@@ -232,6 +233,11 @@ int star_run(const awb_prior* h, const float* params, const float* x, const floa
 int star_bwd_ctas(int64_t n, int64_t* chunk);
 int star_backward(const awb_prior* h, const float* params, const float* x, const float* dy, int64_t n, float* grads,
                   float* dx, float* part, cudaStream_t st);
+// The fused fit step's forward, loss and backward on the rows of an explicit [B,2,H,W] grid (the fit mode
+// of the tiled backward, k_star_bwd<NU, WL>): star_bwd_ctas(ws.N) gradient partials of P floats in ws.part and as many loss partials in ws.lossp
+// (carve's star layout); *n_ctas receives their number.
+int star_fit(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
+             const awb_loss_spec& loss, const Workspace& ws, int* n_ctas, cudaStream_t st);
 int opt_state_init(const awb_prior* h, void* opt_state, const double* lr, cudaStream_t st);
 int opt_set_lr(const awb_prior* h, void* opt_state, const double* lr, cudaStream_t st);
 

@@ -10,7 +10,7 @@ namespace awb {
 static const int kMaxRec = 256;
 static const char* kNames[PK_COUNT] = {"pack", "input_layer", "gemm_fwd", "out_loss", "gemm_wgrad", "gemm_dgrad",
                                        "input_bwd", "reduce_opt", "flow_fwd", "flow_bwd", "tc_fused", "misc",
-                                       "tangent_fwd", "tangent_out", "star_bwd"};
+                                       "tangent_fwd", "tangent_out", "star_bwd", "star_fit"};
 static struct Prof {
   bool on = false;
   cudaEvent_t ev[PK_COUNT][kMaxRec][2];

@@ -207,8 +207,32 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
-template <int NU>
-__global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
+// The fused fit step on whole frames (awb_prior_fit_step on a star handle): the points are the pixel rows of an explicit
+// planar [B,2,H,W] grid and dy comes from the loss on the target, per point, inside the tile.  WL: the loss carries a
+// weight map and / or an ignore label (the plain instantiation reads neither).
+struct StarFitX {
+  GridDev g;             // explicit grid, C = 2
+  const float* target;   // [N]
+  LossCoef loss;
+  LossPix pix;
+  float* lossp;          // [S] loss partial per CTA
+};
+
+template <bool>
+using StarFitArg = StarFitX;
+__device__ __forceinline__ StarFitX star_fit_arg() { return StarFitX{}; }
+__device__ __forceinline__ StarFitX star_fit_arg(const StarFitX& f) { return f; }
+
+// k_star_bwd<NU> (no fit argument): the backward of awb_star_backward, x [n][2] and dy given.  k_star_bwd<NU, WL> (one
+// StarFitX): the fused fit step, the points are grid rows and dy comes from the loss.  The fit mode splits the b / db loop
+// in two: pass 1 sums s over the lane's units, the lane that owns the point turns y = r (s + b2 + b2_r) - 1 into its loss
+// term and dy, and pass 2 is the backward's loop without the s sum.  The mode is a template parameter pack so that the
+// backward's instantiation is the kernel it always was.
+template <int NU, bool... WLs>
+__global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p, StarFitArg<WLs>... fa) {
+  static_assert(sizeof...(WLs) <= 1, "one fit argument at most");
+  constexpr bool FIT = sizeof...(WLs) == 1, WL = (false || ... || WLs);
+  const StarFitX f = star_fit_arg(fa...);
   constexpr int HP = 32 * NU, LDW = HP + 4, T = kStarT, TM = kStarTM;
   extern __shared__ __align__(16) float sm[];
   float* sW1 = sm;                          // [HP][LDW] W1, zero outside [h][h]
@@ -217,7 +241,7 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
   float* sAcc = sDB + T * HP;               // [warp][SG_N][HP] per-unit gradient sums over each warp's points
   float* sPar = sAcc + kStarWarps * SG_N * HP;   // [SP_N][HP], zero for units >= h
   float* sPt = sPar + SP_N * HP;            // [PT_N][T]
-  __shared__ float red[kStarWarps][3];
+  __shared__ float red[kStarWarps][FIT ? 4 : 3];
   const int tid = threadIdx.x, w = tid >> 5, l = tid & 31, h = p.h;
   const float* par = p.params;
   const int o_W0 = 2, o_b0 = 2 + 2 * h, o_W1 = 2 + 3 * h, o_b1 = o_W1 + h * h, o_W2 = o_b1 + h, o_b2 = o_W2 + h,
@@ -246,6 +270,7 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
 #pragma unroll
     for (int b = 0; b < 2 * NU; b++) dW[a][b] = 0.f;
   float g_ox = 0.f, g_oy = 0.f, g_b2 = 0.f;   // lanes < TM: sums over the points they finish
+  float lacc = 0.f;                            // FIT: the warp's loss, its points in point order (every lane holds it)
   __syncthreads();
   const int64_t c0 = (int64_t)blockIdx.x * p.chunk, c1 = c0 + p.chunk < p.n ? c0 + p.chunk : p.n;
   for (int64_t t0 = c0; t0 < c1; t0 += T) {
@@ -256,11 +281,23 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
       float px = 0.f, py = 0.f, dy = 0.f;
       if (tid < nv) {
         const int64_t n = t0 + tid;
-        px = p.x[2 * n] + off0; py = p.x[2 * n + 1] + off1; dy = p.dy[n];
+        if (FIT) {
+          px = coord(f.g, n, 0) + off0; py = coord(f.g, n, 1) + off1;
+        } else {
+          px = p.x[2 * n] + off0; py = p.x[2 * n + 1] + off1; dy = p.dy[n];
+        }
       }
       const float r = sqrtf(px * px + py * py), q = 0.01f + r;
       sPt[PT_PX * T + tid] = px; sPt[PT_PY * T + tid] = py; sPt[PT_R * T + tid] = r; sPt[PT_Q * T + tid] = q;
-      sPt[PT_UX * T + tid] = px / q; sPt[PT_UY * T + tid] = py / q; sPt[PT_DY * T + tid] = dy; sPt[PT_DYR * T + tid] = dy * r;
+      sPt[PT_UX * T + tid] = px / q; sPt[PT_UY * T + tid] = py / q;
+      if (!FIT) { sPt[PT_DY * T + tid] = dy; sPt[PT_DYR * T + tid] = dy * r; }   // FIT: written by the loss lane below
+    }
+    // FIT: the lane that will finish point w * TM + l fetches its target (and weight) now; the W1 product hides the load
+    float tg = 0.f, wt = 1.f;
+    if (FIT && l < TM && w * TM + l < nv) {
+      const int64_t n = t0 + w * TM + l;
+      tg = f.target[n];
+      if (WL && f.pix.weight) wt = f.pix.weight[n];
     }
     __syncthreads();
     // a = relu(W0 u + b0) of the warp's points
@@ -297,7 +334,48 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
         }
       }
     }
-    // b, db; s and drb = sum_j db_j w1r_j per point; the per-unit sums of dyr a, dyr b, db, db r
+    float s_me = 0.f, drb_me = 0.f;   // lane i < TM keeps point w * TM + i
+    if (FIT) {
+      // pass 1: s = sum_j w2_j a_j + w2r_j b_j per point, then the loss of the lane's point and its dy
+      float s[TM];
+#pragma unroll
+      for (int i = 0; i < TM; i++) s[i] = 0.f;
+#pragma unroll
+      for (int u = 0; u < NU; u++) {
+        const int j = l + 32 * u;
+        const float w2 = sPar[SP_W2 * HP + j], w2r = sPar[SP_W2R * HP + j];
+#pragma unroll
+        for (int i = 0; i < TM; i++) s[i] += fmaf(w2, sA[(w * TM + i) * HP + j], w2r * fmaxf(acc[i][u], 0.f));
+      }
+#pragma unroll
+      for (int i = 0; i < TM; i++) {
+        const float si = warp_sum(s[i]);
+        if (l == i) s_me = si;
+      }
+      // k_star's loss: SE on the sigmoid or BCE with logits, coef by cls_rule (times the weight); padding points and
+      // (WL) ignored pixels are selected out, so their dy and loss term are exactly 0 whatever their inputs
+      float lterm = 0.f;
+      if (l < TM) {
+        const int t = w * TM + l;
+        const float r = sPt[PT_R * T + t];
+        const float y = fmaf(r, s_me + bias2, -1.f);
+        const bool fg = f.loss.cls_rule == AWB_CLS_UNARY_LT_HALF ? (tg < 0.5f) : (tg != 1.0f);
+        float coef = fg ? f.loss.coef_fg : f.loss.coef_bg;
+        if (WL) coef *= wt;
+        const float sg = 1.f / (1.f + expf(-y));
+        float lv, dl;
+        if (f.loss.kind == AWB_LOSS_SE_SIGMOID) { const float d = tg - sg; lv = d * d; dl = -2.f * d * sg * (1.f - sg); }
+        else { lv = fmaxf(y, 0.f) - y * tg + log1pf(expf(-fabsf(y))); dl = sg - tg; }
+        const bool keep = t < nv && (!WL || loss_keep(f.pix, tg));
+        const float dy = keep ? coef * dl : 0.f;
+        lterm = keep ? coef * lv : 0.f;
+        sPt[PT_DY * T + t] = dy; sPt[PT_DYR * T + t] = dy * r;
+      }
+#pragma unroll
+      for (int i = 0; i < TM; i++) lacc += __shfl_sync(0xffffffffu, lterm, i);
+      __syncwarp();
+    }
+    // b, db; (BWD: s and) drb = sum_j db_j w1r_j per point; the per-unit sums of dyr a, dyr b, db, db r
     float s[TM], drb[TM];
 #pragma unroll
     for (int i = 0; i < TM; i++) { s[i] = 0.f; drb[i] = 0.f; }
@@ -312,7 +390,7 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
         const int t = w * TM + i;
         const float a = sA[t * HP + j], b = fmaxf(acc[i][u], 0.f);
         const float dyr = sPt[PT_DYR * T + t], r = sPt[PT_R * T + t];
-        s[i] += fmaf(w2, a, w2r * b);
+        if (!FIT) s[i] += fmaf(w2, a, w2r * b);
         const float db = acc[i][u] > 0.f ? dyr * w2r : 0.f;
         sDB[t * HP + j] = db;
         drb[i] = fmaf(db, w1r, drb[i]);
@@ -321,11 +399,15 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
       }
       ga[SG_W2 * HP] = g_w2; ga[SG_W2R * HP] = g_w2r; ga[SG_B1 * HP] = g_b1; ga[SG_W1R * HP] = g_w1r;
     }
-    float s_me = 0.f, drb_me = 0.f;   // lane i < TM keeps point w * TM + i
 #pragma unroll
     for (int i = 0; i < TM; i++) {
-      const float si = warp_sum(s[i]), di = warp_sum(drb[i]);
-      if (l == i) { s_me = si; drb_me = di; }
+      if (FIT) {
+        const float di = warp_sum(drb[i]);
+        if (l == i) drb_me = di;
+      } else {
+        const float si = warp_sum(s[i]), di = warp_sum(drb[i]);
+        if (l == i) { s_me = si; drb_me = di; }
+      }
     }
     __syncwarp();
     // da = dyr w2 + W1^T db; dapre; the per-unit sums of dapre ux, dapre uy, dapre; du = W0^T dapre per point
@@ -387,7 +469,7 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
         gy = duy_me / q + dr * (py / r);
       }
       g_ox += gx; g_oy += gy;
-      if (p.dx) { const int64_t n = t0 + t; p.dx[2 * n] = gx; p.dx[2 * n + 1] = gy; }
+      if (!FIT && p.dx) { const int64_t n = t0 + t; p.dx[2 * n] = gx; p.dx[2 * n + 1] = gy; }
     }
     __syncthreads();
     // dW1 += db^T a over the tile's points, in point order
@@ -423,14 +505,22 @@ __global__ void __launch_bounds__(kStarWarps * 32, 1) k_star_bwd(StarBwdP p) {
       if (j < h && k < h) out[o_W1 + j * h + k] = dW[a][b];
     }
   g_ox = warp_sum(g_ox); g_oy = warp_sum(g_oy); g_b2 = warp_sum(g_b2);
-  if (l == 0) { red[w][0] = g_ox; red[w][1] = g_oy; red[w][2] = g_b2; }
+  if (l == 0) {
+    red[w][0] = g_ox; red[w][1] = g_oy; red[w][2] = g_b2;
+    if (FIT) red[w][FIT ? 3 : 0] = lacc;
+  }
   __syncthreads();
   if (tid == 0) {
-    float ox = 0.f, oy = 0.f, b2 = 0.f;
-    for (int v = 0; v < kStarWarps; v++) { ox += red[v][0]; oy += red[v][1]; b2 += red[v][2]; }
+    float ox = 0.f, oy = 0.f, b2 = 0.f, ls = 0.f;
+    for (int v = 0; v < kStarWarps; v++) {
+      ox += red[v][0]; oy += red[v][1]; b2 += red[v][2];
+      if (FIT) ls += red[v][FIT ? 3 : 0];
+    }
     out[0] = ox; out[1] = oy; out[o_b2] = b2; out[o_b2r] = b2;
+    if (FIT) f.lossp[blockIdx.x] = ls;
   }
 }
+
 
 // Launch geometry of k_star_bwd.  Size-dependent branches (tests/test_gpu_star_autograd.py covers both sides of each):
 //  - tiles per CTA: ceil(n / kStarT) tiles are dealt to at most kMaxSplits CTAs in runs of ceil(tiles / kMaxSplits):
@@ -470,6 +560,42 @@ int star_backward(const awb_prior* h, const float* params, const float* x, const
   }
   if (rc) return rc;
   return reduce_grads_plain(h, grads, part, S, h->lay.P, st);
+}
+
+template <int NU, bool WL>
+static int star_fit_launch(const StarBwdP& p, const StarFitX& f, int S, cudaStream_t st) {
+  constexpr size_t smem = star_bwd_smem<NU>();
+  AWB_CUDA(cudaFuncSetAttribute(k_star_bwd<NU, WL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  AWB_LAUNCH(PK_STAR_FIT, st, k_star_bwd<NU, WL><<<S, kStarWarps * 32, smem, st>>>(p, f));
+  AWB_CUDA(cudaGetLastError());
+  return AWB_OK;
+}
+
+template <bool WL>
+static int star_fit_dispatch(int hh, const StarBwdP& p, const StarFitX& f, int S, cudaStream_t st) {
+  switch ((hh + 31) / 32) {
+    case 1: return star_fit_launch<1, WL>(p, f, S, st);
+    case 2: return star_fit_launch<2, WL>(p, f, S, st);
+    case 3: return star_fit_launch<3, WL>(p, f, S, st);
+    case 4: return star_fit_launch<4, WL>(p, f, S, st);
+    default: return star_fit_launch<5, WL>(p, f, S, st);
+  }
+}
+
+int star_fit(const awb_prior* h, const float* params, const awb_grid_spec* g, const float* target,
+             const awb_loss_spec& loss, const Workspace& ws, int* n_ctas, cudaStream_t st) {
+  const int hh = h->lay.h;
+  if (hh > 160) { set_error("star prior supports n_hidden <= 160, got %d", hh); return AWB_ERR_UNSUPPORTED; }
+  StarBwdP p = {};
+  p.params = params; p.P = h->lay.P; p.h = hh; p.n = ws.N; p.part = ws.part;
+  const int S = star_bwd_ctas(ws.N, &p.chunk);
+  StarFitX f = {};
+  f.g.mode = g->mode; f.g.B = g->B; f.g.H = g->H; f.g.W = g->W; f.g.C = 2; f.g.grid = g->grid; f.g.row0 = 0;
+  f.target = target; f.loss = loss_coef(loss); f.pix = loss_pix(loss); f.lossp = ws.lossp;
+  const int rc = loss_is_weighted(loss) ? star_fit_dispatch<true>(hh, p, f, S, st) : star_fit_dispatch<false>(hh, p, f, S, st);
+  if (rc) return rc;
+  *n_ctas = S;
+  return AWB_OK;
 }
 
 }  // namespace awb

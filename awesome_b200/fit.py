@@ -170,11 +170,13 @@ class PriorFitter:
     """Fits ``prior`` (a native handle) to ``target`` on ``grid`` in place on ``params``.
 
     params ``[O,P]`` fp32 CUDA (the module's arena), target ``[O,N]`` fp32 CUDA.
-    ``run(steps)`` replays CUDA graphs of ``steps_per_graph`` fused steps.
+    ``run(steps)`` replays CUDA graphs of ``steps_per_graph`` fused steps.  ``active_groups``: the optimizer groups
+    the steps update (``awb_opt_hyper.active_groups``; 0 = all).
     """
 
     def __init__(self, prior: Prior, params: torch.Tensor, grid: GridSpecHost, target: torch.Tensor,
-                 loss: LossConfig, optim: OptimConfig, steps_per_graph: int = 25, use_graph: bool = True):
+                 loss: LossConfig, optim: OptimConfig, steps_per_graph: int = 25, use_graph: bool = True,
+                 active_groups: int = 0):
         L.require_cuda()
         self.prior, self.params, self.grid = prior, params, grid
         self.device = params.device
@@ -194,6 +196,7 @@ class PriorFitter:
             self._specs_list = loss.to_specs(self.target, self._weight)
         self._specs = (L.LossSpec * O)(*self._specs_list)
         self._hyper = optim.to_c()
+        self._hyper.active_groups = int(active_groups)
         self._gs = grid.to_c()
         self.optim = optim
         self.K = max(1, int(steps_per_graph))

@@ -1,7 +1,8 @@
 """Star-shape prior (SURVEY a16): drop-in for the notebook class ``myNet``
 (``notebooks/icml_teaser_code/star_shaped/star.ipynb`` cell 2) -- same constructor argument, parameter names
 (``offset, W0, W1, W2, W1_r, W2_r``), initial weights for a given seed and ``forward(x[n,2]) -> [n,1]`` -- with the
-training loop of cell 3 as fused native steps (``StarFitter``).
+training loop of cell 3 as fused native steps (``StarFitter``).  It also takes ``[B,2,H,W]`` grids and fits whole frames
+with ``make_fitter(grid, target, loss, optim)`` (``PriorFitter``; weight maps, ignore label, ``fit_frames``).
 
 ``forward`` is differentiable w.r.t. the parameters and the points (``awb_star_forward`` / ``awb_star_backward``), so
 the notebook's own loop (``loss = mse(sigmoid(net(x)), t); loss.backward(); optimizer.step()``), a custom loss or a
@@ -16,7 +17,7 @@ import torch
 from torch import nn
 
 from .. import _lib as L
-from ..core import Prior
+from ..core import GridSpecHost, Prior
 from .base import Affine, ArenaPriorModule, _first_order_only, _split_grads, reject_second_order
 
 
@@ -77,23 +78,76 @@ class StarShapedNet(ArenaPriorModule):
         return Prior(L.AWB_KIND_STAR, 2, self.n_hidden, 0)
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        """Native forward, differentiable w.r.t. the parameters and ``x``.  ``make_fitter`` runs the notebook's loop as
-        fused steps."""
-        if x.dim() != 2 or x.shape[1] != 2:
-            raise ValueError(f"expected [n,2] points, got {tuple(x.shape)}")
+        """Native forward, differentiable w.r.t. the parameters and ``x``: points ``[n,2]`` -> ``[n,1]``, a grid
+        ``[B,2,H,W]`` -> ``[B,1,H,W]`` or ``[2,H,W]`` -> ``[1,H,W]`` (pixel rows in ``(b, h, w)`` order through the same
+        kernels: a grid and its rows give the same bits).  ``make_fitter`` runs fused fit steps."""
+        if x.dim() == 2:
+            if x.shape[1] != 2:
+                raise ValueError(f"expected [n,2] points, got {tuple(x.shape)}")
+            return self._points(x)
+        squeeze = x.dim() == 3
+        g = x.unsqueeze(0) if squeeze else x
+        if g.dim() != 4 or g.shape[1] != 2:
+            raise ValueError(f"expected [n,2] points or a [B,2,H,W] grid, got {tuple(x.shape)}")
+        B, _, H, W = g.shape
+        y = self._points(g.permute(0, 2, 3, 1).reshape(-1, 2)).reshape(B, H, W, 1).permute(0, 3, 1, 2)
+        return y[0] if squeeze else y
+
+    def _points(self, x: torch.Tensor) -> torch.Tensor:
         if not x.is_cuda:
             raise L.AwbLibraryError("awesome_b200 priors run on CUDA only (no CPU fallback)")
         self._ensure_flat()
         with torch.cuda.device(x.device):
             return _StarFunction.apply(self, x, *self._arena_params())
 
+    @staticmethod
+    def create_grid(H: int, W: int, B: int = 1, device=None) -> torch.Tensor:
+        """``[B,2,H,W]`` coordinates of an ``H x W`` likelihood image as ``fit_likelihood`` samples them (the notebook's
+        cell 3): channel 0 = ``i / (H - 1) - 0.5`` (row), channel 1 = ``j / (W - 1) - 0.5`` (column)."""
+        if H < 2 or W < 2:
+            raise ValueError(f"the notebook's coordinates need H, W >= 2, got {H}x{W}")
+        i = torch.arange(H, device=device) / (H - 1) - 0.5
+        j = torch.arange(W, device=device) / (W - 1) - 0.5
+        ii, jj = torch.meshgrid(i, j, indexing="ij")
+        return torch.stack([ii, jj], 0).float().unsqueeze(0).expand(B, 2, H, W).contiguous()
+
+    def reset_parameters(self) -> None:
+        """Draw the weights again as the constructor does (``nn.Linear`` init, same order), in place in the arena; the
+        offset goes back to 0 and keeps its ``requires_grad``.  ``fit_frames`` calls it before a retry."""
+        self._ensure_flat()
+        h = self.n_hidden
+        fresh = [_lin(2, h), _lin(h, h), _lin(h, 1), _lin(1, h), _lin(h, 1)]
+        with torch.no_grad():
+            self.offset.zero_()
+            for mod, new in zip((self.W0, self.W1, self.W2, self.W1_r, self.W2_r), fresh):
+                mod.weight.copy_(new.weight)
+                mod.bias.copy_(new.bias)
+
     def enforce_convexity(self) -> None:
         """The notebook's projection: ``W2_r.weight <- relu(W2_r.weight)`` (cell 3)."""
         with torch.no_grad():
             self.W2_r.weight.clamp_(min=0)
 
-    def make_fitter(self, optim=None, loss=None, **kw) -> "StarFitter":
-        return StarFitter(self, optim, loss)
+    def make_fitter(self, grid=None, target=None, loss=None, optim=None, **kw):
+        """With a ``grid`` (``[B,2,H,W]`` tensor or ``GridSpecHost``; a generated one is materialised) and its
+        ``target``: a ``PriorFitter`` of fused whole-frame steps (``awb_prior_fit_step`` on the star handle), taking
+        weight maps and an ignore label like the other priors; ``kw`` goes to ``PriorFitter``.  The offset is trained iff
+        ``offset.requires_grad`` when the fitter is built.  Without a grid: the notebook's sampled-point ``StarFitter``
+        (``make_fitter()``, ``make_fitter(optim=..., loss=...)``)."""
+        if grid is None:
+            return StarFitter(self, optim, loss)
+        from ..fit import LossConfig, OptimConfig, PriorFitter
+        arena = self._ensure_flat()
+        prior = self._prior_for(arena.device)
+        if isinstance(grid, torch.Tensor):
+            grid = GridSpecHost.from_tensor(grid.to(arena.device))
+        elif grid.mode != "explicit":
+            grid = GridSpecHost.from_tensor(grid.materialize(2, arena.device))
+        if target is None:
+            raise ValueError("a grid fit needs its target")
+        groups = 0b110 if self.offset.requires_grad else 0b010      # 1: the network's weights, 2: the offset
+        return PriorFitter(prior, arena, grid, target, loss or LossConfig("mse"), optim or OptimConfig(),
+                           active_groups=groups, **kw)
 
 
 class StarFitter:

@@ -84,6 +84,21 @@ def c3_unaries(H: int = 480, W: int = 640, seed: int = 42, t: float = 0.0, tau: 
     return torch.sigmoid((sdf + 0.05 * torch.randn(H, W, generator=g)) / tau).float()
 
 
+def star_unaries(H: int = 480, W: int = 640, seed: int = 42, r0: float = 0.25, a: float = 0.3, k: int = 5,
+                 tau: float = 0.08, noise: float = 0.05) -> torch.Tensor:
+    """A non-convex star-shaped blob for the star prior: boundary ``r(theta) = r0 (1 + a cos(k theta))`` around a
+    seeded centre near the middle, soft like ``c2_unaries`` (fg = 0 inside).  ``noise = 0``: the clean blob."""
+    g = torch.Generator().manual_seed(seed)
+    xx, yy = _grid01(H, W)
+    c = 0.5 + 0.04 * (torch.rand(2, generator=g) - 0.5)
+    phase = float(torch.rand(1, generator=g)) * 2 * math.pi
+    dx, dy = xx - float(c[0]), yy - float(c[1])
+    rho = torch.sqrt(dx ** 2 + dy ** 2)
+    r = r0 * (1 + a * torch.cos(k * torch.atan2(dy, dx) + phase))
+    sdf = rho / r - 1
+    return torch.sigmoid((sdf + noise * torch.randn(H, W, generator=g)) / tau).float()
+
+
 def multi_object_unaries(H: int = 480, W: int = 640, n_objects: int = 8, seed: int = 42, tau: float = 0.08) -> torch.Tensor:
     """Config 4: ``[1, O+1, H, W]`` -- channel 0 background, channel k+1 the soft unaries of object k (fg = 0): O disjoint
     elliptic blobs on a 4 x 2 lattice (``multiple_object_aware_path_connected_net.py:186-192``)."""

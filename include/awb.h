@@ -95,7 +95,7 @@ typedef struct awb_grid_spec {
  * object's map, device [N] over the pixel rows of the call's grid.  The fused fit steps (awb_prior_fit_step, _fit_steps,
  * _fit_host_frames, _slice_grads) honour weight and ignore; awb_prior_fit_steps and awb_prior_fit_host_frames apply
  * the same map to every target they rotate through, and awb_prior_slice_grads reads it at the global row, like the
- * target.  awb_star_fit_step returns AWB_ERR_UNSUPPORTED for either (awb_flow_identity_step has no loss spec: its loss
+ * target.  On star handles the fit steps honour both too; awb_star_fit_step returns AWB_ERR_UNSUPPORTED for either (awb_flow_identity_step has no loss spec: its loss
  * is the flow's own identity regression).  ignore_enabled with a non-finite ignore_value: AWB_ERR_INVALID.  On the
  * tensor path a weighted loss scales its fp16 deltas by max |w coef| over the kept pixels (one extra reduction over
  * target and weight per step) instead of max |coef|. */
@@ -276,6 +276,15 @@ int awb_prior_inverse_backward(awb_handle h, const float* params, const awb_grid
  * params and nothing has written params since (the caller is inside its own step loop): the tensor path then
  * reuses the fp16 weight image its optimizer kernel left in the workspace instead of re-packing it. */
 #define AWB_FIT_REUSE_PACKED 1
+/* Star handles (AWB_KIND_STAR): awb_prior_fit_step, _fit_steps and _fit_host_frames fit the star prior to the pixel rows
+ * of an explicit [B,2,H,W] grid (points in (b, h, w) order; any other grid mode: AWB_ERR_INVALID), with one loss spec
+ * whose weight map and ignore label are honoured, hyper->active_groups as for awb_star_fit_step (bit 1 the weights, bit 2
+ * the offset, 0 all) and the W2_r.weight clamp.  Forward, loss and backward run in one tiled kernel (64-point tiles, the
+ * structure of awb_star_backward) with per-CTA partials summed in a fixed order; AWB_FIT_REUSE_PACKED is ignored (there is
+ * no packed weight image).  awb_prior_workspace_bytes gives star handles a size for AWB_WS_FIT_STEP only (-1 for the
+ * other layouts), and every other generic entry point (forward, backward, grid-grad, deformation, inverse, slice grads,
+ * rows-opt, ActNorm init, flow identity) returns AWB_ERR_UNSUPPORTED for them: points go through awb_star_forward /
+ * awb_star_backward. */
 int awb_prior_fit_step(awb_handle h, float* params, void* opt_state, const awb_grid_spec* grid,
                        const float* target, const awb_loss_spec* loss, const awb_opt_hyper* hyper,
                        float* loss_out, void* workspace, size_t workspace_bytes, int32_t flags, void* stream);
@@ -364,7 +373,9 @@ int awb_star_forward(awb_handle h, const float* params, const float* x, int64_t 
 int64_t awb_star_workspace_bytes(awb_handle h, int64_t n);
 /* One step of the notebook's training loop (cell 3): y = net(x); loss = sum_n coef(t_n) * l(y_n, t_n) (MSE on the
  * sigmoid with coef = 1/n in the notebook); backward; Adam/Adamax; W2_r.weight <- relu(W2_r.weight).  Optimizer
- * groups: 1 = network weights, 2 = offset (frozen until hyper->active_groups includes bit 2, cell 3 "epoch == 1000"). */
+ * groups: 1 = network weights, 2 = offset (frozen until hyper->active_groups includes bit 2, cell 3 "epoch == 1000").
+ * No weight map or ignore label (AWB_ERR_UNSUPPORTED): awb_prior_fit_step with an explicit [1,2,1,n] grid of the sampled
+ * points runs the same step with both. */
 int awb_star_fit_step(awb_handle h, float* params, void* opt_state, const float* x, const float* target, int64_t n,
                       const awb_loss_spec* loss, const awb_opt_hyper* hyper, float* loss_out, void* workspace,
                       size_t workspace_bytes, void* stream);
